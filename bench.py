@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/*.npy
 
 Workload: BASELINE.json configs[1], synthetic 2,000-bin Hi-C matrices with nested block TADs and power-law decay,
 max_pcs = 200.  One TADpole() call = bad-column filter, Pearson correlation, PCA to 200 components, the n_pcs sweep
@@ -69,7 +70,14 @@ def parse():
                          "(N = 1 only; 0 = skip)")
     ap.add_argument("--strong-bins", type=int, default=25000, help="bins of the one call spread over all ranks (0 = skip)")
     ap.add_argument("--arm-bins", type=int, default=15000, help="bins of the centromere_search call, arms sharded (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed batch returned in its last step to "
+                                                          "DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 def usable_cpus():
@@ -205,6 +213,33 @@ def h2d_bytes(n):
     (csrc/filter.cu): rows [r, r + band) x columns [r, n)"""
     band = max(n // 32, 64)
     return sum((n - r) * 8 * min(band, n - r) for r in range(0, n, band))
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, results, prefix=""):
+    """Write the per-call results of one step as a caller of tp_call_batch receives them, so that two builds can be
+    compared output for output: <prefix>callNN_scores.npy (CH score matrix) with <prefix>callNN_scored.npy (1 where a
+    level is scored; the library's NaN marks the others, written as 0 so that every dumped value is finite),
+    <prefix>callNN_seqdist.npy (CONISS heights of the chosen candidate), <prefix>callNN_bad.npy (bad-bin mask as 0 / 1)
+    and <prefix>counts.npy (one row per call: nf, k, n_pcs, n_clusters), all float64.  Calls are written in batch order
+    while the total stays within DUMP_LIMIT bytes; at sizes where it would not, the first calls of the step stand for it."""
+    os.makedirs(out_dir, exist_ok=True)
+    total, counts = 0, []
+    for i, r in enumerate(results):
+        if isinstance(r, Exception):
+            raise r
+        unscored = np.isnan(r["scores"])
+        arrays = {"scores": np.where(unscored, 0.0, r["scores"]), "scored": ~unscored, "seqdist": r["seqdist"], "bad": r["bad"]}
+        size = sum(a.size * 8 for a in arrays.values()) + 4 * 8
+        if total + size > DUMP_LIMIT:
+            break
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, f"{prefix}call{i:02d}_{name}.npy"), np.asarray(a, dtype=np.float64))
+        counts.append([r["nf"], r["k"], r["n_pcs"], r["n_clusters"]])
+        total += size
+    np.save(os.path.join(out_dir, f"{prefix}counts.npy"), np.array(counts, dtype=np.float64).reshape(-1, 4))
 
 
 def measure_fp64_peak(torch):
@@ -379,10 +414,13 @@ def run_b200(args, rank, world, local_rank):
     if sync_blocking:
         ctx.set("sync_blocking", 1)
     barrier()
-    ctx.call_batch(None, device_ptrs=ptrs * args.steps, n=n, inflight=S, tables=False, max_pcs=MAX_PCS)
+    last_step = ctx.call_batch(None, device_ptrs=ptrs * args.steps, n=n, inflight=S, tables=False, max_pcs=MAX_PCS)[-B:]
     ms_thr, launches = ctx.last_batch_device_ms, ctx.last_batch_launches
     barrier()
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step, f"rank{rank}_" if world > 1 else "")
+    del last_step
     # ---- e2e: public API, pinned host input, copies + tables + objects inside the timed region ----
     TADpole_batch(host_np, max_pcs=MAX_PCS, ctx=ctx, streams=S)
     barrier()
