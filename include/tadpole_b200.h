@@ -197,14 +197,14 @@ int tp_test_ss_tile(int r_lo, int r_hi, int c_lo, int c_hi, int nranks, int rpr)
  * For candidates i = cand_begin + t*cand_stride < k (0-based: candidate i clusters on the first
  * i+1 score columns): CONISS dendrogram (seqdist), broken-stick level count n_cluster, and the
  * Calinski-Harabasz score of every level min(min_clusters, n_cluster)..n_cluster on ALL k columns.
- * Outputs (host, may be NULL): n_cluster[k] (0 for candidates not run); scores[k * ld_scores]
- * row-major NaN padded (row = candidate, column = n_clusters-1); ld_scores is chosen by the
- * caller and must be >= the largest n_cluster, otherwise *maxlev_out tells the width needed and
- * TP_ERR_ARG is returned. */
+ * Outputs (host, may be NULL): n_cluster[k] (0 for candidates not run); *maxlev_out = the largest
+ * n_cluster, the width of the score matrix (tp_get_sweep_scores). */
 int tp_sweep(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stride,
-             int *n_cluster_out, double *scores_out, int ld_scores, int *maxlev_out);
-/* score matrix of the last sweep (tp_sweep, tp_call, tp_call_arm): k x maxlev, NaN padded, row pitch ld_scores */
-int tp_get_sweep_scores(tp_ctx *ctx, double *scores_out, int ld_scores);
+             int *n_cluster_out, int *maxlev_out);
+/* score matrix of the last sweep (tp_sweep, tp_call, tp_call_arm, tp_recall): exactly k x maxlev doubles row-major
+ * (row = candidate, column = n_clusters-1), NaN where a level is not scored; k and maxlev as the sweep reported them
+ * (or tp_ctx_dims).  A host copy the sweep made: no device work. */
+int tp_get_sweep_scores(tp_ctx *ctx, double *scores_out);
 /* seqdist (nf-1 doubles) and merge order (nf-1 ints: boundary removed at each step) of one
  * candidate of the last sweep; either pointer may be NULL.  After a sweep that was dealt out over several GPUs the
  * dendrogram lives on the device that ran the candidate: a multi-device context fetches it from there; with one process
@@ -217,28 +217,26 @@ int tp_select(const double *scores, int k, int ld, int maxlev, int *opt_cand, in
 
 /* ---- one-shot: filter -> compact -> correlation -> PCA -> sweep -> selection -------------------
  * The non-centromere path of TADpole() (R/TADpole.R:444-468) from an in-memory matrix.
- * bad_out[n]; scores_out[k * ld_scores] (k = min(max_pcs, nf)); seqdist_out[nf-1] of the optimal
- * candidate.  nf_out/k_out/maxlev_out report the sizes actually used.  When ld_scores < *maxlev_out the call returns
- * TP_ERR_ARG with every other output filled: fetch the scores with tp_get_sweep_scores, nothing has to be recomputed. */
+ * bad_out[n]; seqdist_out[nf-1] of the optimal candidate.  nf_out/k_out/maxlev_out report the sizes actually used
+ * (k = min(max_pcs, nf)); the k x maxlev score matrix is read afterwards with tp_get_sweep_scores. */
 int tp_call(tp_ctx *ctx, const double *mat, int n, int colmajor, int on_device,
             int max_pcs, int min_clusters, double bad_frac,
             uint8_t *bad_out, int *nf_out, int *k_out,
             int *n_pcs_out, int *n_clusters_out,
-            double *scores_out, int ld_scores, int *maxlev_out,
-            double *seqdist_out);
+            int *maxlev_out, double *seqdist_out);
 /* same, starting from an explicit keep list (chromosome arms, R/TADpole.R:357-374) on the matrix
  * already held by the context after tp_filter */
 int tp_call_arm(tp_ctx *ctx, const int *keep, int nf, int max_pcs, int min_clusters,
-                int *k_out, int *n_pcs_out, int *n_clusters_out,
-                double *scores_out, int ld_scores, int *maxlev_out, double *seqdist_out);
+                int *k_out, int *n_pcs_out, int *n_clusters_out, int *maxlev_out, double *seqdist_out);
 
 /* Both chromosome arms of a centromere_search call (R/TADpole.R:357-374: the arms are independent from load_mat on), after
  * tp_filter: on a multi-device context the first half of the devices works on p while the second half works on q; on one
- * device p then q.  Outputs as tp_call_arm, element [0] / the _p buffers for p and [1] / _q for q; a too small ld_scores
- * fails with TP_ERR_ARG and maxlev_out2 filled (call again with wider buffers). */
+ * device p then q.  The results are a tp_batch (below) of two items, p then q, read with tp_batch_dims / tp_batch_get and
+ * released with tp_batch_free: n = 0 (no bad flags: the filtering was tp_filter's), nf, k, maxlev, n_pcs, n_clusters,
+ * scores, seqdist and device ms as tp_call_arm gives them, no tables. */
+typedef struct tp_batch tp_batch;
 int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int *keep_q, int nf_q, int max_pcs, int min_clusters,
-                 int *k_out2, int *n_pcs_out2, int *n_clusters_out2, double *scores_p, double *scores_q, int ld_scores,
-                 int *maxlev_out2, double *seqdist_p, double *seqdist_q);
+                 tp_batch **out);
 
 /* ---- batches of independent calls (genome-wide use: one TADpole() per chromosome) -----------------------------------
  * ncalls matrices (mats[i]: n[i] x n[i], host -- or device when on_device, single-device contexts only), same arguments
@@ -250,7 +248,6 @@ int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int *keep_q, in
  *   tp_batch_dims   sizes to allocate: n, nf, k, maxlev, number of scored levels, total table rows;
  *   tp_batch_get    bad[n], n_pcs, n_clusters, scores[k x maxlev] row-major NaN padded, seqdist[nf-1], levels[nlevels],
  *                   offsets[nlevels+1], start/end[nrows] (1-based inclusive), device ms of the call; NULL = skip. */
-typedef struct tp_batch tp_batch;
 int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
                   int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, tp_batch **out);
 int tp_batch_size(const tp_batch *b);
@@ -274,7 +271,7 @@ int tp_batch_free(tp_batch *b);
  * fresh tp_call with those arguments; the reference has to repeat load_mat, cor and prcomp for this.
  * Outputs as tp_call_arm. */
 int tp_recall(tp_ctx *ctx, int max_pcs, int min_clusters, int *k_out, int *n_pcs_out, int *n_clusters_out,
-              double *scores_out, int ld_scores, int *maxlev_out, double *seqdist_out);
+              int *maxlev_out, double *seqdist_out);
 
 /* ---- stage 6: diffT (R/DiffT.R:41-49) on padded label vectors -------------------------------------
  * labels_x / labels_y: npairs x L int32 row-major (0 = uncovered bin); out: npairs x L doubles =

@@ -148,20 +148,19 @@ SEXP C_tp_filter(SEXP ctx, SEXP mat, SEXP bad_frac) {
     return bad;
 }
 
-/* list(n_pcs, optimal_n_clusters, seqdist, scores) from the outputs of tp_call_arm / tp_recall */
-static SEXP pack_call(tp_ctx *c, int rc, int k, int npcs, int ncl, int maxlev, int ld, double *sc, int kmax, SEXP seq) {
-    if (rc == TP_ERR_ARG && maxlev > ld) {       /* more levels than the buffer: everything else is filled in */
-        ld = maxlev;
-        sc = (double *)R_alloc((size_t)kmax * ld, sizeof(double));
-        rc = tp_get_sweep_scores(c, sc, ld);
-    }
-    if (rc != TP_OK) error("%s", tp_last_error());
-    SEXP scores = PROTECT(allocMatrix(REALSXP, k, maxlev));        /* column-major for R, NaN padding -> NA */
+/* a row-major k x maxlev score matrix, NaN where a level is not scored -> an R matrix (column-major, NA); unprotected */
+static SEXP score_matrix(const double *sc, int k, int maxlev) {
+    SEXP scores = allocMatrix(REALSXP, k, maxlev);
     for (int r = 0; r < k; r++)
         for (int l = 0; l < maxlev; l++) {
-            double v = sc[(size_t)r * ld + l];
+            double v = sc[(size_t)r * maxlev + l];
             REAL(scores)[r + (size_t)l * k] = ISNAN(v) ? NA_REAL : v;
         }
+    return scores;
+}
+
+/* list(n_pcs, optimal_n_clusters, seqdist, scores, generation) of one matrix or arm; seq and scores protected by the caller */
+static SEXP call_result(tp_ctx *c, int npcs, int ncl, SEXP seq, SEXP scores) {
     SEXP out = PROTECT(allocVector(VECSXP, 5));
     SET_VECTOR_ELT(out, 0, ScalarInteger(npcs));
     SET_VECTOR_ELT(out, 1, ScalarInteger(ncl));
@@ -170,7 +169,18 @@ static SEXP pack_call(tp_ctx *c, int rc, int k, int npcs, int ncl, int maxlev, i
     SEXP gen = PROTECT(allocVector(REALSXP, 1));
     REAL(gen)[0] = (double)tp_ctx_generation(c);          /* the state this result was read from */
     SET_VECTOR_ELT(out, 4, gen);
-    UNPROTECT(3);
+    UNPROTECT(2);
+    return out;
+}
+
+/* the result of tp_call_arm / tp_recall (return code rc), with the score matrix of its sweep */
+static SEXP pack_call(tp_ctx *c, int rc, int k, int npcs, int ncl, int maxlev, SEXP seq) {
+    if (rc != TP_OK) error("%s", tp_last_error());
+    double *sc = (double *)R_alloc((size_t)k * maxlev + 1, sizeof(double));
+    if (tp_get_sweep_scores(c, sc) != TP_OK) error("%s", tp_last_error());
+    SEXP scores = PROTECT(score_matrix(sc, k, maxlev));
+    SEXP out = call_result(c, npcs, ncl, seq, scores);
+    UNPROTECT(1);
     return out;
 }
 
@@ -178,14 +188,12 @@ static SEXP pack_call(tp_ctx *c, int rc, int k, int npcs, int ncl, int maxlev, i
  * keep = 0-based original indices of the rows load_mat keeps */
 SEXP C_tp_call_arm(SEXP ctx, SEXP keep, SEXP max_pcs, SEXP min_clusters) {
     tp_ctx *c = ctx_of(ctx);
-    int nf = length(keep), k = 0, npcs = 0, ncl = 0, maxlev = 0, ld = 256;
+    int nf = length(keep), k = 0, npcs = 0, ncl = 0, maxlev = 0;
     if (nf < 3) error("TADpole: fewer than 3 good bins left after filtering");
-    int kmax = asInteger(max_pcs) < nf ? asInteger(max_pcs) : nf;
     SEXP seq = PROTECT(allocVector(REALSXP, nf - 1));
-    double *sc = (double *)R_alloc((size_t)kmax * ld, sizeof(double));
-    int rc = tp_call_arm(c, INTEGER(keep), nf, asInteger(max_pcs), asInteger(min_clusters), &k, &npcs, &ncl, sc, ld,
-                         &maxlev, REAL(seq));
-    SEXP out = pack_call(c, rc, k, npcs, ncl, maxlev, ld, sc, kmax, seq);
+    int rc = tp_call_arm(c, INTEGER(keep), nf, asInteger(max_pcs), asInteger(min_clusters), &k, &npcs, &ncl, &maxlev,
+                         REAL(seq));
+    SEXP out = pack_call(c, rc, k, npcs, ncl, maxlev, seq);
     UNPROTECT(1);
     return out;
 }
@@ -195,15 +203,13 @@ SEXP C_tp_call_arm(SEXP ctx, SEXP keep, SEXP max_pcs, SEXP min_clusters) {
 SEXP C_tp_recall(SEXP ctx, SEXP generation, SEXP max_pcs, SEXP min_clusters) {
     tp_ctx *c = ctx_of(ctx);
     check_generation(c, generation);
-    int nf = 0, kfull = 0, k = 0, npcs = 0, ncl = 0, maxlev = 0, ld = 256;
+    int nf = 0, kfull = 0, k = 0, npcs = 0, ncl = 0, maxlev = 0;
     if (tp_ctx_dims(c, NULL, &nf, NULL, &kfull, NULL) != TP_OK) error("%s", tp_last_error());
     if (nf < 3 || kfull < 1) error("TADpole: the context holds no PC scores");
-    int kmax = asInteger(max_pcs) < nf ? asInteger(max_pcs) : nf;
-    if (kmax < 1) error("TADpole: max_pcs must be positive");
+    if (asInteger(max_pcs) < 1) error("TADpole: max_pcs must be positive");
     SEXP seq = PROTECT(allocVector(REALSXP, nf - 1));
-    double *sc = (double *)R_alloc((size_t)kmax * ld, sizeof(double));
-    int rc = tp_recall(c, asInteger(max_pcs), asInteger(min_clusters), &k, &npcs, &ncl, sc, ld, &maxlev, REAL(seq));
-    SEXP out = pack_call(c, rc, k, npcs, ncl, maxlev, ld, sc, kmax, seq);
+    int rc = tp_recall(c, asInteger(max_pcs), asInteger(min_clusters), &k, &npcs, &ncl, &maxlev, REAL(seq));
+    SEXP out = pack_call(c, rc, k, npcs, ncl, maxlev, seq);
     UNPROTECT(1);
     return out;
 }
@@ -253,35 +259,64 @@ SEXP C_tp_find_groups(SEXP seqdist) {
     return m;
 }
 
+/* item i of a tp_batch: list(bad, n_pcs, optimal_n_clusters, seqdist, scores, levels, tables = list of 2-column
+ * (start, end) matrices), or the call's error message; unprotected */
+static SEXP batch_item(tp_batch *b, int i) {
+    if (tp_batch_status(b, i) != TP_OK) {
+        SEXP msg = PROTECT(allocVector(STRSXP, 1));
+        SET_STRING_ELT(msg, 0, mkChar(tp_batch_error(b, i)));
+        UNPROTECT(1);
+        return msg;
+    }
+    int nn, nf, k, maxlev, nlev, nrow;
+    tp_batch_dims(b, i, &nn, &nf, &k, &maxlev, &nlev, &nrow);
+    SEXP bad = PROTECT(allocVector(LGLSXP, nn)), seq = PROTECT(allocVector(REALSXP, nf - 1));
+    SEXP levels = PROTECT(allocVector(INTSXP, nlev)), tables = PROTECT(allocVector(VECSXP, nlev));
+    unsigned char *tb = (unsigned char *)R_alloc((size_t)nn, 1);
+    double *sc = (double *)R_alloc((size_t)k * maxlev + 1, sizeof(double));
+    int *off = (int *)R_alloc((size_t)nlev + 1, sizeof(int)), *st = (int *)R_alloc((size_t)nrow + 1, sizeof(int)),
+        *en = (int *)R_alloc((size_t)nrow + 1, sizeof(int));
+    int npcs = 0, ncl = 0;
+    tp_batch_get(b, i, tb, &npcs, &ncl, sc, REAL(seq), INTEGER(levels), off, st, en, NULL);
+    for (int j = 0; j < nn; j++) LOGICAL(bad)[j] = tb[j];
+    SEXP scores = PROTECT(score_matrix(sc, k, maxlev));
+    for (int l = 0; l < nlev; l++) {
+        int rows = off[l + 1] - off[l];
+        SEXP m = PROTECT(allocMatrix(INTSXP, rows, 2));
+        for (int r = 0; r < rows; r++) { INTEGER(m)[r] = st[off[l] + r]; INTEGER(m)[r + rows] = en[off[l] + r]; }
+        SET_VECTOR_ELT(tables, l, m);
+        UNPROTECT(1);
+    }
+    SEXP item = PROTECT(allocVector(VECSXP, 7));
+    SET_VECTOR_ELT(item, 0, bad);
+    SET_VECTOR_ELT(item, 1, ScalarInteger(npcs));
+    SET_VECTOR_ELT(item, 2, ScalarInteger(ncl));
+    SET_VECTOR_ELT(item, 3, seq);
+    SET_VECTOR_ELT(item, 4, scores);
+    SET_VECTOR_ELT(item, 5, levels);
+    SET_VECTOR_ELT(item, 6, tables);
+    UNPROTECT(6);
+    return item;
+}
+
 /* both arms of a centromere_search call at once (R/TADpole.R:357-374); on a multi-device context the two halves of the
  * devices work on the two arms at the same time.  list(p = <as C_tp_call_arm>, q = ...) */
 SEXP C_tp_call_arms(SEXP ctx, SEXP keep_p, SEXP keep_q, SEXP max_pcs, SEXP min_clusters) {
     tp_ctx *c = ctx_of(ctx);
-    SEXP keep[2] = {keep_p, keep_q};
-    int nf[2] = {length(keep_p), length(keep_q)}, kmax[2], k[2], npcs[2], ncl[2], maxlev[2] = {0, 0}, ld = 256, rc;
-    if (nf[0] < 3 || nf[1] < 3) error("TADpole: fewer than 3 good bins left in an arm after filtering");
-    SEXP seq0 = PROTECT(allocVector(REALSXP, nf[0] - 1)), seq1 = PROTECT(allocVector(REALSXP, nf[1] - 1));
-    SEXP seq[2] = {seq0, seq1};
-    double *sc[2];
-    for (;;) {
-        for (int a = 0; a < 2; a++) {
-            kmax[a] = asInteger(max_pcs) < nf[a] ? asInteger(max_pcs) : nf[a];
-            sc[a] = (double *)R_alloc((size_t)kmax[a] * ld, sizeof(double));
-        }
-        rc = tp_call_arms(c, INTEGER(keep[0]), nf[0], INTEGER(keep[1]), nf[1], asInteger(max_pcs), asInteger(min_clusters),
-                          k, npcs, ncl, sc[0], sc[1], ld, maxlev, REAL(seq[0]), REAL(seq[1]));
-        int need = maxlev[0] > maxlev[1] ? maxlev[0] : maxlev[1];
-        if (rc == TP_ERR_ARG && need > ld) { ld = need; continue; }       /* rare: more levels than the buffers hold */
-        break;
-    }
-    if (rc != TP_OK) {
-        UNPROTECT(2);
+    if (length(keep_p) < 3 || length(keep_q) < 3) error("TADpole: fewer than 3 good bins left in an arm after filtering");
+    tp_batch *b = NULL;
+    if (tp_call_arms(c, INTEGER(keep_p), length(keep_p), INTEGER(keep_q), length(keep_q), asInteger(max_pcs),
+                     asInteger(min_clusters), &b) != TP_OK)
         error("%s", tp_last_error());
-    }
     SEXP out = PROTECT(allocVector(VECSXP, 2));
-    for (int a = 0; a < 2; a++)
-        SET_VECTOR_ELT(out, a, pack_call(c, TP_OK, k[a], npcs[a], ncl[a], maxlev[a], ld, sc[a], kmax[a], seq[a]));
-    UNPROTECT(3);
+    for (int a = 0; a < 2; a++) {
+        SEXP it = PROTECT(batch_item(b, a));
+        SET_VECTOR_ELT(out, a, call_result(c, asInteger(VECTOR_ELT(it, 1)), asInteger(VECTOR_ELT(it, 2)), VECTOR_ELT(it, 3),
+                                           VECTOR_ELT(it, 4)));
+        UNPROTECT(1);
+    }
+    tp_batch_free(b);
+    UNPROTECT(1);
     return out;
 }
 
@@ -305,49 +340,7 @@ SEXP C_tp_call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP 
         error("%s", tp_last_error());
     /* (an R allocation failure below longjmps past tp_batch_free: the batch, plain host memory, is then leaked) */
     SEXP out = PROTECT(allocVector(VECSXP, nc));
-    for (int i = 0; i < nc; i++) {
-        if (tp_batch_status(b, i) != TP_OK) {
-            SEXP msg = PROTECT(allocVector(STRSXP, 1));
-            SET_STRING_ELT(msg, 0, mkChar(tp_batch_error(b, i)));
-            SET_VECTOR_ELT(out, i, msg);
-            UNPROTECT(1);
-            continue;
-        }
-        int nn, nf, k, maxlev, nlev, nrow;
-        tp_batch_dims(b, i, &nn, &nf, &k, &maxlev, &nlev, &nrow);
-        SEXP bad = PROTECT(allocVector(LGLSXP, nn)), seq = PROTECT(allocVector(REALSXP, nf - 1));
-        SEXP scores = PROTECT(allocMatrix(REALSXP, k, maxlev)), levels = PROTECT(allocVector(INTSXP, nlev));
-        SEXP tables = PROTECT(allocVector(VECSXP, nlev));
-        unsigned char *tb = (unsigned char *)R_alloc((size_t)nn, 1);
-        double *sc = (double *)R_alloc((size_t)k * maxlev + 1, sizeof(double));
-        int *off = (int *)R_alloc((size_t)nlev + 1, sizeof(int)), *st = (int *)R_alloc((size_t)nrow + 1, sizeof(int)),
-            *en = (int *)R_alloc((size_t)nrow + 1, sizeof(int));
-        int npcs = 0, ncl = 0;
-        tp_batch_get(b, i, tb, &npcs, &ncl, sc, REAL(seq), INTEGER(levels), off, st, en, NULL);
-        for (int j = 0; j < nn; j++) LOGICAL(bad)[j] = tb[j];
-        for (int r = 0; r < k; r++)
-            for (int l = 0; l < maxlev; l++) {
-                double v = sc[(size_t)r * maxlev + l];
-                REAL(scores)[r + (size_t)l * k] = ISNAN(v) ? NA_REAL : v;
-            }
-        for (int l = 0; l < nlev; l++) {
-            int rows = off[l + 1] - off[l];
-            SEXP m = PROTECT(allocMatrix(INTSXP, rows, 2));
-            for (int r = 0; r < rows; r++) { INTEGER(m)[r] = st[off[l] + r]; INTEGER(m)[r + rows] = en[off[l] + r]; }
-            SET_VECTOR_ELT(tables, l, m);
-            UNPROTECT(1);
-        }
-        SEXP item = PROTECT(allocVector(VECSXP, 7));
-        SET_VECTOR_ELT(item, 0, bad);
-        SET_VECTOR_ELT(item, 1, ScalarInteger(npcs));
-        SET_VECTOR_ELT(item, 2, ScalarInteger(ncl));
-        SET_VECTOR_ELT(item, 3, seq);
-        SET_VECTOR_ELT(item, 4, scores);
-        SET_VECTOR_ELT(item, 5, levels);
-        SET_VECTOR_ELT(item, 6, tables);
-        SET_VECTOR_ELT(out, i, item);
-        UNPROTECT(6);
-    }
+    for (int i = 0; i < nc; i++) SET_VECTOR_ELT(out, i, batch_item(b, i));
     tp_batch_free(b);
     UNPROTECT(1);
     return out;

@@ -61,7 +61,7 @@ def load():
         "tp_ctx_devices": (c_int, [vp, ip, c_int]),
         "tp_ctx_generation": (c_longlong, [vp]),
         "tp_ctx_dims": (c_int, [vp, ip, ip, ip, ip, ip]),
-        "tp_call_arms": (c_int, [vp, ip, c_int, ip, c_int, c_int, c_int, ip, ip, ip, dp, dp, c_int, ip, dp, dp]),
+        "tp_call_arms": (c_int, [vp, ip, c_int, ip, c_int, c_int, c_int, POINTER(vp)]),
         "tp_call_batch": (c_int, [vp, c_int, POINTER(vp), ip, c_int, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
         "tp_batch_size": (c_int, [vp]),
         "tp_batch_device_ms": (c_double, [vp]),
@@ -109,13 +109,13 @@ def load():
         "tp_test_ss_tile": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int]),
         "tp_get_scores": (c_int, [vp, dp]),
         "tp_set_scores": (c_int, [vp, dp, c_int, c_int]),
-        "tp_sweep": (c_int, [vp, c_int, c_int, c_int, ip, dp, c_int, ip]),
+        "tp_sweep": (c_int, [vp, c_int, c_int, c_int, ip, ip]),
         "tp_get_dendro": (c_int, [vp, c_int, dp, ip]),
-        "tp_get_sweep_scores": (c_int, [vp, dp, c_int]),
+        "tp_get_sweep_scores": (c_int, [vp, dp]),
         "tp_select": (c_int, [dp, c_int, c_int, c_int, ip, ip]),
-        "tp_call": (c_int, [vp, vp, c_int, c_int, c_int, c_int, c_int, c_double, u8p, ip, ip, ip, ip, dp, c_int, ip, dp]),
-        "tp_call_arm": (c_int, [vp, ip, c_int, c_int, c_int, ip, ip, ip, dp, c_int, ip, dp]),
-        "tp_recall": (c_int, [vp, c_int, c_int, ip, ip, ip, dp, c_int, ip, dp]),
+        "tp_call": (c_int, [vp, vp, c_int, c_int, c_int, c_int, c_int, c_double, u8p, ip, ip, ip, ip, ip, dp]),
+        "tp_call_arm": (c_int, [vp, ip, c_int, c_int, c_int, ip, ip, ip, ip, dp]),
+        "tp_recall": (c_int, [vp, c_int, c_int, ip, ip, ip, ip, dp]),
         "tp_difft_batch": (c_int, [vp, vp, vp, c_int, c_int, c_int, vp]),
         "tp_difft_null": (c_int, [vp, vp, c_int, c_int, c_int, c_int, vp, c_int, ctypes.c_ulonglong, c_int, vp, vp, vp, vp]),
         "tp_assemble": (c_int, [dp, c_int, c_int, ip, ip, c_int, ip, ip, ip, ip]),
@@ -406,19 +406,18 @@ class Context:
         check(self.lib.tp_set_scores(self._h, _dp(scores), scores.shape[0], scores.shape[1]))
 
     # ---- stages 4 + 5 ----
-    def sweep(self, k, min_clusters=2, cand_begin=0, cand_stride=1, ld=256):
+    def sweep(self, k, min_clusters=2, cand_begin=0, cand_stride=1):
         """Returns (n_cluster[k], scores[k, maxlev] NaN padded)."""
         ncl = np.zeros(k, dtype=np.int32)
         maxlev = c_int(0)
-        while True:
-            sc = np.empty((k, ld))
-            rc = self.lib.tp_sweep(self._h, int(min_clusters), int(cand_begin), int(cand_stride),
-                                   _ip(ncl), _dp(sc), ld, ctypes.byref(maxlev))
-            if rc == TP_ERR_ARG and maxlev.value > ld:
-                ld = maxlev.value
-                continue
-            check(rc)
-            return ncl, sc[:, :max(maxlev.value, 1)].copy() if maxlev.value else sc[:, :0]
+        check(self.lib.tp_sweep(self._h, int(min_clusters), int(cand_begin), int(cand_stride), _ip(ncl), ctypes.byref(maxlev)))
+        return ncl, self._sweep_scores(k, maxlev.value)
+
+    def _sweep_scores(self, k, maxlev):
+        """tp_get_sweep_scores: the k x maxlev score matrix of the last sweep."""
+        sc = np.empty((k, maxlev))
+        check(self.lib.tp_get_sweep_scores(self._h, _dp(sc)))
+        return sc
 
     def dendro(self, cand, nf):
         seq = np.zeros(nf - 1)
@@ -435,7 +434,7 @@ class Context:
 
     # ---- one-shot ----
     def call(self, mat=None, max_pcs=200, min_clusters=2, bad_frac=0.01, device_ptr=None, n=None, colmajor=None,
-             ld=256, want_scores=True):
+             want_scores=True):
         if device_ptr is None:
             mat = np.asarray(mat)
             if mat.dtype != np.float64 or not (mat.flags.c_contiguous or mat.flags.f_contiguous):
@@ -447,64 +446,53 @@ class Context:
             ptr, ondev, colmajor = int(device_ptr), 1, int(bool(colmajor))
         bad = np.zeros(n, dtype=np.uint8)
         nf, k, npcs, ncl, maxlev = c_int(0), c_int(0), c_int(0), c_int(0), c_int(0)
-        kmax = min(int(max_pcs), n)
         seq = np.zeros(max(n - 1, 1))
-        while True:
-            sc = np.empty((kmax, ld)) if want_scores else None
-            rc = self.lib.tp_call(self._h, ptr, n, colmajor, ondev, int(max_pcs), int(min_clusters), float(bad_frac),
-                                  bad.ctypes.data_as(POINTER(c_uint8)), ctypes.byref(nf), ctypes.byref(k),
-                                  ctypes.byref(npcs), ctypes.byref(ncl),
-                                  _dp(sc) if want_scores else None, ld, ctypes.byref(maxlev), _dp(seq))
-            if rc == TP_ERR_ARG and maxlev.value > ld:       # everything else is filled in: fetch the wider score matrix
-                ld = maxlev.value
-                if want_scores:
-                    sc = np.empty((kmax, ld))
-                    check(self.lib.tp_get_sweep_scores(self._h, _dp(sc), ld))
-                break
-            check(rc)
-            break
+        check(self.lib.tp_call(self._h, ptr, n, colmajor, ondev, int(max_pcs), int(min_clusters), float(bad_frac),
+                               bad.ctypes.data_as(POINTER(c_uint8)), ctypes.byref(nf), ctypes.byref(k),
+                               ctypes.byref(npcs), ctypes.byref(ncl), ctypes.byref(maxlev), _dp(seq)))
         return dict(bad=bad.astype(bool), nf=nf.value, k=k.value, n_pcs=npcs.value, n_clusters=ncl.value,
-                    scores=sc[:k.value, :maxlev.value].copy() if want_scores else None,
+                    scores=self._sweep_scores(k.value, maxlev.value) if want_scores else None,
                     seqdist=seq[:nf.value - 1].copy())
 
-    def call_arm(self, keep, max_pcs=200, min_clusters=2, ld=256):
+    def call_arm(self, keep, max_pcs=200, min_clusters=2):
         keep = np.ascontiguousarray(keep, dtype=np.int32)
         nf = keep.size
         k, npcs, ncl, maxlev = c_int(0), c_int(0), c_int(0), c_int(0)
-        kmax = min(int(max_pcs), nf)
         seq = np.zeros(nf - 1)
-        while True:
-            sc = np.empty((kmax, ld))
-            rc = self.lib.tp_call_arm(self._h, _ip(keep), nf, int(max_pcs), int(min_clusters), ctypes.byref(k),
-                                      ctypes.byref(npcs), ctypes.byref(ncl), _dp(sc), ld, ctypes.byref(maxlev), _dp(seq))
-            if rc == TP_ERR_ARG and maxlev.value > ld:
-                ld = maxlev.value
-                sc = np.empty((kmax, ld))
-                check(self.lib.tp_get_sweep_scores(self._h, _dp(sc), ld))
-                break
-            check(rc)
-            break
+        check(self.lib.tp_call_arm(self._h, _ip(keep), nf, int(max_pcs), int(min_clusters), ctypes.byref(k),
+                                   ctypes.byref(npcs), ctypes.byref(ncl), ctypes.byref(maxlev), _dp(seq)))
         return dict(nf=nf, k=k.value, n_pcs=npcs.value, n_clusters=ncl.value,
-                    scores=sc[:k.value, :maxlev.value].copy(), seqdist=seq)
+                    scores=self._sweep_scores(k.value, maxlev.value), seqdist=seq)
 
-    def call_arms(self, keep_p, keep_q, max_pcs=200, min_clusters=2, ld=256):
+    def call_arms(self, keep_p, keep_q, max_pcs=200, min_clusters=2):
         """tp_call_arms: both chromosome arms (on disjoint halves of the devices of a multi-device context).
         Returns (result_p, result_q), each as call_arm returns."""
         kp = np.ascontiguousarray(keep_p, dtype=np.int32)
         kq = np.ascontiguousarray(keep_q, dtype=np.int32)
-        while True:
-            k, npcs, ncl, ml = (np.zeros(2, np.int32) for _ in range(4))
-            scs = [np.empty((min(int(max_pcs), kk.size), ld)) for kk in (kp, kq)]
-            sqs = [np.zeros(kk.size - 1) for kk in (kp, kq)]
-            rc = self.lib.tp_call_arms(self._h, _ip(kp), kp.size, _ip(kq), kq.size, int(max_pcs), int(min_clusters),
-                                       _ip(k), _ip(npcs), _ip(ncl), _dp(scs[0]), _dp(scs[1]), ld, _ip(ml), _dp(sqs[0]), _dp(sqs[1]))
-            if rc == TP_ERR_ARG and int(ml.max()) > ld:
-                ld = int(ml.max())
-                continue
-            check(rc)
-            break
-        return tuple(dict(nf=int(kk.size), k=int(k[a]), n_pcs=int(npcs[a]), n_clusters=int(ncl[a]),
-                          scores=scs[a][:k[a], :ml[a]].copy(), seqdist=sqs[a]) for a, kk in enumerate((kp, kq)))
+        h = c_void_p()
+        check(self.lib.tp_call_arms(self._h, _ip(kp), kp.size, _ip(kq), kq.size, int(max_pcs), int(min_clusters),
+                                    ctypes.byref(h)))
+        try:
+            items = [self._batch_item(h, a, tables=False) for a in range(2)]
+        finally:
+            self.lib.tp_batch_free(h)
+        return tuple({key: it[key] for key in ("nf", "k", "n_pcs", "n_clusters", "scores", "seqdist")} for it in items)
+
+    def _batch_item(self, h, i, tables):
+        """Item i of a tp_batch as the dict call() returns, plus 'tables' {level: [rows, 2]} (or None) and 'device_ms'."""
+        d = [c_int(0) for _ in range(6)]
+        check(self.lib.tp_batch_dims(h, i, *[ctypes.byref(x) for x in d]))
+        nn, nf, k, ml, nlev, nrows = (x.value for x in d)
+        bad = np.zeros(nn, np.uint8); sc = np.empty((k, ml)); seq = np.empty(nf - 1)
+        lev = np.zeros(nlev, np.int32); off = np.zeros(nlev + 1, np.int32)
+        st = np.zeros(nrows, np.int32); en = np.zeros(nrows, np.int32)
+        npcs, ncl, ms = c_int(0), c_int(0), c_double(0.0)
+        check(self.lib.tp_batch_get(h, i, bad.ctypes.data_as(POINTER(c_uint8)), ctypes.byref(npcs), ctypes.byref(ncl),
+                                    _dp(sc), _dp(seq), _ip(lev), _ip(off), _ip(st), _ip(en), ctypes.byref(ms)))
+        tab = np.stack([st, en], axis=1).astype(np.int64)
+        return dict(bad=bad.astype(bool), nf=nf, k=k, n_pcs=npcs.value, n_clusters=ncl.value, scores=sc, seqdist=seq,
+                    tables={int(l): tab[off[j]: off[j + 1]] for j, l in enumerate(lev)} if tables else None,
+                    device_ms=ms.value)
 
     def call_batch(self, mats, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True, device_ptrs=None, n=None):
         """tp_call_batch: one tp_call per matrix, `inflight` calls per device kept in flight by library-owned threads over
@@ -537,39 +525,19 @@ class Context:
                 if rc != TP_OK:
                     out.append(TadpoleError(rc, self.lib.tp_batch_error(h, i).decode("utf-8", "replace")))
                     continue
-                d = [c_int(0) for _ in range(6)]
-                check(self.lib.tp_batch_dims(h, i, *[ctypes.byref(x) for x in d]))
-                nn, nf, k, ml, nlev, nrows = (x.value for x in d)
-                bad = np.zeros(nn, np.uint8); sc = np.empty((k, ml)); seq = np.empty(nf - 1)
-                lev = np.zeros(nlev, np.int32); off = np.zeros(nlev + 1, np.int32)
-                st = np.zeros(nrows, np.int32); en = np.zeros(nrows, np.int32)
-                npcs, ncl, ms = c_int(0), c_int(0), c_double(0.0)
-                check(self.lib.tp_batch_get(h, i, bad.ctypes.data_as(POINTER(c_uint8)), ctypes.byref(npcs), ctypes.byref(ncl),
-                                            _dp(sc), _dp(seq), _ip(lev), _ip(off), _ip(st), _ip(en), ctypes.byref(ms)))
-                tab = np.stack([st, en], axis=1).astype(np.int64)
-                out.append(dict(bad=bad.astype(bool), nf=nf, k=k, n_pcs=npcs.value, n_clusters=ncl.value, scores=sc, seqdist=seq,
-                                tables={int(l): tab[off[j]: off[j + 1]] for j, l in enumerate(lev)} if tables else None,
-                                device_ms=ms.value))
+                out.append(self._batch_item(h, i, tables))
         finally:
             self.lib.tp_batch_free(h)
         return out
 
-    def recall(self, nf, max_pcs=200, min_clusters=2, ld=256):
+    def recall(self, nf, max_pcs=200, min_clusters=2):
         """tp_recall: the n_pcs sweep and the selection again on the PC scores resident in the context."""
         k, npcs, ncl, maxlev = c_int(0), c_int(0), c_int(0), c_int(0)
-        kmax = min(int(max_pcs), nf)
         seq = np.zeros(nf - 1)
-        sc = np.empty((kmax, ld))
-        rc = self.lib.tp_recall(self._h, int(max_pcs), int(min_clusters), ctypes.byref(k), ctypes.byref(npcs),
-                                ctypes.byref(ncl), _dp(sc), ld, ctypes.byref(maxlev), _dp(seq))
-        if rc == TP_ERR_ARG and maxlev.value > ld:
-            ld = maxlev.value
-            sc = np.empty((kmax, ld))
-            check(self.lib.tp_get_sweep_scores(self._h, _dp(sc), ld))
-        else:
-            check(rc)
+        check(self.lib.tp_recall(self._h, int(max_pcs), int(min_clusters), ctypes.byref(k), ctypes.byref(npcs),
+                                 ctypes.byref(ncl), ctypes.byref(maxlev), _dp(seq)))
         return dict(nf=nf, k=k.value, n_pcs=npcs.value, n_clusters=ncl.value,
-                    scores=sc[:k.value, :maxlev.value].copy(), seqdist=seq)
+                    scores=self._sweep_scores(k.value, maxlev.value), seqdist=seq)
 
     # ---- stage 6 ----
     def difft_batch(self, lx, ly):

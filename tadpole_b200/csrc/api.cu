@@ -8,7 +8,6 @@
 
 int tp_sweep_device(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stride, int *ncand_out);
 int tp_ch_device(tp_ctx *ctx, int min_clusters, int ncand, int ld_chs);
-extern "C" int tp_get_sweep_scores(tp_ctx *ctx, double *scores_out, int ld_scores);
 
 static thread_local char g_err[1024] = "";
 
@@ -20,7 +19,7 @@ void tp_set_error(const char *fmt, ...) {
 }
 
 extern "C" const char *tp_last_error(void) { return g_err; }
-extern "C" int tp_version(void) { return 100; }
+extern "C" int tp_version(void) { return 101; }
 
 int tp_pin_reserve(tp_ctx *ctx, size_t bytes) {
     if (bytes <= ctx->pin_cap) return TP_OK;
@@ -488,15 +487,18 @@ __global__ void zero_foreign_rows_kernel(double *chs, int *ncl, int k, int ld, i
 // collective == true: the candidates are dealt out rank-interleaved over the current communicator (cost grows with
 // the number of PCs) and the level counts / CH rows are combined on every rank; cand_begin / cand_stride are ignored
 static int sweep_impl(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stride,
-                      int *n_cluster_out, double *scores_out, int ld_scores, int *maxlev_out, bool collective = false) {
+                      int *n_cluster_out, int *maxlev_out, bool collective = false) {
     int ncand = 0;
     collective = collective && tp_nranks(ctx) > 1;
     if (collective) { cand_begin = tp_rank(ctx); cand_stride = tp_nranks(ctx); }    // (a rank may end up with no candidate)
     ctx->generation++;
     ctx->last_sweep_ranks = collective ? tp_nranks(ctx) : 1;
+    // a sweep that runs no candidate or fails leaves no width or scores of an earlier sweep readable
+    ctx->last_maxlev = 0;
+    ctx->sweep_scores.clear();
+    if (maxlev_out) *maxlev_out = 0;
     TP_TRY(tp_sweep_device(ctx, min_clusters, cand_begin, cand_stride, &ncand));
     const int k = ctx->k;
-    if (maxlev_out) *maxlev_out = 0;
     if (ncand == 0 && !collective) {
         if (n_cluster_out) std::fill(n_cluster_out, n_cluster_out + k, 0);
         return TP_OK;
@@ -528,44 +530,30 @@ static int sweep_impl(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_st
         if (maxlev <= ld) break;
         ld = round_up(maxlev, 8);          // rare: more levels than the cap; redo the cheap CH pass wider
     }
-    if (maxlev_out) *maxlev_out = maxlev;
-    ctx->last_maxlev = maxlev;
     if (n_cluster_out) memcpy(n_cluster_out, h_ncl, (size_t)k * sizeof(int));
-    if (scores_out) {
-        if (ld_scores < maxlev) {
-            tp_set_error("tp_sweep: ld_scores = %d is smaller than the %d levels found", ld_scores, maxlev);
-            return TP_ERR_ARG;
-        }
-        // NaN-fill, then copy the first maxlev columns of every row
-        for (size_t i = 0; i < (size_t)k * ld_scores; i++) scores_out[i] = NAN;
-        if (maxlev > 0)
-            TP_CUDA(cudaMemcpy2DAsync(scores_out, (size_t)ld_scores * sizeof(double), ctx->chs.p,
-                                      (size_t)ctx->ld_chs * sizeof(double), (size_t)maxlev * sizeof(double), k,
-                                      cudaMemcpyDeviceToHost, ctx->stream));
-        TP_CUDA(tp_stream_sync(ctx));
-    }
-    return TP_OK;
-}
-
-// score matrix of the last sweep: k rows (candidates) x maxlev columns, NaN padded, row pitch ld_scores >= maxlev
-extern "C" int tp_get_sweep_scores(tp_ctx *ctx, double *scores_out, int ld_scores) {
-    TP_ARG(ctx && scores_out && ctx->have_sweep, "tp_get_sweep_scores: run tp_sweep / tp_call first");
-    const int k = ctx->k, maxlev = ctx->last_maxlev;
-    TP_ARG(ld_scores >= maxlev, "tp_get_sweep_scores: ld_scores smaller than the number of levels");
-    for (size_t i = 0; i < (size_t)k * ld_scores; i++) scores_out[i] = NAN;
+    // the first maxlev columns of every row (in a collective sweep the all-reduced rows, complete on every rank)
+    ctx->sweep_scores.resize((size_t)k * maxlev);
     if (maxlev > 0)
-        TP_CUDA(cudaMemcpy2DAsync(scores_out, (size_t)ld_scores * sizeof(double), ctx->chs.p,
+        TP_CUDA(cudaMemcpy2DAsync(ctx->sweep_scores.data(), (size_t)maxlev * sizeof(double), ctx->chs.p,
                                   (size_t)ctx->ld_chs * sizeof(double), (size_t)maxlev * sizeof(double), k,
                                   cudaMemcpyDeviceToHost, ctx->stream));
     TP_CUDA(tp_stream_sync(ctx));
+    ctx->last_maxlev = maxlev;
+    if (maxlev_out) *maxlev_out = maxlev;
     return TP_OK;
 }
 
-extern "C" int tp_sweep(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stride,
-                        int *n_cluster_out, double *scores_out, int ld_scores, int *maxlev_out) {
+extern "C" int tp_get_sweep_scores(tp_ctx *ctx, double *scores_out) {
+    TP_ARG(ctx && scores_out && ctx->have_sweep, "tp_get_sweep_scores: run tp_sweep / tp_call first");
+    std::copy(ctx->sweep_scores.begin(), ctx->sweep_scores.end(), scores_out);
+    return TP_OK;
+}
+
+extern "C" int tp_sweep(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stride, int *n_cluster_out,
+                        int *maxlev_out) {
     TP_ARG(ctx, "tp_sweep: null context");
     TP_CUDA(cudaSetDevice(ctx->device));
-    return sweep_impl(ctx, min_clusters, cand_begin, cand_stride, n_cluster_out, scores_out, ld_scores, maxlev_out);
+    return sweep_impl(ctx, min_clusters, cand_begin, cand_stride, n_cluster_out, maxlev_out);
 }
 
 extern "C" int tp_get_dendro(tp_ctx *ctx, int cand, double *seqdist_out, int *order_out) {
@@ -635,53 +623,34 @@ extern "C" int tp_select(const double *scores, int k, int ld, int maxlev, int *o
 
 // ---- one-shot -----------------------------------------------------------------------------------------
 // stages 4 + 5 and the selection on the context's PC scores (first ctx->k columns)
-static int sweep_and_select(tp_ctx *ctx, int min_clusters, int *n_pcs_out, int *n_clusters_out, double *scores_out,
-                            int ld_scores, int *maxlev_out, double *seqdist_out) {
-    const int k = ctx->k;
-    int maxlev = 0;
-    // the sweep runs once; the score matrix stays on the device (tp_get_sweep_scores) and is copied to the caller's
-    // buffer when that is wide enough.  A narrow buffer makes the call return TP_ERR_ARG with *maxlev_out set and every
-    // other output filled, so the caller only has to fetch the scores again, not to repeat the pipeline.
-    int rc = sweep_impl(ctx, min_clusters, 0, 1, nullptr, nullptr, 0, &maxlev, true);
-    if (maxlev_out) *maxlev_out = maxlev;
-    TP_TRY(rc);
-    const int ld = std::max(maxlev, 1);
-    std::vector<double> local((size_t)k * ld);
-    TP_TRY(tp_get_sweep_scores(ctx, local.data(), ld));
-    const double *sc = local.data();
+static int sweep_and_select(tp_ctx *ctx, int min_clusters, int *n_pcs_out, int *n_clusters_out, int *maxlev_out,
+                            double *seqdist_out) {
+    TP_TRY(sweep_impl(ctx, min_clusters, 0, 1, nullptr, maxlev_out, true));
+    const int maxlev = ctx->last_maxlev;
     int oc = 0, ol = 0;
-    TP_TRY(tp_select(sc, k, ld, maxlev, &oc, &ol));
+    TP_TRY(tp_select(ctx->sweep_scores.data(), ctx->k, maxlev, maxlev, &oc, &ol));
     if (n_pcs_out) *n_pcs_out = oc + 1;
     if (n_clusters_out) *n_clusters_out = ol + 1;
-    if (tp_nranks(ctx) > 1) {       // the optimal candidate's dendrogram lives on the rank that ran it
-        const int n1 = ctx->nf - 1, ldd = round_up(n1, 8);
-        TP_TRY(tp_comm_bcast(ctx, ctx->seqdist.as<double>() + (size_t)oc * ldd, (size_t)n1, oc % tp_nranks(ctx)));
+    // the optimal candidate's dendrogram lives on the rank that ran it: after the broadcast every rank holds the row
+    const int n1 = ctx->nf - 1, ldd = round_up(n1, 8);
+    double *row = ctx->seqdist.as<double>() + (size_t)oc * ldd;
+    if (tp_nranks(ctx) > 1) TP_TRY(tp_comm_bcast(ctx, row, (size_t)n1, oc % tp_nranks(ctx)));
+    if (seqdist_out) {
+        TP_CUDA(cudaMemcpyAsync(seqdist_out, row, (size_t)n1 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        TP_CUDA(tp_stream_sync(ctx));
     }
-    if (seqdist_out) TP_TRY(tp_get_dendro(ctx, oc, seqdist_out, nullptr));
     TP_MARK(ctx, EV_TOTAL1);
-    if (scores_out) {
-        if (ld_scores < maxlev) {
-            tp_set_error("tp_call: ld_scores = %d is smaller than the %d levels found (fetch them with tp_get_sweep_scores)",
-                         ld_scores, maxlev);
-            return TP_ERR_ARG;
-        }
-        for (int r = 0; r < k; r++) {
-            memcpy(scores_out + (size_t)r * ld_scores, local.data() + (size_t)r * ld, (size_t)maxlev * sizeof(double));
-            for (int c = maxlev; c < ld_scores; c++) scores_out[(size_t)r * ld_scores + c] = NAN;
-        }
-    }
     return TP_OK;
 }
 
 static int call_from_compacted(tp_ctx *ctx, int max_pcs, int min_clusters, int *k_out, int *n_pcs_out,
-                               int *n_clusters_out, double *scores_out, int ld_scores, int *maxlev_out,
-                               double *seqdist_out) {
+                               int *n_clusters_out, int *maxlev_out, double *seqdist_out) {
     int k = 0;
     TP_TRY(tp_correlation(ctx));
     TP_TRY(tp_pca(ctx, max_pcs, &k));
     if (k_out) *k_out = k;
     if (ctx->after_pca) ctx->after_pca();                // batch worker: the next matrix uploads under the sweep
-    return sweep_and_select(ctx, min_clusters, n_pcs_out, n_clusters_out, scores_out, ld_scores, maxlev_out, seqdist_out);
+    return sweep_and_select(ctx, min_clusters, n_pcs_out, n_clusters_out, maxlev_out, seqdist_out);
 }
 
 // The PC scores of the last call stay in the context: another (max_pcs, min_clusters) only repeats the n_pcs sweep.
@@ -689,12 +658,12 @@ static int call_from_compacted(tp_ctx *ctx, int max_pcs, int min_clusters, int *
 // their first k' columns is what a fresh call with max_pcs = k' computes (R/TADpole.R:366-367; CH on those k'
 // columns, quirk Q2).
 extern "C" int tp_recall(tp_ctx *ctx, int max_pcs, int min_clusters, int *k_out, int *n_pcs_out, int *n_clusters_out,
-                         double *scores_out, int ld_scores, int *maxlev_out, double *seqdist_out) {
+                         int *maxlev_out, double *seqdist_out) {
     TP_ARG(ctx, "tp_recall: null context");
     if (tp_group_dispatch(ctx))
         return tp_group_run(ctx, [&](tp_ctx *gc, int gr) -> int {
-            return gr ? tp_recall(gc, max_pcs, min_clusters, nullptr, nullptr, nullptr, nullptr, 0, nullptr, nullptr)
-                      : tp_recall(gc, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, scores_out, ld_scores, maxlev_out, seqdist_out);
+            return gr ? tp_recall(gc, max_pcs, min_clusters, nullptr, nullptr, nullptr, nullptr, nullptr)
+                      : tp_recall(gc, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, maxlev_out, seqdist_out);
         });
     TP_ARG(ctx->have_scores && ctx->k_full >= 1, "tp_recall: no PC scores in the context (run tp_call / tp_call_arm / tp_pca first)");
     TP_ARG(max_pcs >= 1, "tp_recall: max_pcs must be positive");
@@ -708,22 +677,22 @@ extern "C" int tp_recall(tp_ctx *ctx, int max_pcs, int min_clusters, int *k_out,
     ctx->k = want;
     ctx->have_sweep = false;
     if (k_out) *k_out = want;
-    return sweep_and_select(ctx, min_clusters, n_pcs_out, n_clusters_out, scores_out, ld_scores, maxlev_out, seqdist_out);
+    return sweep_and_select(ctx, min_clusters, n_pcs_out, n_clusters_out, maxlev_out, seqdist_out);
 }
 
 extern "C" int tp_call(tp_ctx *ctx, const double *mat, int n, int colmajor, int on_device,
                        int max_pcs, int min_clusters, double bad_frac,
                        uint8_t *bad_out, int *nf_out, int *k_out, int *n_pcs_out, int *n_clusters_out,
-                       double *scores_out, int ld_scores, int *maxlev_out, double *seqdist_out) {
+                       int *maxlev_out, double *seqdist_out) {
     TP_ARG(ctx && mat && bad_out, "tp_call: null argument");
     if (tp_group_dispatch(ctx))
         return tp_group_run(ctx, [&](tp_ctx *gc, int gr) -> int {
             if (gr == 0)
                 return tp_call(gc, mat, n, colmajor, on_device, max_pcs, min_clusters, bad_frac, bad_out, nf_out, k_out, n_pcs_out,
-                               n_clusters_out, scores_out, ld_scores, maxlev_out, seqdist_out);
+                               n_clusters_out, maxlev_out, seqdist_out);
             std::vector<uint8_t> tmp((size_t)(n > 0 ? n : 1));
             return tp_call(gc, mat, n, colmajor, on_device, max_pcs, min_clusters, bad_frac, tmp.data(), nullptr, nullptr, nullptr,
-                           nullptr, nullptr, 0, nullptr, nullptr);
+                           nullptr, nullptr, nullptr);
         });
     TP_CUDA(cudaSetDevice(ctx->device));
     TP_MARK(ctx, EV_TOTAL0);
@@ -736,25 +705,22 @@ extern "C" int tp_call(tp_ctx *ctx, const double *mat, int n, int colmajor, int 
     if (nf_out) *nf_out = (int)keep.size();
     TP_ARG(keep.size() >= 3, "tp_call: fewer than 3 good bins left after filtering");
     TP_TRY(tp_compact(ctx, keep.data(), (int)keep.size()));
-    return call_from_compacted(ctx, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, scores_out, ld_scores,
-                               maxlev_out, seqdist_out);
+    return call_from_compacted(ctx, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, maxlev_out, seqdist_out);
 }
 
 extern "C" int tp_call_arm(tp_ctx *ctx, const int *keep, int nf, int max_pcs, int min_clusters,
                            int *k_out, int *n_pcs_out, int *n_clusters_out,
-                           double *scores_out, int ld_scores, int *maxlev_out, double *seqdist_out) {
+                           int *maxlev_out, double *seqdist_out) {
     TP_ARG(ctx && keep, "tp_call_arm: null argument");
     if (tp_group_dispatch(ctx))
         return tp_group_run(ctx, [&](tp_ctx *gc, int gr) -> int {
-            return gr ? tp_call_arm(gc, keep, nf, max_pcs, min_clusters, nullptr, nullptr, nullptr, nullptr, 0, nullptr, nullptr)
-                      : tp_call_arm(gc, keep, nf, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, scores_out, ld_scores,
-                                    maxlev_out, seqdist_out);
+            return gr ? tp_call_arm(gc, keep, nf, max_pcs, min_clusters, nullptr, nullptr, nullptr, nullptr, nullptr)
+                      : tp_call_arm(gc, keep, nf, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, maxlev_out, seqdist_out);
         });
     TP_CUDA(cudaSetDevice(ctx->device));
     TP_MARK(ctx, EV_TOTAL0);
     TP_TRY(tp_compact(ctx, keep, nf));
-    return call_from_compacted(ctx, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, scores_out, ld_scores,
-                               maxlev_out, seqdist_out);
+    return call_from_compacted(ctx, max_pcs, min_clusters, k_out, n_pcs_out, n_clusters_out, maxlev_out, seqdist_out);
 }
 
 // ---- result assembly (host integer logic) ------------------------------------------------------------

@@ -162,6 +162,7 @@ struct tp_ctx {
     DevBuf P, Qp, d0, seqdist, order, ncl, chs, bsbuf, links, harm;
     int ld_chs = 0;
     int last_maxlev = 0;         // levels (columns) of the score matrix of the last sweep
+    std::vector<double> sweep_scores;   // that score matrix on the host: k x last_maxlev row-major, NaN where unscored
     bool have_sweep = false;
     // diffT
     DevBuf lx, ly, dout, dhash, lhash;

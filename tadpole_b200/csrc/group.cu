@@ -186,44 +186,6 @@ extern "C" int tp_ctx_dims(tp_ctx *ctx, int *n_out, int *nf_out, int *k_out, int
     return TP_OK;
 }
 
-// ---- chromosome arms on disjoint halves of the devices (R/TADpole.R:357-374: the arms are independent) --------------
-extern "C" int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int *keep_q, int nf_q, int max_pcs, int min_clusters,
-                            int *k_out2, int *n_pcs_out2, int *n_clusters_out2, double *scores_p, double *scores_q,
-                            int ld_scores, int *maxlev_out2, double *seqdist_p, double *seqdist_q) {
-    TP_ARG(ctx && keep_p && keep_q, "tp_call_arms: null argument");
-    int k2[2] = {0, 0}, np2[2] = {0, 0}, nc2[2] = {0, 0}, ml2[2] = {0, 0};
-    const int *keep[2] = {keep_p, keep_q};
-    const int nf[2] = {nf_p, nf_q};
-    double *sc[2] = {scores_p, scores_q}, *sq[2] = {seqdist_p, seqdist_q};
-    int rc = TP_OK;
-    const int R = tp_group_dispatch(ctx) ? tp_group_size(ctx) : 1;
-    if (R >= 2) {
-        const int half = R / 2;
-        rc = tp_group_run(ctx, [&](tp_ctx *c, int r) -> int {
-            const int arm = r < half ? 0 : 1;
-            const bool lead = r == (arm ? half : 0);
-            const int prev = c->comm_cur;
-            c->comm_cur = c->comm[1].handle ? 1 : -1;
-            const int e = tp_call_arm(c, keep[arm], nf[arm], max_pcs, min_clusters, lead ? &k2[arm] : nullptr,
-                                      lead ? &np2[arm] : nullptr, lead ? &nc2[arm] : nullptr, lead ? sc[arm] : nullptr, ld_scores,
-                                      lead ? &ml2[arm] : nullptr, lead ? sq[arm] : nullptr);
-            c->comm_cur = prev;
-            return e;
-        });
-    } else {
-        for (int arm = 0; arm < 2 && rc == TP_OK; arm++)
-            rc = tp_call_arm(ctx, keep[arm], nf[arm], max_pcs, min_clusters, &k2[arm], &np2[arm], &nc2[arm], sc[arm], ld_scores,
-                             &ml2[arm], sq[arm]);
-    }
-    for (int a = 0; a < 2; a++) {
-        if (k_out2) k_out2[a] = k2[a];
-        if (n_pcs_out2) n_pcs_out2[a] = np2[a];
-        if (n_clusters_out2) n_clusters_out2[a] = nc2[a];
-        if (maxlev_out2) maxlev_out2[a] = ml2[a];
-    }
-    return rc;
-}
-
 // ---- rioja's .find.groups: the hclust merge matrix of a chclust dendrogram ------------------------------------------------
 // n1 - 1... for step s = 1..n1: j = which.min(x) (first index on ties); the operands are -(j) / -(j+1) (1-based objects)
 // while they are singletons, else the step that last absorbed them.  merge_out: n1 x 2 column-major (R matrix).
@@ -261,31 +223,28 @@ struct TpBatchItem {
 };
 struct tp_batch { std::vector<TpBatchItem> items; double device_ms = 0.0; };
 
+// The outputs of a call that has just finished on c, into its batch item: k, maxlev and the score matrix from the context
+// (the host copy the sweep made) and the call's device time.  n_pcs, n_clusters, nf and seqdist the call wrote there itself.
+static void finish_item(tp_ctx *c, TpBatchItem &it) {
+    it.k = c->k;
+    it.maxlev = c->last_maxlev;
+    it.scores = c->sweep_scores;
+    it.seqdist.resize((size_t)it.nf - 1);
+    double tm[10];
+    if (tp_ctx_timings(c, tm) == TP_OK) it.device_ms = tm[6];
+}
+
 static int batch_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_device, int max_pcs, int min_clusters,
                      double bad_frac, int want_tables, TpBatchItem &it) {
     it.n = n;
     const long long launches0 = c->launches;
     struct Count { TpBatchItem &it; tp_ctx *c; long long l0; ~Count() { it.launches = c->launches - l0; } } count{it, c, launches0};
     it.bad.assign((size_t)n, 0);
-    int ld = c->level_cap > 8 ? c->level_cap : 8;
-    const int kmax = max_pcs < n ? max_pcs : n;
-    TP_ARG(kmax >= 1, "tp_call_batch: max_pcs must be positive");
+    TP_ARG(max_pcs >= 1, "tp_call_batch: max_pcs must be positive");
     it.seqdist.assign((size_t)(n > 1 ? n - 1 : 1), 0.0);
-    std::vector<double> sc((size_t)kmax * ld);
-    int rc = tp_call(c, mat, n, colmajor, on_device, max_pcs, min_clusters, bad_frac, it.bad.data(), &it.nf, &it.k, &it.n_pcs,
-                     &it.n_clusters, sc.data(), ld, &it.maxlev, it.seqdist.data());
-    if (rc == TP_ERR_ARG && it.maxlev > ld) {          // more levels than the cap: everything else is filled in
-        ld = it.maxlev;
-        sc.assign((size_t)kmax * ld, 0.0);
-        rc = tp_get_sweep_scores(c, sc.data(), ld);
-    }
-    TP_TRY(rc);
-    it.seqdist.resize((size_t)it.nf - 1);
-    it.scores.resize((size_t)it.k * it.maxlev);
-    for (int r = 0; r < it.k; r++)
-        memcpy(it.scores.data() + (size_t)r * it.maxlev, sc.data() + (size_t)r * ld, (size_t)it.maxlev * sizeof(double));
-    double tm[10];
-    if (tp_ctx_timings(c, tm) == TP_OK) it.device_ms = tm[6];
+    TP_TRY(tp_call(c, mat, n, colmajor, on_device, max_pcs, min_clusters, bad_frac, it.bad.data(), &it.nf, nullptr, &it.n_pcs,
+                   &it.n_clusters, nullptr, it.seqdist.data()));
+    finish_item(c, it);
     if (!want_tables) return TP_OK;
     // for (k in which(!is.na(scores[n_PCs, ]))) ... the start / end table of every scored level of the optimal candidate
     std::vector<int> names, bad;
@@ -301,6 +260,44 @@ static int batch_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_d
                               (int)bad.size(), it.start.data(), it.end.data(), it.offsets.data()));
     it.start.resize((size_t)it.offsets.back());
     it.end.resize((size_t)it.offsets.back());
+    return TP_OK;
+}
+
+// ---- chromosome arms on disjoint halves of the devices (R/TADpole.R:357-374: the arms are independent) --------------
+extern "C" int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int *keep_q, int nf_q, int max_pcs, int min_clusters,
+                            tp_batch **out) {
+    TP_ARG(ctx && keep_p && keep_q && out, "tp_call_arms: null argument");
+    const int *keep[2] = {keep_p, keep_q};
+    tp_batch *b = new tp_batch();
+    b->items.resize(2);
+    b->items[0].nf = nf_p;
+    b->items[1].nf = nf_q;
+    // arm a on context c; only the lead context of the arm reports its outputs
+    auto arm = [&](tp_ctx *c, int a, bool lead) -> int {
+        TpBatchItem &it = b->items[(size_t)a];
+        if (lead) it.seqdist.assign((size_t)(it.nf > 1 ? it.nf - 1 : 1), 0.0);
+        TP_TRY(tp_call_arm(c, keep[a], it.nf, max_pcs, min_clusters, nullptr, lead ? &it.n_pcs : nullptr,
+                           lead ? &it.n_clusters : nullptr, nullptr, lead ? it.seqdist.data() : nullptr));
+        if (lead) finish_item(c, it);
+        return TP_OK;
+    };
+    int rc = TP_OK;
+    const int R = tp_group_dispatch(ctx) ? tp_group_size(ctx) : 1;
+    if (R >= 2) {
+        const int half = R / 2;
+        rc = tp_group_run(ctx, [&](tp_ctx *c, int r) -> int {
+            const int a = r < half ? 0 : 1;
+            const int prev = c->comm_cur;
+            c->comm_cur = c->comm[1].handle ? 1 : -1;
+            const int e = arm(c, a, r == (a ? half : 0));
+            c->comm_cur = prev;
+            return e;
+        });
+    } else {
+        for (int a = 0; a < 2 && rc == TP_OK; a++) rc = arm(ctx, a, true);
+    }
+    if (rc != TP_OK) { delete b; return rc; }
+    *out = b;
     return TP_OK;
 }
 
