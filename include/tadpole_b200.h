@@ -264,6 +264,41 @@ int tp_batch_get(const tp_batch *b, int i, uint8_t *bad_out, int *n_pcs_out, int
                  double *seqdist_out, int *levels_out, int *offsets_out, int *start_out, int *end_out, double *device_ms_out);
 int tp_batch_free(tp_batch *b);
 
+/* ---- genome-wide input: one pixel list over every chromosome (HiC-Pro *.matrix, cooler dump -t pixels) --------------
+ * The bins are global ids over a bin table: chromosome c holds chrom_bins[c] bins, in file order, the first one starting
+ * at id index_base (0 or 1).  tp_genome_ingest takes host arrays; tp_genome_ingest_file a three-column text
+ * "bin1 <sep> bin2 <sep> count" parsed on the device as tp_ingest_coo_file parses it (exact decimal conversion, a first
+ * line that is not such a row is a header).  On the device every pixel is routed: a bin outside the bin table is an
+ * error naming the entry (arrays) or the row (file); a pixel between two chromosomes (trans) and a pixel below the
+ * diagonal are counted and dropped; every other (cis) pixel goes into its chromosome's bucket as chromosome-local
+ * (i, j, count).  The returned handle holds the buckets on the context's device (devices[0] of a multi-device context),
+ * 16 bytes per cis pixel; the input and parse buffers are released.  Device memory needed at the peak: the text, 16 bytes
+ * per pixel, 16 bytes per cis pixel; TP_ERR_NOMEM when that does not fit.  1 <= nchrom <= 2^20, every chrom_bins[c] >= 1.
+ * The handle is independent of the context's resident state and is released with tp_genome_free (before or after the
+ * context).  tp_ingest_stats describes the last genome ingest as it does the other ingests. */
+typedef struct tp_genome tp_genome;
+int tp_genome_ingest(tp_ctx *ctx, const int32_t *chrom_bins, int nchrom, const int32_t *bin1, const int32_t *bin2,
+                     const double *count, size_t nnz, int index_base, tp_genome **out);
+int tp_genome_ingest_file(tp_ctx *ctx, const int32_t *chrom_bins, int nchrom, const char *path, int sep, int index_base,
+                          tp_genome **out);
+/* cis pixels per chromosome (nchrom values), trans pixels, pixels below the diagonal; any pointer may be NULL */
+int tp_genome_stats(const tp_genome *g, unsigned long long *cis_out, unsigned long long *trans_out,
+                    unsigned long long *below_out);
+/* the dense n_c x n_c matrix of chromosome `chrom` (0-based), row-major, upper triangle (pixels naming the same cell add
+ * up, the lower triangle is 0), as the calls see it; built on the context's device (it replaces the context's resident
+ * matrix) and copied to out */
+int tp_genome_matrix(tp_ctx *ctx, const tp_genome *g, int chrom, double *out);
+/* TADpole() on every selected chromosome: chroms[nsel] (0-based; NULL = all, in bin-table order).  A tp_batch of nsel
+ * items in chroms order, read with tp_batch_dims / tp_batch_get: each item is what tp_call_batch gives for that
+ * chromosome's dense matrix (tables included when want_tables).  The dense matrix of a chromosome is built from its
+ * bucket in HBM by the worker that runs its call, and exists only while that call runs; on a multi-device context a
+ * worker on another device first copies the bucket over (cudaMemcpyPeerAsync).  Workers claim chromosomes largest first.
+ * A chromosome with fewer than 2 bins, or whose call fails, fails as its own item.  The context must be the one the
+ * handle was ingested on (or a context whose first device holds it). */
+int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
+                   double bad_frac, int inflight, int want_tables, tp_batch **out);
+int tp_genome_free(tp_genome *g);
+
 /* The context is a device-resident pipeline handle: after tp_call / tp_call_arm / tp_pca the PC scores stay in HBM, and
  * after a sweep so do all k dendrograms (tp_get_dendro) and the score matrix (tp_get_sweep_scores).  tp_recall repeats
  * only the n_pcs sweep and the selection for another max_pcs (<= the number of PCs computed) and / or min_clusters:

@@ -163,13 +163,69 @@ TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01
                  as.integer(inflight))
     lapply(res, function(r) {
         if (is.character(r)) stop(r)
-        bad <- r[[1L]]; scores <- r[[5L]]; keep <- which(!bad)
-        dimnames(scores) <- list(as.character(seq_len(nrow(scores))), as.character(seq_len(ncol(scores))))
-        clusters <- lapply(r[[7L]], function(m) data.frame(start = m[, 1L], end = m[, 2L]))
-        names(clusters) <- as.character(r[[6L]])
-        structure(list(n_pcs = r[[2L]], optimal_n_clusters = r[[3L]], dendro = .tp_dendro(r[[4L]], keep),
-                       clusters = clusters, scores = scores), class = "tadpole")
+        .tp_batch_object(r)
     })
+}
+
+# the tadpole object of one item of a batch (C_tp_call_batch, C_tp_call_genome)
+.tp_batch_object <- function(r) {
+    bad <- r[[1L]]; scores <- r[[5L]]; keep <- which(!bad)
+    dimnames(scores) <- list(as.character(seq_len(nrow(scores))), as.character(seq_len(ncol(scores))))
+    clusters <- lapply(r[[7L]], function(m) data.frame(start = m[, 1L], end = m[, 2L]))
+    names(clusters) <- as.character(r[[6L]])
+    structure(list(n_pcs = r[[2L]], optimal_n_clusters = r[[3L]], dendro = .tp_dendro(r[[4L]], keep),
+                   clusters = clusters, scores = scores), class = "tadpole")
+}
+
+# chromosome names and bins per chromosome of a bin table: a path (HiC-Pro *_abs.bed, `cooler dump -t bins`, header
+# line allowed), a data.frame with the chromosome of every bin in column 1, or a named integer vector of bin counts
+.tp_bin_table <- function(bins) {
+    if (is.numeric(bins) && !is.null(names(bins))) {
+        if (anyDuplicated(names(bins))) stop("a chromosome appears twice in the bin table")
+        return(list(names = names(bins), n = as.integer(bins)))
+    }
+    if (is.character(bins) && length(bins) == 1L) {
+        first <- strsplit(readLines(bins, n = 1L), "[ \t]+")[[1L]]
+        header <- first[1L] == "chrom" || (length(first) >= 2L && !grepl("^[+-]?[0-9]+$", first[2L]))
+        bins <- utils::read.table(path.expand(bins), header = FALSE, skip = if (header) 1L else 0L, sep = "",
+                                  colClasses = "character", comment.char = "", fill = TRUE)
+    }
+    runs <- rle(as.character(bins[[1L]]))
+    if (anyDuplicated(runs$values))
+        stop("chromosome ", runs$values[anyDuplicated(runs$values)], " reappears after another chromosome in the bin table")
+    list(names = runs$values, n = as.integer(runs$lengths))
+}
+
+# TADpole() on every chromosome of one genome-wide pixel list: pixels = sparse_counts(bin1, bin2, count, index_base =)
+# or sparse_counts(path = , index_base = 1L) with GLOBAL bin ids (HiC-Pro *.matrix, cooler dump -t pixels), bins = the
+# bin table.  The pixels are split by chromosome on the GPU and each chromosome's dense matrix exists only in HBM while
+# its call runs.  A named list of tadpole objects (bin-table order, or chroms order), attr(, "failed") = the messages
+# of the chromosomes whose call failed.
+TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L) {
+    stopifnot(inherits(pixels, "tadpole_pixels"))
+    ctx <- .tp_ctx()
+    tab <- .tp_bin_table(bins)
+    sel <- if (is.null(chroms)) tab$names else as.character(chroms)
+    idx <- match(sel, tab$names)
+    if (anyNA(idx)) stop("unknown chromosome(s): ", paste(sel[is.na(idx)], collapse = ", "))
+    g <- if (is.null(pixels$path)) .Call(C_tp_genome, ctx, tab$n, pixels$bin1, pixels$bin2, pixels$count, pixels$index_base)
+         else .Call(C_tp_genome_file, ctx, tab$n, path.expand(pixels$path), pixels$index_base)
+    res <- .Call(C_tp_call_genome, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
+                 as.numeric(bad_frac), as.integer(inflight), TRUE)
+    out <- list()
+    failed <- list()
+    for (i in seq_along(sel)) {
+        message(paste("Processing chromosome", sel[i]))
+        r <- res[[i]]
+        if (is.character(r)) { failed[[sel[i]]] <- r; next }
+        message(paste(sum(r[[1L]]), "bad columns found at position(s):"))
+        message(paste(which(r[[1L]]), collapse = " "))
+        message(paste("Optimal number of PCs:", r[[2L]]))
+        message(paste("Optimal number of clusters:", r[[3L]]))
+        out[[sel[i]]] <- .tp_batch_object(r)
+    }
+    attr(out, "failed") <- failed
+    out
 }
 
 # the n_pcs sweep again with another max_pcs / min_clusters on the PC scores that are still on the GPU

@@ -346,6 +346,81 @@ SEXP C_tp_call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP 
     return out;
 }
 
+static void genome_finalizer(SEXP p) {
+    tp_genome *g = (tp_genome *)R_ExternalPtrAddr(p);
+    if (g) {
+        tp_genome_free(g);
+        R_ClearExternalPtr(p);
+    }
+}
+
+/* list(handle, cis pixels per chromosome, c(trans, below)) of a freshly ingested genome; the handle is an external
+ * pointer whose finalizer releases the buckets, and it keeps the context alive */
+static SEXP genome_result(SEXP ctx, tp_genome *g, int nchrom) {
+    SEXP p = PROTECT(R_MakeExternalPtr(g, R_NilValue, ctx));
+    R_RegisterCFinalizerEx(p, genome_finalizer, TRUE);
+    SEXP cis = PROTECT(allocVector(REALSXP, nchrom)), tb = PROTECT(allocVector(REALSXP, 2));
+    unsigned long long *tmp = (unsigned long long *)R_alloc((size_t)nchrom, sizeof(unsigned long long)), trans = 0, below = 0;
+    tp_genome_stats(g, tmp, &trans, &below);
+    for (int i = 0; i < nchrom; i++) REAL(cis)[i] = (double)tmp[i];
+    REAL(tb)[0] = (double)trans;
+    REAL(tb)[1] = (double)below;
+    SEXP out = PROTECT(allocVector(VECSXP, 3));
+    SET_VECTOR_ELT(out, 0, p);
+    SET_VECTOR_ELT(out, 1, cis);
+    SET_VECTOR_ELT(out, 2, tb);
+    UNPROTECT(4);
+    return out;
+}
+
+/* A genome-wide pixel list split by chromosome on the GPU (tp_genome_ingest): chrom_bins = bins per chromosome in
+ * bin-table order, the pixels = vectors bin1, bin2 (integer, global ids) and count (numeric).  Returns
+ * list(handle, cis pixels per chromosome, c(trans, below)). */
+SEXP C_tp_genome(SEXP ctx, SEXP chrom_bins, SEXP bin1, SEXP bin2, SEXP count, SEXP index_base) {
+    tp_ctx *c = ctx_of(ctx);
+    if (!isInteger(chrom_bins) || length(chrom_bins) < 1) error("TADpole: the bins per chromosome must be an integer vector");
+    if (!isInteger(bin1) || !isInteger(bin2) || !isReal(count) || XLENGTH(bin1) != XLENGTH(bin2) || XLENGTH(bin1) != XLENGTH(count))
+        error("TADpole: bin1, bin2 (integer) and count (numeric) of equal length are expected");
+    tp_genome *g = NULL;
+    if (tp_genome_ingest(c, INTEGER(chrom_bins), length(chrom_bins), INTEGER(bin1), INTEGER(bin2), REAL(count),
+                         (size_t)XLENGTH(bin1), asInteger(index_base), &g) != TP_OK)
+        error("%s", tp_last_error());
+    return genome_result(ctx, g, length(chrom_bins));
+}
+
+/* the same from a three-column tab-separated pixel file (HiC-Pro *.matrix, cooler dump -t pixels) parsed on the device
+ * (tp_genome_ingest_file) */
+SEXP C_tp_genome_file(SEXP ctx, SEXP chrom_bins, SEXP path, SEXP index_base) {
+    tp_ctx *c = ctx_of(ctx);
+    if (!isInteger(chrom_bins) || length(chrom_bins) < 1) error("TADpole: the bins per chromosome must be an integer vector");
+    tp_genome *g = NULL;
+    if (tp_genome_ingest_file(c, INTEGER(chrom_bins), length(chrom_bins), CHAR(STRING_ELT(path, 0)), '\t', asInteger(index_base),
+                              &g) != TP_OK)
+        error("%s", tp_last_error());
+    return genome_result(ctx, g, length(chrom_bins));
+}
+
+/* TADpole() on the chromosomes `chroms` (0-based) of a C_tp_genome handle, `inflight` calls per device in flight
+ * (tp_call_genome).  Per chromosome, in chroms order: what C_tp_call_batch gives for its dense matrix (the per-level
+ * tables empty unless `tables`), or a character error message. */
+SEXP C_tp_call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
+                      SEXP tables) {
+    tp_ctx *c = ctx_of(ctx);
+    tp_genome *g = (tp_genome *)R_ExternalPtrAddr(genome);
+    if (!g) error("TADpole: the genome pixels have been released");
+    if (!isInteger(chroms)) error("TADpole: chromosome indices must be integers");
+    int ns = length(chroms);
+    tp_batch *b = NULL;
+    if (tp_call_genome(c, g, INTEGER(chroms), ns, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac),
+                       asInteger(inflight), asLogical(tables), &b) != TP_OK)
+        error("%s", tp_last_error());
+    SEXP out = PROTECT(allocVector(VECSXP, ns));
+    for (int i = 0; i < ns; i++) SET_VECTOR_ELT(out, i, batch_item(b, i));
+    tp_batch_free(b);
+    UNPROTECT(1);
+    return out;
+}
+
 /* the cutree / fix_values / rle loop of R/TADpole.R:470-497 for many levels at once: list of 2-column integer
  * matrices (start, end), one per requested level.  bad = integer(0) with nbad_null = TRUE means attr NULL. */
 SEXP C_tp_levels(SEXP seqdist, SEXP levels, SEXP names, SEXP bad, SEXP bad_is_null) {
@@ -460,6 +535,9 @@ static const R_CallMethodDef call_table[] = {
     {"C_tp_find_groups", (DL_FUNC)&C_tp_find_groups, 1},
     {"C_tp_call_arms", (DL_FUNC)&C_tp_call_arms, 5},
     {"C_tp_call_batch", (DL_FUNC)&C_tp_call_batch, 6},
+    {"C_tp_genome", (DL_FUNC)&C_tp_genome, 6},
+    {"C_tp_genome_file", (DL_FUNC)&C_tp_genome_file, 4},
+    {"C_tp_call_genome", (DL_FUNC)&C_tp_call_genome, 8},
     {"C_tp_levels", (DL_FUNC)&C_tp_levels, 5},
     {"C_tp_labels", (DL_FUNC)&C_tp_labels, 5},
     {"C_tp_difft", (DL_FUNC)&C_tp_difft, 5},

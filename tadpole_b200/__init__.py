@@ -7,8 +7,8 @@ libtadpole_b200.so (hand-written CUDA for sm_100a behind a C ABI, include/tadpol
 from .api import TADpole, load_mat, diffT, diffT_batch, diffT_null, random_bed, random_bed_batch, read_matrix, bin_index, Tadpole, LoadedMatrix, SparseCounts, get_context
 from ._lib import Context, TadpoleError, assemble
 from .hclust import Dendro, find_groups, cutree
-from .batch import ContextPool, TADpole_batch
+from .batch import ContextPool, TADpole_batch, GenomePixels, TADpole_genome, read_bins
 
 __all__ = ["TADpole", "load_mat", "diffT", "diffT_batch", "diffT_null", "random_bed", "random_bed_batch", "read_matrix", "bin_index", "Tadpole", "LoadedMatrix", "SparseCounts",
-           "get_context", "ContextPool", "TADpole_batch", "Context", "TadpoleError", "assemble", "Dendro", "find_groups", "cutree"]
+           "get_context", "ContextPool", "TADpole_batch", "GenomePixels", "TADpole_genome", "read_bins", "Context", "TadpoleError", "assemble", "Dendro", "find_groups", "cutree"]
 __version__ = "0.1.0"

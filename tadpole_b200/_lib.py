@@ -29,6 +29,7 @@ EXPORTED = [
     "tp_difft_null", "tp_recall",
     "tp_ctx_create_multi", "tp_device_count", "tp_ctx_devices", "tp_ctx_generation", "tp_ctx_dims", "tp_call_arms", "tp_call_batch",
     "tp_batch_size", "tp_batch_device_ms", "tp_batch_launches", "tp_batch_status", "tp_batch_error", "tp_batch_dims", "tp_batch_get", "tp_batch_free", "tp_find_groups",
+    "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
 ]
 
 
@@ -71,6 +72,12 @@ def load():
         "tp_batch_dims": (c_int, [vp, c_int, ip, ip, ip, ip, ip, ip]),
         "tp_batch_get": (c_int, [vp, c_int, u8p, ip, ip, dp, dp, ip, ip, ip, ip, dp]),
         "tp_batch_free": (c_int, [vp]),
+        "tp_genome_ingest": (c_int, [vp, ip, c_int, ip, ip, dp, ctypes.c_size_t, c_int, POINTER(vp)]),
+        "tp_genome_ingest_file": (c_int, [vp, ip, c_int, c_char_p, c_int, c_int, POINTER(vp)]),
+        "tp_genome_stats": (c_int, [vp, POINTER(ctypes.c_ulonglong), POINTER(ctypes.c_ulonglong), POINTER(ctypes.c_ulonglong)]),
+        "tp_genome_matrix": (c_int, [vp, vp, c_int, dp]),
+        "tp_call_genome": (c_int, [vp, vp, ip, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
+        "tp_genome_free": (c_int, [vp]),
         "tp_find_groups": (c_int, [dp, c_int, ip]),
         "tp_ctx_destroy": (c_int, [vp]),
         "tp_ctx_sync": (c_int, [vp]),
@@ -516,6 +523,10 @@ class Context:
         h = c_void_p()
         check(self.lib.tp_call_batch(self._h, ncalls, ptrs, _ip(ns), colmajor, ondev, int(max_pcs), int(min_clusters),
                                      float(bad_frac), int(inflight), int(bool(tables)), ctypes.byref(h)))
+        return self._batch_results(h, ncalls, tables)
+
+    def _batch_results(self, h, ncalls, tables):
+        """Every item of a tp_batch (freed here) as call_batch returns them."""
         out = []
         self.last_batch_device_ms = float(self.lib.tp_batch_device_ms(h))
         self.last_batch_launches = int(self.lib.tp_batch_launches(h))
@@ -529,6 +540,34 @@ class Context:
         finally:
             self.lib.tp_batch_free(h)
         return out
+
+    # ---- genome-wide input ----
+    def genome_ingest(self, chrom_bins, bin1=None, bin2=None, count=None, index_base=0, path=None, sep="\t"):
+        """tp_genome_ingest[_file]: pixels over the whole genome (global bin ids over chrom_bins, the bins per chromosome)
+        routed into one bucket per chromosome on this context's (first) device.  Returns a Genome handle."""
+        cb = np.ascontiguousarray(chrom_bins, dtype=np.int32)
+        h = c_void_p()
+        if path is not None:
+            check(self.lib.tp_genome_ingest_file(self._h, _ip(cb), cb.size, os.fsencode(path), ord(sep), int(index_base),
+                                                 ctypes.byref(h)))
+        else:
+            b1 = np.ascontiguousarray(bin1, dtype=np.int32)
+            b2 = np.ascontiguousarray(bin2, dtype=np.int32)
+            v = np.ascontiguousarray(count, dtype=np.float64)
+            if not (b1.ndim == 1 and b1.shape == b2.shape == v.shape):
+                raise ValueError("bin1, bin2, count: equal-length vectors expected")
+            check(self.lib.tp_genome_ingest(self._h, _ip(cb), cb.size, _ip(b1), _ip(b2), _dp(v), b1.size, int(index_base),
+                                            ctypes.byref(h)))
+        return Genome(self, h, cb)
+
+    def call_genome(self, genome, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True):
+        """tp_call_genome: one call per selected chromosome (0-based indices, default all), results in that order as
+        call_batch returns them (a failed call's entry is the TadpoleError)."""
+        sel = np.arange(genome.chrom_bins.size, dtype=np.int32) if chroms is None else np.ascontiguousarray(chroms, dtype=np.int32)
+        h = c_void_p()
+        check(self.lib.tp_call_genome(self._h, genome._h, _ip(sel), int(sel.size), int(max_pcs), int(min_clusters),
+                                      float(bad_frac), int(inflight), int(bool(tables)), ctypes.byref(h)))
+        return self._batch_results(h, int(sel.size), tables)
 
     def recall(self, nf, max_pcs=200, min_clusters=2):
         """tp_recall: the n_pcs sweep and the selection again on the PC scores resident in the context."""
@@ -569,6 +608,39 @@ class Context:
 
     def difft_batch_dev(self, lx_ptr, ly_ptr, L, npairs, out_ptr):
         check(self.lib.tp_difft_batch(self._h, int(lx_ptr), int(ly_ptr), int(L), int(npairs), 1, int(out_ptr)))
+
+
+class Genome:
+    """Handle on the per-chromosome buckets of a genome-wide pixel list (tp_genome), held on its context's device."""
+
+    def __init__(self, ctx, h, chrom_bins):
+        self.lib, self.ctx, self._h, self.chrom_bins = ctx.lib, ctx, h, chrom_bins
+
+    def stats(self):
+        """(cis pixels per chromosome, trans pixels, pixels below the diagonal)"""
+        cis = np.zeros(self.chrom_bins.size, dtype=np.uint64)
+        trans, below = ctypes.c_ulonglong(0), ctypes.c_ulonglong(0)
+        check(self.lib.tp_genome_stats(self._h, cis.ctypes.data_as(POINTER(ctypes.c_ulonglong)), ctypes.byref(trans),
+                                       ctypes.byref(below)))
+        return cis.astype(np.int64), int(trans.value), int(below.value)
+
+    def matrix(self, chrom):
+        """The dense upper-triangle matrix of chromosome `chrom` (0-based) as the calls see it (tp_genome_matrix)."""
+        n = int(self.chrom_bins[chrom])
+        out = np.empty((n, n))
+        check(self.lib.tp_genome_matrix(self.ctx._h, self._h, int(chrom), _dp(out)))
+        return out
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self.lib.tp_genome_free(self._h)
+            self._h = c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def parse_field(text):

@@ -267,6 +267,17 @@ int tp_group_size(const tp_ctx *ctx);
 tp_ctx *tp_group_member(const tp_ctx *ctx, int rank);
 void tp_group_destroy(tp_ctx *leader);
 void tp_pool_destroy(tp_ctx *ctx);
+// ---- genome-wide pixels (ingest.cu, S0c): every cis pixel in its chromosome's bucket, on one device ----
+struct tp_genome {
+    int device = 0;
+    std::vector<int> bins;                        // bins per chromosome, file order
+    std::vector<unsigned long long> offs;         // bucket c = cis pixels [offs[c], offs[c + 1])
+    unsigned long long trans = 0, below = 0;
+    DevBuf px;                                    // count[ncis] (double), then i[ncis], j[ncis] (int, chromosome-local)
+};
+// the dense n_c x n_c row-major matrix of chromosome `chrom` into c->raw_own, on c's stream (a bucket held by another device
+// is first copied into c->icoo); *out = c->raw_own
+int tp_genome_dense(tp_ctx *c, const tp_genome *g, int chrom, double **out);
 int tp_upload_range(tp_ctx *ctx, void *dst, const void *src, size_t bytes, cudaStream_t st);   // filter.cu: pageable -> lanes
 int tp_stage_input(tp_ctx *ctx, const double *mat, int n, int colmajor);   // filter.cu: upload under the running call
 int tp_flags_reset(tp_ctx *ctx);                 // zero the status words (stream ordered)

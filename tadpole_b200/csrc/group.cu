@@ -301,10 +301,14 @@ extern "C" int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int 
     return TP_OK;
 }
 
-extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
-                             int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, tp_batch **out) {
-    TP_ARG(ctx && mats && n && out && ncalls >= 0, "tp_call_batch: bad arguments");
-    TP_ARG(!(on_device && ctx->group), "tp_call_batch: device-resident inputs need a single-device context");
+// The worker loop of a batch: up to `inflight` library-owned threads per device of the context, each on its own pool
+// context, claim items (in the order order[0..ncalls), or in input order when order is NULL) until none is left.
+// one(c, i, it) runs item i on context c.  need: device bytes one call in flight holds.  host_inputs: the items' matrices
+// come from host memory; then the first uploads of a device's workers go one after the other, and stage(c, i) starts the
+// upload of item i (claimed ahead) under the call that c is running.
+static int batch_run(tp_ctx *ctx, int ncalls, double need, int inflight, bool host_inputs, const int *order,
+                     const std::function<void(tp_ctx *, int)> &stage, const std::function<int(tp_ctx *, int, TpBatchItem &)> &one,
+                     tp_batch **out) {
     if (inflight < 1) inflight = 4;
     if (inflight > 32) inflight = 32;
     const int ndev = tp_group_size(ctx);
@@ -315,11 +319,7 @@ extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats,
     }
     TpPool *pool = ctx->pool;
     int per_dev = std::max(1, std::min(inflight, (ncalls + ndev - 1) / ndev));
-    {   // every call in flight holds its own working set in HBM (raw + filtered + correlation + M + digit planes +
-        // second input buffer + blocks: ~56 bytes per matrix element, 35 GB at 25k bins): do not keep more in flight than the device has room for
-        size_t nmax = 0;
-        for (int i = 0; i < ncalls; i++) nmax = std::max(nmax, (size_t)(n[i] > 0 ? n[i] : 0));
-        const double need = 56.0 * (double)nmax * (double)nmax + 64e6;
+    {   // do not keep more calls in flight than the device has room for
         for (int d = 0; d < ndev; d++) {
             size_t fr = 0, tot = 0;
             cudaSetDevice(pool->devices[d]);
@@ -371,7 +371,7 @@ extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats,
     // first call starts computing after ONE upload instead of after all of them sharing the PCIe link; (2) from then on a
     // worker claims its next matrix while the current call is in the n_pcs sweep and uploads it on its copy stream into the
     // second input buffer (tp_stage_input): the upload leaves the critical path of the call.
-    const bool prefetch = !on_device && !ctx->group && getenv("TADPOLE_BATCH_NOPREFETCH") == nullptr;
+    const bool prefetch = host_inputs && !ctx->group && getenv("TADPOLE_BATCH_NOPREFETCH") == nullptr;
     std::vector<std::mutex> first_upload((size_t)ndev);
     auto worker = [&](tp_ctx *c, cudaEvent_t done, int d) {
         cudaSetDevice(c->device);
@@ -382,20 +382,22 @@ extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats,
             if (!prefetch || claimed >= 0) return;
             const int j = next.fetch_add(1);
             if (j >= ncalls) return;
-            claimed = j;
-            if (mats[j] && n[j] >= 2) (void)tp_stage_input(c, mats[j], n[j], colmajor);    // a failure leaves the normal upload
+            claimed = order ? order[j] : j;
+            stage(c, claimed);
         };
         bool first = true;
         for (;;) {
             int i = claimed;
             claimed = -1;
-            if (i < 0) i = next.fetch_add(1);
-            if (i >= ncalls) break;
-            if (first && !on_device) { first_upload[(size_t)d].lock(); holding = true; }
+            if (i < 0) {
+                const int t = next.fetch_add(1);
+                if (t >= ncalls) break;
+                i = order ? order[t] : t;
+            }
+            if (first && host_inputs) { first_upload[(size_t)d].lock(); holding = true; }
             first = false;
             TpBatchItem &it = b->items[(size_t)i];
-            it.rc = mats[i] ? batch_one(c, mats[i], n[i], colmajor, on_device, max_pcs, min_clusters, bad_frac, want_tables, it)
-                            : (tp_set_error("tp_call_batch: matrix %d is null", i), (int)TP_ERR_ARG);
+            it.rc = one(c, i, it);
             if (holding) { first_upload[(size_t)d].unlock(); holding = false; }
             if (it.rc != TP_OK) it.err = tp_last_error();
         }
@@ -425,6 +427,65 @@ extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats,
     cudaSetDevice(ctx->device);
     *out = b;
     return TP_OK;
+}
+
+extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
+                             int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, tp_batch **out) {
+    TP_ARG(ctx && mats && n && out && ncalls >= 0, "tp_call_batch: bad arguments");
+    TP_ARG(!(on_device && ctx->group), "tp_call_batch: device-resident inputs need a single-device context");
+    // every call in flight holds its own working set in HBM (raw + filtered + correlation + M + digit planes + second
+    // input buffer + blocks: ~56 bytes per matrix element, 35 GB at 25k bins)
+    size_t nmax = 0;
+    for (int i = 0; i < ncalls; i++) nmax = std::max(nmax, (size_t)(n[i] > 0 ? n[i] : 0));
+    const double need = 56.0 * (double)nmax * (double)nmax + 64e6;
+    auto stage = [&](tp_ctx *c, int j) {
+        if (mats[j] && n[j] >= 2) (void)tp_stage_input(c, mats[j], n[j], colmajor);    // a failure leaves the normal upload
+    };
+    auto one = [&](tp_ctx *c, int i, TpBatchItem &it) -> int {
+        return mats[i] ? batch_one(c, mats[i], n[i], colmajor, on_device, max_pcs, min_clusters, bad_frac, want_tables, it)
+                       : (tp_set_error("tp_call_batch: matrix %d is null", i), (int)TP_ERR_ARG);
+    };
+    return batch_run(ctx, ncalls, need, inflight, !on_device, nullptr, stage, one, out);
+}
+
+// ---- genome-wide calls: one per chromosome, each dense matrix built from its bucket in HBM (ingest.cu, S0c) ---------
+extern "C" int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
+                              double bad_frac, int inflight, int want_tables, tp_batch **out) {
+    TP_ARG(ctx && g && out && nsel >= 0 && (chroms || nsel == 0 || nsel == (int)g->bins.size()), "tp_call_genome: bad arguments");
+    TP_ARG(g->device == ctx->device, "tp_call_genome: the handle was ingested on another device than the context's first");
+    std::vector<int> sel((size_t)(nsel > 0 ? nsel : 0));
+    for (int s = 0; s < nsel; s++) {
+        sel[(size_t)s] = chroms ? chroms[s] : s;
+        if (sel[(size_t)s] < 0 || sel[(size_t)s] >= (int)g->bins.size()) {
+            tp_set_error("tp_call_genome: chromosome index %d is outside 0..%d", sel[(size_t)s], (int)g->bins.size() - 1);
+            return TP_ERR_ARG;
+        }
+    }
+    // the cost of a call grows roughly as n^3: the largest chromosomes are claimed first
+    std::vector<int> order((size_t)nsel);
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return g->bins[(size_t)sel[a]] > g->bins[(size_t)sel[b]]; });
+    // per call in flight: the working set of tp_call_batch plus the copy of a bucket held by another device.  The buckets
+    // themselves are resident on devices[0] and already missing from its free memory.
+    double nmax = 0.0, pmax = 0.0;
+    for (int c : sel) {
+        nmax = std::max(nmax, (double)g->bins[(size_t)c]);
+        pmax = std::max(pmax, (double)(g->offs[(size_t)c + 1] - g->offs[(size_t)c]));
+    }
+    const double need = 56.0 * nmax * nmax + 16.0 * pmax + 64e6;
+    auto one = [&](tp_ctx *c, int s, TpBatchItem &it) -> int {
+        const int chrom = sel[(size_t)s], n = g->bins[(size_t)chrom];
+        it.n = n;
+        if (n < 2) {
+            it.bad.assign((size_t)n, 0);
+            tp_set_error("tp_call_genome: chromosome %d has %d bin; a call needs at least 2", chrom, n);
+            return TP_ERR_ARG;
+        }
+        double *mat = nullptr;
+        TP_TRY(tp_genome_dense(c, g, chrom, &mat));
+        return batch_one(c, mat, n, 0, 1, max_pcs, min_clusters, bad_frac, want_tables, it);
+    };
+    return batch_run(ctx, nsel, need, inflight, false, order.data(), [](tp_ctx *, int) {}, one, out);
 }
 
 extern "C" double tp_batch_device_ms(const tp_batch *b) { return b ? b->device_ms : 0.0; }

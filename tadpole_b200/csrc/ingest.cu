@@ -575,40 +575,54 @@ extern "C" int tp_ingest_coo(tp_ctx *ctx, const int32_t *bin1, const int32_t *bi
     return TP_OK;
 }
 
-extern "C" int tp_ingest_coo_file(tp_ctx *ctx, const char *path, int sep, int n, int index_base, int *n_out,
-                                  unsigned long long *nnz_out, unsigned long long *below_out) {
-    TP_ARG(ctx && path, "tp_ingest_coo_file: null argument");
-    TP_ARG(sep > 0 && sep < 128 && sep != '\n' && sep != '\r' && sep != '.' && sep != '-' && sep != '+' && !(sep >= '0' && sep <= '9'),
-           "tp_ingest_coo_file: bad separator");
-    TP_ARG(n <= 200000, "tp_ingest_coo_file: more than 200000 bins");
-    TP_ARG(index_base == 0 || index_base == 1, "tp_ingest_coo_file: index_base must be 0 or 1");
-    TextSource src;
-    src.fd = open(path, O_RDONLY);
-    if (src.fd < 0) {
-        tp_set_error("tp_ingest_coo_file: cannot open '%s' (%s)", path, strerror(errno));
+static int open_text_file(const char *path, const char *who, TextSource *src) {
+    src->fd = open(path, O_RDONLY);
+    if (src->fd < 0) {
+        tp_set_error("%s: cannot open '%s' (%s)", who, path, strerror(errno));
         return TP_ERR_ARG;
     }
-    struct Closer { int fd; ~Closer() { close(fd); } } closer{src.fd};
     struct stat sb;
-    if (fstat(src.fd, &sb) != 0 || !S_ISREG(sb.st_mode)) {
-        tp_set_error("tp_ingest_coo_file: '%s' is not a regular file", path);
+    if (fstat(src->fd, &sb) != 0 || !S_ISREG(sb.st_mode)) {
+        tp_set_error("%s: '%s' is not a regular file", who, path);
         return TP_ERR_ARG;
     }
-    src.size = (size_t)sb.st_size;
+    src->size = (size_t)sb.st_size;
 #ifdef POSIX_FADV_SEQUENTIAL
-    posix_fadvise(src.fd, 0, 0, POSIX_FADV_SEQUENTIAL);
+    posix_fadvise(src->fd, 0, 0, POSIX_FADV_SEQUENTIAL);
 #endif
-    TP_CUDA(cudaSetDevice(ctx->device));
+    return TP_OK;
+}
+
+// fail with a plain message when `bytes` more cannot fit on ctx's device (`held`: bytes of the buffer about to be grown,
+// which its reserve frees first)
+static int device_room(tp_ctx *ctx, double bytes, size_t held, const char *who, const char *what) {
+    size_t fr = 0, tot = 0;
+    if (cudaMemGetInfo(&fr, &tot) != cudaSuccess) { (void)cudaGetLastError(); return TP_OK; }
+    if (bytes > (double)fr + (double)held) {
+        tp_set_error("%s: %s need %.2f GB on device %d and %.2f GB are free; inputs larger than the device memory are not "
+                     "supported", who, what, bytes / 1e9, ctx->device, ((double)fr + (double)held) / 1e9);
+        return TP_ERR_NOMEM;
+    }
+    return TP_OK;
+}
+
+// The pixels of a three-column text "bin1 <sep> bin2 <sep> count", parsed on ctx's device: on return row r of the file is
+// (d1[r], d2[r], dv[r]) in ctx->icoo, rows [first, nrows) are pixels (first = 1 after a header line), status64 (8 words,
+// then the slow list, in ctx->islow) as coo_parse_kernel left it.
+static int coo_text_pixels(tp_ctx *ctx, const TextSource &src, int sep, const char *who, double *extra_per_row, int **d1_out,
+                           int **d2_out, double **dv_out, long long *nrows_out, unsigned *first_out, unsigned *nslow_out,
+                           size_t *nbytes_out, unsigned long long **status_out) {
     cudaStream_t st = ctx->stream;
-    const auto t_begin = std::chrono::steady_clock::now();
-    ctx->raw = nullptr; ctx->n = 0; ctx->ingested_n = 0;
-    ctx->have_X = ctx->have_C = ctx->have_scores = ctx->have_sweep = false;
     unsigned char *text = nullptr;
     size_t nbytes = 0;
     int nb = 0;
     long long *offs = nullptr, nrows = 0;
-    TP_TRY(text_rows(ctx, src, "tp_ingest_coo_file", &text, &nbytes, &nb, &offs, &nrows));
-    TP_ARG(nrows >= 1 && nrows < 0x7fffffffLL, "tp_ingest_coo_file: the file must hold between 1 and 2^31 - 2 rows");
+    TP_TRY(text_rows(ctx, src, who, &text, &nbytes, &nb, &offs, &nrows));
+    if (nrows < 1 || nrows >= 0x7fffffffLL) {
+        tp_set_error("%s: the file must hold between 1 and 2^31 - 2 rows", who);
+        return TP_ERR_ARG;
+    }
+    if (extra_per_row) TP_TRY(device_room(ctx, (24.0 + *extra_per_row) * (double)nrows, ctx->irows.cap + ctx->icoo.cap, who, "the pixels"));
     const long long limit = (long long)nbytes + 1;
     const unsigned slow_cap = 1u << 20;
     unsigned long long *status64 = nullptr;
@@ -629,15 +643,18 @@ extern "C" int tp_ingest_coo_file(tp_ctx *ctx, const char *path, int sep, int n,
     TP_CUDA(cudaMemcpyAsync(hs, status64, sizeof(hs), cudaMemcpyDeviceToHost, st));
     TP_CUDA(tp_stream_sync(ctx));
     if (hs[2] == ~0ull - 1) {
-        tp_set_error("tp_ingest_coo_file: more than %u counts need the host conversion path", slow_cap);
+        tp_set_error("%s: more than %u counts need the host conversion path", who, slow_cap);
         return TP_ERR_ARG;
     }
     if (hs[2] != ~0ull) {
-        tp_set_error("tp_ingest_coo_file: row %llu is not 'bin1 <sep> bin2 <sep> count' with non-negative integer bins", hs[2] + 1);
+        tp_set_error("%s: row %llu is not 'bin1 <sep> bin2 <sep> count' with non-negative integer bins", who, hs[2] + 1);
         return TP_ERR_ARG;
     }
     const unsigned first = hs[4] ? 1u : 0u;                     // a header line is skipped
-    TP_ARG((unsigned long long)nrows > first, "tp_ingest_coo_file: the file holds a header and no pixels");
+    if ((unsigned long long)nrows <= first) {
+        tp_set_error("%s: the file holds a header and no pixels", who);
+        return TP_ERR_ARG;
+    }
     const unsigned nslow = (unsigned)(hs[5] & 0xffffffffu);
     if (nslow) {
         std::vector<SlowTok> list(nslow);
@@ -646,7 +663,7 @@ extern "C" int tp_ingest_coo_file(tp_ctx *ctx, const char *path, int sep, int n,
         std::vector<double> val(nslow);
         std::vector<char> buf(4096 + 1);
         for (unsigned i = 0; i < nslow; i++) {
-            TP_TRY(host_field(src, nbytes, (size_t)list[i].off, sep, buf, &val[i], "tp_ingest_coo_file", list[i].row, 2));
+            TP_TRY(host_field(src, nbytes, (size_t)list[i].off, sep, buf, &val[i], who, list[i].row, 2));
             idx[i] = list[i].row;
         }
         unsigned *didx = (unsigned *)slow;
@@ -658,7 +675,36 @@ extern "C" int tp_ingest_coo_file(tp_ctx *ctx, const char *path, int sep, int n,
         TP_CUDA(tp_stream_sync(ctx));
         ctx->launches += 1;
     }
+    *d1_out = d1; *d2_out = d2; *dv_out = dv; *nrows_out = nrows; *first_out = first; *nslow_out = nslow;
+    *nbytes_out = nbytes; *status_out = status64;
+    return TP_OK;
+}
+
+extern "C" int tp_ingest_coo_file(tp_ctx *ctx, const char *path, int sep, int n, int index_base, int *n_out,
+                                  unsigned long long *nnz_out, unsigned long long *below_out) {
+    TP_ARG(ctx && path, "tp_ingest_coo_file: null argument");
+    TP_ARG(sep > 0 && sep < 128 && sep != '\n' && sep != '\r' && sep != '.' && sep != '-' && sep != '+' && !(sep >= '0' && sep <= '9'),
+           "tp_ingest_coo_file: bad separator");
+    TP_ARG(n <= 200000, "tp_ingest_coo_file: more than 200000 bins");
+    TP_ARG(index_base == 0 || index_base == 1, "tp_ingest_coo_file: index_base must be 0 or 1");
+    TextSource src;
+    TP_TRY(open_text_file(path, "tp_ingest_coo_file", &src));
+    struct Closer { int fd; ~Closer() { close(fd); } } closer{src.fd};
+    TP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const auto t_begin = std::chrono::steady_clock::now();
+    ctx->raw = nullptr; ctx->n = 0; ctx->ingested_n = 0;
+    ctx->have_X = ctx->have_C = ctx->have_scores = ctx->have_sweep = false;
+    int *d1 = nullptr, *d2 = nullptr;
+    double *dv = nullptr;
+    long long nrows = 0;
+    unsigned first = 0, nslow = 0;
+    size_t nbytes = 0;
+    unsigned long long *status64 = nullptr;
+    TP_TRY(coo_text_pixels(ctx, src, sep, "tp_ingest_coo_file", nullptr, &d1, &d2, &dv, &nrows, &first, &nslow, &nbytes, &status64));
+    unsigned long long hs[8];
     if (n <= 0) {
+        TP_CUDA(cudaMemcpy(hs, status64, sizeof(hs), cudaMemcpyDeviceToHost));
         const long long nn = (long long)hs[3] - index_base;
         if (nn < 2 || nn > 200000) {
             tp_set_error("tp_ingest_coo_file: the largest bin in the file gives %lld bins; 2..200000 are supported", nn);
@@ -685,6 +731,281 @@ extern "C" int tp_ingest_coo_file(tp_ctx *ctx, const char *path, int sep, int n,
     if (nnz_out) *nnz_out = m;
     if (below_out) *below_out = hs[1];
     coo_done(ctx, out, n, t_begin, (double)nbytes, (double)nslow);
+    return TP_OK;
+}
+
+// ---- genome-wide pixels (S0c): one pixel list over every chromosome -> one bucket of local pixels per chromosome ------
+// Bins are global ids; chromosome c holds [starts[c], starts[c + 1]) (0-based, starts[0] = 0).  A pixel is out of range
+// (a bin outside the table: the lowest entry index goes to status64[0]), trans (two chromosomes: counted in status64[6]
+// and dropped), below the diagonal (counted in status64[1] and dropped, as S0b does) or cis (kept, in chromosome-local
+// bins).  Any number of chromosomes up to 2^20: a binary search over the starts finds the one of a bin.
+__device__ __forceinline__ int genome_chrom_of(const int *__restrict__ starts, int nchrom, int x) {
+    int lo = 0, hi = nchrom - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(starts + mid) <= x) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// the chromosome whose bucket pixel e goes to, and its local bins; -1 when the pixel is dropped
+__device__ __forceinline__ int genome_route(const int *__restrict__ b1, const int *__restrict__ b2, unsigned e, unsigned m, int base,
+                                            const int *__restrict__ starts, int nchrom, unsigned long long first,
+                                            unsigned long long *__restrict__ status64, bool count, int *li, int *lj) {
+    bool trans = false, below = false;
+    int c = -1;
+    if (e < m) {
+        const long long x = (long long)b1[e] - base, y = (long long)b2[e] - base, total = starts[nchrom];
+        if (x < 0 || y < 0 || x >= total || y >= total) {
+            if (count) atomicMin(status64, first + e);
+        } else {
+            const int cx = genome_chrom_of(starts, nchrom, (int)x), cy = genome_chrom_of(starts, nchrom, (int)y);
+            if (cx != cy) trans = true;
+            else if (x > y) below = true;
+            else { c = cx; *li = (int)x - starts[c]; *lj = (int)y - starts[c]; }
+        }
+    }
+    if (count) {
+        const unsigned bt = __ballot_sync(0xffffffffu, trans), bb = __ballot_sync(0xffffffffu, below);
+        if ((threadIdx.x & 31) == 0) {
+            if (bt) atomicAdd(status64 + 6, (unsigned long long)__popc(bt));
+            if (bb) atomicAdd(status64 + 1, (unsigned long long)__popc(bb));
+        }
+    }
+    return c;
+}
+
+// pass 1: cis pixels per chromosome (one atomic per distinct chromosome in a warp)
+__global__ void __launch_bounds__(256)
+genome_route_kernel(const int *__restrict__ b1, const int *__restrict__ b2, unsigned m, int base, const int *__restrict__ starts,
+                    int nchrom, unsigned long long first, unsigned long long *__restrict__ hist,
+                    unsigned long long *__restrict__ status64) {
+    const unsigned e = blockIdx.x * blockDim.x + threadIdx.x;
+    int li = 0, lj = 0;
+    const int c = genome_route(b1, b2, e, m, base, starts, nchrom, first, status64, true, &li, &lj);
+    const unsigned grp = __match_any_sync(0xffffffffu, c);
+    if (c >= 0 && (threadIdx.x & 31) == __ffs(grp) - 1) atomicAdd(hist + c, (unsigned long long)__popc(grp));
+}
+
+// pass 2: every cis pixel into its chromosome's bucket as local (i, j, count); cursor[c] starts at the bucket's offset
+__global__ void __launch_bounds__(256)
+genome_bucket_kernel(const int *__restrict__ b1, const int *__restrict__ b2, const double *__restrict__ v, unsigned m, int base,
+                     const int *__restrict__ starts, int nchrom, unsigned long long *__restrict__ cursor,
+                     double *__restrict__ ov, int *__restrict__ oi, int *__restrict__ oj) {
+    const unsigned e = blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    int li = 0, lj = 0;
+    const int c = genome_route(b1, b2, e, m, base, starts, nchrom, 0, nullptr, false, &li, &lj);
+    const unsigned grp = __match_any_sync(0xffffffffu, c);
+    const int leader = __ffs(grp) - 1;
+    unsigned long long pos = 0;
+    if (c >= 0 && lane == leader) pos = atomicAdd(cursor + c, (unsigned long long)__popc(grp));
+    pos = __shfl_sync(0xffffffffu, pos, leader) + (unsigned long long)__popc(grp & ((1u << lane) - 1));
+    if (c >= 0) { ov[pos] = v[e]; oi[pos] = li; oj[pos] = lj; }
+}
+
+static int genome_new(const int32_t *chrom_bins, int nchrom, int index_base, const char *who, tp_genome **out) {
+    if (!(nchrom >= 1 && nchrom <= (1 << 20))) { tp_set_error("%s: the number of chromosomes must be in 1..2^20", who); return TP_ERR_ARG; }
+    if (index_base != 0 && index_base != 1) { tp_set_error("%s: index_base must be 0 or 1", who); return TP_ERR_ARG; }
+    long long total = 0;
+    for (int c = 0; c < nchrom; c++) {
+        if (chrom_bins[c] < 1) { tp_set_error("%s: chromosome %d has %d bins; at least 1 is needed", who, c, chrom_bins[c]); return TP_ERR_ARG; }
+        total += chrom_bins[c];
+    }
+    if (total >= 0x7fffffffLL) { tp_set_error("%s: the bin table holds %lld bins; at most 2^31 - 2 are supported", who, total); return TP_ERR_ARG; }
+    tp_genome *g = new tp_genome();
+    g->bins.assign(chrom_bins, chrom_bins + nchrom);
+    *out = g;
+    return TP_OK;
+}
+
+// Route the pixels (d1, d2, dv: m of them on ctx's device; pixel e is entry first + e of the input) into g's buckets.
+// hb1 / hb2: the host arrays, to name the bins of an entry outside the table (NULL for a file: the row is named).
+static int genome_bucket(tp_ctx *ctx, tp_genome *g, const int *d1, const int *d2, const double *dv, size_t m, int index_base,
+                         unsigned long long first, unsigned long long *status64, const int32_t *hb1, const int32_t *hb2,
+                         const char *who) {
+    cudaStream_t st = ctx->stream;
+    const int nchrom = (int)g->bins.size();
+    std::vector<int> starts((size_t)nchrom + 1, 0);
+    for (int c = 0; c < nchrom; c++) starts[c + 1] = starts[c] + g->bins[c];
+    struct Aux { DevBuf b; ~Aux() { b.release(); } } aux;         // hist[nchrom], cursor[nchrom] (u64), starts[nchrom + 1]
+    TP_TRY(aux.b.reserve((size_t)nchrom * 16 + ((size_t)nchrom + 1) * sizeof(int)));
+    unsigned long long *hist = aux.b.as<unsigned long long>(), *cursor = hist + nchrom;
+    int *dstarts = (int *)(cursor + nchrom);
+    TP_CUDA(cudaMemsetAsync(hist, 0, (size_t)nchrom * 8, st));
+    TP_CUDA(cudaMemcpyAsync(dstarts, starts.data(), starts.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    const size_t M = (size_t)1 << 30;
+    for (size_t off = 0; off < m; off += M) {
+        const unsigned k = (unsigned)(m - off < M ? m - off : M);
+        genome_route_kernel<<<(k + 255) / 256, 256, 0, st>>>(d1 + off, d2 + off, k, index_base, dstarts, nchrom, first + off, hist, status64);
+        ctx->launches += 1;
+    }
+    TP_CUDA(cudaGetLastError());
+    std::vector<unsigned long long> h((size_t)nchrom);
+    unsigned long long hs[8];
+    TP_CUDA(cudaMemcpyAsync(h.data(), hist, (size_t)nchrom * 8, cudaMemcpyDeviceToHost, st));
+    TP_CUDA(cudaMemcpyAsync(hs, status64, sizeof(hs), cudaMemcpyDeviceToHost, st));
+    TP_CUDA(tp_stream_sync(ctx));
+    if (hs[0] != ~0ull) {
+        if (hb1) tp_set_error("%s: entry %llu is (%d, %d): outside the %d bins of the bin table (index_base %d)", who, hs[0] + 1,
+                              hb1[hs[0]], hb2[hs[0]], starts[nchrom], index_base);
+        else tp_set_error("%s: row %llu names a bin outside the %d bins of the bin table (index_base %d)", who, hs[0] + 1,
+                          starts[nchrom], index_base);
+        return TP_ERR_ARG;
+    }
+    g->offs.assign((size_t)nchrom + 1, 0);
+    for (int c = 0; c < nchrom; c++) g->offs[c + 1] = g->offs[c] + h[c];
+    g->below = hs[1];
+    g->trans = hs[6];
+    const size_t ncis = g->offs[nchrom];
+    TP_TRY(device_room(ctx, 16.0 * (double)ncis, 0, who, "the buckets of the cis pixels"));
+    TP_TRY(g->px.reserve(ncis * 16 + 16));
+    double *ov = g->px.as<double>();
+    int *oi = (int *)(ov + ncis), *oj = oi + ncis;
+    TP_CUDA(cudaMemcpyAsync(cursor, g->offs.data(), (size_t)nchrom * 8, cudaMemcpyHostToDevice, st));
+    for (size_t off = 0; off < m; off += M) {
+        const unsigned k = (unsigned)(m - off < M ? m - off : M);
+        genome_bucket_kernel<<<(k + 255) / 256, 256, 0, st>>>(d1 + off, d2 + off, dv + off, k, index_base, dstarts, nchrom, cursor, ov, oi, oj);
+        ctx->launches += 1;
+    }
+    TP_CUDA(cudaGetLastError());
+    TP_MARK(ctx, EV_INGEST1);
+    TP_CUDA(tp_stream_sync(ctx));
+    return TP_OK;
+}
+
+static void genome_done(tp_ctx *ctx, std::chrono::steady_clock::time_point t_begin, double bytes, double nslow) {
+    // the parse arrays are not needed any more: their memory goes back to the calls
+    ctx->icoo.release();
+    ctx->irows.release();
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ctx->ev[EV_INGEST0], ctx->ev[EV_INGEST1]);
+    ctx->ingest_stats[0] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    ctx->ingest_stats[1] = ms;
+    ctx->ingest_stats[2] = bytes;
+    ctx->ingest_stats[3] = nslow;
+}
+
+struct GenomeOwner { tp_genome *g = nullptr; ~GenomeOwner() { if (g) tp_genome_free(g); } };
+
+extern "C" int tp_genome_ingest(tp_ctx *ctx, const int32_t *chrom_bins, int nchrom, const int32_t *bin1, const int32_t *bin2,
+                                const double *count, size_t nnz, int index_base, tp_genome **out) {
+    TP_ARG(ctx && chrom_bins && out && (nnz == 0 || (bin1 && bin2 && count)), "tp_genome_ingest: null argument");
+    TP_CUDA(cudaSetDevice(ctx->device));
+    const auto t_begin = std::chrono::steady_clock::now();
+    GenomeOwner own;
+    TP_TRY(genome_new(chrom_bins, nchrom, index_base, "tp_genome_ingest", &own.g));
+    own.g->device = ctx->device;
+    cudaStream_t st = ctx->stream;
+    unsigned long long *status64 = nullptr;
+    TP_TRY(coo_status_init(ctx, &status64));
+    TP_TRY(device_room(ctx, 16.0 * (double)nnz, ctx->icoo.cap, "tp_genome_ingest", "the pixels"));
+    TP_TRY(ctx->icoo.reserve(nnz * 16 + 16));
+    double *dv = ctx->icoo.as<double>();
+    int *d1 = (int *)(dv + nnz), *d2 = d1 + nnz;
+    TP_MARK(ctx, EV_INGEST0);
+    TP_TRY(tp_upload_range(ctx, dv, count, nnz * 8, st));
+    TP_TRY(tp_upload_range(ctx, d1, bin1, nnz * 4, st));
+    TP_TRY(tp_upload_range(ctx, d2, bin2, nnz * 4, st));
+    TP_TRY(genome_bucket(ctx, own.g, d1, d2, dv, nnz, index_base, 0, status64, bin1, bin2, "tp_genome_ingest"));
+    genome_done(ctx, t_begin, (double)nnz * 16.0, 0.0);
+    *out = own.g;
+    own.g = nullptr;
+    return TP_OK;
+}
+
+extern "C" int tp_genome_ingest_file(tp_ctx *ctx, const int32_t *chrom_bins, int nchrom, const char *path, int sep, int index_base,
+                                     tp_genome **out) {
+    TP_ARG(ctx && chrom_bins && path && out, "tp_genome_ingest_file: null argument");
+    TP_ARG(sep > 0 && sep < 128 && sep != '\n' && sep != '\r' && sep != '.' && sep != '-' && sep != '+' && !(sep >= '0' && sep <= '9'),
+           "tp_genome_ingest_file: bad separator");
+    GenomeOwner own;
+    TP_TRY(genome_new(chrom_bins, nchrom, index_base, "tp_genome_ingest_file", &own.g));
+    TextSource src;
+    TP_TRY(open_text_file(path, "tp_genome_ingest_file", &src));
+    struct Closer { int fd; ~Closer() { close(fd); } } closer{src.fd};
+    TP_CUDA(cudaSetDevice(ctx->device));
+    own.g->device = ctx->device;
+    const auto t_begin = std::chrono::steady_clock::now();
+    int *d1 = nullptr, *d2 = nullptr;
+    double *dv = nullptr;
+    long long nrows = 0;
+    unsigned first = 0, nslow = 0;
+    size_t nbytes = 0;
+    unsigned long long *status64 = nullptr;
+    double per_row = 16.0;                       // the buckets, if every row is a cis pixel
+    TP_TRY(coo_text_pixels(ctx, src, sep, "tp_genome_ingest_file", &per_row, &d1, &d2, &dv, &nrows, &first, &nslow, &nbytes,
+                           &status64));
+    ctx->itext.release();                        // the text is parsed
+    const size_t m = (size_t)nrows - first;
+    TP_TRY(genome_bucket(ctx, own.g, d1 + first, d2 + first, dv + first, m, index_base, first, status64, nullptr, nullptr,
+                         "tp_genome_ingest_file"));
+    genome_done(ctx, t_begin, (double)nbytes, (double)nslow);
+    *out = own.g;
+    own.g = nullptr;
+    return TP_OK;
+}
+
+extern "C" int tp_genome_stats(const tp_genome *g, unsigned long long *cis_out, unsigned long long *trans_out,
+                               unsigned long long *below_out) {
+    TP_ARG(g, "tp_genome_stats: null handle");
+    if (cis_out)
+        for (size_t c = 0; c + 1 < g->offs.size(); c++) cis_out[c] = g->offs[c + 1] - g->offs[c];
+    if (trans_out) *trans_out = g->trans;
+    if (below_out) *below_out = g->below;
+    return TP_OK;
+}
+
+int tp_genome_dense(tp_ctx *c, const tp_genome *g, int chrom, double **out) {
+    TP_ARG(chrom >= 0 && chrom < (int)g->bins.size(), "tp_genome: chromosome index out of range");
+    TP_CUDA(cudaSetDevice(c->device));
+    const int n = g->bins[(size_t)chrom];
+    const size_t ncis = g->offs.back(), o = g->offs[(size_t)chrom], m = g->offs[(size_t)chrom + 1] - o;
+    const double *v = g->px.as<double>() + o;
+    const int *bi = (const int *)(g->px.as<double>() + ncis) + o, *bj = bi + ncis;
+    const bool remote = c->device != g->device;
+    // status words of the scatter (every bucket pixel is in range and on or above the diagonal: never written)
+    TP_TRY(c->icoo.reserve(64 + (remote ? m * 16 : 0)));
+    unsigned long long *status64 = c->icoo.as<unsigned long long>();
+    TP_CUDA(cudaMemsetAsync(status64, 0, 64, c->stream));
+    if (remote && m) {
+        double *pv = (double *)(status64 + 8);
+        int *pi = (int *)(pv + m), *pj = pi + m;
+        TP_CUDA(cudaMemcpyPeerAsync(pv, c->device, v, g->device, m * 8, c->stream));
+        TP_CUDA(cudaMemcpyPeerAsync(pi, c->device, bi, g->device, m * 4, c->stream));
+        TP_CUDA(cudaMemcpyPeerAsync(pj, c->device, bj, g->device, m * 4, c->stream));
+        v = pv; bi = pi; bj = pj;
+    }
+    c->raw = nullptr; c->n = 0; c->ingested_n = 0;
+    c->have_X = c->have_C = c->have_scores = c->have_sweep = false;
+    c->generation++;
+    TP_TRY(coo_dense_alloc(c, n, out));
+    const size_t M = (size_t)1 << 30;
+    for (size_t off = 0; off < m; off += M) {
+        const unsigned k = (unsigned)(m - off < M ? m - off : M);
+        coo_scatter_kernel<<<(k + 255) / 256, 256, 0, c->stream>>>(*out, n, bi + off, bj + off, v + off, k, 0, off, status64);
+        c->launches += 1;
+    }
+    TP_CUDA(cudaGetLastError());
+    return TP_OK;
+}
+
+extern "C" int tp_genome_matrix(tp_ctx *ctx, const tp_genome *g, int chrom, double *out) {
+    TP_ARG(ctx && g && out, "tp_genome_matrix: null argument");
+    TP_ARG(chrom >= 0 && chrom < (int)g->bins.size(), "tp_genome_matrix: chromosome index out of range");
+    double *dev = nullptr;
+    TP_TRY(tp_genome_dense(ctx, g, chrom, &dev));
+    const size_t n = (size_t)g->bins[(size_t)chrom];
+    TP_CUDA(cudaMemcpyAsync(out, dev, n * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    TP_CUDA(tp_stream_sync(ctx));
+    return TP_OK;
+}
+
+extern "C" int tp_genome_free(tp_genome *g) {
+    if (!g) return TP_OK;
+    cudaSetDevice(g->device);
+    g->px.release();
+    delete g;
     return TP_OK;
 }
 

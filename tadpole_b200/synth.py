@@ -15,7 +15,7 @@ from __future__ import annotations
 
 import numpy as np
 
-__all__ = ["synth_hic", "synth_hic_gpu", "synth_partition_pairs", "write_tsv"]
+__all__ = ["synth_hic", "synth_hic_gpu", "synth_genome_pixels", "synth_partition_pairs", "write_tsv"]
 
 
 def _random_blocks(rng, n, mean_len):
@@ -117,6 +117,35 @@ def synth_hic_gpu(n, seed=1, device=0, centromere=False, centromere_frac=0.03, z
         mat[c0:c0 + ln, :] = 0.0
         mat[:, c0:c0 + ln] = 0.0
     return mat
+
+
+def synth_genome_pixels(sizes, seed=1, trans_per_chrom=100):
+    """A seeded genome-wide pixel list, as HiC-Pro or cooler write one: chromosome c has sizes[c] bins and its contacts
+    are synth_hic(sizes[c], seed + c) (any size, 1 included); its non-zero upper-triangle cells become pixels with global
+    0-based bin ids, and trans_per_chrom pixels per chromosome join one of its bins to a bin of another chromosome.  The
+    pixels are shuffled.  Returns (names, (bin1, bin2, count), mats): names "chr1", ...; bin1 <= bin2 int32, count
+    float64; mats[c] the symmetric matrix of chromosome c, whose upper triangle its cis pixels are."""
+    rng = np.random.default_rng(seed)
+    sizes = [int(n) for n in sizes]
+    starts = np.concatenate(([0], np.cumsum(sizes)))
+    b1, b2, v, mats = [], [], [], []
+    for c, n in enumerate(sizes):
+        m = synth_hic(n, seed=seed + c) if n >= 2 else np.full((n, n), float(rng.integers(1, 9)))
+        mats.append(m)
+        i, j = np.triu_indices(n)
+        sel = m[i, j] != 0
+        b1.append(i[sel] + starts[c]); b2.append(j[sel] + starts[c]); v.append(m[i, j][sel])
+        if len(sizes) > 1 and trans_per_chrom:
+            x = rng.integers(0, n, trans_per_chrom) + starts[c]
+            other = rng.integers(0, len(sizes) - 1, trans_per_chrom)
+            other += other >= c                                          # any chromosome but c
+            y = starts[other] + (rng.random(trans_per_chrom) * np.asarray(sizes)[other]).astype(np.int64)
+            b1.append(np.minimum(x, y)); b2.append(np.maximum(x, y))
+            v.append(rng.integers(1, 5, trans_per_chrom).astype(np.float64))
+    b1, b2, v = np.concatenate(b1), np.concatenate(b2), np.concatenate(v)
+    perm = rng.permutation(b1.size)
+    names = [f"chr{c + 1}" for c in range(len(sizes))]
+    return names, (b1[perm].astype(np.int32), b2[perm].astype(np.int32), v[perm].astype(np.float64)), mats
 
 
 def synth_partition_pairs(npairs, length, ntads, seed=1, zero_frac=0.01):
