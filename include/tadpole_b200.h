@@ -37,7 +37,9 @@ enum {
     TP_ERR_NOLEVEL = 3,    /* a candidate has no significant broken-stick level: the reference
                               errors inside the worker here (R/TADpole.R:113-115, n_cluster = NA) */
     TP_ERR_NOCONV = 4,     /* eigensolver did not reach the residual tolerance */
-    TP_ERR_NOMEM = 5
+    TP_ERR_NOMEM = 5,
+    TP_ERR_NOSPLIT = 6     /* centromere_search: the matrix does not split (no bad columns, or the longest bad stretch
+                              touches an end): the reference errors here (quirk Q4) */
 };
 
 const char *tp_last_error(void);
@@ -250,6 +252,15 @@ int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int *keep_q, in
  *                   offsets[nlevels+1], start/end[nrows] (1-based inclusive), device ms of the call; NULL = skip. */
 int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
                   int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, tp_batch **out);
+/* centromere_search = TRUE on every matrix of a batch (R/TADpole.R:351-442), in the same worker threads: each worker
+ * filters its matrix, splits it (tp_centromere_split, quirk Q3 kept unless centromere_fix) and runs the p arm, then the
+ * q arm, on its own context; the tables of every scored level and the optimal level's fixed labels are built there too.
+ * A matrix that does not split fails as its own item with TP_ERR_NOSPLIT, or, with centromere_fix, is called whole on
+ * its good bins (TADpole(centromere_fix = TRUE)) and read like a tp_call_batch item.  A split item is read with
+ * tp_batch_split and tp_batch_arm_dims / tp_batch_arm_get; tp_batch_get gives its bad flags and device ms (filter and
+ * both arms). */
+int tp_call_batch_arms(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
+                       int max_pcs, int min_clusters, double bad_frac, int centromere_fix, int inflight, tp_batch **out);
 int tp_batch_size(const tp_batch *b);
 /* device milliseconds of the whole batch: CUDA events, from the start of the batch to the end of the last call, max over
  * the streams and devices it ran on */
@@ -262,6 +273,20 @@ int tp_batch_dims(const tp_batch *b, int i, int *n_out, int *nf_out, int *k_out,
                   int *nrows_out);
 int tp_batch_get(const tp_batch *b, int i, uint8_t *bad_out, int *n_pcs_out, int *n_clusters_out, double *scores_out,
                  double *seqdist_out, int *levels_out, int *offsets_out, int *start_out, int *end_out, double *device_ms_out);
+/* items of tp_call_batch_arms / tp_call_genome_arms, whatever their status: *split_out = 1 when item i was split at
+ * the centromere, 0 when it was not (processed whole, or failed after the filter), -1 when its bad flags are not known
+ * (any item of the other batch calls); cs..ce = the longest bad stretch (1-based, 0 when there is no bad bin);
+ * bad_out[n] = the bad flags when split_out >= 0.  Any pointer may be NULL. */
+int tp_batch_split(const tp_batch *b, int i, int *split_out, int *cs_out, int *ce_out, uint8_t *bad_out);
+/* arm `arm` (0 = p, 1 = q) of a split item: sizes (kept bins, nf = kept bins, k, maxlev, scored levels, table rows, bad
+ * columns or -1 for NULL), then keep[nkeep] (0-based original bins), bad[nbad] (original 1-based), n_pcs, n_clusters,
+ * scores[k x maxlev], seqdist[nf-1], levels, offsets, start/end as tp_batch_get gives them, and labels[nf + max(nbad, 0)]
+ * = the optimal level's fixed label vector with the bad columns re-inserted (merging_arms joins the two). */
+int tp_batch_arm_dims(const tp_batch *b, int i, int arm, int *nkeep_out, int *nf_out, int *k_out, int *maxlev_out,
+                      int *nlevels_out, int *nrows_out, int *nbad_out);
+int tp_batch_arm_get(const tp_batch *b, int i, int arm, int *keep_out, int *bad_out, int *n_pcs_out, int *n_clusters_out,
+                     double *scores_out, double *seqdist_out, int *levels_out, int *offsets_out, int *start_out, int *end_out,
+                     int *labels_out);
 int tp_batch_free(tp_batch *b);
 
 /* ---- genome-wide input: one pixel list over every chromosome (HiC-Pro *.matrix, cooler dump -t pixels) --------------
@@ -297,6 +322,10 @@ int tp_genome_matrix(tp_ctx *ctx, const tp_genome *g, int chrom, double *out);
  * handle was ingested on (or a context whose first device holds it). */
 int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
                    double bad_frac, int inflight, int want_tables, tp_batch **out);
+/* centromere_search = TRUE on every selected chromosome: the items of tp_call_batch_arms, with the workers, memory cap
+ * and largest-first order of tp_call_genome. */
+int tp_call_genome_arms(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
+                        double bad_frac, int centromere_fix, int inflight, tp_batch **out);
 int tp_genome_free(tp_genome *g);
 
 /* The context is a device-resident pipeline handle: after tp_call / tp_call_arm / tp_pca the PC scores stay in HBM, and
@@ -351,6 +380,16 @@ int tp_assemble_levels(const double *seqdist, int nf, const int *levels, int nle
  * -object while that object is a singleton, else the step that last absorbed it.  merge_out: n1 x 2 ints, column-major
  * (an R matrix).  Host only, O(n log n). */
 int tp_find_groups(const double *seqdist, int n1, int *merge_out);
+
+/* load_mat's centromere split (R/TADpole.R:58-86) on the bad flags bad[n]; host only.  The longest run of bad bins (the
+ * first one on ties) is the centromere *cs_out..*ce_out (1-based; 0 when there is no bad bin); *split_out = 0 when there
+ * is none or it touches either end.  Split: keep_p[*nkeep_p] / keep_q[*nkeep_q] = the arms' kept bins (0-based original
+ * indices), bad_p[*nbad_p] / bad_q[*nbad_q] = their bad columns (original 1-based; *nbad = -1 when there is none, the
+ * reference's NULL).  fix = 0 keeps quirk Q3: the q arm drops the rows at the ORIGINAL indices of its bad columns used
+ * as positions in the arm, ignoring those past its end; fix = 1 drops the bad columns themselves.  Every output array
+ * needs room for n ints. */
+int tp_centromere_split(const uint8_t *bad, int n, int fix, int *split_out, int *cs_out, int *ce_out, int *keep_p,
+                        int *nkeep_p, int *bad_p, int *nbad_p, int *keep_q, int *nkeep_q, int *bad_q, int *nbad_q);
 
 #ifdef __cplusplus
 }

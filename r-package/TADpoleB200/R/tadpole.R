@@ -37,22 +37,15 @@
     message(paste(idx, collapse = " "))
     whole <- list(keep = which(!bad), bad_columns = as.character(idx))
     if (!centromere_search || length(idx) == 0L) return(whole)
-    runs <- split(idx, cumsum(c(1L, diff(idx) != 1L)))
-    longest <- runs[[which.max(lengths(runs))]]
-    cs <- longest[1L]; ce <- longest[length(longest)]
-    message(paste("centromere position:", cs, ce))
-    if (cs == 1L || ce == n) {
+    # the split itself (longest bad run, quirk Q3 kept) is the library's tp_centromere_split
+    s <- .Call(C_tp_split, bad, FALSE)
+    message(paste("centromere position:", s[[1L]][2L], s[[1L]][3L]))
+    if (!s[[1L]][1L]) {
         message("longest stretch of bad rows/columns at the ends, not splitting the matrix.")
         return(whole)
     }
-    p_bins <- seq_len(cs - 1L); q_bins <- (ce + 1L):n
-    bad_p <- idx[idx < cs]; bad_q <- idx[idx > ce]
-    keep_q <- rep(TRUE, length(q_bins))
-    # the reference drops q-arm rows by ORIGINAL index used as a position in the arm; out-of-range ones are ignored
-    keep_q[bad_q[bad_q <= length(q_bins)]] <- FALSE
-    list(p = list(keep = setdiff(p_bins, bad_p), bad_columns = if (length(bad_p)) bad_p else NULL),
-         q = list(keep = q_bins[keep_q], bad_columns = if (length(bad_q)) bad_q else NULL),
-         centromere = cs:ce)
+    list(p = list(keep = s[[2L]], bad_columns = s[[3L]]), q = list(keep = s[[4L]], bad_columns = s[[5L]]),
+         centromere = s[[1L]][2L]:s[[1L]][3L])
 }
 
 # the numeric core of load_mat on the GPU: which bins stay (index lists; the matrix itself stays in HBM)
@@ -136,16 +129,22 @@ TADpole <- function(mat_file, max_pcs = 200, min_clusters = 2, bad_frac = 0.01,
     both <- .Call(C_tp_call_arms, ctx, as.integer(mat$p$keep - 1L), as.integer(mat$q$keep - 1L),
                   as.integer(max_pcs), as.integer(min_clusters))
     names(both) <- c("p", "q")
+    .tp_arms_object(both, mat)
+}
+
+# the tadpole object of a split chromosome (R/TADpole.R:376-442): both = list(p, q) of arm results (as C_tp_call_arm
+# returns them), parts = list(p, q, centromere) of list(keep, bad_columns)
+.tp_arms_object <- function(both, parts) {
     out <- structure(list(), class = "tadpole")
     joined <- integer(0)
     for (arm in c("p", "q")) {
         message(paste("Processing arm", arm))
-        r <- .tp_pack_part(both[[arm]], mat[[arm]])
+        r <- .tp_pack_part(both[[arm]], parts[[arm]])
         out[[arm]] <- list(n_pcs = r$n_pcs, optimal_n_clusters = r$optimal_n_clusters, dendro = r$dendro,
                            cluster = r$clusters)
-        joined <- c(joined, r$labels_optimal, rep(0L, length(mat$centromere)))
+        joined <- c(joined, r$labels_optimal, rep(0L, length(parts$centromere)))
     }
-    joined <- joined[seq_len(length(joined) - length(mat$centromere))]
+    joined <- joined[seq_len(length(joined) - length(parts$centromere))]
     runs <- rle(joined)
     ends <- cumsum(runs$lengths)
     coord <- data.frame(start = c(1, ends[-length(ends)] + 1), end = ends)
@@ -153,12 +152,33 @@ TADpole <- function(mat_file, max_pcs = 200, min_clusters = 2, bad_frac = 0.01,
     out
 }
 
+# one item of C_tp_call_batch_arms / C_tp_call_genome_arms: list(bad, centromere, p, q), each arm
+# list(n_pcs, optimal_n_clusters, seqdist, scores, keep, bad_columns)
+.tp_arms_batch_object <- function(r) {
+    message(paste(sum(r[[1L]]), "bad columns found at position(s):"))
+    message(paste(which(r[[1L]]), collapse = " "))
+    message(paste("centromere position:", r[[2L]][1L], r[[2L]][length(r[[2L]])]))
+    parts <- list(p = list(keep = r[[3L]][[5L]], bad_columns = r[[3L]][[6L]]),
+                  q = list(keep = r[[4L]][[5L]], bad_columns = r[[4L]][[6L]]), centromere = r[[2L]])
+    .tp_arms_object(list(p = r[[3L]], q = r[[4L]]), parts)
+}
+
 # TADpole() on a list of matrices (genome-wide use: one per chromosome), `inflight` calls per GPU kept in flight by the
 # library's own threads over every GPU of options(tadpole.gpus); same objects, same order, as calling TADpole() on each
-TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L) {
+# centromere_search = TRUE: every matrix is split at its centromere and both arms run in those threads; a matrix that does
+# not split stops, as TADpole(centromere_search = TRUE) does
+TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L, centromere_search = FALSE) {
     ctx <- .tp_ctx()
     mats <- lapply(mats, function(m) if (is.character(m)) {
         .Call(C_tp_ingest, ctx, path.expand(m)); .Call(C_tp_ingested_matrix, ctx) } else as.matrix(m) + 0)
+    if (centromere_search) {
+        res <- .Call(C_tp_call_batch_arms, ctx, mats, as.integer(max_pcs), as.integer(min_clusters), as.numeric(bad_frac),
+                     as.integer(inflight))
+        return(lapply(res, function(r) {
+            if (is.character(r)) stop(r)
+            .tp_arms_batch_object(r)
+        }))
+    }
     res <- .Call(C_tp_call_batch, ctx, mats, as.integer(max_pcs), as.integer(min_clusters), as.numeric(bad_frac),
                  as.integer(inflight))
     lapply(res, function(r) {
@@ -200,8 +220,10 @@ TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01
 # or sparse_counts(path = , index_base = 1L) with GLOBAL bin ids (HiC-Pro *.matrix, cooler dump -t pixels), bins = the
 # bin table.  The pixels are split by chromosome on the GPU and each chromosome's dense matrix exists only in HBM while
 # its call runs.  A named list of tadpole objects (bin-table order, or chroms order), attr(, "failed") = the messages
-# of the chromosomes whose call failed.
-TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L) {
+# of the chromosomes whose call failed.  centromere_search = TRUE: as TADpole(centromere_search = TRUE) on each
+# chromosome; one that does not split fails.
+TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L,
+                           centromere_search = FALSE) {
     stopifnot(inherits(pixels, "tadpole_pixels"))
     ctx <- .tp_ctx()
     tab <- .tp_bin_table(bins)
@@ -210,14 +232,18 @@ TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clust
     if (anyNA(idx)) stop("unknown chromosome(s): ", paste(sel[is.na(idx)], collapse = ", "))
     g <- if (is.null(pixels$path)) .Call(C_tp_genome, ctx, tab$n, pixels$bin1, pixels$bin2, pixels$count, pixels$index_base)
          else .Call(C_tp_genome_file, ctx, tab$n, path.expand(pixels$path), pixels$index_base)
-    res <- .Call(C_tp_call_genome, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
-                 as.numeric(bad_frac), as.integer(inflight), TRUE)
+    res <- if (centromere_search)
+        .Call(C_tp_call_genome_arms, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
+              as.numeric(bad_frac), as.integer(inflight), FALSE)
+    else .Call(C_tp_call_genome, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
+               as.numeric(bad_frac), as.integer(inflight), TRUE)
     out <- list()
     failed <- list()
     for (i in seq_along(sel)) {
         message(paste("Processing chromosome", sel[i]))
         r <- res[[i]]
         if (is.character(r)) { failed[[sel[i]]] <- r; next }
+        if (centromere_search) { out[[sel[i]]] <- .tp_arms_batch_object(r); next }
         message(paste(sum(r[[1L]]), "bad columns found at position(s):"))
         message(paste(which(r[[1L]]), collapse = " "))
         message(paste("Optimal number of PCs:", r[[2L]]))

@@ -346,6 +346,105 @@ SEXP C_tp_call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP 
     return out;
 }
 
+/* an integer vector of n values plus `add` (NULL when n < 0); unprotected */
+static SEXP int_vector(const int *v, int n, int add) {
+    if (n < 0) return R_NilValue;
+    SEXP x = allocVector(INTSXP, n);
+    for (int i = 0; i < n; i++) INTEGER(x)[i] = v[i] + add;
+    return x;
+}
+
+/* load_mat's centromere split of the bad flags (tp_centromere_split, R/TADpole.R:58-86): list(c(split, cs, ce),
+ * p keep, p bad_columns, q keep, q bad_columns) with keep 1-based, bad_columns NULL when empty, the arms NULL when the
+ * matrix is not split; fix = the repair of quirk Q3 */
+SEXP C_tp_split(SEXP bad, SEXP fix) {
+    int n = length(bad);
+    uint8_t *b = (uint8_t *)R_alloc((size_t)n + 1, 1);
+    for (int i = 0; i < n; i++) b[i] = INTEGER(bad)[i] != 0;
+    int *kp = (int *)R_alloc((size_t)n + 1, sizeof(int)), *bp = (int *)R_alloc((size_t)n + 1, sizeof(int));
+    int *kq = (int *)R_alloc((size_t)n + 1, sizeof(int)), *bq = (int *)R_alloc((size_t)n + 1, sizeof(int));
+    int split = 0, cs = 0, ce = 0, nkp = 0, nbp = 0, nkq = 0, nbq = 0;
+    if (tp_centromere_split(b, n, asLogical(fix), &split, &cs, &ce, kp, &nkp, bp, &nbp, kq, &nkq, bq, &nbq) != TP_OK)
+        error("%s", tp_last_error());
+    SEXP out = PROTECT(allocVector(VECSXP, 5));
+    SEXP head = allocVector(INTSXP, 3);
+    SET_VECTOR_ELT(out, 0, head);
+    INTEGER(head)[0] = split; INTEGER(head)[1] = cs; INTEGER(head)[2] = ce;
+    if (split) {
+        SET_VECTOR_ELT(out, 1, int_vector(kp, nkp, 1));
+        SET_VECTOR_ELT(out, 2, int_vector(bp, nbp, 0));
+        SET_VECTOR_ELT(out, 3, int_vector(kq, nkq, 1));
+        SET_VECTOR_ELT(out, 4, int_vector(bq, nbq, 0));
+    } else {
+        for (int i = 1; i < 5; i++) SET_VECTOR_ELT(out, i, R_NilValue);
+    }
+    UNPROTECT(1);
+    return out;
+}
+
+/* item i of a tp_call_batch_arms / tp_call_genome_arms batch: a split item is list(bad, centromere = cs:ce, p, q), each
+ * arm list(n_pcs, optimal_n_clusters, seqdist, scores, keep (1-based), bad_columns (NULL when empty)); any other item as
+ * batch_item gives it; unprotected */
+static SEXP arms_item(tp_batch *b, int i) {
+    int split = -1, cs = 0, ce = 0, nn = 0;
+    tp_batch_split(b, i, &split, &cs, &ce, NULL);
+    if (tp_batch_status(b, i) != TP_OK || split != 1) return batch_item(b, i);
+    tp_batch_dims(b, i, &nn, NULL, NULL, NULL, NULL, NULL);
+    SEXP item = PROTECT(allocVector(VECSXP, 4));
+    SEXP bad = allocVector(LGLSXP, nn);
+    SET_VECTOR_ELT(item, 0, bad);
+    unsigned char *tb = (unsigned char *)R_alloc((size_t)nn + 1, 1);
+    tp_batch_split(b, i, NULL, NULL, NULL, tb);
+    for (int j = 0; j < nn; j++) LOGICAL(bad)[j] = tb[j];
+    SEXP cen = allocVector(INTSXP, ce - cs + 1);
+    SET_VECTOR_ELT(item, 1, cen);
+    for (int j = cs; j <= ce; j++) INTEGER(cen)[j - cs] = j;
+    for (int a = 0; a < 2; a++) {
+        int nk, nf, k, maxlev, nbad, npcs = 0, ncl = 0;
+        tp_batch_arm_dims(b, i, a, &nk, &nf, &k, &maxlev, NULL, NULL, &nbad);
+        SEXP arm = PROTECT(allocVector(VECSXP, 6));
+        SET_VECTOR_ELT(item, 2 + a, arm);
+        UNPROTECT(1);
+        SEXP seq = allocVector(REALSXP, nf - 1);
+        SET_VECTOR_ELT(arm, 2, seq);
+        int *keep = (int *)R_alloc((size_t)nk + 1, sizeof(int)), *bc = (int *)R_alloc((size_t)(nbad > 0 ? nbad : 0) + 1, sizeof(int));
+        double *sc = (double *)R_alloc((size_t)k * maxlev + 1, sizeof(double));
+        tp_batch_arm_get(b, i, a, keep, bc, &npcs, &ncl, sc, REAL(seq), NULL, NULL, NULL, NULL, NULL);
+        SET_VECTOR_ELT(arm, 0, ScalarInteger(npcs));
+        SET_VECTOR_ELT(arm, 1, ScalarInteger(ncl));
+        SET_VECTOR_ELT(arm, 3, score_matrix(sc, k, maxlev));
+        SET_VECTOR_ELT(arm, 4, int_vector(keep, nk, 1));
+        SET_VECTOR_ELT(arm, 5, int_vector(bc, nbad, 0));
+    }
+    UNPROTECT(1);
+    return item;
+}
+
+/* TADpole(centromere_search = TRUE) on a list of matrices (tp_call_batch_arms): every matrix is split at its centromere
+ * and both arms run in the library's workers.  Per matrix: arms_item, or a character error message (a matrix that does
+ * not split fails, as the reference's TADpole() does). */
+SEXP C_tp_call_batch_arms(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight) {
+    tp_ctx *c = ctx_of(ctx);
+    int nc = length(mats);
+    const double **ptr = (const double **)R_alloc((size_t)(nc ? nc : 1), sizeof(double *));
+    int *n = (int *)R_alloc((size_t)(nc ? nc : 1), sizeof(int));
+    for (int i = 0; i < nc; i++) {
+        SEXP m = VECTOR_ELT(mats, i);
+        if (!isReal(m) || nrows(m) != ncols(m)) error("TADpole: element %d is not a square numeric matrix", i + 1);
+        ptr[i] = REAL(m);
+        n[i] = nrows(m);
+    }
+    tp_batch *b = NULL;
+    if (tp_call_batch_arms(c, nc, ptr, n, 1, 0, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac), 0,
+                           asInteger(inflight), &b) != TP_OK)
+        error("%s", tp_last_error());
+    SEXP out = PROTECT(allocVector(VECSXP, nc));
+    for (int i = 0; i < nc; i++) SET_VECTOR_ELT(out, i, arms_item(b, i));
+    tp_batch_free(b);
+    UNPROTECT(1);
+    return out;
+}
+
 static void genome_finalizer(SEXP p) {
     tp_genome *g = (tp_genome *)R_ExternalPtrAddr(p);
     if (g) {
@@ -416,6 +515,27 @@ SEXP C_tp_call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min
         error("%s", tp_last_error());
     SEXP out = PROTECT(allocVector(VECSXP, ns));
     for (int i = 0; i < ns; i++) SET_VECTOR_ELT(out, i, batch_item(b, i));
+    tp_batch_free(b);
+    UNPROTECT(1);
+    return out;
+}
+
+/* TADpole(centromere_search = TRUE) on the chromosomes `chroms` of a C_tp_genome handle (tp_call_genome_arms).  Per
+ * chromosome, in chroms order: arms_item, or a character error message.  fix: centromere_fix of the Python host (the
+ * repair of quirks Q3 and Q4); R's TADpole() has no such flag and passes FALSE. */
+SEXP C_tp_call_genome_arms(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
+                           SEXP fix) {
+    tp_ctx *c = ctx_of(ctx);
+    tp_genome *g = (tp_genome *)R_ExternalPtrAddr(genome);
+    if (!g) error("TADpole: the genome pixels have been released");
+    if (!isInteger(chroms)) error("TADpole: chromosome indices must be integers");
+    int ns = length(chroms);
+    tp_batch *b = NULL;
+    if (tp_call_genome_arms(c, g, INTEGER(chroms), ns, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac),
+                            asLogical(fix), asInteger(inflight), &b) != TP_OK)
+        error("%s", tp_last_error());
+    SEXP out = PROTECT(allocVector(VECSXP, ns));
+    for (int i = 0; i < ns; i++) SET_VECTOR_ELT(out, i, arms_item(b, i));
     tp_batch_free(b);
     UNPROTECT(1);
     return out;
@@ -538,6 +658,9 @@ static const R_CallMethodDef call_table[] = {
     {"C_tp_genome", (DL_FUNC)&C_tp_genome, 6},
     {"C_tp_genome_file", (DL_FUNC)&C_tp_genome_file, 4},
     {"C_tp_call_genome", (DL_FUNC)&C_tp_call_genome, 8},
+    {"C_tp_split", (DL_FUNC)&C_tp_split, 2},
+    {"C_tp_call_batch_arms", (DL_FUNC)&C_tp_call_batch_arms, 6},
+    {"C_tp_call_genome_arms", (DL_FUNC)&C_tp_call_genome_arms, 8},
     {"C_tp_levels", (DL_FUNC)&C_tp_levels, 5},
     {"C_tp_labels", (DL_FUNC)&C_tp_labels, 5},
     {"C_tp_difft", (DL_FUNC)&C_tp_difft, 5},

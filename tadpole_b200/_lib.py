@@ -14,7 +14,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libtadpole_b200.so")
 
-TP_OK, TP_ERR_ARG, TP_ERR_CUDA, TP_ERR_NOLEVEL, TP_ERR_NOCONV, TP_ERR_NOMEM = range(6)
+TP_OK, TP_ERR_ARG, TP_ERR_CUDA, TP_ERR_NOLEVEL, TP_ERR_NOCONV, TP_ERR_NOMEM, TP_ERR_NOSPLIT = range(7)
 
 # every symbol include/tadpole_b200.h declares
 EXPORTED = [
@@ -30,6 +30,7 @@ EXPORTED = [
     "tp_ctx_create_multi", "tp_device_count", "tp_ctx_devices", "tp_ctx_generation", "tp_ctx_dims", "tp_call_arms", "tp_call_batch",
     "tp_batch_size", "tp_batch_device_ms", "tp_batch_launches", "tp_batch_status", "tp_batch_error", "tp_batch_dims", "tp_batch_get", "tp_batch_free", "tp_find_groups",
     "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
+    "tp_centromere_split", "tp_call_batch_arms", "tp_call_genome_arms", "tp_batch_split", "tp_batch_arm_dims", "tp_batch_arm_get",
 ]
 
 
@@ -72,6 +73,12 @@ def load():
         "tp_batch_dims": (c_int, [vp, c_int, ip, ip, ip, ip, ip, ip]),
         "tp_batch_get": (c_int, [vp, c_int, u8p, ip, ip, dp, dp, ip, ip, ip, ip, dp]),
         "tp_batch_free": (c_int, [vp]),
+        "tp_call_batch_arms": (c_int, [vp, c_int, POINTER(vp), ip, c_int, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
+        "tp_call_genome_arms": (c_int, [vp, vp, ip, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
+        "tp_batch_split": (c_int, [vp, c_int, ip, ip, ip, u8p]),
+        "tp_batch_arm_dims": (c_int, [vp, c_int, c_int, ip, ip, ip, ip, ip, ip, ip]),
+        "tp_batch_arm_get": (c_int, [vp, c_int, c_int, ip, ip, ip, ip, dp, dp, ip, ip, ip, ip, ip]),
+        "tp_centromere_split": (c_int, [u8p, c_int, c_int, ip, ip, ip, ip, ip, ip, ip, ip, ip, ip, ip]),
         "tp_genome_ingest": (c_int, [vp, ip, c_int, ip, ip, dp, ctypes.c_size_t, c_int, POINTER(vp)]),
         "tp_genome_ingest_file": (c_int, [vp, ip, c_int, c_char_p, c_int, c_int, POINTER(vp)]),
         "tp_genome_stats": (c_int, [vp, POINTER(ctypes.c_ulonglong), POINTER(ctypes.c_ulonglong), POINTER(ctypes.c_ulonglong)]),
@@ -501,11 +508,15 @@ class Context:
                     tables={int(l): tab[off[j]: off[j + 1]] for j, l in enumerate(lev)} if tables else None,
                     device_ms=ms.value)
 
-    def call_batch(self, mats, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True, device_ptrs=None, n=None):
+    def call_batch(self, mats, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True, device_ptrs=None, n=None,
+                   centromere_search=False, centromere_fix=False):
         """tp_call_batch: one tp_call per matrix, `inflight` calls per device kept in flight by library-owned threads over
         every device of the context.  mats: list of square float64 arrays (all C or all F order); or device_ptrs + n
         (row-major, single-device contexts).  Returns a list of dicts as call() returns, plus 'tables' {level: [rows, 2]}
-        and 'device_ms'; a failed call's entry is the TadpoleError."""
+        and 'device_ms'; a failed call's entry is the TadpoleError.
+        centromere_search: tp_call_batch_arms, each matrix split at its centromere and its two arms called in the same
+        workers; a split matrix's entry is the dict of _split_item, an unsplit one's (centromere_fix) the dict above, and
+        one that does not split without centromere_fix fails with TP_ERR_NOSPLIT."""
         if device_ptrs is None:
             mats = [m if (m.dtype == np.float64 and (m.flags.c_contiguous or m.flags.f_contiguous))
                     else np.ascontiguousarray(m, dtype=np.float64) for m in (np.asarray(m) for m in mats)]
@@ -521,9 +532,49 @@ class Context:
             colmajor, ondev = 0, 1
         ncalls = int(ns.size)
         h = c_void_p()
+        if centromere_search:
+            check(self.lib.tp_call_batch_arms(self._h, ncalls, ptrs, _ip(ns), colmajor, ondev, int(max_pcs), int(min_clusters),
+                                              float(bad_frac), int(bool(centromere_fix)), int(inflight), ctypes.byref(h)))
+            return self._batch_results(h, ncalls, True)
         check(self.lib.tp_call_batch(self._h, ncalls, ptrs, _ip(ns), colmajor, ondev, int(max_pcs), int(min_clusters),
                                      float(bad_frac), int(inflight), int(bool(tables)), ctypes.byref(h)))
         return self._batch_results(h, ncalls, tables)
+
+    def _split_state(self, h, i, n):
+        """(split: -1 / 0 / 1, the longest bad stretch cs..ce (1-based bins) or None, bad flags or None) of item i
+        (tp_batch_split)."""
+        sp, cs, ce = c_int(0), c_int(0), c_int(0)
+        bad = np.zeros(max(n, 1), np.uint8)
+        check(self.lib.tp_batch_split(h, i, ctypes.byref(sp), ctypes.byref(cs), ctypes.byref(ce),
+                                      bad.ctypes.data_as(POINTER(c_uint8))))
+        return (sp.value, np.arange(cs.value, ce.value + 1) if cs.value else None,
+                bad[:n].astype(bool) if sp.value >= 0 else None)
+
+    def _arm_item(self, h, i, arm):
+        """Arm `arm` (0 = p, 1 = q) of split item i: dict(keep (0-based), bad_columns (original 1-based, or None), nf, k,
+        n_pcs, n_clusters, scores, seqdist, tables {level: [rows, 2]}, labels (fixed labels of the optimal level))."""
+        d = [c_int(0) for _ in range(7)]
+        check(self.lib.tp_batch_arm_dims(h, i, arm, *[ctypes.byref(x) for x in d]))
+        nk, nf, k, ml, nlev, nrows, nbad = (x.value for x in d)
+        keep = np.zeros(nk, np.int32); bad = np.zeros(max(nbad, 0), np.int32)
+        sc = np.empty((k, ml)); seq = np.empty(nf - 1)
+        lev = np.zeros(nlev, np.int32); off = np.zeros(nlev + 1, np.int32)
+        st = np.zeros(nrows, np.int32); en = np.zeros(nrows, np.int32)
+        lab = np.zeros(nf + max(nbad, 0), np.int32)
+        npcs, ncl = c_int(0), c_int(0)
+        check(self.lib.tp_batch_arm_get(h, i, arm, _ip(keep), _ip(bad), ctypes.byref(npcs), ctypes.byref(ncl), _dp(sc),
+                                        _dp(seq), _ip(lev), _ip(off), _ip(st), _ip(en), _ip(lab)))
+        tab = np.stack([st, en], axis=1).astype(np.int64)
+        return dict(keep=keep, bad_columns=bad if nbad >= 0 else None, nf=nf, k=k, n_pcs=npcs.value, n_clusters=ncl.value,
+                    scores=sc, seqdist=seq, tables={int(l): tab[off[j]: off[j + 1]] for j, l in enumerate(lev)}, labels=lab)
+
+    def _split_item(self, h, i, n, centromere):
+        """A split item: dict(split=True, centromere (1-based bins cs..ce), bad, device_ms, p, q) with p / q as _arm_item."""
+        ms = c_double(0.0)
+        check(self.lib.tp_batch_get(h, i, None, None, None, None, None, None, None, None, None, ctypes.byref(ms)))
+        _, _, bad = self._split_state(h, i, n)
+        return dict(split=True, centromere=centromere, bad=bad, device_ms=ms.value, p=self._arm_item(h, i, 0),
+                    q=self._arm_item(h, i, 1))
 
     def _batch_results(self, h, ncalls, tables):
         """Every item of a tp_batch (freed here) as call_batch returns them."""
@@ -534,9 +585,24 @@ class Context:
             for i in range(ncalls):
                 rc = self.lib.tp_batch_status(h, i)
                 if rc != TP_OK:
-                    out.append(TadpoleError(rc, self.lib.tp_batch_error(h, i).decode("utf-8", "replace")))
+                    err = TadpoleError(rc, self.lib.tp_batch_error(h, i).decode("utf-8", "replace"))
+                    # a centromere_search item that failed after its filter: split (-1 = not reached), the longest bad
+                    # stretch and the bad flags, for load_mat's messages
+                    nn = c_int(0)
+                    check(self.lib.tp_batch_dims(h, i, ctypes.byref(nn), None, None, None, None, None))
+                    err.split, err.centromere, err.bad = self._split_state(h, i, nn.value)
+                    out.append(err)
                     continue
-                out.append(self._batch_item(h, i, tables))
+                nn = c_int(0)
+                check(self.lib.tp_batch_dims(h, i, ctypes.byref(nn), None, None, None, None, None))
+                split, cen, _ = self._split_state(h, i, nn.value)
+                if split == 1:
+                    out.append(self._split_item(h, i, nn.value, cen))
+                    continue
+                item = self._batch_item(h, i, tables)
+                if split == 0:                       # centromere_search, not split: processed whole (centromere_fix)
+                    item.update(split=False, centromere=cen)
+                out.append(item)
         finally:
             self.lib.tp_batch_free(h)
         return out
@@ -560,11 +626,17 @@ class Context:
                                             ctypes.byref(h)))
         return Genome(self, h, cb)
 
-    def call_genome(self, genome, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True):
+    def call_genome(self, genome, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True,
+                    centromere_search=False, centromere_fix=False):
         """tp_call_genome: one call per selected chromosome (0-based indices, default all), results in that order as
-        call_batch returns them (a failed call's entry is the TadpoleError)."""
+        call_batch returns them (a failed call's entry is the TadpoleError); centromere_search: tp_call_genome_arms, the
+        entries as call_batch(centromere_search=True) gives them."""
         sel = np.arange(genome.chrom_bins.size, dtype=np.int32) if chroms is None else np.ascontiguousarray(chroms, dtype=np.int32)
         h = c_void_p()
+        if centromere_search:
+            check(self.lib.tp_call_genome_arms(self._h, genome._h, _ip(sel), int(sel.size), int(max_pcs), int(min_clusters),
+                                               float(bad_frac), int(bool(centromere_fix)), int(inflight), ctypes.byref(h)))
+            return self._batch_results(h, int(sel.size), True)
         check(self.lib.tp_call_genome(self._h, genome._h, _ip(sel), int(sel.size), int(max_pcs), int(min_clusters),
                                       float(bad_frac), int(inflight), int(bool(tables)), ctypes.byref(h)))
         return self._batch_results(h, int(sel.size), tables)
@@ -677,6 +749,26 @@ def assemble(seqdist, n_clusters, names, bad):
     check(lib.tp_assemble(_dp(seqdist), nf, int(n_clusters), _ip(names), _ip(badarr), nbad, _ip(start), _ip(end),
                           ctypes.byref(nrows), _ip(labels)))
     return np.stack([start[:nrows.value], end[:nrows.value]], axis=1).astype(np.int64), labels
+
+
+def centromere_split(bad, fix=False):
+    """tp_centromere_split (host only): load_mat's split of the bad flags at the longest bad stretch (R/TADpole.R:58-86).
+    Returns (split, (cs, ce) or None when there is no bad bin, (keep_p, bad_p), (keep_q, bad_q)): keep 0-based, bad
+    columns original 1-based or None (NULL); the arms are None when split is False."""
+    lib = load()
+    b = np.ascontiguousarray(bad, dtype=np.uint8)
+    n = b.size
+    bufs = [np.zeros(max(n, 1), np.int32) for _ in range(4)]
+    v = [c_int(0) for _ in range(7)]
+    sp, cs, ce, nkp, nbp, nkq, nbq = v
+    check(lib.tp_centromere_split(b.ctypes.data_as(POINTER(c_uint8)), n, int(bool(fix)), ctypes.byref(sp), ctypes.byref(cs),
+                                  ctypes.byref(ce), _ip(bufs[0]), ctypes.byref(nkp), _ip(bufs[1]), ctypes.byref(nbp),
+                                  _ip(bufs[2]), ctypes.byref(nkq), _ip(bufs[3]), ctypes.byref(nbq)))
+    span = (cs.value, ce.value) if cs.value else None
+    if not sp.value:
+        return False, span, None, None
+    arm = lambda k, nk, bb, nb: (k[:nk.value].copy(), bb[:nb.value].copy() if nb.value >= 0 else None)
+    return True, span, arm(bufs[0], nkp, bufs[1], nbp), arm(bufs[2], nkq, bufs[3], nbq)
 
 
 def assemble_levels(seqdist, levels, names, bad):

@@ -120,34 +120,35 @@ class LoadedMatrix:
 
 
 def _split_centromere(bad, fix=False):
-    """R/TADpole.R:58-86 on the bad flags.  Returns None when the matrix is not split.
+    """R/TADpole.R:58-86 on the bad flags (tp_centromere_split).  Returns None when the matrix is not split.
     fix=True removes the q-arm bad columns by their position within the arm (quirk Q3 repaired)."""
-    n = bad.size
-    idx = np.flatnonzero(bad) + 1
-    brk = np.flatnonzero(np.diff(idx) > 1) + 1
-    runs = np.split(idx, brk)
-    longest = runs[int(np.argmax([len(r) for r in runs]))]       # which.max: first on ties
-    cs, ce = int(longest[0]), int(longest[-1])
-    message(f"centromere position: {cs} {ce}")
-    if cs == 1 or ce == n:
-        message("longest stretch of bad rows/columns at the ends, not splitting the matrix.")
+    split, span, arm_p, arm_q = _lib.centromere_split(bad, fix)
+    cen = None if span is None else np.arange(span[0], span[1] + 1)
+    _messages_split(cen, split)
+    if not split:
         return None
-    idx_p = np.arange(1, cs)
-    idx_q = np.arange(ce + 1, n + 1)
-    bad_p = idx[idx < cs]
-    bad_q = idx[idx > ce]
-    keep_p = np.ones(idx_p.size, bool)
-    keep_p[bad_p - 1] = False
-    keep_q = np.ones(idx_q.size, bool)
-    # R/TADpole.R:80 applies the ORIGINAL indices of the q-arm bad columns as negative positional
-    # indices to the re-based q matrix; out-of-range ones are silently ignored (SURVEY.md quirk Q3).
-    if fix:
-        keep_q[bad_q - ce - 1] = False
-    else:
-        inr = bad_q[bad_q <= idx_q.size]
-        keep_q[inr - 1] = False
-    return (idx_p[keep_p] - 1, bad_p if bad_p.size else None), (idx_q[keep_q] - 1, bad_q if bad_q.size else None), \
-        np.arange(cs, ce + 1)
+    as64 = lambda a: None if a is None else a.astype(np.int64)
+    return (arm_p[0].astype(np.int64), as64(arm_p[1])), (arm_q[0].astype(np.int64), as64(arm_q[1])), cen
+
+
+def _messages_split(cen, split):
+    """load_mat's messages about the centromere cen = cs..ce (R/TADpole.R:64-70); None: no bad bin, nothing is said."""
+    if cen is None:
+        return
+    message(f"centromere position: {cen[0]} {cen[-1]}")
+    if not split:
+        message("longest stretch of bad rows/columns at the ends, not splitting the matrix.")
+
+
+def _messages_bad(bad):
+    message(f"{int(bad.sum())} bad columns found at position(s):")
+    message(" ".join(str(i) for i in np.flatnonzero(bad) + 1))
+
+
+# TADpole(centromere_search=TRUE) on a matrix that load_mat does not split: R/TADpole.R:356-359 then does
+# mat$centromer / mat[['p']] on a plain matrix and errors (quirk Q4)
+NOSPLIT_MESSAGE = ("centromere_search=TRUE but load_mat did not split the matrix "
+                   "(no bad columns, or the longest bad stretch touches an end); the reference errors here")
 
 
 def load_mat(mat_file, chr=None, start=None, end=None, resol=None, bad_frac=0.01, centromere_search=False,
@@ -161,9 +162,7 @@ def load_mat(mat_file, chr=None, start=None, end=None, resol=None, bad_frac=0.01
 
 def _loaded_from_flags(ctx, bad, centromere_search, fix=False):
     n = bad.size
-    bad_names = [str(i) for i in np.flatnonzero(bad) + 1]
-    message(f"{int(bad.sum())} bad columns found at position(s):")
-    message(" ".join(bad_names))
+    _messages_bad(bad)
     if bad.any() and centromere_search:
         split = _split_centromere(bad, fix)
         if split is not None:
@@ -263,9 +262,7 @@ def TADpole(mat_file, max_pcs=200, min_clusters=2, bad_frac=0.01, chr=None, star
     mat = _matrix_args(mat_file, ctx)
     if not centromere_search:
         res = ctx.call(max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac, **mat)
-        bad = res["bad"]
-        message(f"{int(bad.sum())} bad columns found at position(s):")
-        message(" ".join(str(i) for i in np.flatnonzero(bad) + 1))
+        _messages_bad(res["bad"])
         return _tadpole_from_result(res, ctx)
 
     bad, _, _ = ctx.filter(bad_frac=bad_frac, **mat)
@@ -275,12 +272,7 @@ def TADpole(mat_file, max_pcs=200, min_clusters=2, bad_frac=0.01, chr=None, star
         res["bad"] = bad
         return _tadpole_from_result(res, ctx)
     if not lm.is_split:
-        # R/TADpole.R:356-359 then does mat$centromer / mat[['p']] on a plain matrix and errors (quirk Q4)
-        raise ValueError("centromere_search=TRUE but load_mat did not split the matrix "
-                         "(no bad columns, or the longest bad stretch touches an end); the reference errors here")
-    tp = Tadpole()
-    fixed_arms = []
-    ncen = len(lm.centromere)
+        raise ValueError(NOSPLIT_MESSAGE)
     arm_res = {}
     if dist is not None and dist.world > 1:
         # every rank runs its own arm (collectively with the other ranks of that arm); the small result summaries
@@ -294,32 +286,46 @@ def TADpole(mat_file, max_pcs=200, min_clusters=2, bad_frac=0.01, chr=None, star
     else:
         # tp_call_arms: on a multi-device context the two halves of the devices work on the two arms at the same time
         arm_res["p"], arm_res["q"] = ctx.call_arms(lm.p.keep, lm.q.keep, max_pcs=max_pcs, min_clusters=min_clusters)
+    tp = Tadpole()
+    labels = []
     for arm in ("p", "q"):
-        message(f"Processing arm {arm}")
         la = getattr(lm, arm)
-        res = arm_res[arm]
-        _messages_optimal(res)
-        a = _Obj()
-        a.n_pcs = res["n_pcs"]
-        a.optimal_n_clusters = res["n_clusters"]
-        a.dendro = Dendro(res["seqdist"], labels=la.names)
-        a.cluster = _levels_table(res, la.names.astype(np.int32), la.bad_columns)
-        if centromere_fix:
-            a.clusters, a.scores = a.cluster, res["scores"]
-        tp[arm] = a
-        # optimal level of this arm, bad columns re-inserted, fix_values applied (R/TADpole.R:411-431)
-        bad_for_merge = la.bad_columns if la.bad_columns is not None else np.zeros(0, np.int32)
-        _, labels = _lib.assemble(res["seqdist"], res["n_clusters"], la.names.astype(np.int32), bad_for_merge)
-        fixed_arms.append(labels.astype(np.int64))
-        fixed_arms.append(np.zeros(ncen, dtype=np.int64))
-    allv = np.concatenate(fixed_arms)
-    allv = allv[: allv.size - ncen]                      # R/TADpole.R:438
+        names = la.names.astype(np.int32)
+        tp[arm] = _arm_object(arm, arm_res[arm], names, _levels_table(arm_res[arm], names, la.bad_columns), centromere_fix)
+        labels.append(_arm_labels(arm_res[arm], names, la.bad_columns))
+    tp.merging_arms = _merging_arms(labels[0], labels[1], len(lm.centromere))
+    return tp
+
+
+def _arm_object(arm, res, names, tables, centromere_fix):
+    """One arm of a centromere_search result (R/TADpole.R:376-408): n_pcs, optimal_n_clusters, dendro and the per-level
+    tables as `cluster`; with centromere_fix also `clusters` and `scores`."""
+    message(f"Processing arm {arm}")
+    _messages_optimal(res)
+    a = _Obj()
+    a.n_pcs = res["n_pcs"]
+    a.optimal_n_clusters = res["n_clusters"]
+    a.dendro = Dendro(res["seqdist"], labels=names)
+    a.cluster = tables
+    if centromere_fix:
+        a.clusters, a.scores = a.cluster, res["scores"]
+    return a
+
+
+def _arm_labels(res, names, bad_columns):
+    """The optimal level of an arm, bad columns re-inserted, fix_values applied (R/TADpole.R:411-431)."""
+    bad_for_merge = bad_columns if bad_columns is not None else np.zeros(0, np.int32)
+    return _lib.assemble(res["seqdist"], res["n_clusters"], names, bad_for_merge)[1]
+
+
+def _merging_arms(labels_p, labels_q, ncen):
+    """c(p labels, centromere zeros, q labels) -> start / end of its non-zero runs (R/TADpole.R:432-442)."""
+    allv = np.concatenate([labels_p.astype(np.int64), np.zeros(ncen, np.int64), labels_q.astype(np.int64)])
     brk = np.flatnonzero(allv[1:] != allv[:-1]) + 1
     starts = np.concatenate(([0], brk))
     ends = np.concatenate((brk, [allv.size]))
     keep = allv[starts] != 0
-    tp.merging_arms = np.stack([starts[keep] + 1, ends[keep]], axis=1)
-    return tp
+    return np.stack([starts[keep] + 1, ends[keep]], axis=1)
 
 
 # ---- diffT -------------------------------------------------------------------------------------------

@@ -19,7 +19,8 @@ import os
 import numpy as np
 
 from . import _lib
-from .api import Tadpole, _messages_optimal, get_context, message, read_matrix
+from .api import (NOSPLIT_MESSAGE, Tadpole, _arm_object, _merging_arms, _messages_bad, _messages_optimal, _messages_split,
+                  message, read_matrix)
 from .hclust import Dendro
 
 __all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "TADpole_genome", "read_bins"]
@@ -38,10 +39,21 @@ class ContextPool:
         self.ctx.close()
 
 
-def _tadpole_from_batch_item(res):
+def _tadpole_from_batch_item(res, centromere_fix=False):
+    """The object and the messages TADpole() gives for one item of a batch; a centromere_search item
+    (call_batch(centromere_search=True)) as TADpole(centromere_search=True, centromere_fix=centromere_fix) gives it."""
     bad = res["bad"]
-    message(f"{int(bad.sum())} bad columns found at position(s):")
-    message(" ".join(str(i) for i in np.flatnonzero(bad) + 1))
+    _messages_bad(bad)
+    if "split" in res:
+        _messages_split(res["centromere"], res["split"])
+    if res.get("split"):
+        tp = Tadpole()
+        for arm in ("p", "q"):
+            a = res[arm]
+            tp[arm] = _arm_object(arm, a, (a["keep"] + 1).astype(np.int32), {str(k): t for k, t in a["tables"].items()},
+                                  centromere_fix)
+        tp.merging_arms = _merging_arms(res["p"]["labels"], res["q"]["labels"], res["centromere"].size)
+        return tp
     _messages_optimal(res)
     tp = Tadpole()
     tp.n_pcs = res["n_pcs"]
@@ -52,21 +64,36 @@ def _tadpole_from_batch_item(res):
     return tp                          # no device handle: the per-call contexts are reused by the next call
 
 
+def _failed_item(err):
+    """What TADpole(centromere_search=True) says and raises for a matrix whose batch item failed: load_mat's messages when
+    the filter ran, then the ValueError of an unsplit matrix (quirk Q4) or the library's error."""
+    if getattr(err, "split", -1) >= 0:
+        _messages_bad(err.bad)
+        _messages_split(err.centromere, err.split)
+    return ValueError(NOSPLIT_MESSAGE) if err.code == _lib.TP_ERR_NOSPLIT else err
+
+
 def TADpole_batch(mat_files, max_pcs=200, min_clusters=2, bad_frac=0.01, centromere_search=False, pool=None,
-                  device=0, streams=4, ctx=None):
-    """TADpole() on every matrix of `mat_files` (paths or arrays), `streams` calls in flight per GPU."""
-    if centromere_search:
-        from .api import TADpole
-        c = ctx or (pool.ctx if pool else get_context(device if isinstance(device, int) else device[0]))
-        return [TADpole(m, max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac, centromere_search=True, ctx=c)
-                for m in mat_files]
+                  device=0, streams=4, ctx=None, centromere_fix=False):
+    """TADpole() on every matrix of `mat_files` (paths or arrays), `streams` calls in flight per GPU.  centromere_search
+    (and centromere_fix, see TADpole()): every matrix is split at its centromere and both arms are called in the library's
+    workers; the objects and messages are TADpole(centromere_search=True)'s, and the first matrix TADpole() would fail on
+    raises its exception."""
     own = pool is None and ctx is None
     if ctx is None:
         pool = pool or ContextPool(device, streams)
         ctx, streams = pool.ctx, pool.streams
     try:
         mats = [read_matrix(m, ctx) for m in mat_files]
-        res = ctx.call_batch(mats, max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac, inflight=streams)
+        res = ctx.call_batch(mats, max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac, inflight=streams,
+                             centromere_search=centromere_search, centromere_fix=centromere_fix)
+        if centromere_search:
+            out = []
+            for r in res:                   # messages in input order, up to the first matrix that fails
+                if isinstance(r, Exception):
+                    raise _failed_item(r)
+                out.append(_tadpole_from_batch_item(r, centromere_fix))
+            return out
         for r in res:
             if isinstance(r, Exception):
                 raise r
@@ -157,10 +184,13 @@ class GenomeResult(dict):
     stats: dict
 
 
-def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, ctx=None, device=0, streams=4):
+def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, ctx=None, device=0, streams=4,
+                   centromere_search=False, centromere_fix=False):
     """TADpole() on every chromosome of a genome-wide pixel list (GenomePixels), `streams` calls in flight per GPU.
-    Each chromosome's Tadpole is the one TADpole() returns for that chromosome's dense matrix.  Returns a GenomeResult in
-    bin-table order, or in `chroms` order when chroms (a list of names) is given."""
+    Each chromosome's Tadpole is the one TADpole() returns for that chromosome's dense matrix (with centromere_search /
+    centromere_fix as TADpole() takes them: p, q and merging_arms; a chromosome that does not split fails with
+    TADpole()'s message unless centromere_fix).  Returns a GenomeResult in bin-table order, or in `chroms` order when
+    chroms (a list of names) is given."""
     index = {nm: c for c, nm in enumerate(pixels.names)}
     sel = list(pixels.names) if chroms is None else [str(c) for c in chroms]
     unknown = [c for c in sel if c not in index]
@@ -173,7 +203,7 @@ def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.
         try:
             cis, trans, below = g.stats()
             res = ctx.call_genome(g, [index[c] for c in sel], max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac,
-                                  inflight=streams)
+                                  inflight=streams, centromere_search=centromere_search, centromere_fix=centromere_fix)
         finally:
             g.close()
     finally:
@@ -185,7 +215,7 @@ def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.
     for nm, r in zip(sel, res):
         message(f"Processing chromosome {nm}")
         if isinstance(r, Exception):
-            out.failed[nm] = str(r)
+            out.failed[nm] = NOSPLIT_MESSAGE if r.code == _lib.TP_ERR_NOSPLIT else str(r)
             continue
-        out[nm] = _tadpole_from_batch_item(r)
+        out[nm] = _tadpole_from_batch_item(r, centromere_fix)
     return out

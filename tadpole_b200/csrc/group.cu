@@ -7,9 +7,10 @@
 //     torchrun job runs with one process per GPU -- same kernels, same collectives, same bits.
 //   * chromosome arms on disjoint halves of the devices at the same time (tp_call_arms, R/TADpole.R:357-374).
 //   * batches of independent calls kept in flight by library-owned threads (tp_call_batch): genome-wide use loops over
-//     chromosomes, and one 2000-bin call leaves most of a B200 idle.
+//     chromosomes, and one 2000-bin call leaves most of a B200 idle.  With centromere_search (tp_call_batch_arms,
+//     tp_call_genome_arms) each worker splits its matrix at the centromere and runs both arms one after the other.
 //   * small host-side pieces the R wrapper would otherwise do in interpreted loops: the hclust merge matrix of a
-//     chclust dendrogram (rioja's .find.groups rule) in O(n log n).
+//     chclust dendrogram (rioja's .find.groups rule) in O(n log n), and load_mat's centromere split (tp_centromere_split).
 //
 // The R API never sees threads: every entry point returns when all member devices are done, worker threads never touch
 // R (SURVEY.md 8b, "Threading").
@@ -210,6 +211,52 @@ extern "C" int tp_find_groups(const double *seqdist, int n1, int *merge_out) {
     return TP_OK;
 }
 
+// ---- load_mat's centromere split (R/TADpole.R:58-86) on the bad flags ------------------------------------------------
+// runs <- split(idx, cumsum(c(1, diff(idx) != 1))); the longest run (which.max: the first one on ties) is the centromere
+// cs..ce; no split when it touches either end.  keep_p / keep_q: 0-based original bins of each arm; bad_p / bad_q: the
+// arm's bad columns as original 1-based bins, *nbad = -1 when there is none (attr NULL).  The reference drops the q arm's
+// rows by the ORIGINAL index of its bad columns used as a position in the arm, ignoring those past the arm's end (quirk
+// Q3); fix = 1 drops the bad columns themselves.
+extern "C" int tp_centromere_split(const uint8_t *bad, int n, int fix, int *split_out, int *cs_out, int *ce_out, int *keep_p,
+                                   int *nkeep_p, int *bad_p, int *nbad_p, int *keep_q, int *nkeep_q, int *bad_q, int *nbad_q) {
+    TP_ARG(bad && n >= 0 && split_out && cs_out && ce_out && keep_p && nkeep_p && bad_p && nbad_p && keep_q && nkeep_q && bad_q &&
+           nbad_q, "tp_centromere_split: null argument");
+    *split_out = *cs_out = *ce_out = *nkeep_p = *nkeep_q = 0;
+    *nbad_p = *nbad_q = -1;
+    int cs = 0, ce = 0;
+    for (int i = 0; i < n;) {
+        if (!bad[i]) { i++; continue; }
+        int j = i;
+        while (j + 1 < n && bad[j + 1]) j++;
+        if (cs == 0 || j - i > ce - cs) { cs = i + 1; ce = j + 1; }
+        i = j + 1;
+    }
+    *cs_out = cs;
+    *ce_out = ce;
+    if (cs == 0 || cs == 1 || ce == n) return TP_OK;
+    const int nq = n - ce;
+    std::vector<uint8_t> drop_q((size_t)nq, 0);
+    int np = 0, bp = 0, bq = 0;
+    for (int i = 0; i < cs - 1; i++) {
+        if (bad[i]) bad_p[bp++] = i + 1;
+        else keep_p[np++] = i;
+    }
+    for (int i = ce; i < n; i++)
+        if (bad[i]) {
+            bad_q[bq++] = i + 1;
+            const int pos = fix ? i - ce : i;              // 0-based position in the arm of the row that is dropped
+            if (pos < nq) drop_q[(size_t)pos] = 1;
+        }
+    int nk = 0;
+    for (int t = 0; t < nq; t++) if (!drop_q[(size_t)t]) keep_q[nk++] = ce + t;
+    *split_out = 1;
+    *nkeep_p = np;
+    *nkeep_q = nk;
+    *nbad_p = bp ? bp : -1;
+    *nbad_q = bq ? bq : -1;
+    return TP_OK;
+}
+
 // ---- batches of independent calls ----------------------------------------------------------------------------------------
 struct TpBatchItem {
     int rc = TP_OK;
@@ -220,6 +267,14 @@ struct TpBatchItem {
     std::vector<int> levels, offsets, start, end; // per-level start / end tables (R/TADpole.R:470-497)
     double device_ms = 0.0;
     long long launches = 0;
+    // centromere_search items (tp_call_batch_arms, tp_call_genome_arms): split = -1 until the bad flags are known, then
+    // 0 (processed whole or failed) or 1 (arms[0] = p, arms[1] = q); cs..ce = the longest bad run (1-based, 0 = none)
+    int split = -1, cs = 0, ce = 0;
+    std::vector<TpBatchItem> arms;
+    // an arm: its 0-based original bins, its bad columns (original 1-based; nbad = -1: attr NULL) and the fixed label
+    // vector of its optimal level, bad columns re-inserted (R/TADpole.R:411-431)
+    std::vector<int> keep, badcols, labels;
+    int nbad = -1;
 };
 struct tp_batch { std::vector<TpBatchItem> items; double device_ms = 0.0; };
 
@@ -234,6 +289,29 @@ static void finish_item(tp_ctx *c, TpBatchItem &it) {
     if (tp_ctx_timings(c, tm) == TP_OK) it.device_ms = tm[6];
 }
 
+// for (k in which(!is.na(scores[n_PCs, ]))) ... the start / end table of every scored level of the optimal candidate of a
+// finished item (R/TADpole.R:381-408, 470-497).  names[nf]: original 1-based bin of each kept row; bad[nbad]: the bad
+// columns (nbad < 0: attr NULL).
+static int level_tables(TpBatchItem &it, const int *names, const int *bad, int nbad) {
+    const double *row = it.scores.data() + (size_t)(it.n_pcs - 1) * it.maxlev;
+    size_t cap = 0;
+    for (int l = 0; l < it.maxlev; l++)
+        if (row[l] == row[l]) { it.levels.push_back(l + 1); cap += (size_t)(l + 1) + (size_t)std::max(nbad, 0) + 1; }
+    it.offsets.assign(it.levels.size() + 1, 0);
+    it.start.assign(cap + 1, 0);
+    it.end.assign(cap + 1, 0);
+    TP_TRY(tp_assemble_levels(it.seqdist.data(), it.nf, it.levels.data(), (int)it.levels.size(), names, bad, nbad,
+                              it.start.data(), it.end.data(), it.offsets.data()));
+    it.start.resize((size_t)it.offsets.back());
+    it.end.resize((size_t)it.offsets.back());
+    return TP_OK;
+}
+
+// names and bad columns of a whole matrix from its bad flags, as TADpole() packs it
+static void whole_lists(const TpBatchItem &it, std::vector<int> &names, std::vector<int> &bad) {
+    for (int i = 0; i < it.n; i++) (it.bad[(size_t)i] ? bad : names).push_back(i + 1);
+}
+
 static int batch_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_device, int max_pcs, int min_clusters,
                      double bad_frac, int want_tables, TpBatchItem &it) {
     it.n = n;
@@ -246,20 +324,91 @@ static int batch_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_d
                    &it.n_clusters, nullptr, it.seqdist.data()));
     finish_item(c, it);
     if (!want_tables) return TP_OK;
-    // for (k in which(!is.na(scores[n_PCs, ]))) ... the start / end table of every scored level of the optimal candidate
     std::vector<int> names, bad;
-    for (int i = 0; i < n; i++) (it.bad[i] ? bad : names).push_back(i + 1);
-    const double *row = it.scores.data() + (size_t)(it.n_pcs - 1) * it.maxlev;
-    size_t cap = 0;
-    for (int l = 0; l < it.maxlev; l++)
-        if (row[l] == row[l]) { it.levels.push_back(l + 1); cap += (size_t)(l + 1) + bad.size() + 1; }
-    it.offsets.assign(it.levels.size() + 1, 0);
-    it.start.assign(cap + 1, 0);
-    it.end.assign(cap + 1, 0);
-    TP_TRY(tp_assemble_levels(it.seqdist.data(), it.nf, it.levels.data(), (int)it.levels.size(), names.data(), bad.data(),
-                              (int)bad.size(), it.start.data(), it.end.data(), it.offsets.data()));
-    it.start.resize((size_t)it.offsets.back());
-    it.end.resize((size_t)it.offsets.back());
+    whole_lists(it, names, bad);
+    return level_tables(it, names.data(), bad.data(), (int)bad.size());
+}
+
+// one chromosome arm on c, after tp_filter: the arm's call (tp_call_arm on its keep list), its tables and its fixed labels
+static int arm_one(tp_ctx *c, int max_pcs, int min_clusters, TpBatchItem &a) {
+    a.nf = (int)a.keep.size();
+    a.seqdist.assign((size_t)(a.nf > 1 ? a.nf - 1 : 1), 0.0);
+    TP_TRY(tp_call_arm(c, a.keep.data(), a.nf, max_pcs, min_clusters, nullptr, &a.n_pcs, &a.n_clusters, nullptr,
+                       a.seqdist.data()));
+    finish_item(c, a);
+    std::vector<int> names(a.keep.size());
+    for (size_t t = 0; t < names.size(); t++) names[t] = a.keep[t] + 1;
+    TP_TRY(level_tables(a, names.data(), a.badcols.data(), a.nbad));
+    // the optimal level with the bad columns re-inserted and fix_values applied, for merging_arms
+    const int nb = std::max(a.nbad, 0);
+    std::vector<int> st((size_t)a.n_clusters + nb + 2), en(st.size());
+    int rows = 0;
+    a.labels.assign((size_t)a.nf + nb, 0);
+    return tp_assemble(a.seqdist.data(), a.nf, a.n_clusters, names.data(), a.badcols.data(), nb, st.data(), en.data(), &rows,
+                       a.labels.data());
+}
+
+static const char *const NOSPLIT_MSG = "centromere_search=TRUE but load_mat did not split the matrix (no bad columns, or the "
+                                       "longest bad stretch touches an end); the reference errors here";
+
+// TADpole(centromere_search = TRUE) on one matrix (R/TADpole.R:351-442): filter, split at the longest bad stretch, then the
+// p arm and the q arm one after the other on c.  Unsplit: TP_ERR_NOSPLIT (the reference errors, quirk Q4), or with fix the
+// whole matrix's good bins as TADpole(centromere_fix = TRUE) does.  device_ms covers the filter and both arms.
+static int arms_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_device, int max_pcs, int min_clusters,
+                    double bad_frac, int fix, TpBatchItem &it) {
+    it.n = n;
+    const long long launches0 = c->launches;
+    struct Count { TpBatchItem &it; tp_ctx *c; long long l0; ~Count() { it.launches = c->launches - l0; } } count{it, c, launches0};
+    it.bad.assign((size_t)n, 0);
+    TP_ARG(max_pcs >= 1, "tp_call_batch_arms: max_pcs must be positive");
+    struct Events {
+        cudaEvent_t e[2] = {nullptr, nullptr};
+        ~Events() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
+    } ev;
+    TP_CUDA(cudaSetDevice(c->device));
+    TP_CUDA(cudaEventCreate(&ev.e[0]));
+    TP_CUDA(cudaEventCreate(&ev.e[1]));
+    TP_CUDA(cudaEventRecord(ev.e[0], c->stream));
+    // tp_call calls the hook itself; here the worker runs tp_filter directly, and the hook releases the first-upload lock
+    const int frc = tp_filter(c, mat, n, colmajor, on_device, bad_frac, it.bad.data(), nullptr, nullptr);
+    if (c->after_filter) c->after_filter();
+    TP_TRY(frc);
+    std::vector<int> kp((size_t)n), bp((size_t)n), kq((size_t)n), bq((size_t)n);
+    int split = 0, nkp = 0, nbp = 0, nkq = 0, nbq = 0;
+    TP_TRY(tp_centromere_split(it.bad.data(), n, fix, &split, &it.cs, &it.ce, kp.data(), &nkp, bp.data(), &nbp, kq.data(), &nkq,
+                               bq.data(), &nbq));
+    it.split = split;
+    if (split) {
+        // The p arm's after_pca hook may stage the next matrix while the q arm still has to compact from this one.  The
+        // staged upload (tp_stage_input) writes raw_next only, on the copy stream; the matrix the arms read is c->raw, which
+        // tp_filter pointed at raw_own (after swapping in the previous staged upload), at the caller's device matrix or at
+        // the genome worker's dense build in raw_own.  raw_own changes hands only in the next tp_filter, so the q arm reads
+        // what the p arm read.
+        it.arms.resize(2);
+        it.arms[0].keep.assign(kp.begin(), kp.begin() + nkp);
+        it.arms[1].keep.assign(kq.begin(), kq.begin() + nkq);
+        it.arms[0].nbad = nbp;
+        it.arms[1].nbad = nbq;
+        if (nbp > 0) it.arms[0].badcols.assign(bp.begin(), bp.begin() + nbp);
+        if (nbq > 0) it.arms[1].badcols.assign(bq.begin(), bq.begin() + nbq);
+        for (TpBatchItem &a : it.arms) TP_TRY(arm_one(c, max_pcs, min_clusters, a));
+    } else {
+        if (!fix) { tp_set_error("%s", NOSPLIT_MSG); return TP_ERR_NOSPLIT; }
+        std::vector<int> names, bad, keep;
+        whole_lists(it, names, bad);
+        for (int v : names) keep.push_back(v - 1);
+        it.nf = (int)keep.size();
+        it.seqdist.assign((size_t)(it.nf > 1 ? it.nf - 1 : 1), 0.0);
+        TP_TRY(tp_call_arm(c, keep.data(), it.nf, max_pcs, min_clusters, nullptr, &it.n_pcs, &it.n_clusters, nullptr,
+                           it.seqdist.data()));
+        finish_item(c, it);
+        TP_TRY(level_tables(it, names.data(), bad.data(), (int)bad.size()));
+    }
+    TP_CUDA(cudaEventRecord(ev.e[1], c->stream));
+    TP_CUDA(cudaEventSynchronize(ev.e[1]));
+    float ms = 0.f;
+    TP_CUDA(cudaEventElapsedTime(&ms, ev.e[0], ev.e[1]));
+    it.device_ms = ms;
     return TP_OK;
 }
 
@@ -448,16 +597,34 @@ extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats,
     return batch_run(ctx, ncalls, need, inflight, !on_device, nullptr, stage, one, out);
 }
 
+extern "C" int tp_call_batch_arms(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
+                                  int max_pcs, int min_clusters, double bad_frac, int centromere_fix, int inflight, tp_batch **out) {
+    TP_ARG(ctx && mats && n && out && ncalls >= 0, "tp_call_batch_arms: bad arguments");
+    TP_ARG(!(on_device && ctx->group), "tp_call_batch_arms: device-resident inputs need a single-device context");
+    // the working set of a whole-matrix call: an arm is smaller than its chromosome
+    size_t nmax = 0;
+    for (int i = 0; i < ncalls; i++) nmax = std::max(nmax, (size_t)(n[i] > 0 ? n[i] : 0));
+    const double need = 56.0 * (double)nmax * (double)nmax + 64e6;
+    auto stage = [&](tp_ctx *c, int j) {
+        if (mats[j] && n[j] >= 2) (void)tp_stage_input(c, mats[j], n[j], colmajor);    // a failure leaves the normal upload
+    };
+    auto one = [&](tp_ctx *c, int i, TpBatchItem &it) -> int {
+        return mats[i] ? arms_one(c, mats[i], n[i], colmajor, on_device, max_pcs, min_clusters, bad_frac, centromere_fix, it)
+                       : (tp_set_error("tp_call_batch_arms: matrix %d is null", i), (int)TP_ERR_ARG);
+    };
+    return batch_run(ctx, ncalls, need, inflight, !on_device, nullptr, stage, one, out);
+}
+
 // ---- genome-wide calls: one per chromosome, each dense matrix built from its bucket in HBM (ingest.cu, S0c) ---------
-extern "C" int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
-                              double bad_frac, int inflight, int want_tables, tp_batch **out) {
-    TP_ARG(ctx && g && out && nsel >= 0 && (chroms || nsel == 0 || nsel == (int)g->bins.size()), "tp_call_genome: bad arguments");
-    TP_ARG(g->device == ctx->device, "tp_call_genome: the handle was ingested on another device than the context's first");
+// The selected chromosomes (checked against the handle), claimed largest first; call(c, mat, n, it) runs one chromosome's
+// dense matrix (device pointer, row-major) on context c.
+static int genome_run(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int inflight, const char *who,
+                      const std::function<int(tp_ctx *, const double *, int, TpBatchItem &)> &call, tp_batch **out) {
     std::vector<int> sel((size_t)(nsel > 0 ? nsel : 0));
     for (int s = 0; s < nsel; s++) {
         sel[(size_t)s] = chroms ? chroms[s] : s;
         if (sel[(size_t)s] < 0 || sel[(size_t)s] >= (int)g->bins.size()) {
-            tp_set_error("tp_call_genome: chromosome index %d is outside 0..%d", sel[(size_t)s], (int)g->bins.size() - 1);
+            tp_set_error("%s: chromosome index %d is outside 0..%d", who, sel[(size_t)s], (int)g->bins.size() - 1);
             return TP_ERR_ARG;
         }
     }
@@ -478,14 +645,32 @@ extern "C" int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms
         it.n = n;
         if (n < 2) {
             it.bad.assign((size_t)n, 0);
-            tp_set_error("tp_call_genome: chromosome %d has %d bin; a call needs at least 2", chrom, n);
+            tp_set_error("%s: chromosome %d has %d bin; a call needs at least 2", who, chrom, n);
             return TP_ERR_ARG;
         }
         double *mat = nullptr;
         TP_TRY(tp_genome_dense(c, g, chrom, &mat));
-        return batch_one(c, mat, n, 0, 1, max_pcs, min_clusters, bad_frac, want_tables, it);
+        return call(c, mat, n, it);
     };
     return batch_run(ctx, nsel, need, inflight, false, order.data(), [](tp_ctx *, int) {}, one, out);
+}
+
+extern "C" int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
+                              double bad_frac, int inflight, int want_tables, tp_batch **out) {
+    TP_ARG(ctx && g && out && nsel >= 0 && (chroms || nsel == 0 || nsel == (int)g->bins.size()), "tp_call_genome: bad arguments");
+    TP_ARG(g->device == ctx->device, "tp_call_genome: the handle was ingested on another device than the context's first");
+    return genome_run(ctx, g, chroms, nsel, inflight, "tp_call_genome", [&](tp_ctx *c, const double *mat, int n, TpBatchItem &it) {
+        return batch_one(c, mat, n, 0, 1, max_pcs, min_clusters, bad_frac, want_tables, it);
+    }, out);
+}
+
+extern "C" int tp_call_genome_arms(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
+                                   double bad_frac, int centromere_fix, int inflight, tp_batch **out) {
+    TP_ARG(ctx && g && out && nsel >= 0 && (chroms || nsel == 0 || nsel == (int)g->bins.size()), "tp_call_genome_arms: bad arguments");
+    TP_ARG(g->device == ctx->device, "tp_call_genome_arms: the handle was ingested on another device than the context's first");
+    return genome_run(ctx, g, chroms, nsel, inflight, "tp_call_genome_arms", [&](tp_ctx *c, const double *mat, int n, TpBatchItem &it) {
+        return arms_one(c, mat, n, 0, 1, max_pcs, min_clusters, bad_frac, centromere_fix, it);
+    }, out);
 }
 
 extern "C" double tp_batch_device_ms(const tp_batch *b) { return b ? b->device_ms : 0.0; }
@@ -503,16 +688,31 @@ extern "C" const char *tp_batch_error(const tp_batch *b, int i) {
     if (!b || i < 0 || i >= (int)b->items.size()) return "tp_batch_error: index out of range";
     return b->items[(size_t)i].err.c_str();
 }
-extern "C" int tp_batch_dims(const tp_batch *b, int i, int *n_out, int *nf_out, int *k_out, int *maxlev_out, int *nlevels_out,
-                             int *nrows_out) {
-    TP_ARG(b && i >= 0 && i < (int)b->items.size(), "tp_batch_dims: index out of range");
-    const TpBatchItem &it = b->items[(size_t)i];
-    if (n_out) *n_out = it.n;
+// the sizes and the outputs of one finished item (a top-level item or an arm of a split one)
+static void item_dims(const TpBatchItem &it, int *nf_out, int *k_out, int *maxlev_out, int *nlevels_out, int *nrows_out) {
     if (nf_out) *nf_out = it.nf;
     if (k_out) *k_out = it.k;
     if (maxlev_out) *maxlev_out = it.maxlev;
     if (nlevels_out) *nlevels_out = (int)it.levels.size();
     if (nrows_out) *nrows_out = (int)it.start.size();
+}
+static void item_get(const TpBatchItem &it, int *n_pcs_out, int *n_clusters_out, double *scores_out, double *seqdist_out,
+                     int *levels_out, int *offsets_out, int *start_out, int *end_out) {
+    if (n_pcs_out) *n_pcs_out = it.n_pcs;
+    if (n_clusters_out) *n_clusters_out = it.n_clusters;
+    if (scores_out) memcpy(scores_out, it.scores.data(), it.scores.size() * sizeof(double));
+    if (seqdist_out) memcpy(seqdist_out, it.seqdist.data(), it.seqdist.size() * sizeof(double));
+    if (levels_out) memcpy(levels_out, it.levels.data(), it.levels.size() * sizeof(int));
+    if (offsets_out) memcpy(offsets_out, it.offsets.data(), it.offsets.size() * sizeof(int));
+    if (start_out) memcpy(start_out, it.start.data(), it.start.size() * sizeof(int));
+    if (end_out) memcpy(end_out, it.end.data(), it.end.size() * sizeof(int));
+}
+extern "C" int tp_batch_dims(const tp_batch *b, int i, int *n_out, int *nf_out, int *k_out, int *maxlev_out, int *nlevels_out,
+                             int *nrows_out) {
+    TP_ARG(b && i >= 0 && i < (int)b->items.size(), "tp_batch_dims: index out of range");
+    const TpBatchItem &it = b->items[(size_t)i];
+    if (n_out) *n_out = it.n;
+    item_dims(it, nf_out, k_out, maxlev_out, nlevels_out, nrows_out);
     return TP_OK;
 }
 extern "C" int tp_batch_get(const tp_batch *b, int i, uint8_t *bad_out, int *n_pcs_out, int *n_clusters_out, double *scores_out,
@@ -522,15 +722,42 @@ extern "C" int tp_batch_get(const tp_batch *b, int i, uint8_t *bad_out, int *n_p
     const TpBatchItem &it = b->items[(size_t)i];
     if (it.rc != TP_OK) { tp_set_error("%s", it.err.c_str()); return it.rc; }
     if (bad_out) memcpy(bad_out, it.bad.data(), it.bad.size());
-    if (n_pcs_out) *n_pcs_out = it.n_pcs;
-    if (n_clusters_out) *n_clusters_out = it.n_clusters;
-    if (scores_out) memcpy(scores_out, it.scores.data(), it.scores.size() * sizeof(double));
-    if (seqdist_out) memcpy(seqdist_out, it.seqdist.data(), it.seqdist.size() * sizeof(double));
-    if (levels_out) memcpy(levels_out, it.levels.data(), it.levels.size() * sizeof(int));
-    if (offsets_out) memcpy(offsets_out, it.offsets.data(), it.offsets.size() * sizeof(int));
-    if (start_out) memcpy(start_out, it.start.data(), it.start.size() * sizeof(int));
-    if (end_out) memcpy(end_out, it.end.data(), it.end.size() * sizeof(int));
+    item_get(it, n_pcs_out, n_clusters_out, scores_out, seqdist_out, levels_out, offsets_out, start_out, end_out);
     if (device_ms_out) *device_ms_out = it.device_ms;
+    return TP_OK;
+}
+extern "C" int tp_batch_split(const tp_batch *b, int i, int *split_out, int *cs_out, int *ce_out, uint8_t *bad_out) {
+    TP_ARG(b && i >= 0 && i < (int)b->items.size(), "tp_batch_split: index out of range");
+    const TpBatchItem &it = b->items[(size_t)i];
+    if (split_out) *split_out = it.split;
+    if (cs_out) *cs_out = it.cs;
+    if (ce_out) *ce_out = it.ce;
+    if (bad_out && it.split >= 0) memcpy(bad_out, it.bad.data(), it.bad.size());
+    return TP_OK;
+}
+static const TpBatchItem *arm_of(const tp_batch *b, int i, int arm) {
+    if (!b || i < 0 || i >= (int)b->items.size() || arm < 0 || arm > 1) return nullptr;
+    const TpBatchItem &it = b->items[(size_t)i];
+    return it.rc == TP_OK && it.split == 1 ? &it.arms[(size_t)arm] : nullptr;
+}
+extern "C" int tp_batch_arm_dims(const tp_batch *b, int i, int arm, int *nkeep_out, int *nf_out, int *k_out, int *maxlev_out,
+                                 int *nlevels_out, int *nrows_out, int *nbad_out) {
+    const TpBatchItem *a = arm_of(b, i, arm);
+    TP_ARG(a, "tp_batch_arm_dims: no such arm (index out of range, or the item was not split)");
+    if (nkeep_out) *nkeep_out = (int)a->keep.size();
+    item_dims(*a, nf_out, k_out, maxlev_out, nlevels_out, nrows_out);
+    if (nbad_out) *nbad_out = a->nbad;
+    return TP_OK;
+}
+extern "C" int tp_batch_arm_get(const tp_batch *b, int i, int arm, int *keep_out, int *bad_out, int *n_pcs_out,
+                                int *n_clusters_out, double *scores_out, double *seqdist_out, int *levels_out, int *offsets_out,
+                                int *start_out, int *end_out, int *labels_out) {
+    const TpBatchItem *a = arm_of(b, i, arm);
+    TP_ARG(a, "tp_batch_arm_get: no such arm (index out of range, or the item was not split)");
+    if (keep_out) memcpy(keep_out, a->keep.data(), a->keep.size() * sizeof(int));
+    if (bad_out) memcpy(bad_out, a->badcols.data(), a->badcols.size() * sizeof(int));
+    item_get(*a, n_pcs_out, n_clusters_out, scores_out, seqdist_out, levels_out, offsets_out, start_out, end_out);
+    if (labels_out) memcpy(labels_out, a->labels.data(), a->labels.size() * sizeof(int));
     return TP_OK;
 }
 extern "C" int tp_batch_free(tp_batch *b) {

@@ -119,18 +119,21 @@ def synth_hic_gpu(n, seed=1, device=0, centromere=False, centromere_frac=0.03, z
     return mat
 
 
-def synth_genome_pixels(sizes, seed=1, trans_per_chrom=100):
+def synth_genome_pixels(sizes, seed=1, trans_per_chrom=100, centromere=None):
     """A seeded genome-wide pixel list, as HiC-Pro or cooler write one: chromosome c has sizes[c] bins and its contacts
     are synth_hic(sizes[c], seed + c) (any size, 1 included); its non-zero upper-triangle cells become pixels with global
     0-based bin ids, and trans_per_chrom pixels per chromosome join one of its bins to a bin of another chromosome.  The
-    pixels are shuffled.  Returns (names, (bin1, bin2, count), mats): names "chr1", ...; bin1 <= bin2 int32, count
-    float64; mats[c] the symmetric matrix of chromosome c, whose upper triangle its cis pixels are."""
+    pixels are shuffled.  centromere: indices of the chromosomes (of 2 bins or more) drawn with
+    synth_hic(..., centromere=True); the others, and the random stream, are the same as without it.  Returns (names,
+    (bin1, bin2, count), mats): names "chr1", ...; bin1 <= bin2 int32, count float64; mats[c] the symmetric matrix of
+    chromosome c, whose upper triangle its cis pixels are."""
     rng = np.random.default_rng(seed)
     sizes = [int(n) for n in sizes]
+    cen = set() if centromere is None else {int(c) for c in centromere}
     starts = np.concatenate(([0], np.cumsum(sizes)))
     b1, b2, v, mats = [], [], [], []
     for c, n in enumerate(sizes):
-        m = synth_hic(n, seed=seed + c) if n >= 2 else np.full((n, n), float(rng.integers(1, 9)))
+        m = synth_hic(n, seed=seed + c, centromere=c in cen) if n >= 2 else np.full((n, n), float(rng.integers(1, 9)))
         mats.append(m)
         i, j = np.triu_indices(n)
         sel = m[i, j] != 0
