@@ -233,9 +233,9 @@ int tp_call_arm(tp_ctx *ctx, const int *keep, int nf, int max_pcs, int min_clust
 
 /* Both chromosome arms of a centromere_search call (R/TADpole.R:357-374: the arms are independent from load_mat on), after
  * tp_filter: on a multi-device context the first half of the devices works on p while the second half works on q; on one
- * device p then q.  The results are a tp_batch (below) of two items, p then q, read with tp_batch_dims / tp_batch_get and
- * released with tp_batch_free: n = 0 (no bad flags: the filtering was tp_filter's), nf, k, maxlev, n_pcs, n_clusters,
- * scores, seqdist and device ms as tp_call_arm gives them, no tables. */
+ * device p then q.  The results are a tp_batch (below) of two items, p then q, read with tp_batch_dims / tp_batch_get
+ * (part = -1) and released with tp_batch_free: n = 0 (no bad flags: the filtering was tp_filter's), nf, k, maxlev, n_pcs,
+ * n_clusters, scores, seqdist and device ms as tp_call_arm gives them, no tables. */
 typedef struct tp_batch tp_batch;
 int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int *keep_q, int nf_q, int max_pcs, int min_clusters,
                  tp_batch **out);
@@ -245,22 +245,27 @@ int tp_call_arms(tp_ctx *ctx, const int *keep_p, int nf_p, const int *keep_q, in
  * as tp_call.  `inflight` calls per device are kept in flight by library-owned host threads, each on its own context and
  * stream (a lone 2000-bin call leaves most of a B200 idle), over every device of the context; the caller's one thread
  * just waits.  want_tables: also build the start / end table of every scored level of the optimal candidate
- * (R/TADpole.R:470-497) in those threads.  Results are held by the returned tp_batch, in input order:
+ * (R/TADpole.R:470-497) in those threads.
+ * centromere: 0 = TADpole() on every matrix.  1 = centromere_search = TRUE (R/TADpole.R:351-442): each worker filters
+ * its matrix, splits it (tp_centromere_split, quirk Q3 kept) and runs the p arm, then the q arm, on its own context; the
+ * tables of every scored level and the optimal level's fixed labels are built there too, whatever want_tables says.  A
+ * matrix that does not split fails as its own item with TP_ERR_NOSPLIT.  2 = the same with centromere_fix: the split
+ * repairs quirk Q3, and a matrix that does not split is called whole on its good bins (TADpole(centromere_fix = TRUE)).
+ * Results are held by the returned tp_batch, in input order:
  *   tp_batch_status / tp_batch_error  per-call return code and message (a failed call does not stop the others);
- *   tp_batch_dims   sizes to allocate: n, nf, k, maxlev, number of scored levels, total table rows;
+ *   tp_batch_split  the split state of a centromere_search item;
+ *   tp_batch_dims   sizes to allocate: n, nf, k, maxlev, number of scored levels, total table rows, kept bins, bad
+ *                   columns (-1 for NULL);
  *   tp_batch_get    bad[n], n_pcs, n_clusters, scores[k x maxlev] row-major NaN padded, seqdist[nf-1], levels[nlevels],
- *                   offsets[nlevels+1], start/end[nrows] (1-based inclusive), device ms of the call; NULL = skip. */
+ *                   offsets[nlevels+1], start/end[nrows] (1-based inclusive), device ms of the call, keep[nkeep] (0-based
+ *                   original bins), bad columns[nbad] (original 1-based), labels[nf + max(nbad, 0)] = the optimal level's
+ *                   fixed label vector with the bad columns re-inserted (merging_arms joins the two arms'); NULL = skip.
+ * The two readers take `part`: -1 = item i itself, 0 / 1 = the p / q arm of item i when it was split (TP_ERR_ARG
+ * otherwise).  Kept bins, bad columns and labels exist for arms only; an arm has n = 0.  A split item itself has its bad
+ * flags and its device ms (filter and both arms); an unsplit centromere_fix item reads like a whole-matrix item. */
 int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
-                  int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, tp_batch **out);
-/* centromere_search = TRUE on every matrix of a batch (R/TADpole.R:351-442), in the same worker threads: each worker
- * filters its matrix, splits it (tp_centromere_split, quirk Q3 kept unless centromere_fix) and runs the p arm, then the
- * q arm, on its own context; the tables of every scored level and the optimal level's fixed labels are built there too.
- * A matrix that does not split fails as its own item with TP_ERR_NOSPLIT, or, with centromere_fix, is called whole on
- * its good bins (TADpole(centromere_fix = TRUE)) and read like a tp_call_batch item.  A split item is read with
- * tp_batch_split and tp_batch_arm_dims / tp_batch_arm_get; tp_batch_get gives its bad flags and device ms (filter and
- * both arms). */
-int tp_call_batch_arms(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
-                       int max_pcs, int min_clusters, double bad_frac, int centromere_fix, int inflight, tp_batch **out);
+                  int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, int centromere,
+                  tp_batch **out);
 int tp_batch_size(const tp_batch *b);
 /* device milliseconds of the whole batch: CUDA events, from the start of the batch to the end of the last call, max over
  * the streams and devices it ran on */
@@ -269,24 +274,16 @@ double tp_batch_device_ms(const tp_batch *b);
 long long tp_batch_launches(const tp_batch *b);
 int tp_batch_status(const tp_batch *b, int i);
 const char *tp_batch_error(const tp_batch *b, int i);
-int tp_batch_dims(const tp_batch *b, int i, int *n_out, int *nf_out, int *k_out, int *maxlev_out, int *nlevels_out,
-                  int *nrows_out);
-int tp_batch_get(const tp_batch *b, int i, uint8_t *bad_out, int *n_pcs_out, int *n_clusters_out, double *scores_out,
-                 double *seqdist_out, int *levels_out, int *offsets_out, int *start_out, int *end_out, double *device_ms_out);
-/* items of tp_call_batch_arms / tp_call_genome_arms, whatever their status: *split_out = 1 when item i was split at
- * the centromere, 0 when it was not (processed whole, or failed after the filter), -1 when its bad flags are not known
- * (any item of the other batch calls); cs..ce = the longest bad stretch (1-based, 0 when there is no bad bin);
- * bad_out[n] = the bad flags when split_out >= 0.  Any pointer may be NULL. */
+int tp_batch_dims(const tp_batch *b, int i, int part, int *n_out, int *nf_out, int *k_out, int *maxlev_out,
+                  int *nlevels_out, int *nrows_out, int *nkeep_out, int *nbad_out);
+int tp_batch_get(const tp_batch *b, int i, int part, uint8_t *bad_out, int *n_pcs_out, int *n_clusters_out,
+                 double *scores_out, double *seqdist_out, int *levels_out, int *offsets_out, int *start_out, int *end_out,
+                 double *device_ms_out, int *keep_out, int *badcols_out, int *labels_out);
+/* item i of a batch, whatever its status: *split_out = 1 when it was split at the centromere, 0 when it was not
+ * (processed whole, or failed after the filter), -1 when its bad flags are not known (any item of another
+ * batch); cs..ce = the longest bad stretch (1-based, 0 when there is no bad bin); bad_out[n] = the bad flags
+ * when split_out >= 0.  Any pointer may be NULL. */
 int tp_batch_split(const tp_batch *b, int i, int *split_out, int *cs_out, int *ce_out, uint8_t *bad_out);
-/* arm `arm` (0 = p, 1 = q) of a split item: sizes (kept bins, nf = kept bins, k, maxlev, scored levels, table rows, bad
- * columns or -1 for NULL), then keep[nkeep] (0-based original bins), bad[nbad] (original 1-based), n_pcs, n_clusters,
- * scores[k x maxlev], seqdist[nf-1], levels, offsets, start/end as tp_batch_get gives them, and labels[nf + max(nbad, 0)]
- * = the optimal level's fixed label vector with the bad columns re-inserted (merging_arms joins the two). */
-int tp_batch_arm_dims(const tp_batch *b, int i, int arm, int *nkeep_out, int *nf_out, int *k_out, int *maxlev_out,
-                      int *nlevels_out, int *nrows_out, int *nbad_out);
-int tp_batch_arm_get(const tp_batch *b, int i, int arm, int *keep_out, int *bad_out, int *n_pcs_out, int *n_clusters_out,
-                     double *scores_out, double *seqdist_out, int *levels_out, int *offsets_out, int *start_out, int *end_out,
-                     int *labels_out);
 int tp_batch_free(tp_batch *b);
 
 /* ---- genome-wide input: one pixel list over every chromosome (HiC-Pro *.matrix, cooler dump -t pixels) --------------
@@ -314,18 +311,14 @@ int tp_genome_stats(const tp_genome *g, unsigned long long *cis_out, unsigned lo
  * matrix) and copied to out */
 int tp_genome_matrix(tp_ctx *ctx, const tp_genome *g, int chrom, double *out);
 /* TADpole() on every selected chromosome: chroms[nsel] (0-based; NULL = all, in bin-table order).  A tp_batch of nsel
- * items in chroms order, read with tp_batch_dims / tp_batch_get: each item is what tp_call_batch gives for that
- * chromosome's dense matrix (tables included when want_tables).  The dense matrix of a chromosome is built from its
+ * items in chroms order: each item is what tp_call_batch gives for that chromosome's dense matrix with the same
+ * want_tables and centromere.  The dense matrix of a chromosome is built from its
  * bucket in HBM by the worker that runs its call, and exists only while that call runs; on a multi-device context a
  * worker on another device first copies the bucket over (cudaMemcpyPeerAsync).  Workers claim chromosomes largest first.
  * A chromosome with fewer than 2 bins, or whose call fails, fails as its own item.  The context must be the one the
  * handle was ingested on (or a context whose first device holds it). */
 int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
-                   double bad_frac, int inflight, int want_tables, tp_batch **out);
-/* centromere_search = TRUE on every selected chromosome: the items of tp_call_batch_arms, with the workers, memory cap
- * and largest-first order of tp_call_genome. */
-int tp_call_genome_arms(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
-                        double bad_frac, int centromere_fix, int inflight, tp_batch **out);
+                   double bad_frac, int inflight, int want_tables, int centromere, tp_batch **out);
 int tp_genome_free(tp_genome *g);
 
 /* The context is a device-resident pipeline handle: after tp_call / tp_call_arm / tp_pca the PC scores stay in HBM, and

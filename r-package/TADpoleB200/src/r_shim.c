@@ -269,7 +269,7 @@ static SEXP batch_item(tp_batch *b, int i) {
         return msg;
     }
     int nn, nf, k, maxlev, nlev, nrow;
-    tp_batch_dims(b, i, &nn, &nf, &k, &maxlev, &nlev, &nrow);
+    tp_batch_dims(b, i, -1, &nn, &nf, &k, &maxlev, &nlev, &nrow, NULL, NULL);
     SEXP bad = PROTECT(allocVector(LGLSXP, nn)), seq = PROTECT(allocVector(REALSXP, nf - 1));
     SEXP levels = PROTECT(allocVector(INTSXP, nlev)), tables = PROTECT(allocVector(VECSXP, nlev));
     unsigned char *tb = (unsigned char *)R_alloc((size_t)nn, 1);
@@ -277,7 +277,7 @@ static SEXP batch_item(tp_batch *b, int i) {
     int *off = (int *)R_alloc((size_t)nlev + 1, sizeof(int)), *st = (int *)R_alloc((size_t)nrow + 1, sizeof(int)),
         *en = (int *)R_alloc((size_t)nrow + 1, sizeof(int));
     int npcs = 0, ncl = 0;
-    tp_batch_get(b, i, tb, &npcs, &ncl, sc, REAL(seq), INTEGER(levels), off, st, en, NULL);
+    tp_batch_get(b, i, -1, tb, &npcs, &ncl, sc, REAL(seq), INTEGER(levels), off, st, en, NULL, NULL, NULL, NULL);
     for (int j = 0; j < nn; j++) LOGICAL(bad)[j] = tb[j];
     SEXP scores = PROTECT(score_matrix(sc, k, maxlev));
     for (int l = 0; l < nlev; l++) {
@@ -320,32 +320,6 @@ SEXP C_tp_call_arms(SEXP ctx, SEXP keep_p, SEXP keep_q, SEXP max_pcs, SEXP min_c
     return out;
 }
 
-/* TADpole() on a list of matrices, `inflight` calls per device kept in flight by the library's own threads over every
- * device of the context (tp_call_batch); this thread only waits.  Per matrix: list(bad, n_pcs, optimal_n_clusters,
- * seqdist, scores, levels, tables = list of 2-column (start, end) matrices), or a character error message. */
-SEXP C_tp_call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight) {
-    tp_ctx *c = ctx_of(ctx);
-    int nc = length(mats);
-    const double **ptr = (const double **)R_alloc((size_t)(nc ? nc : 1), sizeof(double *));
-    int *n = (int *)R_alloc((size_t)(nc ? nc : 1), sizeof(int));
-    for (int i = 0; i < nc; i++) {
-        SEXP m = VECTOR_ELT(mats, i);
-        if (!isReal(m) || nrows(m) != ncols(m)) error("TADpole: element %d is not a square numeric matrix", i + 1);
-        ptr[i] = REAL(m);
-        n[i] = nrows(m);
-    }
-    tp_batch *b = NULL;
-    if (tp_call_batch(c, nc, ptr, n, 1, 0, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac), asInteger(inflight),
-                      1, &b) != TP_OK)
-        error("%s", tp_last_error());
-    /* (an R allocation failure below longjmps past tp_batch_free: the batch, plain host memory, is then leaked) */
-    SEXP out = PROTECT(allocVector(VECSXP, nc));
-    for (int i = 0; i < nc; i++) SET_VECTOR_ELT(out, i, batch_item(b, i));
-    tp_batch_free(b);
-    UNPROTECT(1);
-    return out;
-}
-
 /* an integer vector of n values plus `add` (NULL when n < 0); unprotected */
 static SEXP int_vector(const int *v, int n, int add) {
     if (n < 0) return R_NilValue;
@@ -382,14 +356,14 @@ SEXP C_tp_split(SEXP bad, SEXP fix) {
     return out;
 }
 
-/* item i of a tp_call_batch_arms / tp_call_genome_arms batch: a split item is list(bad, centromere = cs:ce, p, q), each
- * arm list(n_pcs, optimal_n_clusters, seqdist, scores, keep (1-based), bad_columns (NULL when empty)); any other item as
- * batch_item gives it; unprotected */
+/* item i of a batch: a split centromere_search item is list(bad, centromere = cs:ce, p, q), each arm list(n_pcs,
+ * optimal_n_clusters, seqdist, scores, keep (1-based), bad_columns (NULL when empty)); any other item as batch_item gives
+ * it; unprotected */
 static SEXP arms_item(tp_batch *b, int i) {
     int split = -1, cs = 0, ce = 0, nn = 0;
     tp_batch_split(b, i, &split, &cs, &ce, NULL);
     if (tp_batch_status(b, i) != TP_OK || split != 1) return batch_item(b, i);
-    tp_batch_dims(b, i, &nn, NULL, NULL, NULL, NULL, NULL);
+    tp_batch_dims(b, i, -1, &nn, NULL, NULL, NULL, NULL, NULL, NULL, NULL);
     SEXP item = PROTECT(allocVector(VECSXP, 4));
     SEXP bad = allocVector(LGLSXP, nn);
     SET_VECTOR_ELT(item, 0, bad);
@@ -401,7 +375,7 @@ static SEXP arms_item(tp_batch *b, int i) {
     for (int j = cs; j <= ce; j++) INTEGER(cen)[j - cs] = j;
     for (int a = 0; a < 2; a++) {
         int nk, nf, k, maxlev, nbad, npcs = 0, ncl = 0;
-        tp_batch_arm_dims(b, i, a, &nk, &nf, &k, &maxlev, NULL, NULL, &nbad);
+        tp_batch_dims(b, i, a, NULL, &nf, &k, &maxlev, NULL, NULL, &nk, &nbad);
         SEXP arm = PROTECT(allocVector(VECSXP, 6));
         SET_VECTOR_ELT(item, 2 + a, arm);
         UNPROTECT(1);
@@ -409,7 +383,7 @@ static SEXP arms_item(tp_batch *b, int i) {
         SET_VECTOR_ELT(arm, 2, seq);
         int *keep = (int *)R_alloc((size_t)nk + 1, sizeof(int)), *bc = (int *)R_alloc((size_t)(nbad > 0 ? nbad : 0) + 1, sizeof(int));
         double *sc = (double *)R_alloc((size_t)k * maxlev + 1, sizeof(double));
-        tp_batch_arm_get(b, i, a, keep, bc, &npcs, &ncl, sc, REAL(seq), NULL, NULL, NULL, NULL, NULL);
+        tp_batch_get(b, i, a, NULL, &npcs, &ncl, sc, REAL(seq), NULL, NULL, NULL, NULL, NULL, keep, bc, NULL);
         SET_VECTOR_ELT(arm, 0, ScalarInteger(npcs));
         SET_VECTOR_ELT(arm, 1, ScalarInteger(ncl));
         SET_VECTOR_ELT(arm, 3, score_matrix(sc, k, maxlev));
@@ -420,10 +394,10 @@ static SEXP arms_item(tp_batch *b, int i) {
     return item;
 }
 
-/* TADpole(centromere_search = TRUE) on a list of matrices (tp_call_batch_arms): every matrix is split at its centromere
- * and both arms run in the library's workers.  Per matrix: arms_item, or a character error message (a matrix that does
- * not split fails, as the reference's TADpole() does). */
-SEXP C_tp_call_batch_arms(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight) {
+/* TADpole() on a list of matrices, `inflight` calls per device kept in flight by the library's own threads over every
+ * device of the context (tp_call_batch with `centromere`); this thread only waits.  Per matrix: arms_item, or a character
+ * error message. */
+static SEXP call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight, int centromere) {
     tp_ctx *c = ctx_of(ctx);
     int nc = length(mats);
     const double **ptr = (const double **)R_alloc((size_t)(nc ? nc : 1), sizeof(double *));
@@ -435,14 +409,27 @@ SEXP C_tp_call_batch_arms(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, 
         n[i] = nrows(m);
     }
     tp_batch *b = NULL;
-    if (tp_call_batch_arms(c, nc, ptr, n, 1, 0, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac), 0,
-                           asInteger(inflight), &b) != TP_OK)
+    if (tp_call_batch(c, nc, ptr, n, 1, 0, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac), asInteger(inflight),
+                      1, centromere, &b) != TP_OK)
         error("%s", tp_last_error());
+    /* (an R allocation failure below longjmps past tp_batch_free: the batch, plain host memory, is then leaked) */
     SEXP out = PROTECT(allocVector(VECSXP, nc));
     for (int i = 0; i < nc; i++) SET_VECTOR_ELT(out, i, arms_item(b, i));
     tp_batch_free(b);
     UNPROTECT(1);
     return out;
+}
+
+/* Per matrix: list(bad, n_pcs, optimal_n_clusters, seqdist, scores, levels, tables = list of 2-column (start, end)
+ * matrices), or a character error message. */
+SEXP C_tp_call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight) {
+    return call_batch(ctx, mats, max_pcs, min_clusters, bad_frac, inflight, 0);
+}
+
+/* TADpole(centromere_search = TRUE) on a list of matrices: every matrix is split at its centromere and both arms run in
+ * the library's workers (a matrix that does not split fails, as the reference's TADpole() does). */
+SEXP C_tp_call_batch_arms(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight) {
+    return call_batch(ctx, mats, max_pcs, min_clusters, bad_frac, inflight, 1);
 }
 
 static void genome_finalizer(SEXP p) {
@@ -500,10 +487,9 @@ SEXP C_tp_genome_file(SEXP ctx, SEXP chrom_bins, SEXP path, SEXP index_base) {
 }
 
 /* TADpole() on the chromosomes `chroms` (0-based) of a C_tp_genome handle, `inflight` calls per device in flight
- * (tp_call_genome).  Per chromosome, in chroms order: what C_tp_call_batch gives for its dense matrix (the per-level
- * tables empty unless `tables`), or a character error message. */
-SEXP C_tp_call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
-                      SEXP tables) {
+ * (tp_call_genome with `centromere`).  Per chromosome, in chroms order: arms_item, or a character error message. */
+static SEXP call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
+                        int tables, int centromere) {
     tp_ctx *c = ctx_of(ctx);
     tp_genome *g = (tp_genome *)R_ExternalPtrAddr(genome);
     if (!g) error("TADpole: the genome pixels have been released");
@@ -511,34 +497,26 @@ SEXP C_tp_call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min
     int ns = length(chroms);
     tp_batch *b = NULL;
     if (tp_call_genome(c, g, INTEGER(chroms), ns, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac),
-                       asInteger(inflight), asLogical(tables), &b) != TP_OK)
-        error("%s", tp_last_error());
-    SEXP out = PROTECT(allocVector(VECSXP, ns));
-    for (int i = 0; i < ns; i++) SET_VECTOR_ELT(out, i, batch_item(b, i));
-    tp_batch_free(b);
-    UNPROTECT(1);
-    return out;
-}
-
-/* TADpole(centromere_search = TRUE) on the chromosomes `chroms` of a C_tp_genome handle (tp_call_genome_arms).  Per
- * chromosome, in chroms order: arms_item, or a character error message.  fix: centromere_fix of the Python host (the
- * repair of quirks Q3 and Q4); R's TADpole() has no such flag and passes FALSE. */
-SEXP C_tp_call_genome_arms(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
-                           SEXP fix) {
-    tp_ctx *c = ctx_of(ctx);
-    tp_genome *g = (tp_genome *)R_ExternalPtrAddr(genome);
-    if (!g) error("TADpole: the genome pixels have been released");
-    if (!isInteger(chroms)) error("TADpole: chromosome indices must be integers");
-    int ns = length(chroms);
-    tp_batch *b = NULL;
-    if (tp_call_genome_arms(c, g, INTEGER(chroms), ns, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac),
-                            asLogical(fix), asInteger(inflight), &b) != TP_OK)
+                       asInteger(inflight), tables, centromere, &b) != TP_OK)
         error("%s", tp_last_error());
     SEXP out = PROTECT(allocVector(VECSXP, ns));
     for (int i = 0; i < ns; i++) SET_VECTOR_ELT(out, i, arms_item(b, i));
     tp_batch_free(b);
     UNPROTECT(1);
     return out;
+}
+
+/* Per chromosome: what C_tp_call_batch gives for its dense matrix (the per-level tables empty unless `tables`). */
+SEXP C_tp_call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
+                      SEXP tables) {
+    return call_genome(ctx, genome, chroms, max_pcs, min_clusters, bad_frac, inflight, asLogical(tables), 0);
+}
+
+/* TADpole(centromere_search = TRUE) on each chromosome.  fix: centromere_fix of the Python host (the repair of quirks Q3
+ * and Q4); R's TADpole() has no such flag and passes FALSE. */
+SEXP C_tp_call_genome_arms(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
+                           SEXP fix) {
+    return call_genome(ctx, genome, chroms, max_pcs, min_clusters, bad_frac, inflight, 1, asLogical(fix) ? 2 : 1);
 }
 
 /* the cutree / fix_values / rle loop of R/TADpole.R:470-497 for many levels at once: list of 2-column integer

@@ -30,7 +30,7 @@ EXPORTED = [
     "tp_ctx_create_multi", "tp_device_count", "tp_ctx_devices", "tp_ctx_generation", "tp_ctx_dims", "tp_call_arms", "tp_call_batch",
     "tp_batch_size", "tp_batch_device_ms", "tp_batch_launches", "tp_batch_status", "tp_batch_error", "tp_batch_dims", "tp_batch_get", "tp_batch_free", "tp_find_groups",
     "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
-    "tp_centromere_split", "tp_call_batch_arms", "tp_call_genome_arms", "tp_batch_split", "tp_batch_arm_dims", "tp_batch_arm_get",
+    "tp_centromere_split", "tp_batch_split",
 ]
 
 
@@ -64,26 +64,23 @@ def load():
         "tp_ctx_generation": (c_longlong, [vp]),
         "tp_ctx_dims": (c_int, [vp, ip, ip, ip, ip, ip]),
         "tp_call_arms": (c_int, [vp, ip, c_int, ip, c_int, c_int, c_int, POINTER(vp)]),
-        "tp_call_batch": (c_int, [vp, c_int, POINTER(vp), ip, c_int, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
+        "tp_call_batch": (c_int, [vp, c_int, POINTER(vp), ip, c_int, c_int, c_int, c_int, c_double, c_int, c_int, c_int,
+                                  POINTER(vp)]),
         "tp_batch_size": (c_int, [vp]),
         "tp_batch_device_ms": (c_double, [vp]),
         "tp_batch_launches": (c_longlong, [vp]),
         "tp_batch_status": (c_int, [vp, c_int]),
         "tp_batch_error": (c_char_p, [vp, c_int]),
-        "tp_batch_dims": (c_int, [vp, c_int, ip, ip, ip, ip, ip, ip]),
-        "tp_batch_get": (c_int, [vp, c_int, u8p, ip, ip, dp, dp, ip, ip, ip, ip, dp]),
+        "tp_batch_dims": (c_int, [vp, c_int, c_int, ip, ip, ip, ip, ip, ip, ip, ip]),
+        "tp_batch_get": (c_int, [vp, c_int, c_int, u8p, ip, ip, dp, dp, ip, ip, ip, ip, dp, ip, ip, ip]),
         "tp_batch_free": (c_int, [vp]),
-        "tp_call_batch_arms": (c_int, [vp, c_int, POINTER(vp), ip, c_int, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
-        "tp_call_genome_arms": (c_int, [vp, vp, ip, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
         "tp_batch_split": (c_int, [vp, c_int, ip, ip, ip, u8p]),
-        "tp_batch_arm_dims": (c_int, [vp, c_int, c_int, ip, ip, ip, ip, ip, ip, ip]),
-        "tp_batch_arm_get": (c_int, [vp, c_int, c_int, ip, ip, ip, ip, dp, dp, ip, ip, ip, ip, ip]),
         "tp_centromere_split": (c_int, [u8p, c_int, c_int, ip, ip, ip, ip, ip, ip, ip, ip, ip, ip, ip]),
         "tp_genome_ingest": (c_int, [vp, ip, c_int, ip, ip, dp, ctypes.c_size_t, c_int, POINTER(vp)]),
         "tp_genome_ingest_file": (c_int, [vp, ip, c_int, c_char_p, c_int, c_int, POINTER(vp)]),
         "tp_genome_stats": (c_int, [vp, POINTER(ctypes.c_ulonglong), POINTER(ctypes.c_ulonglong), POINTER(ctypes.c_ulonglong)]),
         "tp_genome_matrix": (c_int, [vp, vp, c_int, dp]),
-        "tp_call_genome": (c_int, [vp, vp, ip, c_int, c_int, c_int, c_double, c_int, c_int, POINTER(vp)]),
+        "tp_call_genome": (c_int, [vp, vp, ip, c_int, c_int, c_int, c_double, c_int, c_int, c_int, POINTER(vp)]),
         "tp_genome_free": (c_int, [vp]),
         "tp_find_groups": (c_int, [dp, c_int, ip]),
         "tp_ctx_destroy": (c_int, [vp]),
@@ -169,6 +166,12 @@ def _dp(a):
 
 def _ip(a):
     return a.ctypes.data_as(POINTER(c_int))
+
+
+def _centromere(search, fix):
+    """The `centromere` argument of tp_call_batch / tp_call_genome: 0 whole matrices, 1 centromere_search, 2 with
+    centromere_fix."""
+    return (2 if fix else 1) if search else 0
 
 
 class Context:
@@ -492,21 +495,28 @@ class Context:
             self.lib.tp_batch_free(h)
         return tuple({key: it[key] for key in ("nf", "k", "n_pcs", "n_clusters", "scores", "seqdist")} for it in items)
 
-    def _batch_item(self, h, i, tables):
-        """Item i of a tp_batch as the dict call() returns, plus 'tables' {level: [rows, 2]} (or None) and 'device_ms'."""
-        d = [c_int(0) for _ in range(6)]
-        check(self.lib.tp_batch_dims(h, i, *[ctypes.byref(x) for x in d]))
-        nn, nf, k, ml, nlev, nrows = (x.value for x in d)
+    def _batch_item(self, h, i, tables, part=-1):
+        """Item i of a tp_batch as the dict call() returns, plus 'tables' {level: [rows, 2]} (or None) and 'device_ms'.
+        part 0 / 1: the p / q arm of split item i instead, with 'tables', 'keep' (0-based), 'bad_columns' (original 1-based,
+        or None) and 'labels' (fixed labels of the optimal level) in place of 'bad' and 'device_ms'."""
+        d = [c_int(0) for _ in range(8)]
+        check(self.lib.tp_batch_dims(h, i, part, *[ctypes.byref(x) for x in d]))
+        nn, nf, k, ml, nlev, nrows, nk, nbad = (x.value for x in d)
         bad = np.zeros(nn, np.uint8); sc = np.empty((k, ml)); seq = np.empty(nf - 1)
         lev = np.zeros(nlev, np.int32); off = np.zeros(nlev + 1, np.int32)
         st = np.zeros(nrows, np.int32); en = np.zeros(nrows, np.int32)
+        keep = np.zeros(nk, np.int32); badc = np.zeros(max(nbad, 0), np.int32)
+        lab = np.zeros(nf + max(nbad, 0) if part >= 0 else 0, np.int32)
         npcs, ncl, ms = c_int(0), c_int(0), c_double(0.0)
-        check(self.lib.tp_batch_get(h, i, bad.ctypes.data_as(POINTER(c_uint8)), ctypes.byref(npcs), ctypes.byref(ncl),
-                                    _dp(sc), _dp(seq), _ip(lev), _ip(off), _ip(st), _ip(en), ctypes.byref(ms)))
+        check(self.lib.tp_batch_get(h, i, part, bad.ctypes.data_as(POINTER(c_uint8)), ctypes.byref(npcs), ctypes.byref(ncl),
+                                    _dp(sc), _dp(seq), _ip(lev), _ip(off), _ip(st), _ip(en), ctypes.byref(ms), _ip(keep),
+                                    _ip(badc), _ip(lab)))
         tab = np.stack([st, en], axis=1).astype(np.int64)
-        return dict(bad=bad.astype(bool), nf=nf, k=k, n_pcs=npcs.value, n_clusters=ncl.value, scores=sc, seqdist=seq,
-                    tables={int(l): tab[off[j]: off[j + 1]] for j, l in enumerate(lev)} if tables else None,
-                    device_ms=ms.value)
+        item = dict(nf=nf, k=k, n_pcs=npcs.value, n_clusters=ncl.value, scores=sc, seqdist=seq,
+                    tables={int(l): tab[off[j]: off[j + 1]] for j, l in enumerate(lev)} if tables else None)
+        if part >= 0:
+            return dict(keep=keep, bad_columns=badc if nbad >= 0 else None, **item, labels=lab)
+        return dict(bad=bad.astype(bool), **item, device_ms=ms.value)
 
     def call_batch(self, mats, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True, device_ptrs=None, n=None,
                    centromere_search=False, centromere_fix=False):
@@ -514,8 +524,9 @@ class Context:
         every device of the context.  mats: list of square float64 arrays (all C or all F order); or device_ptrs + n
         (row-major, single-device contexts).  Returns a list of dicts as call() returns, plus 'tables' {level: [rows, 2]}
         and 'device_ms'; a failed call's entry is the TadpoleError.
-        centromere_search: tp_call_batch_arms, each matrix split at its centromere and its two arms called in the same
-        workers; a split matrix's entry is the dict of _split_item, an unsplit one's (centromere_fix) the dict above, and
+        centromere_search: each matrix split at its centromere and its two arms called in the same workers, tables always
+        built; a split matrix's entry is dict(split=True, centromere (1-based bins), bad, device_ms, p, q) with p / q as
+        _batch_item reads an arm, an unsplit one's (centromere_fix) the dict above plus split=False and centromere, and
         one that does not split without centromere_fix fails with TP_ERR_NOSPLIT."""
         if device_ptrs is None:
             mats = [m if (m.dtype == np.float64 and (m.flags.c_contiguous or m.flags.f_contiguous))
@@ -532,12 +543,10 @@ class Context:
             colmajor, ondev = 0, 1
         ncalls = int(ns.size)
         h = c_void_p()
-        if centromere_search:
-            check(self.lib.tp_call_batch_arms(self._h, ncalls, ptrs, _ip(ns), colmajor, ondev, int(max_pcs), int(min_clusters),
-                                              float(bad_frac), int(bool(centromere_fix)), int(inflight), ctypes.byref(h)))
-            return self._batch_results(h, ncalls, True)
+        tables = bool(tables or centromere_search)
         check(self.lib.tp_call_batch(self._h, ncalls, ptrs, _ip(ns), colmajor, ondev, int(max_pcs), int(min_clusters),
-                                     float(bad_frac), int(inflight), int(bool(tables)), ctypes.byref(h)))
+                                     float(bad_frac), int(inflight), int(tables), _centromere(centromere_search, centromere_fix),
+                                     ctypes.byref(h)))
         return self._batch_results(h, ncalls, tables)
 
     def _split_state(self, h, i, n):
@@ -549,32 +558,6 @@ class Context:
                                       bad.ctypes.data_as(POINTER(c_uint8))))
         return (sp.value, np.arange(cs.value, ce.value + 1) if cs.value else None,
                 bad[:n].astype(bool) if sp.value >= 0 else None)
-
-    def _arm_item(self, h, i, arm):
-        """Arm `arm` (0 = p, 1 = q) of split item i: dict(keep (0-based), bad_columns (original 1-based, or None), nf, k,
-        n_pcs, n_clusters, scores, seqdist, tables {level: [rows, 2]}, labels (fixed labels of the optimal level))."""
-        d = [c_int(0) for _ in range(7)]
-        check(self.lib.tp_batch_arm_dims(h, i, arm, *[ctypes.byref(x) for x in d]))
-        nk, nf, k, ml, nlev, nrows, nbad = (x.value for x in d)
-        keep = np.zeros(nk, np.int32); bad = np.zeros(max(nbad, 0), np.int32)
-        sc = np.empty((k, ml)); seq = np.empty(nf - 1)
-        lev = np.zeros(nlev, np.int32); off = np.zeros(nlev + 1, np.int32)
-        st = np.zeros(nrows, np.int32); en = np.zeros(nrows, np.int32)
-        lab = np.zeros(nf + max(nbad, 0), np.int32)
-        npcs, ncl = c_int(0), c_int(0)
-        check(self.lib.tp_batch_arm_get(h, i, arm, _ip(keep), _ip(bad), ctypes.byref(npcs), ctypes.byref(ncl), _dp(sc),
-                                        _dp(seq), _ip(lev), _ip(off), _ip(st), _ip(en), _ip(lab)))
-        tab = np.stack([st, en], axis=1).astype(np.int64)
-        return dict(keep=keep, bad_columns=bad if nbad >= 0 else None, nf=nf, k=k, n_pcs=npcs.value, n_clusters=ncl.value,
-                    scores=sc, seqdist=seq, tables={int(l): tab[off[j]: off[j + 1]] for j, l in enumerate(lev)}, labels=lab)
-
-    def _split_item(self, h, i, n, centromere):
-        """A split item: dict(split=True, centromere (1-based bins cs..ce), bad, device_ms, p, q) with p / q as _arm_item."""
-        ms = c_double(0.0)
-        check(self.lib.tp_batch_get(h, i, None, None, None, None, None, None, None, None, None, ctypes.byref(ms)))
-        _, _, bad = self._split_state(h, i, n)
-        return dict(split=True, centromere=centromere, bad=bad, device_ms=ms.value, p=self._arm_item(h, i, 0),
-                    q=self._arm_item(h, i, 1))
 
     def _batch_results(self, h, ncalls, tables):
         """Every item of a tp_batch (freed here) as call_batch returns them."""
@@ -589,15 +572,19 @@ class Context:
                     # a centromere_search item that failed after its filter: split (-1 = not reached), the longest bad
                     # stretch and the bad flags, for load_mat's messages
                     nn = c_int(0)
-                    check(self.lib.tp_batch_dims(h, i, ctypes.byref(nn), None, None, None, None, None))
+                    check(self.lib.tp_batch_dims(h, i, -1, ctypes.byref(nn), None, None, None, None, None, None, None))
                     err.split, err.centromere, err.bad = self._split_state(h, i, nn.value)
                     out.append(err)
                     continue
                 nn = c_int(0)
-                check(self.lib.tp_batch_dims(h, i, ctypes.byref(nn), None, None, None, None, None))
-                split, cen, _ = self._split_state(h, i, nn.value)
-                if split == 1:
-                    out.append(self._split_item(h, i, nn.value, cen))
+                check(self.lib.tp_batch_dims(h, i, -1, ctypes.byref(nn), None, None, None, None, None, None, None))
+                split, cen, bad = self._split_state(h, i, nn.value)
+                if split == 1:                       # centromere_search, split: the item's bad flags and device time, the arms
+                    ms = c_double(0.0)
+                    check(self.lib.tp_batch_get(h, i, -1, None, None, None, None, None, None, None, None, None,
+                                                ctypes.byref(ms), None, None, None))
+                    out.append(dict(split=True, centromere=cen, bad=bad, device_ms=ms.value,
+                                    p=self._batch_item(h, i, True, 0), q=self._batch_item(h, i, True, 1)))
                     continue
                 item = self._batch_item(h, i, tables)
                 if split == 0:                       # centromere_search, not split: processed whole (centromere_fix)
@@ -629,16 +616,13 @@ class Context:
     def call_genome(self, genome, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True,
                     centromere_search=False, centromere_fix=False):
         """tp_call_genome: one call per selected chromosome (0-based indices, default all), results in that order as
-        call_batch returns them (a failed call's entry is the TadpoleError); centromere_search: tp_call_genome_arms, the
-        entries as call_batch(centromere_search=True) gives them."""
+        call_batch returns them (a failed call's entry is the TadpoleError), with centromere_search too."""
         sel = np.arange(genome.chrom_bins.size, dtype=np.int32) if chroms is None else np.ascontiguousarray(chroms, dtype=np.int32)
         h = c_void_p()
-        if centromere_search:
-            check(self.lib.tp_call_genome_arms(self._h, genome._h, _ip(sel), int(sel.size), int(max_pcs), int(min_clusters),
-                                               float(bad_frac), int(bool(centromere_fix)), int(inflight), ctypes.byref(h)))
-            return self._batch_results(h, int(sel.size), True)
+        tables = bool(tables or centromere_search)
         check(self.lib.tp_call_genome(self._h, genome._h, _ip(sel), int(sel.size), int(max_pcs), int(min_clusters),
-                                      float(bad_frac), int(inflight), int(bool(tables)), ctypes.byref(h)))
+                                      float(bad_frac), int(inflight), int(tables), _centromere(centromere_search, centromere_fix),
+                                      ctypes.byref(h)))
         return self._batch_results(h, int(sel.size), tables)
 
     def recall(self, nf, max_pcs=200, min_clusters=2):

@@ -19,7 +19,7 @@ void tp_set_error(const char *fmt, ...) {
 }
 
 extern "C" const char *tp_last_error(void) { return g_err; }
-extern "C" int tp_version(void) { return 103; }
+extern "C" int tp_version(void) { return 104; }
 
 int tp_pin_reserve(tp_ctx *ctx, size_t bytes) {
     if (bytes <= ctx->pin_cap) return TP_OK;

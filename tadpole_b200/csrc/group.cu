@@ -7,8 +7,9 @@
 //     torchrun job runs with one process per GPU -- same kernels, same collectives, same bits.
 //   * chromosome arms on disjoint halves of the devices at the same time (tp_call_arms, R/TADpole.R:357-374).
 //   * batches of independent calls kept in flight by library-owned threads (tp_call_batch): genome-wide use loops over
-//     chromosomes, and one 2000-bin call leaves most of a B200 idle.  With centromere_search (tp_call_batch_arms,
-//     tp_call_genome_arms) each worker splits its matrix at the centromere and runs both arms one after the other.
+//     chromosomes, and one 2000-bin call leaves most of a B200 idle.  With centromere_search (the `centromere` argument
+//     of tp_call_batch and tp_call_genome) each worker splits its matrix at the centromere and runs both arms one after
+//     the other.
 //   * small host-side pieces the R wrapper would otherwise do in interpreted loops: the hclust merge matrix of a
 //     chclust dendrogram (rioja's .find.groups rule) in O(n log n), and load_mat's centromere split (tp_centromere_split).
 //
@@ -267,7 +268,7 @@ struct TpBatchItem {
     std::vector<int> levels, offsets, start, end; // per-level start / end tables (R/TADpole.R:470-497)
     double device_ms = 0.0;
     long long launches = 0;
-    // centromere_search items (tp_call_batch_arms, tp_call_genome_arms): split = -1 until the bad flags are known, then
+    // centromere_search items (centromere != 0): split = -1 until the bad flags are known, then
     // 0 (processed whole or failed) or 1 (arms[0] = p, arms[1] = q); cs..ce = the longest bad run (1-based, 0 = none)
     int split = -1, cs = 0, ce = 0;
     std::vector<TpBatchItem> arms;
@@ -307,25 +308,13 @@ static int level_tables(TpBatchItem &it, const int *names, const int *bad, int n
     return TP_OK;
 }
 
-// names and bad columns of a whole matrix from its bad flags, as TADpole() packs it
-static void whole_lists(const TpBatchItem &it, std::vector<int> &names, std::vector<int> &bad) {
-    for (int i = 0; i < it.n; i++) (it.bad[(size_t)i] ? bad : names).push_back(i + 1);
-}
-
-static int batch_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_device, int max_pcs, int min_clusters,
-                     double bad_frac, int want_tables, TpBatchItem &it) {
-    it.n = n;
-    const long long launches0 = c->launches;
-    struct Count { TpBatchItem &it; tp_ctx *c; long long l0; ~Count() { it.launches = c->launches - l0; } } count{it, c, launches0};
-    it.bad.assign((size_t)n, 0);
-    TP_ARG(max_pcs >= 1, "tp_call_batch: max_pcs must be positive");
-    it.seqdist.assign((size_t)(n > 1 ? n - 1 : 1), 0.0);
-    TP_TRY(tp_call(c, mat, n, colmajor, on_device, max_pcs, min_clusters, bad_frac, it.bad.data(), &it.nf, nullptr, &it.n_pcs,
-                   &it.n_clusters, nullptr, it.seqdist.data()));
+// The result tail of a matrix called whole: finish_item, then (tables) the start / end table of every scored level, with
+// the names and bad columns TADpole() packs from the bad flags.
+static int finish_whole(tp_ctx *c, TpBatchItem &it, bool tables) {
     finish_item(c, it);
-    if (!want_tables) return TP_OK;
+    if (!tables) return TP_OK;
     std::vector<int> names, bad;
-    whole_lists(it, names, bad);
+    for (int i = 0; i < it.n; i++) (it.bad[(size_t)i] ? bad : names).push_back(i + 1);
     return level_tables(it, names.data(), bad.data(), (int)bad.size());
 }
 
@@ -351,16 +340,31 @@ static int arm_one(tp_ctx *c, int max_pcs, int min_clusters, TpBatchItem &a) {
 static const char *const NOSPLIT_MSG = "centromere_search=TRUE but load_mat did not split the matrix (no bad columns, or the "
                                        "longest bad stretch touches an end); the reference errors here";
 
-// TADpole(centromere_search = TRUE) on one matrix (R/TADpole.R:351-442): filter, split at the longest bad stretch, then the
-// p arm and the q arm one after the other on c.  Unsplit: TP_ERR_NOSPLIT (the reference errors, quirk Q4), or with fix the
-// whole matrix's good bins as TADpole(centromere_fix = TRUE) does.  device_ms covers the filter and both arms.
-static int arms_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_device, int max_pcs, int min_clusters,
-                    double bad_frac, int fix, TpBatchItem &it) {
+// What every item of a batch call is run with.  centromere: 0 = TADpole(), 1 = centromere_search, 2 = centromere_search
+// with centromere_fix.
+struct ItemArgs {
+    int max_pcs, min_clusters;
+    double bad_frac;
+    int want_tables, centromere;
+};
+
+// One matrix of a batch on c.  centromere = 0: tp_call, then its outputs and (want_tables) its tables.  Otherwise
+// TADpole(centromere_search = TRUE) on one matrix (R/TADpole.R:351-442): filter, split at the longest bad stretch, then
+// the p arm and the q arm one after the other on c, tables always built.  Unsplit: TP_ERR_NOSPLIT (the reference errors,
+// quirk Q4), or with centromere_fix the whole matrix's good bins as TADpole(centromere_fix = TRUE) does.  device_ms of
+// a centromere_search item covers the filter and both arms.
+static int item_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_device, const ItemArgs &a, TpBatchItem &it) {
     it.n = n;
     const long long launches0 = c->launches;
     struct Count { TpBatchItem &it; tp_ctx *c; long long l0; ~Count() { it.launches = c->launches - l0; } } count{it, c, launches0};
     it.bad.assign((size_t)n, 0);
-    TP_ARG(max_pcs >= 1, "tp_call_batch_arms: max_pcs must be positive");
+    TP_ARG(a.max_pcs >= 1, "tp_call_batch: max_pcs must be positive");
+    if (!a.centromere) {
+        it.seqdist.assign((size_t)(n > 1 ? n - 1 : 1), 0.0);
+        TP_TRY(tp_call(c, mat, n, colmajor, on_device, a.max_pcs, a.min_clusters, a.bad_frac, it.bad.data(), &it.nf, nullptr,
+                       &it.n_pcs, &it.n_clusters, nullptr, it.seqdist.data()));
+        return finish_whole(c, it, a.want_tables);
+    }
     struct Events {
         cudaEvent_t e[2] = {nullptr, nullptr};
         ~Events() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
@@ -370,13 +374,13 @@ static int arms_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_de
     TP_CUDA(cudaEventCreate(&ev.e[1]));
     TP_CUDA(cudaEventRecord(ev.e[0], c->stream));
     // tp_call calls the hook itself; here the worker runs tp_filter directly, and the hook releases the first-upload lock
-    const int frc = tp_filter(c, mat, n, colmajor, on_device, bad_frac, it.bad.data(), nullptr, nullptr);
+    const int frc = tp_filter(c, mat, n, colmajor, on_device, a.bad_frac, it.bad.data(), nullptr, nullptr);
     if (c->after_filter) c->after_filter();
     TP_TRY(frc);
     std::vector<int> kp((size_t)n), bp((size_t)n), kq((size_t)n), bq((size_t)n);
     int split = 0, nkp = 0, nbp = 0, nkq = 0, nbq = 0;
-    TP_TRY(tp_centromere_split(it.bad.data(), n, fix, &split, &it.cs, &it.ce, kp.data(), &nkp, bp.data(), &nbp, kq.data(), &nkq,
-                               bq.data(), &nbq));
+    TP_TRY(tp_centromere_split(it.bad.data(), n, a.centromere == 2, &split, &it.cs, &it.ce, kp.data(), &nkp, bp.data(), &nbp,
+                               kq.data(), &nkq, bq.data(), &nbq));
     it.split = split;
     if (split) {
         // The p arm's after_pca hook may stage the next matrix while the q arm still has to compact from this one.  The
@@ -391,18 +395,16 @@ static int arms_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_de
         it.arms[1].nbad = nbq;
         if (nbp > 0) it.arms[0].badcols.assign(bp.begin(), bp.begin() + nbp);
         if (nbq > 0) it.arms[1].badcols.assign(bq.begin(), bq.begin() + nbq);
-        for (TpBatchItem &a : it.arms) TP_TRY(arm_one(c, max_pcs, min_clusters, a));
+        for (TpBatchItem &arm : it.arms) TP_TRY(arm_one(c, a.max_pcs, a.min_clusters, arm));
     } else {
-        if (!fix) { tp_set_error("%s", NOSPLIT_MSG); return TP_ERR_NOSPLIT; }
-        std::vector<int> names, bad, keep;
-        whole_lists(it, names, bad);
-        for (int v : names) keep.push_back(v - 1);
+        if (a.centromere != 2) { tp_set_error("%s", NOSPLIT_MSG); return TP_ERR_NOSPLIT; }
+        std::vector<int> keep;
+        for (int i = 0; i < n; i++) if (!it.bad[(size_t)i]) keep.push_back(i);
         it.nf = (int)keep.size();
         it.seqdist.assign((size_t)(it.nf > 1 ? it.nf - 1 : 1), 0.0);
-        TP_TRY(tp_call_arm(c, keep.data(), it.nf, max_pcs, min_clusters, nullptr, &it.n_pcs, &it.n_clusters, nullptr,
+        TP_TRY(tp_call_arm(c, keep.data(), it.nf, a.max_pcs, a.min_clusters, nullptr, &it.n_pcs, &it.n_clusters, nullptr,
                            it.seqdist.data()));
-        finish_item(c, it);
-        TP_TRY(level_tables(it, names.data(), bad.data(), (int)bad.size()));
+        TP_TRY(finish_whole(c, it, true));
     }
     TP_CUDA(cudaEventRecord(ev.e[1], c->stream));
     TP_CUDA(cudaEventSynchronize(ev.e[1]));
@@ -579,52 +581,39 @@ static int batch_run(tp_ctx *ctx, int ncalls, double need, int inflight, bool ho
 }
 
 extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
-                             int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, tp_batch **out) {
-    TP_ARG(ctx && mats && n && out && ncalls >= 0, "tp_call_batch: bad arguments");
+                             int max_pcs, int min_clusters, double bad_frac, int inflight, int want_tables, int centromere,
+                             tp_batch **out) {
+    TP_ARG(ctx && mats && n && out && ncalls >= 0 && centromere >= 0 && centromere <= 2, "tp_call_batch: bad arguments");
     TP_ARG(!(on_device && ctx->group), "tp_call_batch: device-resident inputs need a single-device context");
     // every call in flight holds its own working set in HBM (raw + filtered + correlation + M + digit planes + second
-    // input buffer + blocks: ~56 bytes per matrix element, 35 GB at 25k bins)
+    // input buffer + blocks: ~56 bytes per matrix element, 35 GB at 25k bins); an arm is smaller than its chromosome
     size_t nmax = 0;
     for (int i = 0; i < ncalls; i++) nmax = std::max(nmax, (size_t)(n[i] > 0 ? n[i] : 0));
     const double need = 56.0 * (double)nmax * (double)nmax + 64e6;
     auto stage = [&](tp_ctx *c, int j) {
         if (mats[j] && n[j] >= 2) (void)tp_stage_input(c, mats[j], n[j], colmajor);    // a failure leaves the normal upload
     };
+    const ItemArgs args{max_pcs, min_clusters, bad_frac, want_tables, centromere};
     auto one = [&](tp_ctx *c, int i, TpBatchItem &it) -> int {
-        return mats[i] ? batch_one(c, mats[i], n[i], colmajor, on_device, max_pcs, min_clusters, bad_frac, want_tables, it)
+        return mats[i] ? item_one(c, mats[i], n[i], colmajor, on_device, args, it)
                        : (tp_set_error("tp_call_batch: matrix %d is null", i), (int)TP_ERR_ARG);
     };
     return batch_run(ctx, ncalls, need, inflight, !on_device, nullptr, stage, one, out);
 }
 
-extern "C" int tp_call_batch_arms(tp_ctx *ctx, int ncalls, const double *const *mats, const int *n, int colmajor, int on_device,
-                                  int max_pcs, int min_clusters, double bad_frac, int centromere_fix, int inflight, tp_batch **out) {
-    TP_ARG(ctx && mats && n && out && ncalls >= 0, "tp_call_batch_arms: bad arguments");
-    TP_ARG(!(on_device && ctx->group), "tp_call_batch_arms: device-resident inputs need a single-device context");
-    // the working set of a whole-matrix call: an arm is smaller than its chromosome
-    size_t nmax = 0;
-    for (int i = 0; i < ncalls; i++) nmax = std::max(nmax, (size_t)(n[i] > 0 ? n[i] : 0));
-    const double need = 56.0 * (double)nmax * (double)nmax + 64e6;
-    auto stage = [&](tp_ctx *c, int j) {
-        if (mats[j] && n[j] >= 2) (void)tp_stage_input(c, mats[j], n[j], colmajor);    // a failure leaves the normal upload
-    };
-    auto one = [&](tp_ctx *c, int i, TpBatchItem &it) -> int {
-        return mats[i] ? arms_one(c, mats[i], n[i], colmajor, on_device, max_pcs, min_clusters, bad_frac, centromere_fix, it)
-                       : (tp_set_error("tp_call_batch_arms: matrix %d is null", i), (int)TP_ERR_ARG);
-    };
-    return batch_run(ctx, ncalls, need, inflight, !on_device, nullptr, stage, one, out);
-}
-
 // ---- genome-wide calls: one per chromosome, each dense matrix built from its bucket in HBM (ingest.cu, S0c) ---------
-// The selected chromosomes (checked against the handle), claimed largest first; call(c, mat, n, it) runs one chromosome's
-// dense matrix (device pointer, row-major) on context c.
-static int genome_run(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int inflight, const char *who,
-                      const std::function<int(tp_ctx *, const double *, int, TpBatchItem &)> &call, tp_batch **out) {
+// The selected chromosomes (checked against the handle), claimed largest first; each worker runs one chromosome's dense
+// matrix (device pointer, row-major) on its context.
+extern "C" int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
+                              double bad_frac, int inflight, int want_tables, int centromere, tp_batch **out) {
+    TP_ARG(ctx && g && out && nsel >= 0 && (chroms || nsel == 0 || nsel == (int)g->bins.size()) && centromere >= 0 &&
+           centromere <= 2, "tp_call_genome: bad arguments");
+    TP_ARG(g->device == ctx->device, "tp_call_genome: the handle was ingested on another device than the context's first");
     std::vector<int> sel((size_t)(nsel > 0 ? nsel : 0));
     for (int s = 0; s < nsel; s++) {
         sel[(size_t)s] = chroms ? chroms[s] : s;
         if (sel[(size_t)s] < 0 || sel[(size_t)s] >= (int)g->bins.size()) {
-            tp_set_error("%s: chromosome index %d is outside 0..%d", who, sel[(size_t)s], (int)g->bins.size() - 1);
+            tp_set_error("tp_call_genome: chromosome index %d is outside 0..%d", sel[(size_t)s], (int)g->bins.size() - 1);
             return TP_ERR_ARG;
         }
     }
@@ -640,37 +629,20 @@ static int genome_run(tp_ctx *ctx, const tp_genome *g, const int *chroms, int ns
         pmax = std::max(pmax, (double)(g->offs[(size_t)c + 1] - g->offs[(size_t)c]));
     }
     const double need = 56.0 * nmax * nmax + 16.0 * pmax + 64e6;
+    const ItemArgs args{max_pcs, min_clusters, bad_frac, want_tables, centromere};
     auto one = [&](tp_ctx *c, int s, TpBatchItem &it) -> int {
         const int chrom = sel[(size_t)s], n = g->bins[(size_t)chrom];
         it.n = n;
         if (n < 2) {
             it.bad.assign((size_t)n, 0);
-            tp_set_error("%s: chromosome %d has %d bin; a call needs at least 2", who, chrom, n);
+            tp_set_error("tp_call_genome: chromosome %d has %d bin; a call needs at least 2", chrom, n);
             return TP_ERR_ARG;
         }
         double *mat = nullptr;
         TP_TRY(tp_genome_dense(c, g, chrom, &mat));
-        return call(c, mat, n, it);
+        return item_one(c, mat, n, 0, 1, args, it);
     };
     return batch_run(ctx, nsel, need, inflight, false, order.data(), [](tp_ctx *, int) {}, one, out);
-}
-
-extern "C" int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
-                              double bad_frac, int inflight, int want_tables, tp_batch **out) {
-    TP_ARG(ctx && g && out && nsel >= 0 && (chroms || nsel == 0 || nsel == (int)g->bins.size()), "tp_call_genome: bad arguments");
-    TP_ARG(g->device == ctx->device, "tp_call_genome: the handle was ingested on another device than the context's first");
-    return genome_run(ctx, g, chroms, nsel, inflight, "tp_call_genome", [&](tp_ctx *c, const double *mat, int n, TpBatchItem &it) {
-        return batch_one(c, mat, n, 0, 1, max_pcs, min_clusters, bad_frac, want_tables, it);
-    }, out);
-}
-
-extern "C" int tp_call_genome_arms(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel, int max_pcs, int min_clusters,
-                                   double bad_frac, int centromere_fix, int inflight, tp_batch **out) {
-    TP_ARG(ctx && g && out && nsel >= 0 && (chroms || nsel == 0 || nsel == (int)g->bins.size()), "tp_call_genome_arms: bad arguments");
-    TP_ARG(g->device == ctx->device, "tp_call_genome_arms: the handle was ingested on another device than the context's first");
-    return genome_run(ctx, g, chroms, nsel, inflight, "tp_call_genome_arms", [&](tp_ctx *c, const double *mat, int n, TpBatchItem &it) {
-        return arms_one(c, mat, n, 0, 1, max_pcs, min_clusters, bad_frac, centromere_fix, it);
-    }, out);
 }
 
 extern "C" double tp_batch_device_ms(const tp_batch *b) { return b ? b->device_ms : 0.0; }
@@ -688,42 +660,48 @@ extern "C" const char *tp_batch_error(const tp_batch *b, int i) {
     if (!b || i < 0 || i >= (int)b->items.size()) return "tp_batch_error: index out of range";
     return b->items[(size_t)i].err.c_str();
 }
-// the sizes and the outputs of one finished item (a top-level item or an arm of a split one)
-static void item_dims(const TpBatchItem &it, int *nf_out, int *k_out, int *maxlev_out, int *nlevels_out, int *nrows_out) {
-    if (nf_out) *nf_out = it.nf;
-    if (k_out) *k_out = it.k;
-    if (maxlev_out) *maxlev_out = it.maxlev;
-    if (nlevels_out) *nlevels_out = (int)it.levels.size();
-    if (nrows_out) *nrows_out = (int)it.start.size();
-}
-static void item_get(const TpBatchItem &it, int *n_pcs_out, int *n_clusters_out, double *scores_out, double *seqdist_out,
-                     int *levels_out, int *offsets_out, int *start_out, int *end_out) {
-    if (n_pcs_out) *n_pcs_out = it.n_pcs;
-    if (n_clusters_out) *n_clusters_out = it.n_clusters;
-    if (scores_out) memcpy(scores_out, it.scores.data(), it.scores.size() * sizeof(double));
-    if (seqdist_out) memcpy(seqdist_out, it.seqdist.data(), it.seqdist.size() * sizeof(double));
-    if (levels_out) memcpy(levels_out, it.levels.data(), it.levels.size() * sizeof(int));
-    if (offsets_out) memcpy(offsets_out, it.offsets.data(), it.offsets.size() * sizeof(int));
-    if (start_out) memcpy(start_out, it.start.data(), it.start.size() * sizeof(int));
-    if (end_out) memcpy(end_out, it.end.data(), it.end.size() * sizeof(int));
-}
-extern "C" int tp_batch_dims(const tp_batch *b, int i, int *n_out, int *nf_out, int *k_out, int *maxlev_out, int *nlevels_out,
-                             int *nrows_out) {
-    TP_ARG(b && i >= 0 && i < (int)b->items.size(), "tp_batch_dims: index out of range");
+// item i of a batch (part -1) or arm `part` (0 = p, 1 = q) of split item i; nullptr when there is no such item or arm
+static const TpBatchItem *batch_part(const tp_batch *b, int i, int part) {
+    if (!b || i < 0 || i >= (int)b->items.size() || part < -1 || part > 1) return nullptr;
     const TpBatchItem &it = b->items[(size_t)i];
-    if (n_out) *n_out = it.n;
-    item_dims(it, nf_out, k_out, maxlev_out, nlevels_out, nrows_out);
+    if (part < 0) return &it;
+    return it.rc == TP_OK && it.split == 1 ? &it.arms[(size_t)part] : nullptr;
+}
+extern "C" int tp_batch_dims(const tp_batch *b, int i, int part, int *n_out, int *nf_out, int *k_out, int *maxlev_out,
+                             int *nlevels_out, int *nrows_out, int *nkeep_out, int *nbad_out) {
+    const TpBatchItem *it = batch_part(b, i, part);
+    TP_ARG(it, part < 0 ? "tp_batch_dims: index out of range"
+                          : "tp_batch_dims: no such arm (index out of range, or the item was not split)");
+    if (n_out) *n_out = it->n;
+    if (nf_out) *nf_out = it->nf;
+    if (k_out) *k_out = it->k;
+    if (maxlev_out) *maxlev_out = it->maxlev;
+    if (nlevels_out) *nlevels_out = (int)it->levels.size();
+    if (nrows_out) *nrows_out = (int)it->start.size();
+    if (nkeep_out) *nkeep_out = (int)it->keep.size();
+    if (nbad_out) *nbad_out = it->nbad;
     return TP_OK;
 }
-extern "C" int tp_batch_get(const tp_batch *b, int i, uint8_t *bad_out, int *n_pcs_out, int *n_clusters_out, double *scores_out,
-                            double *seqdist_out, int *levels_out, int *offsets_out, int *start_out, int *end_out,
-                            double *device_ms_out) {
-    TP_ARG(b && i >= 0 && i < (int)b->items.size(), "tp_batch_get: index out of range");
-    const TpBatchItem &it = b->items[(size_t)i];
-    if (it.rc != TP_OK) { tp_set_error("%s", it.err.c_str()); return it.rc; }
-    if (bad_out) memcpy(bad_out, it.bad.data(), it.bad.size());
-    item_get(it, n_pcs_out, n_clusters_out, scores_out, seqdist_out, levels_out, offsets_out, start_out, end_out);
-    if (device_ms_out) *device_ms_out = it.device_ms;
+extern "C" int tp_batch_get(const tp_batch *b, int i, int part, uint8_t *bad_out, int *n_pcs_out, int *n_clusters_out,
+                            double *scores_out, double *seqdist_out, int *levels_out, int *offsets_out, int *start_out,
+                            int *end_out, double *device_ms_out, int *keep_out, int *badcols_out, int *labels_out) {
+    const TpBatchItem *it = batch_part(b, i, part);
+    TP_ARG(it, part < 0 ? "tp_batch_get: index out of range"
+                          : "tp_batch_get: no such arm (index out of range, or the item was not split)");
+    if (it->rc != TP_OK) { tp_set_error("%s", it->err.c_str()); return it->rc; }
+    if (bad_out) memcpy(bad_out, it->bad.data(), it->bad.size());
+    if (n_pcs_out) *n_pcs_out = it->n_pcs;
+    if (n_clusters_out) *n_clusters_out = it->n_clusters;
+    if (scores_out) memcpy(scores_out, it->scores.data(), it->scores.size() * sizeof(double));
+    if (seqdist_out) memcpy(seqdist_out, it->seqdist.data(), it->seqdist.size() * sizeof(double));
+    if (levels_out) memcpy(levels_out, it->levels.data(), it->levels.size() * sizeof(int));
+    if (offsets_out) memcpy(offsets_out, it->offsets.data(), it->offsets.size() * sizeof(int));
+    if (start_out) memcpy(start_out, it->start.data(), it->start.size() * sizeof(int));
+    if (end_out) memcpy(end_out, it->end.data(), it->end.size() * sizeof(int));
+    if (device_ms_out) *device_ms_out = it->device_ms;
+    if (keep_out) memcpy(keep_out, it->keep.data(), it->keep.size() * sizeof(int));
+    if (badcols_out) memcpy(badcols_out, it->badcols.data(), it->badcols.size() * sizeof(int));
+    if (labels_out) memcpy(labels_out, it->labels.data(), it->labels.size() * sizeof(int));
     return TP_OK;
 }
 extern "C" int tp_batch_split(const tp_batch *b, int i, int *split_out, int *cs_out, int *ce_out, uint8_t *bad_out) {
@@ -733,31 +711,6 @@ extern "C" int tp_batch_split(const tp_batch *b, int i, int *split_out, int *cs_
     if (cs_out) *cs_out = it.cs;
     if (ce_out) *ce_out = it.ce;
     if (bad_out && it.split >= 0) memcpy(bad_out, it.bad.data(), it.bad.size());
-    return TP_OK;
-}
-static const TpBatchItem *arm_of(const tp_batch *b, int i, int arm) {
-    if (!b || i < 0 || i >= (int)b->items.size() || arm < 0 || arm > 1) return nullptr;
-    const TpBatchItem &it = b->items[(size_t)i];
-    return it.rc == TP_OK && it.split == 1 ? &it.arms[(size_t)arm] : nullptr;
-}
-extern "C" int tp_batch_arm_dims(const tp_batch *b, int i, int arm, int *nkeep_out, int *nf_out, int *k_out, int *maxlev_out,
-                                 int *nlevels_out, int *nrows_out, int *nbad_out) {
-    const TpBatchItem *a = arm_of(b, i, arm);
-    TP_ARG(a, "tp_batch_arm_dims: no such arm (index out of range, or the item was not split)");
-    if (nkeep_out) *nkeep_out = (int)a->keep.size();
-    item_dims(*a, nf_out, k_out, maxlev_out, nlevels_out, nrows_out);
-    if (nbad_out) *nbad_out = a->nbad;
-    return TP_OK;
-}
-extern "C" int tp_batch_arm_get(const tp_batch *b, int i, int arm, int *keep_out, int *bad_out, int *n_pcs_out,
-                                int *n_clusters_out, double *scores_out, double *seqdist_out, int *levels_out, int *offsets_out,
-                                int *start_out, int *end_out, int *labels_out) {
-    const TpBatchItem *a = arm_of(b, i, arm);
-    TP_ARG(a, "tp_batch_arm_get: no such arm (index out of range, or the item was not split)");
-    if (keep_out) memcpy(keep_out, a->keep.data(), a->keep.size() * sizeof(int));
-    if (bad_out) memcpy(bad_out, a->badcols.data(), a->badcols.size() * sizeof(int));
-    item_get(*a, n_pcs_out, n_clusters_out, scores_out, seqdist_out, levels_out, offsets_out, start_out, end_out);
-    if (labels_out) memcpy(labels_out, a->labels.data(), a->labels.size() * sizeof(int));
     return TP_OK;
 }
 extern "C" int tp_batch_free(tp_batch *b) {
