@@ -194,6 +194,24 @@ int tp_test_symshard(tp_ctx *ctx, const double *a, int n, int nranks, int kind, 
  * 128 x 64 tile rows [r_lo, r_hi] x columns [c_lo, c_hi] hold any such element (i.e. is it launched)? */
 int tp_test_ss_need(int i, int j, int nranks, int rpr);
 int tp_test_ss_tile(int r_lo, int r_hi, int c_lo, int c_hi, int nranks, int rpr);
+/* test hooks of the two matrix-product engines of stages 2 and 3 (host in / out, row-major; operands go up in buffers of
+ * their own with their padding columns set to NaN, so a kernel reading past an edge shows it).
+ * tp_test_gemm: one FP64 DMMA GEMM, D = alpha A B + beta E1 + gamma E2 (E1 / E2 may be NULL), or, when mean != NULL, the
+ * correlation epilogue ((v - nrows mean_i mean_j) / (nrows - 1) / (sd_i sd_j), NaN -> 0, row i = epi_row0 + local row;
+ * mean / sd hold max(epi_row0 + M, N) entries).  A: M x K (a_kc) or K x M; B: N x K (b_kc) or K x N; E1 / E2: M x N;
+ * sym: only tiles on and above the diagonal are computed and mirrored; splitk > 1: deterministic split-K.  D_inout is
+ * M x ldd (ldd >= N) and comes back whole.  The environment variable TADPOLE_GEMM_CFG = 10 / 11 / 12 forces the
+ * 32x64 / 64x64 / 128x128 tiles.
+ * tp_test_iop: tp_iop_prepare of the symmetric n x n operator S, then napps sliced int8 operator applications in order on
+ * this context, D_a[rows] = alpha S[rows, :] Y_a + beta E1_a[rows] + gamma E2_a[rows] with rows [row_begin, row_end),
+ * block width bs[a] <= 1024 and np = 5 or 8 digit planes; Ys, E1, E2 (may be NULL) and D_inout hold the n x bs[a] blocks
+ * back to back; rows outside the range keep D_inout's values; a write into a padding column of D is an error.  The tile
+ * width follows the context's "io_bn32". */
+int tp_test_gemm(tp_ctx *ctx, int M, int N, int K, const double *A, int a_kc, const double *B, int b_kc, double alpha,
+                 const double *E1, double beta, const double *E2, double gamma, int sym, int splitk, const double *mean,
+                 const double *sd, double nrows, int epi_row0, int ldd, double *D_inout);
+int tp_test_iop(tp_ctx *ctx, const double *S, int n, int napps, const int *bs, const double *Ys, int np, int row_begin,
+                int row_end, double alpha, const double *E1, double beta, const double *E2, double gamma, double *D_inout);
 
 /* ---- stages 4+5: the find_params sweep (R/TADpole.R:104-123) --------------------------------------
  * For candidates i = cand_begin + t*cand_stride < k (0-based: candidate i clusters on the first

@@ -23,6 +23,7 @@ EXPORTED = [
     "tp_get_filtered", "tp_correlation", "tp_get_correlation", "tp_set_correlation", "tp_pca",
     "tp_get_scores", "tp_set_scores", "tp_sweep", "tp_get_sweep_scores", "tp_get_dendro", "tp_select", "tp_call", "tp_call_arm",
     "tp_difft_batch", "tp_assemble", "tp_assemble_levels", "tp_test_cholinv", "tp_test_eig", "tp_test_igram", "tp_test_mgram", "tp_test_symshard", "tp_test_ss_need", "tp_test_ss_tile",
+    "tp_test_gemm", "tp_test_iop",
     "tp_comm_unique_id", "tp_ctx_comm_init", "tp_ctx_comm_select", "tp_ctx_comm_info",
     "tp_ingest_tsv", "tp_ingest_tsv_file", "tp_ingested", "tp_get_ingested", "tp_ingest_stats", "tp_test_parse_field",
     "tp_ingest_coo", "tp_ingest_coo_file",
@@ -118,6 +119,10 @@ def load():
         "tp_test_symshard": (c_int, [vp, dp, c_int, c_int, c_int, c_double, dp]),
         "tp_test_ss_need": (c_int, [c_int, c_int, c_int, c_int]),
         "tp_test_ss_tile": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int]),
+        "tp_test_gemm": (c_int, [vp, c_int, c_int, c_int, dp, c_int, dp, c_int, c_double, dp, c_double, dp, c_double, c_int,
+                                 c_int, dp, dp, c_double, c_int, c_int, dp]),
+        "tp_test_iop": (c_int, [vp, dp, c_int, c_int, ip, dp, c_int, c_int, c_int, c_double, dp, c_double, dp, c_double,
+                                dp]),
         "tp_get_scores": (c_int, [vp, dp]),
         "tp_set_scores": (c_int, [vp, dp, c_int, c_int]),
         "tp_sweep": (c_int, [vp, c_int, c_int, c_int, ip, ip]),
@@ -412,6 +417,46 @@ class Context:
         g = np.zeros((n, n))
         check(self.lib.tp_test_symshard(self._h, _dp(a), n, int(nranks), int(kind), float(fill), _dp(g)))
         return g
+
+    def test_gemm(self, a, b, d, a_kc=True, b_kc=False, alpha=1.0, e1=None, beta=0.0, e2=None, gamma=0.0, sym=False,
+                  splitk=1, mean=None, sd=None, nrows=0.0, epi_row0=0):
+        """One FP64 DMMA GEMM (test hook): a is M x K (a_kc) or K x M, b is N x K (b_kc) or K x N, d is M x ldd
+        (ldd >= N) and comes back as the kernel left it.  alpha a b + beta e1 + gamma e2, or the correlation epilogue
+        when mean is given.  Returns the new d."""
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        b = np.ascontiguousarray(b, dtype=np.float64)
+        m, k = a.shape if a_kc else a.shape[::-1]
+        n = b.shape[0] if b_kc else b.shape[1]
+        assert (b.shape[1] if b_kc else b.shape[0]) == k, "inner dimensions differ"
+        d = np.array(d, dtype=np.float64, order="C")
+        assert d.shape[0] == m and d.shape[1] >= n
+        e = [None if x is None else np.ascontiguousarray(x, dtype=np.float64).reshape(m, n) for x in (e1, e2)]
+        st = [None if x is None else np.ascontiguousarray(x, dtype=np.float64) for x in (mean, sd)]
+        ptr = lambda x: None if x is None else _dp(x)
+        check(self.lib.tp_test_gemm(self._h, m, n, k, _dp(a), int(bool(a_kc)), _dp(b), int(bool(b_kc)), float(alpha),
+                                    ptr(e[0]), float(beta), ptr(e[1]), float(gamma), int(bool(sym)), int(splitk),
+                                    ptr(st[0]), ptr(st[1]), float(nrows), int(epi_row0), d.shape[1], _dp(d)))
+        return d
+
+    def test_iop(self, s, ys, d, np_=8, row_begin=0, row_end=None, alpha=1.0, e1=None, beta=0.0, e2=None, gamma=0.0):
+        """One tp_iop_prepare of the symmetric operator s (n x n), then one sliced operator application per block of the
+        list ys (n x b_a each), in order (test hook).  d, e1, e2: lists of blocks shaped like ys (e1 / e2 may be None).
+        Returns the list of output blocks; rows outside [row_begin, row_end) keep d's values."""
+        s = np.ascontiguousarray(s, dtype=np.float64)
+        n = s.shape[0]
+        bs = np.array([y.shape[1] for y in ys], dtype=np.int32)
+        cat = lambda xs: np.concatenate([np.ascontiguousarray(x, dtype=np.float64).ravel() for x in xs])
+        yv, dv = cat(ys), cat(d)
+        ev = [None if x is None else cat(x) for x in (e1, e2)]
+        ptr = lambda x: None if x is None else _dp(x)
+        check(self.lib.tp_test_iop(self._h, _dp(s), n, bs.size, _ip(bs), _dp(yv), int(np_), int(row_begin),
+                                   n if row_end is None else int(row_end), float(alpha), ptr(ev[0]), float(beta), ptr(ev[1]),
+                                   float(gamma), _dp(dv)))
+        out, off = [], 0
+        for b in bs:
+            out.append(dv[off: off + n * b].reshape(n, b))
+            off += n * b
+        return out
 
     def get_scores(self, nf, k):
         out = np.zeros((nf, k))

@@ -1,5 +1,6 @@
 // api.cu -- context management, one-shot pipeline, host-side reductions and result assembly.
 #include "common.cuh"
+#include "gemm.cuh"
 #include <stdarg.h>
 #include <algorithm>
 #include <mutex>
@@ -406,6 +407,133 @@ extern "C" int tp_test_symshard(tp_ctx *ctx, const double *a, int n, int nranks,
     TP_CUDA(cudaMemcpy2DAsync(gram_out, (size_t)n * sizeof(double), out.p, (size_t)ld * sizeof(double),
                               (size_t)n * sizeof(double), n, cudaMemcpyDeviceToHost, ctx->stream));
     TP_CUDA(tp_stream_sync(ctx));
+    return TP_OK;
+}
+
+// ---- test hooks of the two matrix-product engines of stages 2 and 3 ---------------------------------------------------
+// Operands live in buffers of their own (no pipeline buffer or have_* flag of the context changes).  A host matrix of
+// rows x cols goes up with its leading dimension rounded up to 8 and the padding columns set to NaN (all bits one), so a
+// kernel that reads past the logical edge shows it in its result.
+struct TestBufs {
+    DevBuf b[5];
+    ~TestBufs() { for (DevBuf &x : b) x.release(); }
+};
+
+static int upload_nan_padded(tp_ctx *ctx, DevBuf &buf, size_t off, const double *h, int rows, int cols, int ld) {
+    double *d = buf.as<double>() + off;
+    TP_CUDA(cudaMemsetAsync(d, 0xff, (size_t)rows * ld * sizeof(double), ctx->stream));
+    TP_CUDA(cudaMemcpy2DAsync(d, (size_t)ld * sizeof(double), h, (size_t)cols * sizeof(double), (size_t)cols * sizeof(double),
+                              rows, cudaMemcpyHostToDevice, ctx->stream));
+    return TP_OK;
+}
+
+// One tp_gemm: D = alpha A B + beta E1 + gamma E2, or the EPI_CORR epilogue when mean != NULL (mean / sd hold
+// max(epi_row0 + M, N) entries).  A is M x K row-major (a_kc) or K x M; B is N x K (b_kc) or K x N; E1 / E2 (may be NULL)
+// are M x N.  D_inout (M x ldd, ldd >= N) goes up whole and comes back whole.  TADPOLE_GEMM_CFG = 10 / 11 / 12 forces the
+// 32x64 / 64x64 / 128x128 tiles.
+extern "C" int tp_test_gemm(tp_ctx *ctx, int M, int N, int K, const double *A, int a_kc, const double *B, int b_kc,
+                            double alpha, const double *E1, double beta, const double *E2, double gamma, int sym, int splitk,
+                            const double *mean, const double *sd, double nrows, int epi_row0, int ldd, double *D_inout) {
+    TP_ARG(ctx && M >= 1 && N >= 1 && K >= 1 && A && B && ldd >= N && D_inout && (!mean || (sd && epi_row0 >= 0)),
+           "tp_test_gemm: bad arguments");
+    TP_CUDA(cudaSetDevice(ctx->device));
+    const int ar = a_kc ? M : K, ac = a_kc ? K : M, br = b_kc ? N : K, bc = b_kc ? K : N;
+    const int lda = round_up(ac, 8), ldb = round_up(bc, 8), lde = round_up(N, 8);
+    const int nv = std::max(epi_row0 + M, N);
+    TestBufs t;
+    TP_TRY(t.b[0].reserve((size_t)ar * lda * sizeof(double)));
+    TP_TRY(t.b[1].reserve((size_t)br * ldb * sizeof(double)));
+    TP_TRY(t.b[2].reserve((size_t)2 * M * lde * sizeof(double)));
+    TP_TRY(t.b[3].reserve((size_t)M * ldd * sizeof(double)));
+    TP_TRY(t.b[4].reserve((size_t)2 * nv * sizeof(double)));
+    TP_TRY(upload_nan_padded(ctx, t.b[0], 0, A, ar, ac, lda));
+    TP_TRY(upload_nan_padded(ctx, t.b[1], 0, B, br, bc, ldb));
+    if (E1) TP_TRY(upload_nan_padded(ctx, t.b[2], 0, E1, M, N, lde));
+    if (E2) TP_TRY(upload_nan_padded(ctx, t.b[2], (size_t)M * lde, E2, M, N, lde));
+    TP_CUDA(cudaMemcpyAsync(t.b[3].p, D_inout, (size_t)M * ldd * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    GemmArgs g;
+    g.A = t.b[0].as<double>(); g.lda = lda; g.a_kc = a_kc ? 1 : 0;
+    g.B = t.b[1].as<double>(); g.ldb = ldb; g.b_kc = b_kc ? 1 : 0;
+    g.D = t.b[3].as<double>(); g.ldd = ldd;
+    g.M = M; g.N = N; g.K = K;
+    g.alpha = alpha; g.beta = beta; g.gamma = gamma;
+    if (E1) { g.E1 = t.b[2].as<double>(); g.lde1 = lde; }
+    if (E2) { g.E2 = t.b[2].as<double>() + (size_t)M * lde; g.lde2 = lde; }
+    g.sym = sym ? 1 : 0; g.splitk = splitk;
+    if (mean) {
+        double *st = t.b[4].as<double>();
+        TP_CUDA(cudaMemcpyAsync(st, mean, (size_t)nv * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        TP_CUDA(cudaMemcpyAsync(st + nv, sd, (size_t)nv * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        g.epi = EPI_CORR; g.mean = st; g.sd = st + nv; g.nrows = nrows; g.epi_row0 = epi_row0;
+    }
+    TP_TRY(tp_gemm(ctx, g));
+    TP_CUDA(cudaMemcpyAsync(D_inout, t.b[3].p, (size_t)M * ldd * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    TP_CUDA(tp_stream_sync(ctx));
+    return TP_OK;
+}
+
+int tp_iop_prepare(tp_ctx *ctx, const double *S, int n, int ld);
+int tp_iop_apply(tp_ctx *ctx, const double *Yin, int b, int ldy, double *D, int ldd, double alpha, const double *E1,
+                 int lde1, double beta, const double *E2, int lde2, double gamma, int row_begin, int row_end, int np);
+
+// tp_iop_prepare of the symmetric n x n operator S once, then `napps` tp_iop_apply in order on this context:
+// D_a[rows] = alpha S[rows, :] Y_a + beta E1_a[rows] + gamma E2_a[rows], rows = [row_begin, row_end), block width bs[a]
+// (<= 1024), np = 5 or 8 digit planes.  Ys, E1, E2 (may be NULL) and D_inout hold the n x bs[a] blocks back to back.
+// Rows of D outside the range keep their values; a write into the padding columns of a D block is reported as an error.
+// Tile width: the context's "io_bn32".
+extern "C" int tp_test_iop(tp_ctx *ctx, const double *S, int n, int napps, const int *bs, const double *Ys, int np,
+                           int row_begin, int row_end, double alpha, const double *E1, double beta, const double *E2,
+                           double gamma, double *D_inout) {
+    TP_ARG(ctx && S && n >= 1 && napps >= 1 && bs && Ys && D_inout && 0 <= row_begin && row_begin < row_end && row_end <= n,
+           "tp_test_iop: bad arguments");
+    TP_CUDA(cudaSetDevice(ctx->device));
+    size_t tot = 0;
+    for (int a = 0; a < napps; a++) {
+        TP_ARG(bs[a] >= 1 && bs[a] <= 1024, "tp_test_iop: block widths 1..1024");
+        tot += (size_t)n * round_up(bs[a], 8);
+    }
+    const int lds = round_up(n, 8);
+    TestBufs t;
+    TP_TRY(t.b[0].reserve((size_t)n * lds * sizeof(double)));
+    for (int i = 1; i < 5; i++) TP_TRY(t.b[i].reserve(tot * sizeof(double)));
+    TP_TRY(upload_nan_padded(ctx, t.b[0], 0, S, n, n, lds));
+    size_t ho = 0, dof = 0;                 // host / device offsets of block a
+    for (int a = 0; a < napps; a++) {
+        const int b = bs[a], ld = round_up(b, 8);
+        TP_TRY(upload_nan_padded(ctx, t.b[1], dof, Ys + ho, n, b, ld));
+        if (E1) TP_TRY(upload_nan_padded(ctx, t.b[2], dof, E1 + ho, n, b, ld));
+        if (E2) TP_TRY(upload_nan_padded(ctx, t.b[3], dof, E2 + ho, n, b, ld));
+        TP_TRY(upload_nan_padded(ctx, t.b[4], dof, D_inout + ho, n, b, ld));
+        ho += (size_t)n * b; dof += (size_t)n * ld;
+    }
+    TP_TRY(tp_iop_prepare(ctx, t.b[0].as<double>(), n, lds));
+    ho = dof = 0;
+    for (int a = 0; a < napps; a++) {
+        const int b = bs[a], ld = round_up(b, 8);
+        TP_TRY(tp_iop_apply(ctx, t.b[1].as<double>() + dof, b, ld, t.b[4].as<double>() + dof, ld, alpha,
+                            E1 ? t.b[2].as<double>() + dof : nullptr, ld, beta, E2 ? t.b[3].as<double>() + dof : nullptr, ld,
+                            gamma, row_begin, row_end, np));
+        dof += (size_t)n * ld;
+    }
+    std::vector<double> h(tot);
+    TP_CUDA(cudaMemcpyAsync(h.data(), t.b[4].p, tot * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    TP_CUDA(tp_stream_sync(ctx));
+    ho = dof = 0;
+    for (int a = 0; a < napps; a++) {
+        const int b = bs[a], ld = round_up(b, 8);
+        for (int r = 0; r < n; r++) {
+            memcpy(D_inout + ho + (size_t)r * b, h.data() + dof + (size_t)r * ld, (size_t)b * sizeof(double));
+            for (int c = b; c < ld; c++) {
+                unsigned long long bits;
+                memcpy(&bits, h.data() + dof + (size_t)r * ld + c, sizeof(bits));
+                if (bits != ~0ull) {
+                    tp_set_error("tp_test_iop: application %d wrote D[%d][%d], a padding column of its block", a, r, c);
+                    return TP_ERR_CUDA;
+                }
+            }
+        }
+        ho += (size_t)n * b; dof += (size_t)n * ld;
+    }
     return TP_OK;
 }
 
