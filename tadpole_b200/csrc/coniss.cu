@@ -105,6 +105,9 @@ __device__ __forceinline__ unsigned lds_u32(unsigned a) { unsigned v; asm volati
 __device__ __forceinline__ void sts_u32(unsigned a, unsigned v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 __device__ __forceinline__ int lds_s32(unsigned a) { int v; asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; }
 __device__ __forceinline__ void sts_s32(unsigned a, int v) { asm volatile("st.shared.s32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+// the dSS leaf array in global memory (DSS_GLOBAL), through L2 only: one lane writes what the whole warp reads next
+__device__ __forceinline__ double ldcg_f64(const double *p) { double v; asm volatile("ld.global.cg.f64 %0, [%1];" : "=d"(v) : "l"(p) : "memory"); return v; }
+__device__ __forceinline__ void stcg_f64(double *p, double v) { asm volatile("st.global.cg.f64 [%0], %1;" ::"l"(p), "d"(v) : "memory"); }
 
 template <typename LinkT, bool SMEM> struct Links {
     unsigned sp, sn;          // shared addresses (SMEM)
@@ -140,7 +143,13 @@ template <typename LinkT, bool SMEM> struct Links {
 // TRACE: cycles of one merge step by phase, summed over the merge loop of the first candidate of the list (the widest),
 // written to trace[0..5] = find, links, P rows + dot products, shuffle reduce + scale, write back + level-1 re-reduce,
 // level-2 re-reduce; trace[6] = steps (TADPOLE_SWEEP_TRACE; profiles/r02_coniss_merge_step.md)
-template <typename LinkT, bool LINKS_SMEM, bool INV_SMEM, bool TRACE>
+// DSS_GLOBAL: the leaf level of the dSS array (n1 doubles) stays in the candidate's own row of d0 in global memory, read
+// and written through L2; only the two min-tree levels and the live-boundary bitmap are in shared memory (~19 KB at 50k
+// bins instead of ~400 KB).  The leaf block of the minimum is loaded once by the find step and kept in registers, the
+// blocks of the two neighbours are loaded beside the P rows of the dot products, and the re-reductions patch those
+// registers with the values written back: the same operations on the same values as the shared-memory path, so the same
+// bits, for one more L2 round trip per merge step.
+template <typename LinkT, bool LINKS_SMEM, bool INV_SMEM, bool TRACE, bool DSS_GLOBAL>
 __global__ void __launch_bounds__(256)
 coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
                     const double *__restrict__ d0, int ldd,
@@ -167,8 +176,8 @@ coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
     const int cand = cand_list[slot];
     const int ncol = cand + 1;
     const unsigned sbase = sbase0 + (unsigned)warp * cand_smem;
-    const unsigned sd = sbase;                       // d[n1p]
-    const unsigned sm1 = sd + 8u * n1p;              // m1[B1p]
+    const unsigned sd = sbase;                       // d[n1p] (not DSS_GLOBAL)
+    const unsigned sm1 = DSS_GLOBAL ? sbase : sd + 8u * n1p;      // m1[B1p]
     const unsigned sm2 = sm1 + 8u * B1p;             // m2[B2p]
     // Neighbours of a boundary (previous / next boundary still alive).  LINKS_SMEM: two link arrays in shared memory, two
     // dependent loads per merge.  Otherwise (the arrays do not fit beside the dSS array: above ~18k bins; or they would push
@@ -211,8 +220,13 @@ coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
     const double *d0row = d0 + (size_t)cand * ldd;
     double *seq = seqdist + (size_t)cand * ldd;
     int4 *mrg = merges + (size_t)cand * ldd;
+    // DSS_GLOBAL: this candidate's row of d0 (written by d0_kernel of this sweep, read by nobody else) becomes its leaf
+    // array; entries n1..n1p-1 are not stored: a load there reads +inf, as the padding of the shared array does
+    double *const gd = const_cast<double *>(d0row);
+    auto ld_leaf = [&](int b) -> double { const int q = (b << 5) + lane; return q < n1 ? ldcg_f64(gd + q) : INF_D; };
 
-    for (int j = lane; j < n1p; j += 32) sts_f64(sd + 8u * j, (j < n1) ? d0row[j] : INF_D);
+    if (!DSS_GLOBAL)
+        for (int j = lane; j < n1p; j += 32) sts_f64(sd + 8u * j, (j < n1) ? d0row[j] : INF_D);
     if (LINKS_SMEM) {
         for (int j = lane; j < n1; j += 32) { lk.set_prv(j, j); lk.set_nxt(j, j + 1); }   // prv holds index+1, 0 = none
     } else {
@@ -222,9 +236,23 @@ coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
     for (int b = lane; b < B1p; b += 32) sts_f64(sm1 + 8u * b, INF_D);
     for (int b = lane; b < B2p; b += 32) sts_f64(sm2 + 8u * b, INF_D);
     __syncwarp();
-    for (int b = 0; b < B1; b++) {
-        double v = warp_min_nonneg(lds_f64(sd + 8u * ((b << 5) + lane)));
-        if (lane == 0) sts_f64(sm1 + 8u * b, v);
+    if (DSS_GLOBAL) {
+        // eight leaf blocks per L2 round trip
+        for (int b0 = 0; b0 < B1; b0 += 8) {
+            double x[8];
+#pragma unroll
+            for (int u = 0; u < 8; u++) x[u] = b0 + u < B1 ? ld_leaf(b0 + u) : INF_D;
+#pragma unroll
+            for (int u = 0; u < 8; u++) {
+                const double v = warp_min_nonneg(x[u]);
+                if (lane == 0 && b0 + u < B1) sts_f64(sm1 + 8u * (b0 + u), v);
+            }
+        }
+    } else {
+        for (int b = 0; b < B1; b++) {
+            double v = warp_min_nonneg(lds_f64(sd + 8u * ((b << 5) + lane)));
+            if (lane == 0) sts_f64(sm1 + 8u * b, v);
+        }
     }
     __syncwarp();
     for (int b = 0; b < B2; b++) {
@@ -269,7 +297,7 @@ coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
         const double thr = fma(mn, TIE_REL, mn) + tie_abs;
         const unsigned bal1 = __ballot_sync(0xffffffffu, lds_f64(sm1 + 8u * ((b2 << 5) + lane)) <= thr);
         const int b1 = (b2 << 5) + __ffs(bal1) - 1;
-        const double leaf = lds_f64(sd + 8u * ((b1 << 5) + lane));
+        const double leaf = DSS_GLOBAL ? ld_leaf(b1) : lds_f64(sd + 8u * ((b1 << 5) + lane));
         const unsigned bal0 = __ballot_sync(0xffffffffu, leaf <= thr);
         const int j = (b1 << 5) + __ffs(bal0) - 1;
         mn = __shfl_sync(0xffffffffu, leaf, j & 31);          // the increase of the boundary that is merged
@@ -293,6 +321,13 @@ coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
         const double *Pc = Plane + (size_t)c * ldk, *Pe = Plane + (size_t)e * ldk;
         const int cC = c - b, cLL = b - a, cRR = e - c;
         const double iC = inv_of(cC), iLL = inv_of(cLL), iRR = inv_of(cRR);
+        // DSS_GLOBAL: the leaf blocks of the neighbours, when not the one in registers, in flight with the P rows
+        double xk1 = 0.0, xk2 = 0.0;
+        if (DSS_GLOBAL) {
+            const int q0 = j >> 5, q1 = hasL ? (pj >> 5) : q0, q2 = hasR ? (nj >> 5) : q0;
+            if (q1 != q0) xk1 = ld_leaf(q1);
+            if (q2 != q0 && q2 != q1) xk2 = ld_leaf(q2);
+        }
         double accL = 0.0, accR = 0.0;
         if (TRACE) { asm volatile("" ::"d"(iC), "d"(iLL), "d"(iRR)); CS_TR(1); }
         for (int c0 = 0; c0 < ncol; c0 += 32 * CS_CHUNK) {
@@ -336,9 +371,10 @@ coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
         if (TRACE) { asm volatile("" ::"d"(accL), "d"(accR)); CS_TR(3); }
         // ---- write back: boundary j dies, its neighbours get new increases ---------------
         if (lane == 0) {
-            sts_f64(sd + 8u * j, INF_D);
-            if (hasL) { sts_f64(sd + 8u * pj, accL); if (LINKS_SMEM) lk.set_nxt(pj, nj); }
-            if (hasR) { sts_f64(sd + 8u * nj, accR); if (LINKS_SMEM) lk.set_prv(nj, pj + 1); }
+            auto st_d = [&](int q, double v) { if (DSS_GLOBAL) stcg_f64(gd + q, v); else sts_f64(sd + 8u * q, v); };
+            st_d(j, INF_D);
+            if (hasL) { st_d(pj, accL); if (LINKS_SMEM) lk.set_nxt(pj, nj); }
+            if (hasR) { st_d(nj, accR); if (LINKS_SMEM) lk.set_prv(nj, pj + 1); }
             if (!LINKS_SMEM) sts_u32(sbits + 4u * (j >> 5), lds_u32(sbits + 4u * (j >> 5)) & ~(1u << (j & 31)));
         }
         __syncwarp();
@@ -346,9 +382,25 @@ coniss_sweep_kernel(const double *__restrict__ P, int ldk, int n,
         const int k1 = hasL ? (pj >> 5) : k0;
         const int k2 = hasR ? (nj >> 5) : k0;
         // independent re-reductions issued back to back (ILP), then stored
-        const double x0 = lds_f64(sd + 8u * ((k0 << 5) + lane));
-        const double x1 = lds_f64(sd + 8u * ((k1 << 5) + lane));
-        const double x2 = lds_f64(sd + 8u * ((k2 << 5) + lane));
+        double x0, x1, x2;
+        if (DSS_GLOBAL) {
+            // the blocks as loaded, with this step's write-back applied (accL / accR are the same on every lane: the
+            // butterfly adds the same two values on both lanes of each pair)
+            auto patch = [&](double x, int blk) -> double {
+                const int q = (blk << 5) + lane;
+                if (q == j) x = INF_D;
+                if (hasL && q == pj) x = accL;
+                if (hasR && q == nj) x = accR;
+                return x;
+            };
+            x0 = patch(leaf, k0);
+            x1 = k1 != k0 ? patch(xk1, k1) : x0;
+            x2 = k2 == k0 ? x0 : (k2 == k1 ? x1 : patch(xk2, k2));
+        } else {
+            x0 = lds_f64(sd + 8u * ((k0 << 5) + lane));
+            x1 = lds_f64(sd + 8u * ((k1 << 5) + lane));
+            x2 = lds_f64(sd + 8u * ((k2 << 5) + lane));
+        }
         const double r0 = warp_min_nonneg(x0);
         const double r1 = (k1 != k0) ? warp_min_nonneg(x1) : r0;
         const double r2 = (k2 != k0) ? warp_min_nonneg(x2) : r0;
@@ -557,24 +609,30 @@ int tp_sweep_device(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stri
     ctx->launches += 4;
 
     // shared memory plan: per candidate the dSS array with its min tree (+ the boundary links when they fit); several
-    // candidates per CTA (one warp each) sharing one reciprocal table while that fits
+    // candidates per CTA (one warp each) sharing one reciprocal table while that fits.  When the dSS array does not fit
+    // (above ~27 700 bins) its leaf level goes to global memory (DSS_GLOBAL) and only the tree and the bitmap stay.
     const int n1p = round_up(n1, 32), B1p = round_up(n1p / 32, 32), B2p = round_up(B1p / 32, 32);
     const size_t base = (size_t)(n1p + B1p + B2p) * sizeof(double);
+    const size_t tree = (size_t)(B1p + B2p) * sizeof(double);
     const bool small_links = n <= 65535;
     const size_t link_bytes = round_up((int)((size_t)2 * n1 * (small_links ? 2 : 4)), 8);
     const size_t bitmap_bytes = (size_t)round_up(((n1 + 31) / 32) * 4, 16);
     const size_t inv_bytes = (size_t)(n + 1) * sizeof(double);
     const size_t limit = (size_t)ctx->max_smem_optin;
-    TP_ARG(base + bitmap_bytes <= limit, "tp_sweep: matrix too large for the shared-memory dSS array (n > ~28k bins); split by centromere");
+    const char *e_dss = getenv("TADPOLE_SWEEP_DSS");             // "global": the global leaf array at any size (tests)
+    const bool dss_global = base + bitmap_bytes > limit || (e_dss && e_dss[0] == 'g');
     // link arrays while they fit (two dependent loads: ~90 cycles per merge against ~400 for the bitmap searches), else the
-    // bitmap (32 x smaller: above ~18k bins)
+    // bitmap (32 x smaller: above ~18k bins; always beside a global leaf array)
     const char *force = getenv("TADPOLE_SWEEP_LINKS");           // "bitmap" / "array": experiments
     bool links_smem = base + link_bytes <= limit;
     if (force && force[0] == 'b') links_smem = false;
     if (force && force[0] == 'a' && base + link_bytes <= limit) links_smem = true;
-    const size_t cand_smem = round_up((int)(links_smem ? base + link_bytes : base + bitmap_bytes), 16);
-    // the reciprocal table goes to shared memory while at least two candidates still fit beside it
-    bool inv_smem = 2 * cand_smem + inv_bytes <= limit;
+    if (dss_global) links_smem = false;
+    const size_t cand_smem = round_up((int)(links_smem ? base + link_bytes : (dss_global ? tree : base) + bitmap_bytes), 16);
+    TP_ARG(cand_smem <= limit, "tp_sweep: matrix too large for the shared-memory min tree of the dSS array (n > ~600k bins)");
+    // the reciprocal table goes to shared memory while at least two candidates still fit beside it (never beside a global
+    // leaf array: that only runs where the table would not fit either)
+    bool inv_smem = !dss_global && 2 * cand_smem + inv_bytes <= limit;
     const char *e_inv = getenv("TADPOLE_SWEEP_INV"), *e_wpc = getenv("TADPOLE_SWEEP_WPC");       // experiments
     if (e_inv && e_inv[0] == 'g') inv_smem = false;
     int wpc = (int)((limit - (inv_smem ? inv_bytes : 0)) / cand_smem);
@@ -588,21 +646,23 @@ int tp_sweep_device(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stri
     long long *trace = nullptr;
     DevBuf trbuf;
     if (getenv("TADPOLE_SWEEP_TRACE")) { TP_TRY(trbuf.reserve(8 * sizeof(long long))); trace = trbuf.as<long long>(); }
-#define LAUNCH_SWEEP2(LT, LS, IS, TR)                                                                     \
+#define LAUNCH_SWEEP2(LT, LS, IS, TR, DG)                                                                 \
     do {                                                                                                  \
-        TP_CUDA(tp_optin_smem(coniss_sweep_kernel<LT, LS, IS, TR>, ctx)); \
+        TP_CUDA(tp_optin_smem(coniss_sweep_kernel<LT, LS, IS, TR, DG>, ctx)); \
         tp_prof_begin(ctx, PC_SWEEP);                                                                     \
-        coniss_sweep_kernel<LT, LS, IS, TR><<<nblocks, 32 * wpc, smem, st>>>(ctx->P.as<double>(), ldk, n, ctx->d0.as<double>(), ldd, \
+        coniss_sweep_kernel<LT, LS, IS, TR, DG><<<nblocks, 32 * wpc, smem, st>>>(ctx->P.as<double>(), ldk, n, ctx->d0.as<double>(), ldd, \
                                                                  d_cands, ncand, (unsigned)cand_smem, ctx->seqdist.as<double>(), \
                                                                  ctx->order.as<int4>(), (LT *)glinks, ctx->Qp.as<double>() + n, trace); \
         tp_prof_end(ctx);                                                                                 \
     } while (0)
-#define LAUNCH_SWEEP(LT, LS, IS) do { if (trace) LAUNCH_SWEEP2(LT, LS, IS, true); else LAUNCH_SWEEP2(LT, LS, IS, false); } while (0)
-    if (links_smem) {
-        if (small_links) { if (inv_smem) LAUNCH_SWEEP(unsigned short, true, true); else LAUNCH_SWEEP(unsigned short, true, false); }
-        else { if (inv_smem) LAUNCH_SWEEP(int, true, true); else LAUNCH_SWEEP(int, true, false); }
+#define LAUNCH_SWEEP(LT, LS, IS, DG) do { if (trace) LAUNCH_SWEEP2(LT, LS, IS, true, DG); else LAUNCH_SWEEP2(LT, LS, IS, false, DG); } while (0)
+    if (dss_global) {
+        LAUNCH_SWEEP(unsigned short, false, false, true);
+    } else if (links_smem) {
+        if (small_links) { if (inv_smem) LAUNCH_SWEEP(unsigned short, true, true, false); else LAUNCH_SWEEP(unsigned short, true, false, false); }
+        else { if (inv_smem) LAUNCH_SWEEP(int, true, true, false); else LAUNCH_SWEEP(int, true, false, false); }
     } else {
-        if (inv_smem) LAUNCH_SWEEP(unsigned short, false, true); else LAUNCH_SWEEP(unsigned short, false, false);
+        if (inv_smem) LAUNCH_SWEEP(unsigned short, false, true, false); else LAUNCH_SWEEP(unsigned short, false, false, false);
     }
 #undef LAUNCH_SWEEP2
 #undef LAUNCH_SWEEP
@@ -614,7 +674,8 @@ int tp_sweep_device(tp_ctx *ctx, int min_clusters, int cand_begin, int cand_stri
         TP_CUDA(cudaStreamSynchronize(st));
         TP_CUDA(cudaMemcpy(h, trace, sizeof(h), cudaMemcpyDeviceToHost));
         static const char *ph[6] = {"find", "links", "p_rows_dot", "reduce_scale", "writeback_l1", "l2"};
-        fprintf(stderr, "[sweep trace] n=%d cols=%lld wpc=%d links_smem=%d inv_smem=%d cycles per merge step:", n, h[7], wpc, (int)links_smem, (int)inv_smem);
+        fprintf(stderr, "[sweep trace] n=%d cols=%lld wpc=%d links_smem=%d inv_smem=%d dss_global=%d cycles per merge step:", n, h[7], wpc,
+                (int)links_smem, (int)inv_smem, (int)dss_global);
         for (int p = 0; p < 6; p++) fprintf(stderr, " %s %.0f", ph[p], (double)h[p] / (double)h[6]);
         fprintf(stderr, "\n");
         trbuf.release();
