@@ -370,6 +370,24 @@ int tp_difft_null(tp_ctx *ctx, const int32_t *labels_x, int L, int pad_left, int
                   const int32_t *bad_positions, int nbad, unsigned long long seed, int nperm,
                   int32_t *borders_out, int32_t *labels_out, double *curves_out, double *totals_out);
 
+/* nprob diffT comparisons of different lengths, each with its own null distribution, in one call (diffT_genome: one
+ * problem per chromosome and level shared by two samples).
+ * Problem p: labels_x / labels_y hold its L_p = off[p+1] - off[p] padded labels from off[p] (as tp_difft_batch takes
+ * them; off[0] = 0); pad_left[p], pad_right[p], ntads[p] and bad_positions[bad_off[p] .. bad_off[p+1]) (bad_off[0] = 0)
+ * describe the random partitions exactly as tp_difft_null takes them; the draws of problem p are tp_difft_null's with
+ * seed + p (mod 2^64) and permutations 0 .. nperm-1, scored against labels_x of problem p.
+ * Outputs (host, each may be NULL): curves_out[off[nprob]] observed normalised curves, totals_out[nprob] observed
+ * un-normalised totals, null_totals_out[nprob x nperm] (row-major) totals of the random partitions, status_out[nprob] =
+ * TP_OK, or TP_ERR_ARG for a problem tp_difft_null would refuse ("sample larger than the population"): its null row is
+ * NaN, its observed curve and total are still written, and the other problems are unaffected.  Malformed arguments
+ * (offsets not increasing, a pad outside the extent, ntads < 1, a bad position 0) fail the whole call.
+ * The random label vectors never leave the GPU: one CTA draws and scores each partition.  Launches and host
+ * synchronisations do not grow with nprob.  Runs on the context's first device. */
+int tp_difft_multi(tp_ctx *ctx, int nprob, const int64_t *off, const int32_t *labels_x, const int32_t *labels_y,
+                   const int32_t *pad_left, const int32_t *pad_right, const int32_t *ntads, const int64_t *bad_off,
+                   const int32_t *bad_positions, unsigned long long seed, int nperm, double *curves_out,
+                   double *totals_out, double *null_totals_out, int *status_out);
+
 /* ---- result assembly (host integer logic, R/TADpole.R:470-497 and fix_values :503-510) ----------
  * Cuts the dendrogram `seqdist` (nf-1) into n_clusters contiguous clusters, re-inserts the bad bins
  * as 0 by original position, absorbs interior 0 runs flanked by the same id, and writes the

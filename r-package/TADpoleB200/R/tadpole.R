@@ -318,3 +318,73 @@ diffT_null <- function(bed_x, bed_y = bed_x, nperm = 1000L, bad_columns = NULL, 
                  nrow(bed_y), bad, as.numeric(seed), as.integer(nperm))
     list(borders = t(res[[1L]]) + bed_y[1, 2], totals = res[[2L]], curves = t(res[[3L]]))
 }
+
+# diffT between two TADpole_genome() results, level by level, every comparison with its own null distribution, all in
+# one .Call.  One problem per chromosome present in both as a whole-chromosome object (control's order) and per level
+# scored in both (or listed in `levels`), ascending: diffT(control[[chr]]$clusters[[k]], case[[chr]]$clusters[[k]]) and
+# nperm random partitions of the case's extent with its TAD count, drawn with seed + p for problem p (0-based).  The
+# null's bad columns are the case's filtered bins inside its table's extent, as positions within start:end.
+# Returns data.frame(chrom, level, total, p_value) with attr(, "curves"), attr(, "null_totals") (problems x nperm) and
+# attr(, "skipped") (reasons, named by chromosome or "chromosome:level").  p_value = (1 + #{null totals <= total}) /
+# (nperm + 1) is not in the reference.
+diffT_genome <- function(control, case, levels = NULL, nperm = 1000L, seed = 0) {
+    skipped <- list()
+    failed_x <- attr(control, "failed"); failed_y <- attr(case, "failed")
+    probs <- list()
+    for (chr in names(control)) {
+        if (is.null(case[[chr]])) {
+            skipped[[chr]] <- if (!is.null(failed_y[[chr]])) paste("failed in case:", failed_y[[chr]]) else "missing from case"
+            next
+        }
+        a <- control[[chr]]; b <- case[[chr]]
+        if (is.null(a$clusters) || is.null(b$clusters)) {
+            skipped[[chr]] <- "centromere_search result: comparing the arms is not supported"
+            next
+        }
+        shared <- sort(as.integer(intersect(names(a$clusters), names(b$clusters))))
+        ks <- if (is.null(levels)) shared else {
+            want <- sort(unique(as.integer(levels)))
+            for (k in setdiff(want, shared))
+                skipped[[paste0(chr, ":", k)]] <- paste("level", k, "is not scored in",
+                                                        if (is.null(a$clusters[[as.character(k)]])) "control" else "case")
+            intersect(want, shared)
+        }
+        kept <- as.integer(b$dendro$labels)
+        for (k in ks) {
+            bx <- a$clusters[[as.character(k)]]; by <- b$clusters[[as.character(k)]]
+            if (nrow(bx) != nrow(by)) {
+                skipped[[paste0(chr, ":", k)]] <- "Both calls must have the same number of TADs."
+                next
+            }
+            # .tp_padded_labels reads BED columns 2:3
+            lab <- .tp_padded_labels(cbind(0, bx$start, bx$end), cbind(0, by$start, by$end))
+            span <- by$start[1L]:by$end[nrow(by)]
+            probs[[length(probs) + 1L]] <- list(chrom = chr, level = k, x = lab$x, y = lab$y, pl = lab$pad_left_y,
+                                                pr = lab$pad_right_y, ntads = nrow(by),
+                                                bad = as.integer(span[!(span %in% kept)] - by$start[1L] + 1L))
+        }
+    }
+    for (chr in setdiff(names(case), names(control)))
+        skipped[[chr]] <- if (!is.null(failed_x[[chr]])) paste("failed in control:", failed_x[[chr]]) else "missing from control"
+    np <- length(probs)
+    lens <- vapply(probs, function(p) length(p$x), 0)
+    nbad <- vapply(probs, function(p) length(p$bad), 0)
+    off <- c(0, cumsum(lens)); boff <- c(0, cumsum(nbad))
+    pm <- matrix(as.integer(c(sapply(probs, `[[`, "pl"), sapply(probs, `[[`, "pr"), sapply(probs, `[[`, "ntads"))),
+                 nrow = np, ncol = 3L)
+    res <- .Call(C_tp_difft_multi, .tp_ctx(), as.numeric(off),
+                 list(as.integer(unlist(lapply(probs, `[[`, "x"))), as.integer(unlist(lapply(probs, `[[`, "y")))), pm,
+                 as.numeric(boff), as.integer(unlist(lapply(probs, `[[`, "bad"))), as.numeric(seed), as.integer(nperm))
+    ok <- res[[4L]] == 0L
+    for (i in which(!ok))
+        skipped[[paste0(probs[[i]]$chrom, ":", probs[[i]]$level)]] <- "the library refused it: random_bed cannot draw the borders (sample() errors here)"
+    keep <- which(ok)
+    null <- t(res[[3L]])[keep, , drop = FALSE]
+    total <- res[[2L]][keep]
+    out <- data.frame(chrom = as.character(sapply(probs[keep], `[[`, "chrom")), level = as.integer(sapply(probs[keep], `[[`, "level")),
+                      total = total, p_value = (1 + rowSums(null <= total)) / (nperm + 1), stringsAsFactors = FALSE)
+    attr(out, "curves") <- lapply(keep, function(i) res[[1L]][(off[i] + 1):off[i + 1L]])
+    attr(out, "null_totals") <- null
+    attr(out, "skipped") <- skipped
+    out
+}

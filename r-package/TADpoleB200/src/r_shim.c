@@ -595,6 +595,41 @@ SEXP C_tp_difft_null(SEXP ctx, SEXP lx, SEXP pad_left, SEXP pad_right, SEXP ntad
     return out;
 }
 
+/* nprob diffT comparisons of different lengths, each with its own null distribution (tp_difft_multi; diffT_genome).
+ * off / bad_off: numeric (doubles: R has no 64-bit integers), nprob + 1 offsets into the labels and bad; labels =
+ * list(x, y) of integer vectors; problems = integer matrix nprob x 3 (pad_left, pad_right, ntads).  Returns
+ * list(curves [off[nprob]], totals [nprob], null_totals [nperm x nprob] -- column per problem, status [nprob]) */
+SEXP C_tp_difft_multi(SEXP ctx, SEXP off, SEXP labels, SEXP problems, SEXP bad_off, SEXP bad, SEXP seed, SEXP nperm) {
+    int nprob = length(off) - 1, P = asInteger(nperm);
+    if (nprob < 0 || length(bad_off) != nprob + 1 || length(problems) != 3 * nprob || length(labels) != 2)
+        error("TADpole: off, bad_off, labels and the problem matrix do not describe the same problems");
+    SEXP lx = VECTOR_ELT(labels, 0), ly = VECTOR_ELT(labels, 1);
+    int64_t *o = (int64_t *)R_alloc((size_t)nprob + 1, sizeof(int64_t));
+    int64_t *bo = (int64_t *)R_alloc((size_t)nprob + 1, sizeof(int64_t));
+    for (int i = 0; i <= nprob; i++) { o[i] = (int64_t)REAL(off)[i]; bo[i] = (int64_t)REAL(bad_off)[i]; }
+    if (nprob > 0 && ((int64_t)length(lx) != o[nprob] || (int64_t)length(ly) != o[nprob] || (int64_t)length(bad) != bo[nprob]))
+        error("TADpole: label or bad-position vectors do not match the offsets");
+    const int *pm = INTEGER(problems);                    /* column-major: pad_left, pad_right, ntads */
+    SEXP curves = PROTECT(allocVector(REALSXP, nprob > 0 ? (size_t)o[nprob] : 0));
+    SEXP totals = PROTECT(allocVector(REALSXP, nprob));
+    SEXP null = PROTECT(allocMatrix(REALSXP, P, nprob));
+    SEXP status = PROTECT(allocVector(INTSXP, nprob));
+    int rc = tp_difft_multi(ctx_of(ctx), nprob, o, INTEGER(lx), INTEGER(ly), pm, pm + nprob, pm + 2 * (size_t)nprob, bo,
+                            length(bad) ? INTEGER(bad) : NULL, (unsigned long long)asReal(seed), P, REAL(curves),
+                            REAL(totals), REAL(null), INTEGER(status));
+    if (rc != TP_OK) {
+        UNPROTECT(4);
+        error("%s", tp_last_error());
+    }
+    SEXP out = PROTECT(allocVector(VECSXP, 4));
+    SET_VECTOR_ELT(out, 0, curves);
+    SET_VECTOR_ELT(out, 1, totals);
+    SET_VECTOR_ELT(out, 2, null);
+    SET_VECTOR_ELT(out, 3, status);
+    UNPROTECT(5);
+    return out;
+}
+
 /* several GPUs: one R process per GPU; rank 0 makes the id, every rank joins (csrc/comm.cu) */
 SEXP C_tp_comm_unique_id(void) {
     SEXP id = PROTECT(allocVector(RAWSXP, 128));
@@ -643,6 +678,7 @@ static const R_CallMethodDef call_table[] = {
     {"C_tp_labels", (DL_FUNC)&C_tp_labels, 5},
     {"C_tp_difft", (DL_FUNC)&C_tp_difft, 5},
     {"C_tp_difft_null", (DL_FUNC)&C_tp_difft_null, 8},
+    {"C_tp_difft_multi", (DL_FUNC)&C_tp_difft_multi, 8},
     {"C_tp_comm_unique_id", (DL_FUNC)&C_tp_comm_unique_id, 0},
     {"C_tp_ctx_comm_init", (DL_FUNC)&C_tp_ctx_comm_init, 5},
     {"C_tp_ctx_comm_select", (DL_FUNC)&C_tp_ctx_comm_select, 2},

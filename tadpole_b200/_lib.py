@@ -27,7 +27,7 @@ EXPORTED = [
     "tp_comm_unique_id", "tp_ctx_comm_init", "tp_ctx_comm_select", "tp_ctx_comm_info",
     "tp_ingest_tsv", "tp_ingest_tsv_file", "tp_ingested", "tp_get_ingested", "tp_ingest_stats", "tp_test_parse_field",
     "tp_ingest_coo", "tp_ingest_coo_file",
-    "tp_difft_null", "tp_recall",
+    "tp_difft_null", "tp_difft_multi", "tp_recall",
     "tp_ctx_create_multi", "tp_device_count", "tp_ctx_devices", "tp_ctx_generation", "tp_ctx_dims", "tp_call_arms", "tp_call_batch",
     "tp_batch_size", "tp_batch_device_ms", "tp_batch_launches", "tp_batch_status", "tp_batch_error", "tp_batch_dims", "tp_batch_get", "tp_batch_free", "tp_find_groups",
     "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
@@ -134,6 +134,7 @@ def load():
         "tp_recall": (c_int, [vp, c_int, c_int, ip, ip, ip, ip, dp]),
         "tp_difft_batch": (c_int, [vp, vp, vp, c_int, c_int, c_int, vp]),
         "tp_difft_null": (c_int, [vp, vp, c_int, c_int, c_int, c_int, vp, c_int, ctypes.c_ulonglong, c_int, vp, vp, vp, vp]),
+        "tp_difft_multi": (c_int, [vp, c_int, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.c_ulonglong, c_int, vp, vp, vp, vp]),
         "tp_assemble": (c_int, [dp, c_int, c_int, ip, ip, c_int, ip, ip, ip, ip]),
         "tp_assemble_levels": (c_int, [dp, c_int, ip, c_int, ip, ip, c_int, ip, ip, ip]),
     }
@@ -706,6 +707,31 @@ class Context:
                                      labels.ctypes.data if want_labels else None,
                                      curves.ctypes.data if want_curves else None, totals.ctypes.data))
         return dict(borders=borders, totals=totals, curves=curves, labels=labels)
+
+    def difft_multi(self, off, labels_x, labels_y, pad_left, pad_right, ntads, bad_off, bad_positions, seed=0, nperm=1000,
+                    want_curves=True):
+        """tp_difft_multi: nprob = off.size - 1 ragged diffT comparisons, each with nperm random partitions drawn with
+        seed + p.  Returns dict(curves [off[-1]] (concatenated) or None, totals [nprob], null_totals [nprob, nperm],
+        status [nprob])."""
+        off = np.ascontiguousarray(off, dtype=np.int64)
+        nprob = off.size - 1
+        arr32 = lambda a: np.ascontiguousarray(a, dtype=np.int32)
+        lx, ly = arr32(labels_x), arr32(labels_y)
+        pl, pr, nt = arr32(pad_left), arr32(pad_right), arr32(ntads)
+        boff = np.ascontiguousarray(bad_off, dtype=np.int64)
+        bad = arr32(bad_positions)
+        if not (lx.size == ly.size == off[-1] and pl.size == pr.size == nt.size == nprob and boff.size == nprob + 1
+                and bad.size == boff[-1]):
+            raise ValueError("difft_multi: array sizes do not match the offsets")
+        curves = np.empty(int(off[-1])) if want_curves else None
+        totals = np.empty(nprob)
+        null = np.empty((nprob, int(nperm)))
+        status = np.empty(nprob, dtype=np.int32)
+        ptr = lambda a: a.ctypes.data if a.size else None
+        check(self.lib.tp_difft_multi(self._h, nprob, off.ctypes.data, ptr(lx), ptr(ly), ptr(pl), ptr(pr), ptr(nt),
+                                      boff.ctypes.data, ptr(bad), int(seed) & (2 ** 64 - 1), int(nperm),
+                                      ptr(curves) if want_curves else None, ptr(totals), ptr(null), ptr(status)))
+        return dict(curves=curves, totals=totals, null_totals=null, status=status)
 
     def difft_batch_dev(self, lx_ptr, ly_ptr, L, npairs, out_ptr):
         check(self.lib.tp_difft_batch(self._h, int(lx_ptr), int(ly_ptr), int(L), int(npairs), 1, int(out_ptr)))

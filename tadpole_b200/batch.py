@@ -19,11 +19,11 @@ import os
 import numpy as np
 
 from . import _lib
-from .api import (NOSPLIT_MESSAGE, Tadpole, _arm_object, _merging_arms, _messages_bad, _messages_optimal, _messages_split,
-                  message, read_matrix)
+from .api import (NOSPLIT_MESSAGE, Tadpole, _Obj, _arm_object, _bed_rows, _difft_labels, _merging_arms, _messages_bad,
+                  _messages_optimal, _messages_split, get_context, message, read_matrix)
 from .hclust import Dendro
 
-__all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "TADpole_genome", "read_bins"]
+__all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "TADpole_genome", "read_bins", "diffT_genome"]
 
 
 class ContextPool:
@@ -218,4 +218,122 @@ def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.
             out.failed[nm] = NOSPLIT_MESSAGE if r.code == _lib.TP_ERR_NOSPLIT else str(r)
             continue
         out[nm] = _tadpole_from_batch_item(r, centromere_fix)
+    return out
+
+
+# ---- comparing two genome-wide calls ---------------------------------------------------------------------------------
+
+def _field(obj, name):
+    if isinstance(obj, dict):
+        return obj.get(name)
+    return getattr(obj, name, None)
+
+
+def _difft_genome_problems(control, case, levels=None):
+    """The problems of diffT_genome (one per chromosome and level compared) and the `skipped` dict.  Each problem is a
+    dict: chrom, level, x / y (the control's and the case's start / end tables), tx / ty (padded labels, as diffT pads
+    them), pad_left / pad_right / ntads (of y within the common extent) and bad (1-based positions within y's start:end
+    of the case's filtered bins there).  Host bookkeeping only."""
+    skipped = {}
+    failed_x, failed_y = getattr(control, "failed", None) or {}, getattr(case, "failed", None) or {}
+    problems = []
+    for chrom, tx_obj in control.items():
+        if chrom not in case:
+            skipped[chrom] = (f"failed in case: {failed_y[chrom]}" if chrom in failed_y else "missing from case")
+            continue
+        ty_obj = case[chrom]
+        if _field(tx_obj, "clusters") is None or _field(ty_obj, "clusters") is None:
+            skipped[chrom] = "centromere_search result: comparing the arms is not supported"
+            continue
+        cx = {int(k): v for k, v in _field(tx_obj, "clusters").items()}
+        cy = {int(k): v for k, v in _field(ty_obj, "clusters").items()}
+        if levels is None:
+            ks = sorted(set(cx) & set(cy))
+        else:
+            ks = []
+            for k in sorted({int(k) for k in levels}):
+                if k not in cx or k not in cy:
+                    skipped[(chrom, k)] = f"level {k} is not scored in {'control' if k not in cx else 'case'}"
+                else:
+                    ks.append(k)
+        dendro = _field(ty_obj, "dendro")
+        kept = np.asarray(_field(dendro, "labels"), dtype=np.int64)
+        for k in ks:
+            bx, by = _bed_rows(cx[k]), _bed_rows(cy[k])
+            if bx.shape[0] != by.shape[0]:
+                skipped[(chrom, k)] = "Both calls must have the same number of TADs."      # R/DiffT.R:20
+                continue
+            tx, ty = _difft_labels(bx, by)
+            sx, sy, ex, ey = int(bx[0, 0]), int(by[0, 0]), int(bx[-1, 1]), int(by[-1, 1])
+            span = np.arange(sy, ey + 1)
+            bad = (span[~np.isin(span, kept)] - sy + 1).astype(np.int32)
+            problems.append(dict(chrom=chrom, level=k, x=bx, y=by, tx=tx, ty=ty, pad_left=max(0, sy - sx),
+                                 pad_right=max(0, ex - ey), ntads=int(by.shape[0]), bad=bad))
+    for chrom in case:
+        if chrom not in control:
+            skipped[chrom] = (f"failed in control: {failed_x[chrom]}" if chrom in failed_x else "missing from control")
+    for chrom, msg in failed_x.items():
+        if chrom not in control and chrom not in skipped:
+            skipped[chrom] = f"failed in control: {msg}"
+    for chrom, msg in failed_y.items():
+        if chrom not in case and chrom not in control and chrom not in skipped:
+            skipped[chrom] = f"failed in case: {msg}"
+    return problems, skipped
+
+
+def _population(pr):
+    """Candidate border positions of a problem's random partitions (tp_difft_null's count)."""
+    size = int(pr["ty"].size) - pr["pad_left"] - pr["pad_right"]
+    bad = np.unique(pr["bad"][(pr["bad"] >= 1) & (pr["bad"] <= size)])
+    return max(size - bad.size - 1, 0)
+
+
+def diffT_genome(control, case, levels=None, nperm=1000, seed=0, ctx=None):
+    """diffT (R/DiffT.R:19-50) between two genome-wide calls, level by level, each comparison with its own null
+    distribution; every comparison and every random partition is computed in one call to the library.
+
+    control, case: GenomeResults of TADpole_genome (or {chromosome: Tadpole} mappings).  One problem per chromosome
+    present in both as a whole-chromosome object (in control's order) and per level k scored in both (or listed in
+    `levels`), ascending: diffT(control[chrom].clusters[k], case[chrom].clusters[k]), and diffT against nperm random
+    partitions of the case's extent with its TAD count, as diffT_null(x, y, bad_columns=...) draws them.  The bad columns
+    of the null are the case's filtered bins inside its table's extent, as positions within start:end
+    (bin - start + 1): the reference's random_bed takes positions, so the chromosome's own bad_columns would be
+    misplaced whenever the table does not start at bin 1.  Problem p (0-based, in this order) draws with seed + p.
+
+    Returns an object of parallel lists / arrays, one entry per compared problem: chrom, level, total (observed,
+    un-normalised), p_value = (1 + #{null totals <= total}) / (nperm + 1), curves (observed normalised curves),
+    null_totals [nproblems, nperm] and seed (per problem); and skipped: {chromosome or (chromosome, level): reason}.
+    p_value (the share of random partitions at least as close to the control as the case is) is not in the reference."""
+    ctx = ctx or get_context()
+    problems, skipped = _difft_genome_problems(control, case, levels)
+    nperm = int(nperm)
+    out = _Obj(chrom=[], level=np.zeros(0, np.int64), total=np.zeros(0), p_value=np.zeros(0), curves=[],
+               null_totals=np.zeros((0, nperm)), seed=[], skipped=skipped)
+    if not problems:
+        return out
+    lens = np.array([pr["tx"].size for pr in problems], dtype=np.int64)
+    off = np.concatenate(([0], np.cumsum(lens)))
+    nbad = np.array([pr["bad"].size for pr in problems], dtype=np.int64)
+    res = ctx.difft_multi(off, np.concatenate([pr["tx"] for pr in problems]), np.concatenate([pr["ty"] for pr in problems]),
+                          [pr["pad_left"] for pr in problems], [pr["pad_right"] for pr in problems],
+                          [pr["ntads"] for pr in problems], np.concatenate(([0], np.cumsum(nbad))),
+                          np.concatenate([pr["bad"] for pr in problems]), seed=seed, nperm=nperm)
+    keep = []
+    for p, pr in enumerate(problems):
+        if res["status"][p] != _lib.TP_OK:
+            skipped[(pr["chrom"], pr["level"])] = (
+                f"the library refused it: random_bed cannot draw {pr['ntads'] - 1} borders from {_population(pr)} "
+                "candidate bins (sample() errors here, R/DiffT.R:69)")
+            continue
+        keep.append(p)
+    keep = np.array(keep, dtype=np.int64)
+    null = res["null_totals"][keep]
+    total = res["totals"][keep]
+    out.chrom = [problems[p]["chrom"] for p in keep]
+    out.level = np.array([problems[p]["level"] for p in keep], dtype=np.int64)
+    out.total = total
+    out.p_value = (1 + (null <= total[:, None]).sum(axis=1)) / (nperm + 1)
+    out.curves = [res["curves"][off[p]:off[p + 1]] for p in keep]
+    out.null_totals = null
+    out.seed = [(int(seed) + int(p)) % 2 ** 64 for p in keep]
     return out
