@@ -81,9 +81,12 @@ long long tp_ctx_launches(tp_ctx *ctx);
  * "shard_sym" (0: ranks of a sharded call compute full-width row blocks of the symmetric products),
  * "mgram_min_n" (smallest nf whose M = Xc Xc^T is formed by the sliced int8 Gram; 0 = FP64 DMMA),
  * "io_bn32" (operator applications on 32-column tiles: -1 auto, 0 never, 1 always),
+ * "batch_resident" (1: batch and genome calls keep resident stores for tp_batch_recall, see there; default 0),
  * "upload_lanes" (helper threads that stage a pageable host matrix or pixel array of 64 MB and more through pinned
  * buffers, default 4; 0 = leave pageable memory to the driver's own staging) */
 int tp_ctx_set(tp_ctx *ctx, const char *key, double value);
+/* the current value of a tp_ctx_set key (TP_ERR_ARG for an unknown key) */
+int tp_ctx_get(tp_ctx *ctx, const char *key, double *value_out);
 /* The environment variable TADPOLE_TUNE="key=value,key=value" applies tp_ctx_set to every context at creation. */
 /* per-stage device milliseconds of the last tp_call / stage call, measured with CUDA events on
  * the context stream: [0] filter [1] compact [2] correlation [3] pca [4] sweep (CONISS) [5] CH
@@ -347,6 +350,34 @@ int tp_genome_free(tp_genome *g);
  * Outputs as tp_call_arm. */
 int tp_recall(tp_ctx *ctx, int max_pcs, int min_clusters, int *k_out, int *n_pcs_out, int *n_clusters_out,
               int *maxlev_out, double *seqdist_out);
+
+/* ---- the same handle for batches and genome-wide calls ----------------------------------------------------------------
+ * With tp_ctx_set(ctx, "batch_resident", 1), tp_call_batch and tp_call_genome on ctx keep a resident store for every
+ * item that succeeds and for every arm: the item's PC scores (nf x k_full, in the worker's row-major layout with k_full
+ * rounded up to 8 columns) and the seqdist of all k candidates of its sweep (k x (nf - 1), each row padded to a multiple
+ * of 8), on the device whose worker ran it.  Cost: 16 bytes per (good bin x PC computed) plus that padding, e.g. about
+ * 0.9 GB for a human genome at 10 kb with max_pcs = 200 (arithmetic, not measured).  The store belongs to the returned
+ * tp_batch and is released by the last tp_batch_free that refers to it, before or after the context is destroyed.  An
+ * item whose store cannot be allocated fails with TP_ERR_NOMEM.  Default 0: no store.
+ *
+ * tp_batch_recall: tp_recall on each selected part of src -- items[s] with parts[s] = -1 for the item (both arms of a
+ * split item) or 0 / 1 for its p / q arm -- run in the worker threads of tp_call_batch (`inflight` per device).  The
+ * result is a tp_batch of nsel items read with tp_batch_dims / tp_batch_get / tp_batch_split: item s is what the batch
+ * call gives for that part, computed from its resident PC scores (for a selected arm, the arm as item s, part -1).  It
+ * equals a fresh call with max_pcs = the source's followed by tp_recall bit for bit (the same sweep and CH kernels on the
+ * same scores).  Its items share the source's score stores and hold stores of their own new dendrograms, so a recall can
+ * be recalled again.  Errors are per item: max_pcs above the item's k_full is tp_recall's TP_ERR_ARG, no level
+ * TP_ERR_NOLEVEL; a part that failed, does not exist or holds no store, or whose store is on a device the context does
+ * not have, is TP_ERR_ARG.  The store is installed on another device of the context with cudaMemcpyPeerAsync. */
+int tp_batch_recall(tp_ctx *ctx, const tp_batch *src, const int *items, const int *parts, int nsel, int max_pcs,
+                    int min_clusters, int inflight, tp_batch **out);
+/* the seqdist (nf - 1 doubles) of candidate cand (0-based: cand + 1 PCs) of a resident item or arm */
+int tp_batch_dendro(const tp_batch *b, int item, int part, int cand, double *seqdist_out);
+/* device bytes of the resident stores a batch refers to, each store counted once (0 without "batch_resident") */
+long long tp_batch_resident_bytes(const tp_batch *b);
+/* the devices of an item's (or arm's) two stores: its PC scores, and its dendrograms -- the device that ran it.  For an
+ * item of tp_batch_recall the two differ when the recall ran on another device than the store it was made from. */
+int tp_batch_resident_devices(const tp_batch *b, int item, int part, int *scores_device_out, int *dendro_device_out);
 
 /* ---- stage 6: diffT (R/DiffT.R:41-49) on padded label vectors -------------------------------------
  * labels_x / labels_y: npairs x L int32 row-major (0 = uncovered bin); out: npairs x L doubles =

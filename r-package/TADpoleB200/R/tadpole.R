@@ -167,24 +167,67 @@ TADpole <- function(mat_file, max_pcs = 200, min_clusters = 2, bad_frac = 0.01,
 # library's own threads over every GPU of options(tadpole.gpus); same objects, same order, as calling TADpole() on each
 # centromere_search = TRUE: every matrix is split at its centromere and both arms run in those threads; a matrix that does
 # not split stops, as TADpole(centromere_search = TRUE) does
-TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L, centromere_search = FALSE) {
+# resident = TRUE: every object keeps its PC scores and all its candidates' dendrograms on the GPU (16 bytes per good bin
+# and PC), so tadpole_recall() and tadpole_dendro() accept it (and tadpole_dendro() each arm); the memory goes with the
+# last object that refers to it.
+TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L, centromere_search = FALSE,
+                          resident = FALSE) {
     ctx <- .tp_ctx()
     mats <- lapply(mats, function(m) if (is.character(m)) {
         .Call(C_tp_ingest, ctx, path.expand(m)); .Call(C_tp_ingested_matrix, ctx) } else as.matrix(m) + 0)
     if (centromere_search) {
-        res <- .Call(C_tp_call_batch_arms, ctx, mats, as.integer(max_pcs), as.integer(min_clusters), as.numeric(bad_frac),
-                     as.integer(inflight))
-        return(lapply(res, function(r) {
+        res <- .tp_with_resident(ctx, resident, function()
+            .Call(C_tp_call_batch_arms, ctx, mats, as.integer(max_pcs), as.integer(min_clusters), as.numeric(bad_frac),
+                  as.integer(inflight)))
+        return(lapply(seq_along(res$items), function(i) {
+            r <- res$items[[i]]
             if (is.character(r)) stop(r)
-            .tp_arms_batch_object(r)
+            .tp_attach(.tp_arms_batch_object(r), res$batch, i - 1L)
         }))
     }
-    res <- .Call(C_tp_call_batch, ctx, mats, as.integer(max_pcs), as.integer(min_clusters), as.numeric(bad_frac),
-                 as.integer(inflight))
-    lapply(res, function(r) {
+    res <- .tp_with_resident(ctx, resident, function()
+        .Call(C_tp_call_batch, ctx, mats, as.integer(max_pcs), as.integer(min_clusters), as.numeric(bad_frac),
+              as.integer(inflight)))
+    lapply(seq_along(res$items), function(i) {
+        r <- res$items[[i]]
         if (is.character(r)) stop(r)
-        .tp_batch_object(r)
+        .tp_attach(.tp_batch_object(r), res$batch, i - 1L)
     })
+}
+
+# a batch or genome .Call with "batch_resident" = resident on ctx (the previous value restored): list(items, batch), where
+# batch is the external pointer on the resident batch (NULL without resident)
+.tp_with_resident <- function(ctx, resident, call) {
+    prev <- .Call(C_tp_ctx_set, ctx, "batch_resident", as.numeric(isTRUE(resident)))
+    on.exit(.Call(C_tp_ctx_set, ctx, "batch_resident", prev))
+    res <- call()
+    if (!isTRUE(resident)) return(list(items = res, batch = NULL))
+    list(items = res[-length(res)], batch = res[[length(res)]])
+}
+
+# attr(, "resident") of an object read from item `item` (0-based) of a resident batch: list(batch, item, part, keep);
+# a split object gets part -1 (tadpole_recall recalls both arms), each arm part 0 / 1 and its kept bins
+.tp_attach <- function(obj, batch, item) {
+    if (is.null(batch)) return(obj)
+    if (!is.null(obj[["p"]])) {
+        for (a in c("p", "q"))
+            attr(obj[[a]], "resident") <- list(batch = batch, item = item, part = if (a == "p") 0L else 1L,
+                                               keep = as.integer(obj[[a]]$dendro$labels))
+        attr(obj, "resident") <- list(batch = batch, item = item, part = -1L, keep = NULL)
+    } else {
+        attr(obj, "resident") <- list(batch = batch, item = item, part = -1L, keep = as.integer(obj$dendro$labels))
+    }
+    obj
+}
+
+# the object and messages of one genome item (C_tp_call_genome[_arms], C_tp_batch_recall)
+.tp_item_object <- function(r) {
+    if (length(r) == 4L) return(.tp_arms_batch_object(r))       # split at the centromere: list(bad, centromere, p, q)
+    message(paste(sum(r[[1L]]), "bad columns found at position(s):"))
+    message(paste(which(r[[1L]]), collapse = " "))
+    message(paste("Optimal number of PCs:", r[[2L]]))
+    message(paste("Optimal number of clusters:", r[[3L]]))
+    .tp_batch_object(r)
 }
 
 # the tadpole object of one item of a batch (C_tp_call_batch, C_tp_call_genome)
@@ -223,7 +266,7 @@ TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01
 # of the chromosomes whose call failed.  centromere_search = TRUE: as TADpole(centromere_search = TRUE) on each
 # chromosome; one that does not split fails.
 TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L,
-                           centromere_search = FALSE) {
+                           centromere_search = FALSE, resident = FALSE) {
     stopifnot(inherits(pixels, "tadpole_pixels"))
     ctx <- .tp_ctx()
     tab <- .tp_bin_table(bins)
@@ -232,32 +275,56 @@ TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clust
     if (anyNA(idx)) stop("unknown chromosome(s): ", paste(sel[is.na(idx)], collapse = ", "))
     g <- if (is.null(pixels$path)) .Call(C_tp_genome, ctx, tab$n, pixels$bin1, pixels$bin2, pixels$count, pixels$index_base)
          else .Call(C_tp_genome_file, ctx, tab$n, path.expand(pixels$path), pixels$index_base)
-    res <- if (centromere_search)
+    res <- .tp_with_resident(ctx, resident, function() if (centromere_search)
         .Call(C_tp_call_genome_arms, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
               as.numeric(bad_frac), as.integer(inflight), FALSE)
     else .Call(C_tp_call_genome, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
-               as.numeric(bad_frac), as.integer(inflight), TRUE)
+               as.numeric(bad_frac), as.integer(inflight), TRUE))
+    .tp_genome_list(sel, res$items, res$batch, list())
+}
+
+# the named list TADpole_genome() returns from the items of a genome call or recall; failed: the earlier failures
+.tp_genome_list <- function(sel, items, batch, failed) {
     out <- list()
-    failed <- list()
     for (i in seq_along(sel)) {
         message(paste("Processing chromosome", sel[i]))
-        r <- res[[i]]
+        r <- items[[i]]
         if (is.character(r)) { failed[[sel[i]]] <- r; next }
-        if (centromere_search) { out[[sel[i]]] <- .tp_arms_batch_object(r); next }
-        message(paste(sum(r[[1L]]), "bad columns found at position(s):"))
-        message(paste(which(r[[1L]]), collapse = " "))
-        message(paste("Optimal number of PCs:", r[[2L]]))
-        message(paste("Optimal number of clusters:", r[[3L]]))
-        out[[sel[i]]] <- .tp_batch_object(r)
+        out[[sel[i]]] <- .tp_attach(.tp_item_object(r), batch, i - 1L)
     }
     attr(out, "failed") <- failed
     out
+}
+
+# TADpole_genome() again with another max_pcs (<= the one computed) / min_clusters on every chromosome of a result of
+# TADpole_genome(resident = TRUE), or on `chroms`, in one .Call: only the n_pcs sweep and the selection run.  Shaped like
+# TADpole_genome()'s result; attr(, "failed") = the earlier failures plus this recall's.
+tadpole_genome_recall <- function(result, max_pcs = 200, min_clusters = 2, chroms = NULL) {
+    sel <- if (is.null(chroms)) names(result) else as.character(chroms)
+    miss <- setdiff(sel, names(result))
+    if (length(miss)) stop("chromosome(s) not in this result: ", paste(miss, collapse = ", "))
+    hs <- lapply(sel, function(nm) attr(result[[nm]], "resident"))
+    if (any(vapply(hs, function(h) is.null(h$batch), TRUE))) stop("this tadpole object carries no device handle")
+    if (!all(vapply(hs, function(h) identical(h$batch, hs[[1L]]$batch), TRUE)))
+        stop("the chromosomes come from different genome calls: recall them separately")
+    failed <- attr(result, "failed")
+    if (!length(sel)) return(structure(list(), failed = failed))
+    res <- .Call(C_tp_batch_recall, .tp_ctx(), hs[[1L]]$batch, vapply(hs, function(h) as.integer(h$item), 0L),
+                 rep(-1L, length(sel)), as.integer(max_pcs), as.integer(min_clusters))
+    .tp_genome_list(sel, res[-length(res)], res[[length(res)]], failed)
 }
 
 # the n_pcs sweep again with another max_pcs / min_clusters on the PC scores that are still on the GPU
 tadpole_recall <- function(tadpole, max_pcs = 200, min_clusters = 2) {
     h <- attr(tadpole, "resident")
     if (is.null(h)) stop("this tadpole object carries no device handle")
+    if (!is.null(h$batch)) {            # an object of TADpole_batch / TADpole_genome(resident = TRUE)
+        if (h$part >= 0L) stop("recall the whole centromere_search object (both arms); its arms offer tadpole_dendro()")
+        res <- .Call(C_tp_batch_recall, .tp_ctx(), h$batch, as.integer(h$item), -1L, as.integer(max_pcs),
+                     as.integer(min_clusters))
+        if (is.character(res[[1L]])) stop(res[[1L]])
+        return(.tp_attach(.tp_item_object(res[[1L]]), res[[2L]], 0L))
+    }
     # the shim stops when the context has been used for another matrix since (generation), and sizes every buffer from
     # the context, never from this object
     res <- .Call(C_tp_recall, h$ctx, h$generation, as.integer(max_pcs), as.integer(min_clusters))
@@ -273,6 +340,11 @@ tadpole_recall <- function(tadpole, max_pcs = 200, min_clusters = 2) {
 tadpole_dendro <- function(tadpole, n_pcs) {
     h <- attr(tadpole, "resident")
     if (is.null(h)) stop("this tadpole object carries no device handle")
+    if (!is.null(h$batch)) {
+        if (is.null(h$keep)) stop("a centromere_search object has no dendrogram of its own: use its arms p / q")
+        return(.tp_dendro(.Call(C_tp_batch_dendro, h$batch, as.integer(h$item), as.integer(h$part), as.integer(n_pcs)),
+                          h$keep))
+    }
     .tp_dendro(.Call(C_tp_dendro, h$ctx, h$generation, as.integer(n_pcs)), h$part$keep)
 }
 

@@ -394,6 +394,35 @@ static SEXP arms_item(tp_batch *b, int i) {
     return item;
 }
 
+static void batch_finalizer(SEXP p) {
+    tp_batch *b = (tp_batch *)R_ExternalPtrAddr(p);
+    if (b) {
+        tp_batch_free(b);
+        R_ClearExternalPtr(p);
+    }
+}
+
+/* list(item 0, ..., item n-1) of a batch as arms_item reads them; with `keep` the batch itself follows as element n, an
+ * external pointer whose finalizer frees it (its resident stores live as long as an R object refers to it), otherwise
+ * the batch is freed here */
+static SEXP batch_items(tp_batch *b, int n, int keep) {
+    SEXP p = PROTECT(keep ? R_MakeExternalPtr(b, R_NilValue, R_NilValue) : R_NilValue);
+    if (keep) R_RegisterCFinalizerEx(p, batch_finalizer, TRUE);
+    /* (without keep, an R allocation failure below longjmps past tp_batch_free: the batch, plain host memory, leaks) */
+    SEXP out = PROTECT(allocVector(VECSXP, n + (keep ? 1 : 0)));
+    for (int i = 0; i < n; i++) SET_VECTOR_ELT(out, i, arms_item(b, i));
+    if (keep) SET_VECTOR_ELT(out, n, p);
+    else tp_batch_free(b);
+    UNPROTECT(2);
+    return out;
+}
+
+/* is "batch_resident" set on the context (TADpole_batch / TADpole_genome with resident = TRUE)? */
+static int resident_on(tp_ctx *c) {
+    double v = 0.0;
+    return tp_ctx_get(c, "batch_resident", &v) == TP_OK && v != 0.0;
+}
+
 /* TADpole() on a list of matrices, `inflight` calls per device kept in flight by the library's own threads over every
  * device of the context (tp_call_batch with `centromere`); this thread only waits.  Per matrix: arms_item, or a character
  * error message. */
@@ -412,16 +441,12 @@ static SEXP call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEX
     if (tp_call_batch(c, nc, ptr, n, 1, 0, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac), asInteger(inflight),
                       1, centromere, &b) != TP_OK)
         error("%s", tp_last_error());
-    /* (an R allocation failure below longjmps past tp_batch_free: the batch, plain host memory, is then leaked) */
-    SEXP out = PROTECT(allocVector(VECSXP, nc));
-    for (int i = 0; i < nc; i++) SET_VECTOR_ELT(out, i, arms_item(b, i));
-    tp_batch_free(b);
-    UNPROTECT(1);
-    return out;
+    return batch_items(b, nc, resident_on(c));
 }
 
 /* Per matrix: list(bad, n_pcs, optimal_n_clusters, seqdist, scores, levels, tables = list of 2-column (start, end)
- * matrices), or a character error message. */
+ * matrices), or a character error message; with "batch_resident" set (C_tp_ctx_set) the batch follows as a last
+ * element (an external pointer for C_tp_batch_recall / C_tp_batch_dendro).  The same holds for the routines below. */
 SEXP C_tp_call_batch(SEXP ctx, SEXP mats, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight) {
     return call_batch(ctx, mats, max_pcs, min_clusters, bad_frac, inflight, 0);
 }
@@ -499,11 +524,58 @@ static SEXP call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP m
     if (tp_call_genome(c, g, INTEGER(chroms), ns, asInteger(max_pcs), asInteger(min_clusters), asReal(bad_frac),
                        asInteger(inflight), tables, centromere, &b) != TP_OK)
         error("%s", tp_last_error());
-    SEXP out = PROTECT(allocVector(VECSXP, ns));
-    for (int i = 0; i < ns; i++) SET_VECTOR_ELT(out, i, arms_item(b, i));
-    tp_batch_free(b);
+    return batch_items(b, ns, resident_on(c));
+}
+
+/* tp_ctx_set(ctx, key, value); returns the key's previous value (so that the R host can restore it) */
+SEXP C_tp_ctx_set(SEXP ctx, SEXP key, SEXP value) {
+    tp_ctx *c = ctx_of(ctx);
+    if (length(key) != 1) error("TADpole: the key must be one string");
+    double prev = 0.0;
+    if (tp_ctx_get(c, CHAR(STRING_ELT(key, 0)), &prev) != TP_OK || tp_ctx_set(c, CHAR(STRING_ELT(key, 0)), asReal(value)) != TP_OK)
+        error("%s", tp_last_error());
+    SEXP out = PROTECT(allocVector(REALSXP, 1));
+    REAL(out)[0] = prev;
     UNPROTECT(1);
     return out;
+}
+
+static tp_batch *batch_of(SEXP p) {
+    tp_batch *b = (tp_batch *)R_ExternalPtrAddr(p);
+    if (!b) error("TADpole: the resident batch has been released");
+    return b;
+}
+
+/* tp_batch_recall of items (0-based) / parts (-1 = the item, 0 / 1 = an arm) of a resident batch, 8 recalls in flight per
+ * device (TADpole_genome()'s default): per selection what arms_item gives (a character message for a selection that
+ * failed), then the new batch as the last element (it shares the source's PC scores and holds its own dendrograms). */
+SEXP C_tp_batch_recall(SEXP ctx, SEXP batch, SEXP items, SEXP parts, SEXP max_pcs, SEXP min_clusters) {
+    tp_ctx *c = ctx_of(ctx);
+    tp_batch *src = batch_of(batch);
+    if (!isInteger(items) || !isInteger(parts) || length(items) != length(parts))
+        error("TADpole: items and parts must be integer vectors of equal length");
+    int ns = length(items);
+    tp_batch *b = NULL;
+    if (tp_batch_recall(c, src, INTEGER(items), INTEGER(parts), ns, asInteger(max_pcs), asInteger(min_clusters), 8, &b) !=
+        TP_OK)
+        error("%s", tp_last_error());
+    return batch_items(b, ns, 1);
+}
+
+/* seqdist of the candidate that clusters on the first n_pcs PCs (1-based) of item (0-based) / part of a resident batch;
+ * the buffer is sized from the batch (tp_batch_dims), never from the R object */
+SEXP C_tp_batch_dendro(SEXP batch, SEXP item, SEXP part, SEXP n_pcs) {
+    tp_batch *b = batch_of(batch);
+    int nf = 0, k = 0;
+    if (tp_batch_dims(b, asInteger(item), asInteger(part), NULL, &nf, &k, NULL, NULL, NULL, NULL, NULL) != TP_OK)
+        error("%s", tp_last_error());
+    if (nf < 3) error("TADpole: this item holds no dendrogram");
+    if (asInteger(n_pcs) < 1 || asInteger(n_pcs) > k) error("TADpole: n_pcs must be between 1 and %d", k);
+    SEXP seq = PROTECT(allocVector(REALSXP, nf - 1));
+    int rc = tp_batch_dendro(b, asInteger(item), asInteger(part), asInteger(n_pcs) - 1, REAL(seq));
+    UNPROTECT(1);
+    if (rc != TP_OK) error("%s", tp_last_error());
+    return seq;
 }
 
 /* Per chromosome: what C_tp_call_batch gives for its dense matrix (the per-level tables empty unless `tables`). */
@@ -682,6 +754,9 @@ static const R_CallMethodDef call_table[] = {
     {"C_tp_comm_unique_id", (DL_FUNC)&C_tp_comm_unique_id, 0},
     {"C_tp_ctx_comm_init", (DL_FUNC)&C_tp_ctx_comm_init, 5},
     {"C_tp_ctx_comm_select", (DL_FUNC)&C_tp_ctx_comm_select, 2},
+    {"C_tp_ctx_set", (DL_FUNC)&C_tp_ctx_set, 3},
+    {"C_tp_batch_recall", (DL_FUNC)&C_tp_batch_recall, 6},
+    {"C_tp_batch_dendro", (DL_FUNC)&C_tp_batch_dendro, 4},
     {NULL, NULL, 0}};
 
 void R_init_TADpoleB200(DllInfo *dll) {

@@ -5,6 +5,7 @@ product fails loudly.  Nothing under oracle/ is imported here.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 import os
 from ctypes import POINTER, c_char_p, c_double, c_int, c_int32, c_longlong, c_uint8, c_void_p
@@ -31,7 +32,8 @@ EXPORTED = [
     "tp_ctx_create_multi", "tp_device_count", "tp_ctx_devices", "tp_ctx_generation", "tp_ctx_dims", "tp_call_arms", "tp_call_batch",
     "tp_batch_size", "tp_batch_device_ms", "tp_batch_launches", "tp_batch_status", "tp_batch_error", "tp_batch_dims", "tp_batch_get", "tp_batch_free", "tp_find_groups",
     "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
-    "tp_centromere_split", "tp_batch_split",
+    "tp_centromere_split", "tp_batch_split", "tp_batch_recall", "tp_batch_dendro", "tp_batch_resident_bytes",
+    "tp_batch_resident_devices", "tp_ctx_get",
 ]
 
 
@@ -76,6 +78,10 @@ def load():
         "tp_batch_get": (c_int, [vp, c_int, c_int, u8p, ip, ip, dp, dp, ip, ip, ip, ip, dp, ip, ip, ip]),
         "tp_batch_free": (c_int, [vp]),
         "tp_batch_split": (c_int, [vp, c_int, ip, ip, ip, u8p]),
+        "tp_batch_recall": (c_int, [vp, vp, ip, ip, c_int, c_int, c_int, c_int, POINTER(vp)]),
+        "tp_batch_dendro": (c_int, [vp, c_int, c_int, c_int, dp]),
+        "tp_batch_resident_bytes": (c_longlong, [vp]),
+        "tp_batch_resident_devices": (c_int, [vp, c_int, c_int, ip, ip]),
         "tp_centromere_split": (c_int, [u8p, c_int, c_int, ip, ip, ip, ip, ip, ip, ip, ip, ip, ip, ip]),
         "tp_genome_ingest": (c_int, [vp, ip, c_int, ip, ip, dp, ctypes.c_size_t, c_int, POINTER(vp)]),
         "tp_genome_ingest_file": (c_int, [vp, ip, c_int, c_char_p, c_int, c_int, POINTER(vp)]),
@@ -89,6 +95,7 @@ def load():
         "tp_ctx_stream": (vp, [vp]),
         "tp_ctx_launches": (c_longlong, [vp]),
         "tp_ctx_set": (c_int, [vp, c_char_p, c_double]),
+        "tp_ctx_get": (c_int, [vp, c_char_p, dp]),
         "tp_ctx_timings": (c_int, [vp, dp]),
         "tp_ctx_profile": (c_int, [vp, c_int, dp, POINTER(c_longlong)]),
         "tp_ingest_tsv": (c_int, [vp, c_char_p, ctypes.c_size_t, c_int, ip]),
@@ -226,6 +233,11 @@ class Context:
     # ---- plumbing ----
     def set(self, key, value):
         check(self.lib.tp_ctx_set(self._h, key.encode(), float(value)))
+
+    def get(self, key):
+        v = c_double(0.0)
+        check(self.lib.tp_ctx_get(self._h, key.encode(), ctypes.byref(v)))
+        return v.value
 
     def sync(self):
         check(self.lib.tp_ctx_sync(self._h))
@@ -565,7 +577,7 @@ class Context:
         return dict(bad=bad.astype(bool), **item, device_ms=ms.value)
 
     def call_batch(self, mats, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True, device_ptrs=None, n=None,
-                   centromere_search=False, centromere_fix=False):
+                   centromere_search=False, centromere_fix=False, resident=False):
         """tp_call_batch: one tp_call per matrix, `inflight` calls per device kept in flight by library-owned threads over
         every device of the context.  mats: list of square float64 arrays (all C or all F order); or device_ptrs + n
         (row-major, single-device contexts).  Returns a list of dicts as call() returns, plus 'tables' {level: [rows, 2]}
@@ -573,7 +585,8 @@ class Context:
         centromere_search: each matrix split at its centromere and its two arms called in the same workers, tables always
         built; a split matrix's entry is dict(split=True, centromere (1-based bins), bad, device_ms, p, q) with p / q as
         _batch_item reads an arm, an unsplit one's (centromere_fix) the dict above plus split=False and centromere, and
-        one that does not split without centromere_fix fails with TP_ERR_NOSPLIT."""
+        one that does not split without centromere_fix fails with TP_ERR_NOSPLIT.
+        resident: "batch_resident" for this call; returns (results, ResidentBatch) instead of the results."""
         if device_ptrs is None:
             mats = [m if (m.dtype == np.float64 and (m.flags.c_contiguous or m.flags.f_contiguous))
                     else np.ascontiguousarray(m, dtype=np.float64) for m in (np.asarray(m) for m in mats)]
@@ -590,10 +603,21 @@ class Context:
         ncalls = int(ns.size)
         h = c_void_p()
         tables = bool(tables or centromere_search)
-        check(self.lib.tp_call_batch(self._h, ncalls, ptrs, _ip(ns), colmajor, ondev, int(max_pcs), int(min_clusters),
-                                     float(bad_frac), int(inflight), int(tables), _centromere(centromere_search, centromere_fix),
-                                     ctypes.byref(h)))
-        return self._batch_results(h, ncalls, tables)
+        with self._resident(resident):
+            check(self.lib.tp_call_batch(self._h, ncalls, ptrs, _ip(ns), colmajor, ondev, int(max_pcs), int(min_clusters),
+                                         float(bad_frac), int(inflight), int(tables),
+                                         _centromere(centromere_search, centromere_fix), ctypes.byref(h)))
+        return self._batch_results(h, ncalls, tables, resident)
+
+    @contextlib.contextmanager
+    def _resident(self, on):
+        """"batch_resident" = on for the batch or genome call inside the block only; the previous value is restored."""
+        prev = self.get("batch_resident")
+        self.set("batch_resident", int(bool(on)))
+        try:
+            yield
+        finally:
+            self.set("batch_resident", prev)
 
     def _split_state(self, h, i, n):
         """(split: -1 / 0 / 1, the longest bad stretch cs..ce (1-based bins) or None, bad flags or None) of item i
@@ -605,9 +629,11 @@ class Context:
         return (sp.value, np.arange(cs.value, ce.value + 1) if cs.value else None,
                 bad[:n].astype(bool) if sp.value >= 0 else None)
 
-    def _batch_results(self, h, ncalls, tables):
-        """Every item of a tp_batch (freed here) as call_batch returns them."""
+    def _batch_results(self, h, ncalls, tables, resident=False):
+        """Every item of a tp_batch as call_batch returns them; the batch is freed here, or with resident kept by the
+        ResidentBatch returned beside them."""
         out = []
+        keep = ResidentBatch(self, h) if resident else None
         self.last_batch_device_ms = float(self.lib.tp_batch_device_ms(h))
         self.last_batch_launches = int(self.lib.tp_batch_launches(h))
         try:
@@ -637,8 +663,9 @@ class Context:
                     item.update(split=False, centromere=cen)
                 out.append(item)
         finally:
-            self.lib.tp_batch_free(h)
-        return out
+            if keep is None:
+                self.lib.tp_batch_free(h)
+        return out if keep is None else (out, keep)
 
     # ---- genome-wide input ----
     def genome_ingest(self, chrom_bins, bin1=None, bin2=None, count=None, index_base=0, path=None, sep="\t"):
@@ -660,16 +687,17 @@ class Context:
         return Genome(self, h, cb)
 
     def call_genome(self, genome, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True,
-                    centromere_search=False, centromere_fix=False):
+                    centromere_search=False, centromere_fix=False, resident=False):
         """tp_call_genome: one call per selected chromosome (0-based indices, default all), results in that order as
-        call_batch returns them (a failed call's entry is the TadpoleError), with centromere_search too."""
+        call_batch returns them (a failed call's entry is the TadpoleError), with centromere_search and resident too."""
         sel = np.arange(genome.chrom_bins.size, dtype=np.int32) if chroms is None else np.ascontiguousarray(chroms, dtype=np.int32)
         h = c_void_p()
         tables = bool(tables or centromere_search)
-        check(self.lib.tp_call_genome(self._h, genome._h, _ip(sel), int(sel.size), int(max_pcs), int(min_clusters),
-                                      float(bad_frac), int(inflight), int(tables), _centromere(centromere_search, centromere_fix),
-                                      ctypes.byref(h)))
-        return self._batch_results(h, int(sel.size), tables)
+        with self._resident(resident):
+            check(self.lib.tp_call_genome(self._h, genome._h, _ip(sel), int(sel.size), int(max_pcs), int(min_clusters),
+                                          float(bad_frac), int(inflight), int(tables),
+                                          _centromere(centromere_search, centromere_fix), ctypes.byref(h)))
+        return self._batch_results(h, int(sel.size), tables, resident)
 
     def recall(self, nf, max_pcs=200, min_clusters=2):
         """tp_recall: the n_pcs sweep and the selection again on the PC scores resident in the context."""
@@ -735,6 +763,66 @@ class Context:
 
     def difft_batch_dev(self, lx_ptr, ly_ptr, L, npairs, out_ptr):
         check(self.lib.tp_difft_batch(self._h, int(lx_ptr), int(ly_ptr), int(L), int(npairs), 1, int(out_ptr)))
+
+
+class ResidentBatch:
+    """A tp_batch whose items keep their resident stores (PC scores and every candidate's dendrogram, "batch_resident").
+    Objects read from it hold a reference; the batch is freed with the last one.  Recalls run on the context of the call
+    that made it, or -- after detach() -- on a context of their own, made for the recall on the same devices and closed
+    after it, so that the batch holds nothing but its stores."""
+
+    def __init__(self, ctx, h):
+        self.ctx, self.lib, self._h, self.devices = ctx, ctx.lib, h, list(ctx.devices)
+
+    def detach(self):
+        """Forget the context (the caller closes it): the stores outlive it."""
+        self.ctx = None
+        return self
+
+    def devices_of(self, item, part=-1):
+        """(device of the PC scores, device of the dendrograms) of an item or arm (tp_batch_resident_devices)"""
+        a, b = c_int(0), c_int(0)
+        check(self.lib.tp_batch_resident_devices(self._h, int(item), int(part), ctypes.byref(a), ctypes.byref(b)))
+        return a.value, b.value
+
+    def nbytes(self):
+        """device bytes of the stores this batch refers to (tp_batch_resident_bytes)"""
+        return int(self.lib.tp_batch_resident_bytes(self._h))
+
+    def recall(self, items, parts=None, max_pcs=200, min_clusters=2, inflight=4):
+        """tp_batch_recall of the selected items (parts: -1 = the item, 0 / 1 = an arm; default -1): (results as
+        call_batch returns them, the ResidentBatch that holds them)."""
+        it = np.ascontiguousarray(items, dtype=np.int32)
+        pt = np.full(it.size, -1, np.int32) if parts is None else np.ascontiguousarray(parts, dtype=np.int32)
+        if pt.size != it.size:
+            raise ValueError("items and parts: equal lengths expected")
+        ctx = self.ctx or Context(self.devices if len(self.devices) > 1 else self.devices[0])
+        try:
+            h = c_void_p()
+            check(self.lib.tp_batch_recall(ctx._h, self._h, _ip(it), _ip(pt), int(it.size), int(max_pcs),
+                                           int(min_clusters), int(inflight), ctypes.byref(h)))
+            out, store = ctx._batch_results(h, int(it.size), True, resident=True)
+        finally:
+            if self.ctx is None:
+                ctx.close()
+        return out, (store.detach() if self.ctx is None else store)
+
+    def dendro(self, item, part, cand, nf):
+        """seqdist of candidate cand (0-based) of item / arm (tp_batch_dendro)"""
+        seq = np.empty(max(nf - 1, 0))
+        check(self.lib.tp_batch_dendro(self._h, int(item), int(part), int(cand), _dp(seq)))
+        return seq
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self.lib.tp_batch_free(self._h)
+            self._h = c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class Genome:

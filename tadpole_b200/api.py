@@ -190,12 +190,16 @@ class Tadpole(_Obj):
     Beyond the reference: a whole-chromosome object is also a handle on the pipeline state that stays in HBM
     (PC scores, all k dendrograms): recall() repeats only the n_pcs sweep for another max_pcs / min_clusters, and
     dendro_for() returns the dendrogram of any candidate number of PCs (what CH_map / plot_hierarchy browse),
-    as long as the context has not been used for another matrix since."""
+    as long as the context has not been used for another matrix since.  The objects of TADpole_batch / TADpole_genome
+    with resident=True are such handles too, on stores of their own that no later call replaces; there recall() of a
+    centromere_search result recalls both arms, and each arm has dendro_for()."""
 
     def _resident(self):
         h = object.__getattribute__(self, "__dict__").get("_handle")
         if h is None:
             raise RuntimeError("this tadpole object carries no device handle (centromere_search results do not)")
+        if "batch" in h:
+            return h
         if h["ctx"].generation != h["generation"]:
             raise RuntimeError("the GPU context has been used for another matrix since this call; its resident state is gone")
         return h
@@ -204,6 +208,9 @@ class Tadpole(_Obj):
         """TADpole() again on the same matrix with another max_pcs (<= the one computed) / min_clusters, from the
         resident PC scores: same result as a fresh call, without load_mat, cor and prcomp."""
         h = self._resident()
+        if "batch" in h:
+            res, store = h["batch"].recall([h["item"]], max_pcs=max_pcs, min_clusters=min_clusters, inflight=1)
+            return _recalled_object(res[0], store, 0, h["centromere_fix"])
         res = h["ctx"].recall(h["nf"], max_pcs=max_pcs, min_clusters=min_clusters)
         res["bad"] = h["bad"]
         return _tadpole_from_result(res, h["ctx"])       # the sweep state was replaced: this object is now stale
@@ -211,8 +218,27 @@ class Tadpole(_Obj):
     def dendro_for(self, n_pcs):
         """chclust dendrogram of the candidate that clusters on the first n_pcs PCs (R/TADpole.R:108)."""
         h = self._resident()
+        if "batch" in h:
+            if "names" not in h:
+                raise ValueError("a centromere_search result has no dendrogram of its own: use dendro_for of its arms p / q")
+            return Dendro(h["batch"].dendro(h["item"], h["part"], int(n_pcs) - 1, h["nf"]), labels=h["names"])
         seq, _ = h["ctx"].dendro(int(n_pcs) - 1, h["nf"])
         return Dendro(seq, labels=h["names"])
+
+
+class ResidentArm(_Obj):
+    """An arm (p or q) of a centromere_search result of TADpole_batch / TADpole_genome with resident=True: the arm
+    object of TADpole(centromere_search=True) plus dendro_for() of any candidate number of PCs."""
+    _resident = Tadpole._resident
+    dendro_for = Tadpole.dendro_for
+
+
+def _recalled_object(res, store, i, centromere_fix):
+    """The object of item i of a recall (an exception is raised)."""
+    if isinstance(res, Exception):
+        raise res
+    from .batch import _tadpole_from_batch_item
+    return _tadpole_from_batch_item(res, centromere_fix, (store, i))
 
 
 def _levels_table(res, names, bad_cols):
@@ -297,12 +323,12 @@ def TADpole(mat_file, max_pcs=200, min_clusters=2, bad_frac=0.01, chr=None, star
     return tp
 
 
-def _arm_object(arm, res, names, tables, centromere_fix):
+def _arm_object(arm, res, names, tables, centromere_fix, cls=_Obj):
     """One arm of a centromere_search result (R/TADpole.R:376-408): n_pcs, optimal_n_clusters, dendro and the per-level
     tables as `cluster`; with centromere_fix also `clusters` and `scores`."""
     message(f"Processing arm {arm}")
     _messages_optimal(res)
-    a = _Obj()
+    a = cls()
     a.n_pcs = res["n_pcs"]
     a.optimal_n_clusters = res["n_clusters"]
     a.dendro = Dendro(res["seqdist"], labels=names)

@@ -19,8 +19,8 @@ import os
 import numpy as np
 
 from . import _lib
-from .api import (NOSPLIT_MESSAGE, Tadpole, _Obj, _arm_object, _bed_rows, _difft_labels, _merging_arms, _messages_bad,
-                  _messages_optimal, _messages_split, get_context, message, read_matrix)
+from .api import (NOSPLIT_MESSAGE, ResidentArm, Tadpole, _Obj, _arm_object, _bed_rows, _difft_labels, _merging_arms,
+                  _messages_bad, _messages_optimal, _messages_split, get_context, message, read_matrix)
 from .hclust import Dendro
 
 __all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "TADpole_genome", "read_bins", "diffT_genome"]
@@ -39,29 +39,45 @@ class ContextPool:
         self.ctx.close()
 
 
-def _tadpole_from_batch_item(res, centromere_fix=False):
+def _handle(obj, resident, **kw):
+    """Attach the device handle of item `resident` = (ResidentBatch, item) to obj."""
+    object.__getattribute__(obj, "__dict__")["_handle"] = dict(batch=resident[0], item=resident[1], **kw)
+
+
+def _tadpole_from_batch_item(res, centromere_fix=False, resident=None):
     """The object and the messages TADpole() gives for one item of a batch; a centromere_search item
-    (call_batch(centromere_search=True)) as TADpole(centromere_search=True, centromere_fix=centromere_fix) gives it."""
+    (call_batch(centromere_search=True)) as TADpole(centromere_search=True, centromere_fix=centromere_fix) gives it.
+    resident: (ResidentBatch, item index) of a batch run with resident=True, which the object (and its arms) then keep
+    as their device handle."""
     bad = res["bad"]
     _messages_bad(bad)
     if "split" in res:
         _messages_split(res["centromere"], res["split"])
     if res.get("split"):
         tp = Tadpole()
-        for arm in ("p", "q"):
+        for part, arm in enumerate(("p", "q")):
             a = res[arm]
-            tp[arm] = _arm_object(arm, a, (a["keep"] + 1).astype(np.int32), {str(k): t for k, t in a["tables"].items()},
-                                  centromere_fix)
+            names = (a["keep"] + 1).astype(np.int32)
+            tp[arm] = _arm_object(arm, a, names, {str(k): t for k, t in a["tables"].items()}, centromere_fix,
+                                  ResidentArm if resident else _Obj)
+            if resident:
+                _handle(tp[arm], resident, part=part, nf=int(a["nf"]), names=names)
         tp.merging_arms = _merging_arms(res["p"]["labels"], res["q"]["labels"], res["centromere"].size)
+        if resident:
+            _handle(tp, resident, part=-1, centromere_fix=centromere_fix)
         return tp
     _messages_optimal(res)
     tp = Tadpole()
+    names = (np.flatnonzero(~bad) + 1).astype(np.int32)
     tp.n_pcs = res["n_pcs"]
     tp.optimal_n_clusters = res["n_clusters"]
-    tp.dendro = Dendro(res["seqdist"], labels=(np.flatnonzero(~bad) + 1).astype(np.int32))
+    tp.dendro = Dendro(res["seqdist"], labels=names)
     tp.clusters = {str(k): t for k, t in res["tables"].items()}
     tp.scores = res["scores"]
-    return tp                          # no device handle: the per-call contexts are reused by the next call
+    if resident:
+        _handle(tp, resident, part=-1, nf=int(names.size), names=names, centromere_fix=centromere_fix)
+    # without resident no device handle: the per-call contexts are reused by the next call
+    return tp
 
 
 def _failed_item(err):
@@ -74,11 +90,15 @@ def _failed_item(err):
 
 
 def TADpole_batch(mat_files, max_pcs=200, min_clusters=2, bad_frac=0.01, centromere_search=False, pool=None,
-                  device=0, streams=4, ctx=None, centromere_fix=False):
+                  device=0, streams=4, ctx=None, centromere_fix=False, resident=False):
     """TADpole() on every matrix of `mat_files` (paths or arrays), `streams` calls in flight per GPU.  centromere_search
     (and centromere_fix, see TADpole()): every matrix is split at its centromere and both arms are called in the library's
     workers; the objects and messages are TADpole(centromere_search=True)'s, and the first matrix TADpole() would fail on
-    raises its exception."""
+    raises its exception.
+    resident: every object keeps its PC scores and all its candidates' dendrograms in HBM (16 bytes per good bin and PC
+    computed), so recall() and dendro_for() work on it (and dendro_for() on its arms) as on TADpole()'s objects; that
+    memory is released with the last object.  Recalls run on the given pool or ctx, or else on a context made for each
+    recall: a context this function makes for the call is closed when it returns, as without resident."""
     own = pool is None and ctx is None
     if ctx is None:
         pool = pool or ContextPool(device, streams)
@@ -86,18 +106,22 @@ def TADpole_batch(mat_files, max_pcs=200, min_clusters=2, bad_frac=0.01, centrom
     try:
         mats = [read_matrix(m, ctx) for m in mat_files]
         res = ctx.call_batch(mats, max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac, inflight=streams,
-                             centromere_search=centromere_search, centromere_fix=centromere_fix)
+                             centromere_search=centromere_search, centromere_fix=centromere_fix, resident=resident)
+        res, store = res if resident else (res, None)
+        if own and store is not None:
+            store.detach()
+        handle = lambda i: (store, i) if resident else None
         if centromere_search:
             out = []
-            for r in res:                   # messages in input order, up to the first matrix that fails
+            for i, r in enumerate(res):     # messages in input order, up to the first matrix that fails
                 if isinstance(r, Exception):
                     raise _failed_item(r)
-                out.append(_tadpole_from_batch_item(r, centromere_fix))
+                out.append(_tadpole_from_batch_item(r, centromere_fix, handle(i)))
             return out
         for r in res:
             if isinstance(r, Exception):
                 raise r
-        return [_tadpole_from_batch_item(r) for r in res]
+        return [_tadpole_from_batch_item(r, False, handle(i)) for i, r in enumerate(res)]
     finally:
         if own:
             pool.close()
@@ -183,14 +207,44 @@ class GenomeResult(dict):
     failed: dict
     stats: dict
 
+    def recall(self, max_pcs=200, min_clusters=2, chroms=None, streams=4):
+        """TADpole_genome() again with another max_pcs (<= the one computed) / min_clusters, from the PC scores resident
+        for every chromosome (TADpole_genome(resident=True)): only the n_pcs sweep and the selection run, all selected
+        chromosomes in one library call.  chroms: names (default every chromosome of this result).  Returns a
+        GenomeResult with the same messages, .stats, and .failed = the earlier failures plus this recall's."""
+        names = list(self) if chroms is None else [str(c) for c in chroms]
+        missing = [c for c in names if c not in self]
+        if missing:
+            raise ValueError(f"chromosome(s) {missing} are not in this result")
+        handles = [self[nm]._resident() for nm in names]
+        stores = {id(h["batch"]): h["batch"] for h in handles}
+        if len(stores) > 1:
+            raise ValueError("the chromosomes come from different genome calls: recall them separately")
+        out = GenomeResult()
+        out.failed = dict(self.failed)
+        out.stats = self.stats
+        if not names:
+            return out
+        res, store = handles[0]["batch"].recall([h["item"] for h in handles], max_pcs=max_pcs, min_clusters=min_clusters,
+                                                inflight=streams)
+        for i, (nm, h, r) in enumerate(zip(names, handles, res)):
+            message(f"Processing chromosome {nm}")
+            if isinstance(r, Exception):
+                out.failed[nm] = str(r)
+                continue
+            out[nm] = _tadpole_from_batch_item(r, h["centromere_fix"], (store, i))
+        return out
+
 
 def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, ctx=None, device=0, streams=4,
-                   centromere_search=False, centromere_fix=False):
+                   centromere_search=False, centromere_fix=False, resident=False):
     """TADpole() on every chromosome of a genome-wide pixel list (GenomePixels), `streams` calls in flight per GPU.
     Each chromosome's Tadpole is the one TADpole() returns for that chromosome's dense matrix (with centromere_search /
     centromere_fix as TADpole() takes them: p, q and merging_arms; a chromosome that does not split fails with
     TADpole()'s message unless centromere_fix).  Returns a GenomeResult in bin-table order, or in `chroms` order when
-    chroms (a list of names) is given."""
+    chroms (a list of names) is given.
+    resident: as TADpole_batch's (recalls run on ctx when it is given, else on a context made for each recall); the
+    result then also has recall() over all its chromosomes at once."""
     index = {nm: c for c, nm in enumerate(pixels.names)}
     sel = list(pixels.names) if chroms is None else [str(c) for c in chroms]
     unknown = [c for c in sel if c not in index]
@@ -203,21 +257,25 @@ def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.
         try:
             cis, trans, below = g.stats()
             res = ctx.call_genome(g, [index[c] for c in sel], max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac,
-                                  inflight=streams, centromere_search=centromere_search, centromere_fix=centromere_fix)
+                                  inflight=streams, centromere_search=centromere_search, centromere_fix=centromere_fix,
+                                  resident=resident)
         finally:
             g.close()
     finally:
         if own:
             ctx.close()
+    res, store = res if resident else (res, None)
+    if own and store is not None:
+        store.detach()
     out = GenomeResult()
     out.failed = {}
     out.stats = dict(cis={nm: int(k) for nm, k in zip(pixels.names, cis)}, trans=trans, below=below)
-    for nm, r in zip(sel, res):
+    for i, (nm, r) in enumerate(zip(sel, res)):
         message(f"Processing chromosome {nm}")
         if isinstance(r, Exception):
             out.failed[nm] = NOSPLIT_MESSAGE if r.code == _lib.TP_ERR_NOSPLIT else str(r)
             continue
-        out[nm] = _tadpole_from_batch_item(r, centromere_fix)
+        out[nm] = _tadpole_from_batch_item(r, centromere_fix, (store, i) if resident else None)
     return out
 
 

@@ -20,7 +20,7 @@ void tp_set_error(const char *fmt, ...) {
 }
 
 extern "C" const char *tp_last_error(void) { return g_err; }
-extern "C" int tp_version(void) { return 105; }
+extern "C" int tp_version(void) { return 106; }
 
 int tp_pin_reserve(tp_ctx *ctx, size_t bytes) {
     if (bytes <= ctx->pin_cap) return TP_OK;
@@ -203,9 +203,37 @@ extern "C" int tp_ctx_set(tp_ctx *ctx, const char *key, double value) {
     else if (k == "upload_lanes") ctx->upload_lanes = (int)value < 0 ? 0 : ((int)value > 16 ? 16 : (int)value);
     else if (k == "iop_switch") ctx->iop_switch = value;
     else if (k == "io_bn32") ctx->io_bn32 = (int)value;
+    else if (k == "batch_resident") ctx->batch_resident = (int)value != 0;
     else if (k == "iop_final") ctx->iop_final = ((int)value == 8) ? 8 : 0;
     else if (k == "iop_final_min_n") ctx->iop_final_min_n = (int)value;
     else { tp_set_error("tp_ctx_set: unknown key '%s'", key); return TP_ERR_ARG; }
+    return TP_OK;
+}
+
+extern "C" int tp_ctx_get(tp_ctx *ctx, const char *key, double *value_out) {
+    TP_ARG(ctx && key && value_out, "tp_ctx_get: null argument");
+    const std::string k(key);
+    double v;
+    if (k == "pca_block") v = ctx->pca_block;
+    else if (k == "pca_tol") v = ctx->pca_tol;
+    else if (k == "pca_maxit") v = ctx->pca_maxit;
+    else if (k == "pca_inner") v = ctx->pca_inner;
+    else if (k == "jacobi_direct_max") v = ctx->jacobi_direct_max;
+    else if (k == "level_cap") v = ctx->level_cap;
+    else if (k == "dist_min_n") v = ctx->dist_min_n;
+    else if (k == "igemm_min_n") v = ctx->igemm_min_n;
+    else if (k == "iop_min_n") v = ctx->iop_min_n;
+    else if (k == "mgram_min_n") v = ctx->mgram_min_n;
+    else if (k == "shard_sym") v = ctx->shard_sym;
+    else if (k == "sync_blocking") v = ctx->sync_blocking;
+    else if (k == "upload_lanes") v = ctx->upload_lanes;
+    else if (k == "iop_switch") v = ctx->iop_switch;
+    else if (k == "io_bn32") v = ctx->io_bn32;
+    else if (k == "batch_resident") v = ctx->batch_resident;
+    else if (k == "iop_final") v = ctx->iop_final;
+    else if (k == "iop_final_min_n") v = ctx->iop_final_min_n;
+    else { tp_set_error("tp_ctx_get: unknown key '%s'", key); return TP_ERR_ARG; }
+    *value_out = v;
     return TP_OK;
 }
 
@@ -782,9 +810,10 @@ static int call_from_compacted(tp_ctx *ctx, int max_pcs, int min_clusters, int *
 }
 
 // The PC scores of the last call stay in the context: another (max_pcs, min_clusters) only repeats the n_pcs sweep.
-// prcomp(rank. = k') returns the first k' columns of the same decomposition, so restricting the resident scores to
-// their first k' columns is what a fresh call with max_pcs = k' computes (R/TADpole.R:366-367; CH on those k'
-// columns, quirk Q2).
+// prcomp(rank. = k') returns the first k' columns of the same decomposition, so the first k' columns of the resident
+// scores are what a fresh call with max_pcs = k' computes (R/TADpole.R:366-367; CH on those k' columns, quirk Q2) --
+// the same decomposition, not the same bits: that call's subspace iteration runs with a narrower block, whose scores
+// differ in the last bits.
 extern "C" int tp_recall(tp_ctx *ctx, int max_pcs, int min_clusters, int *k_out, int *n_pcs_out, int *n_clusters_out,
                          int *maxlev_out, double *seqdist_out) {
     TP_ARG(ctx, "tp_recall: null context");

@@ -107,6 +107,7 @@ struct tp_ctx {
     int mgram_min_n = 1024;      // smallest nf whose M = Xc Xc^T is formed by the sliced int8 Gram (needs the sliced operator; 0 = FP64 DMMA)
     int iop_final_min_n = 1024;  // below this nf the later rounds use the FP64 DMMA operator whatever iop_final says (measured at N = 2000, 8 calls in flight: 224 -> 264 calls/s with the sliced operator)
     int iop_final = 8;           // operator of the later rounds where the sliced one is in use: 8 digit planes, or 0 = FP64 DMMA
+    int batch_resident = 0;      // 1: tp_call_batch / tp_call_genome keep every item's PC scores and dendrograms (tp_batch_recall)
     int io_bn32 = -1;            // operator applications on 32-column tiles: -1 = when 64-column tiles would not fill the SMs, 0 / 1 = never / always
     double iop_switch = 1e-3;    // relative residual below which the 8-plane (or FP64 DMMA) operator takes over (the first iteration always starts with 5 planes)
 

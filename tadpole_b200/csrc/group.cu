@@ -19,8 +19,10 @@
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
+#include <memory>
 #include <mutex>
 #include <numeric>
+#include <set>
 #include <thread>
 
 static thread_local bool tl_in_group = false;
@@ -259,6 +261,22 @@ extern "C" int tp_centromere_split(const uint8_t *bad, int n, int fix, int *spli
 }
 
 // ---- batches of independent calls ----------------------------------------------------------------------------------------
+// Device memory of a resident store (one allocation, exactly `bytes`, on `device`), released with its last reference: by
+// tp_batch_free of the last batch that shares it, before or after the context is destroyed.
+struct TpDevStore {
+    int device = 0;
+    void *p = nullptr;
+    size_t bytes = 0;
+    ~TpDevStore() {
+        if (!p) return;
+        int cur = 0;
+        if (cudaGetDevice(&cur) != cudaSuccess) cur = device;
+        cudaSetDevice(device);
+        cudaFree(p);
+        cudaSetDevice(cur);
+    }
+};
+
 struct TpBatchItem {
     int rc = TP_OK;
     std::string err;
@@ -276,8 +294,47 @@ struct TpBatchItem {
     // vector of its optimal level, bad columns re-inserted (R/TADpole.R:411-431)
     std::vector<int> keep, badcols, labels;
     int nbad = -1;
+    // resident store ("batch_resident" = 1, and every item of tp_batch_recall): the PC scores, nf x ldk row-major in the
+    // worker's layout (k_full PCs, shared by the recalls made from them), and the seqdist of all k candidates (k x ldd,
+    // ldd = nf - 1 rounded up to 8)
+    std::shared_ptr<TpDevStore> rs_scores, rs_dendro;
+    int k_full = 0, ldk = 0;
 };
 struct tp_batch { std::vector<TpBatchItem> items; double device_ms = 0.0; };
+
+static int store_alloc(int device, size_t bytes, std::shared_ptr<TpDevStore> &out) {
+    auto s = std::make_shared<TpDevStore>();
+    s->device = device;
+    const cudaError_t e = cudaMalloc(&s->p, bytes);
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        s->p = nullptr;
+        tp_set_error("batch_resident: cudaMalloc(%zu) of the resident store (PC scores and dendrograms) failed: %s", bytes,
+                     cudaGetErrorString(e));
+        return TP_ERR_NOMEM;
+    }
+    s->bytes = bytes;
+    out = std::move(s);
+    return TP_OK;
+}
+
+// The resident store of an item that has just finished on c: its PC scores (unless `scores` already holds them, as for
+// a recall) and the dendrograms of all its k candidates, copied out of c before the next item replaces them.
+static int keep_resident(tp_ctx *c, TpBatchItem &it, std::shared_ptr<TpDevStore> scores) {
+    const size_t ldd = (size_t)round_up(it.nf - 1, 8);
+    if (!scores) {
+        TP_TRY(store_alloc(c->device, (size_t)it.nf * c->ldk * sizeof(double), scores));
+        TP_CUDA(cudaMemcpyAsync(scores->p, c->scores.p, scores->bytes, cudaMemcpyDeviceToDevice, c->stream));
+        it.k_full = c->k_full;
+        it.ldk = c->ldk;
+    }
+    it.rs_scores = std::move(scores);
+    const int rc = store_alloc(c->device, (size_t)it.k * ldd * sizeof(double), it.rs_dendro);
+    if (rc != TP_OK) { it.rs_scores.reset(); return rc; }       // a failed item holds no store
+    TP_CUDA(cudaMemcpyAsync(it.rs_dendro->p, c->seqdist.p, it.rs_dendro->bytes, cudaMemcpyDeviceToDevice, c->stream));
+    TP_CUDA(tp_stream_sync(c));
+    return TP_OK;
+}
 
 // The outputs of a call that has just finished on c, into its batch item: k, maxlev and the score matrix from the context
 // (the host copy the sweep made) and the call's device time.  n_pcs, n_clusters, nf and seqdist the call wrote there itself.
@@ -308,23 +365,23 @@ static int level_tables(TpBatchItem &it, const int *names, const int *bad, int n
     return TP_OK;
 }
 
-// The result tail of a matrix called whole: finish_item, then (tables) the start / end table of every scored level, with
-// the names and bad columns TADpole() packs from the bad flags.
-static int finish_whole(tp_ctx *c, TpBatchItem &it, bool tables) {
-    finish_item(c, it);
-    if (!tables) return TP_OK;
+// the start / end table of every scored level of a matrix called whole, with the names and bad columns TADpole() packs
+// from the bad flags
+static int whole_tables(TpBatchItem &it) {
     std::vector<int> names, bad;
     for (int i = 0; i < it.n; i++) (it.bad[(size_t)i] ? bad : names).push_back(i + 1);
     return level_tables(it, names.data(), bad.data(), (int)bad.size());
 }
 
-// one chromosome arm on c, after tp_filter: the arm's call (tp_call_arm on its keep list), its tables and its fixed labels
-static int arm_one(tp_ctx *c, int max_pcs, int min_clusters, TpBatchItem &a) {
-    a.nf = (int)a.keep.size();
-    a.seqdist.assign((size_t)(a.nf > 1 ? a.nf - 1 : 1), 0.0);
-    TP_TRY(tp_call_arm(c, a.keep.data(), a.nf, max_pcs, min_clusters, nullptr, &a.n_pcs, &a.n_clusters, nullptr,
-                       a.seqdist.data()));
-    finish_item(c, a);
+// The result tail of a matrix called whole: finish_item, then (tables) whole_tables and (resident) its store.
+static int finish_whole(tp_ctx *c, TpBatchItem &it, bool tables, bool resident) {
+    finish_item(c, it);
+    if (tables) TP_TRY(whole_tables(it));
+    return resident ? keep_resident(c, it, nullptr) : (int)TP_OK;
+}
+
+// the tables of an arm whose seqdist is known, and the fixed labels of its optimal level
+static int arm_tables(TpBatchItem &a) {
     std::vector<int> names(a.keep.size());
     for (size_t t = 0; t < names.size(); t++) names[t] = a.keep[t] + 1;
     TP_TRY(level_tables(a, names.data(), a.badcols.data(), a.nbad));
@@ -341,12 +398,24 @@ static const char *const NOSPLIT_MSG = "centromere_search=TRUE but load_mat did 
                                        "longest bad stretch touches an end); the reference errors here";
 
 // What every item of a batch call is run with.  centromere: 0 = TADpole(), 1 = centromere_search, 2 = centromere_search
-// with centromere_fix.
+// with centromere_fix.  resident: the context's "batch_resident".
 struct ItemArgs {
     int max_pcs, min_clusters;
     double bad_frac;
-    int want_tables, centromere;
+    int want_tables, centromere, resident;
 };
+
+// one chromosome arm on c, after tp_filter: the arm's call (tp_call_arm on its keep list), its tables, its fixed labels
+// and (resident) its store
+static int arm_one(tp_ctx *c, const ItemArgs &args, TpBatchItem &a) {
+    a.nf = (int)a.keep.size();
+    a.seqdist.assign((size_t)(a.nf > 1 ? a.nf - 1 : 1), 0.0);
+    TP_TRY(tp_call_arm(c, a.keep.data(), a.nf, args.max_pcs, args.min_clusters, nullptr, &a.n_pcs, &a.n_clusters, nullptr,
+                       a.seqdist.data()));
+    finish_item(c, a);
+    TP_TRY(arm_tables(a));
+    return args.resident ? keep_resident(c, a, nullptr) : (int)TP_OK;
+}
 
 // One matrix of a batch on c.  centromere = 0: tp_call, then its outputs and (want_tables) its tables.  Otherwise
 // TADpole(centromere_search = TRUE) on one matrix (R/TADpole.R:351-442): filter, split at the longest bad stretch, then
@@ -363,7 +432,7 @@ static int item_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_de
         it.seqdist.assign((size_t)(n > 1 ? n - 1 : 1), 0.0);
         TP_TRY(tp_call(c, mat, n, colmajor, on_device, a.max_pcs, a.min_clusters, a.bad_frac, it.bad.data(), &it.nf, nullptr,
                        &it.n_pcs, &it.n_clusters, nullptr, it.seqdist.data()));
-        return finish_whole(c, it, a.want_tables);
+        return finish_whole(c, it, a.want_tables, a.resident);
     }
     struct Events {
         cudaEvent_t e[2] = {nullptr, nullptr};
@@ -395,7 +464,7 @@ static int item_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_de
         it.arms[1].nbad = nbq;
         if (nbp > 0) it.arms[0].badcols.assign(bp.begin(), bp.begin() + nbp);
         if (nbq > 0) it.arms[1].badcols.assign(bq.begin(), bq.begin() + nbq);
-        for (TpBatchItem &arm : it.arms) TP_TRY(arm_one(c, a.max_pcs, a.min_clusters, arm));
+        for (TpBatchItem &arm : it.arms) TP_TRY(arm_one(c, a, arm));
     } else {
         if (a.centromere != 2) { tp_set_error("%s", NOSPLIT_MSG); return TP_ERR_NOSPLIT; }
         std::vector<int> keep;
@@ -404,7 +473,7 @@ static int item_one(tp_ctx *c, const double *mat, int n, int colmajor, int on_de
         it.seqdist.assign((size_t)(it.nf > 1 ? it.nf - 1 : 1), 0.0);
         TP_TRY(tp_call_arm(c, keep.data(), it.nf, a.max_pcs, a.min_clusters, nullptr, &it.n_pcs, &it.n_clusters, nullptr,
                            it.seqdist.data()));
-        TP_TRY(finish_whole(c, it, true));
+        TP_TRY(finish_whole(c, it, true, a.resident));
     }
     TP_CUDA(cudaEventRecord(ev.e[1], c->stream));
     TP_CUDA(cudaEventSynchronize(ev.e[1]));
@@ -593,7 +662,7 @@ extern "C" int tp_call_batch(tp_ctx *ctx, int ncalls, const double *const *mats,
     auto stage = [&](tp_ctx *c, int j) {
         if (mats[j] && n[j] >= 2) (void)tp_stage_input(c, mats[j], n[j], colmajor);    // a failure leaves the normal upload
     };
-    const ItemArgs args{max_pcs, min_clusters, bad_frac, want_tables, centromere};
+    const ItemArgs args{max_pcs, min_clusters, bad_frac, want_tables, centromere, ctx->batch_resident};
     auto one = [&](tp_ctx *c, int i, TpBatchItem &it) -> int {
         return mats[i] ? item_one(c, mats[i], n[i], colmajor, on_device, args, it)
                        : (tp_set_error("tp_call_batch: matrix %d is null", i), (int)TP_ERR_ARG);
@@ -629,7 +698,7 @@ extern "C" int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms
         pmax = std::max(pmax, (double)(g->offs[(size_t)c + 1] - g->offs[(size_t)c]));
     }
     const double need = 56.0 * nmax * nmax + 16.0 * pmax + 64e6;
-    const ItemArgs args{max_pcs, min_clusters, bad_frac, want_tables, centromere};
+    const ItemArgs args{max_pcs, min_clusters, bad_frac, want_tables, centromere, ctx->batch_resident};
     auto one = [&](tp_ctx *c, int s, TpBatchItem &it) -> int {
         const int chrom = sel[(size_t)s], n = g->bins[(size_t)chrom];
         it.n = n;
@@ -715,5 +784,135 @@ extern "C" int tp_batch_split(const tp_batch *b, int i, int *split_out, int *cs_
 }
 extern "C" int tp_batch_free(tp_batch *b) {
     delete b;
+    return TP_OK;
+}
+
+// ---- recalls from the resident stores of a batch ------------------------------------------------------------------------
+// tp_recall on the store of `src` (a whole item or an arm), run on c, into dst: the store's PC scores installed in c (one
+// contiguous copy, from the peer device when the store is on another one), the sweep and the selection exactly as
+// tp_recall runs them, then the result tail of a call (its tables; for an arm also its fixed labels) and a store of the
+// new dendrograms beside the shared scores.
+static int recall_part(tp_ctx *c, const TpBatchItem &src, bool arm, int max_pcs, int min_clusters, TpBatchItem &dst) {
+    dst.n = src.n; dst.nf = src.nf; dst.bad = src.bad;
+    dst.keep = src.keep; dst.badcols = src.badcols; dst.nbad = src.nbad;
+    dst.k_full = src.k_full; dst.ldk = src.ldk;
+    const TpDevStore &s = *src.rs_scores;
+    TP_CUDA(cudaSetDevice(c->device));
+    TP_TRY(c->scores.reserve(s.bytes));
+    if (s.device == c->device) TP_CUDA(cudaMemcpyAsync(c->scores.p, s.p, s.bytes, cudaMemcpyDeviceToDevice, c->stream));
+    else TP_CUDA(cudaMemcpyPeerAsync(c->scores.p, c->device, s.p, s.device, s.bytes, c->stream));
+    c->generation++;
+    c->nf = src.nf; c->k = c->k_full = src.k_full; c->ldk = src.ldk;
+    c->have_X = c->have_C = c->have_sweep = false;
+    c->have_scores = true;
+    dst.seqdist.assign((size_t)src.nf - 1, 0.0);
+    const long long l0 = c->launches;
+    const int rc = tp_recall(c, max_pcs, min_clusters, nullptr, &dst.n_pcs, &dst.n_clusters, nullptr, dst.seqdist.data());
+    dst.launches = c->launches - l0;
+    TP_TRY(rc);
+    finish_item(c, dst);
+    TP_TRY(arm ? arm_tables(dst) : whole_tables(dst));
+    return keep_resident(c, dst, src.rs_scores);
+}
+
+extern "C" int tp_batch_recall(tp_ctx *ctx, const tp_batch *src, const int *items, const int *parts, int nsel, int max_pcs,
+                               int min_clusters, int inflight, tp_batch **out) {
+    TP_ARG(nsel >= 0, "tp_batch_recall: nsel must not be negative");
+    TP_ARG(nsel == 0 || (items && parts), "tp_batch_recall: null items / parts");
+    TP_ARG(src && out, "tp_batch_recall: null source batch or output");
+    for (int s = 0; s < nsel; s++)
+        if (items[s] < 0 || items[s] >= (int)src->items.size() || parts[s] < -1 || parts[s] > 1) {
+            tp_set_error("tp_batch_recall: selection %d (item %d, part %d) is outside items 0..%d, parts -1..1", s, items[s],
+                         parts[s], (int)src->items.size() - 1);
+            return TP_ERR_ARG;
+        }
+    TP_ARG(ctx, "tp_batch_recall: null context");
+    std::vector<int> devs;
+    for (int r = 0; r < tp_group_size(ctx); r++) devs.push_back(tp_group_member(ctx, r)->device);
+    // per call in flight: the sweep's buffers (scores, prefix sums, d0, seqdist, merge order, broken-stick) ~ 56 bytes per
+    // (good bin x PC), next to the working sets the pool's contexts already hold
+    double need = 64e6;
+    for (int s = 0; s < nsel; s++) {
+        const TpBatchItem &it = src->items[(size_t)items[s]];
+        auto add = [&](const TpBatchItem &p) { need = std::max(need, 64.0 * p.nf * std::max(p.ldk, 8) + 64e6); };
+        add(it);
+        for (const TpBatchItem &a : it.arms) add(a);
+    }
+    // a part with a store this context can reach; otherwise the item's TP_ERR_ARG
+    auto usable = [&](const TpBatchItem *p, int i, int part) -> int {
+        if (!p || p->rc != TP_OK || !p->rs_scores) {
+            tp_set_error("tp_batch_recall: item %d part %d %s", i, part,
+                         !p ? "does not exist (the item failed, or was not split)"
+                            : p->rc != TP_OK ? "failed" : "holds no resident store (its batch ran without \"batch_resident\")");
+            return TP_ERR_ARG;
+        }
+        if (std::find(devs.begin(), devs.end(), p->rs_scores->device) == devs.end()) {
+            tp_set_error("tp_batch_recall: item %d part %d is resident on device %d, which is not a device of the context", i,
+                         part, p->rs_scores->device);
+            return TP_ERR_ARG;
+        }
+        return TP_OK;
+    };
+    auto one = [&](tp_ctx *c, int s, TpBatchItem &it) -> int {
+        const int i = items[s], part = parts[s];
+        const TpBatchItem &whole = src->items[(size_t)i];
+        if (part >= 0 || whole.rc != TP_OK || whole.split != 1) {
+            const TpBatchItem *p = batch_part(src, i, part);
+            TP_TRY(usable(p, i, part));
+            if (part < 0) { it.split = p->split; it.cs = p->cs; it.ce = p->ce; }
+            return recall_part(c, *p, part >= 0, max_pcs, min_clusters, it);
+        }
+        // a split item selected whole: both arms
+        it.n = whole.n; it.bad = whole.bad; it.split = 1; it.cs = whole.cs; it.ce = whole.ce;
+        it.arms.resize(2);
+        for (int a = 0; a < 2; a++) TP_TRY(usable(&whole.arms[(size_t)a], i, a));
+        for (int a = 0; a < 2; a++) {
+            const int rc = recall_part(c, whole.arms[(size_t)a], true, max_pcs, min_clusters, it.arms[(size_t)a]);
+            it.device_ms += it.arms[(size_t)a].device_ms;
+            it.launches += it.arms[(size_t)a].launches;
+            TP_TRY(rc);
+        }
+        return TP_OK;
+    };
+    return batch_run(ctx, nsel, need, inflight, false, nullptr, [](tp_ctx *, int) {}, one, out);
+}
+
+extern "C" int tp_batch_dendro(const tp_batch *b, int item, int part, int cand, double *seqdist_out) {
+    const TpBatchItem *it = batch_part(b, item, part);
+    TP_ARG(it && seqdist_out, "tp_batch_dendro: no such item or arm, or null output");
+    if (it->rc != TP_OK) { tp_set_error("%s", it->err.c_str()); return it->rc; }
+    TP_ARG(it->rs_dendro, "tp_batch_dendro: the item holds no resident store (its batch ran without \"batch_resident\")");
+    TP_ARG(cand >= 0 && cand < it->k, "tp_batch_dendro: candidate out of range");
+    const size_t n1 = (size_t)it->nf - 1, ldd = (size_t)round_up(it->nf - 1, 8);
+    int cur = 0;
+    TP_CUDA(cudaGetDevice(&cur));
+    TP_CUDA(cudaSetDevice(it->rs_dendro->device));
+    const double *row = (const double *)it->rs_dendro->p + (size_t)cand * ldd;
+    cudaError_t e = cudaMemcpyAsync(seqdist_out, row, n1 * sizeof(double), cudaMemcpyDeviceToHost, 0);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+    cudaSetDevice(cur);
+    TP_CUDA(e);
+    return TP_OK;
+}
+
+extern "C" long long tp_batch_resident_bytes(const tp_batch *b) {
+    if (!b) return 0;
+    std::set<const TpDevStore *> seen;
+    long long s = 0;
+    auto add = [&](const std::shared_ptr<TpDevStore> &p) { if (p && seen.insert(p.get()).second) s += (long long)p->bytes; };
+    for (const TpBatchItem &it : b->items) {
+        add(it.rs_scores); add(it.rs_dendro);
+        for (const TpBatchItem &a : it.arms) { add(a.rs_scores); add(a.rs_dendro); }
+    }
+    return s;
+}
+
+extern "C" int tp_batch_resident_devices(const tp_batch *b, int item, int part, int *scores_device_out,
+                                         int *dendro_device_out) {
+    const TpBatchItem *it = batch_part(b, item, part);
+    TP_ARG(it, "tp_batch_resident_devices: no such item or arm");
+    TP_ARG(it->rs_scores && it->rs_dendro, "tp_batch_resident_devices: the item holds no resident store");
+    if (scores_device_out) *scores_device_out = it->rs_scores->device;
+    if (dendro_device_out) *dendro_device_out = it->rs_dendro->device;
     return TP_OK;
 }
