@@ -342,6 +342,30 @@ int tp_call_genome(tp_ctx *ctx, const tp_genome *g, const int *chroms, int nsel,
                    double bad_frac, int inflight, int want_tables, int centromere, tp_batch **out);
 int tp_genome_free(tp_genome *g);
 
+/* ---- equal-depth subsampling: the same genome at fewer reads (DESIGN S0d) ---------------------------------------------
+ * A TADpole call depends on sequencing depth (bad bins, the broken-stick level count), so two samples are compared at the
+ * same number of cis contacts by subsampling the deeper one.  A cell is (c, i, j): chromosome c, chromosome-local bins
+ * i <= j; its count C is the sum of the bucket entries naming it (duplicates merge) and it holds the reads (c, i, j, r),
+ * r = 0 .. C-1.  Every count, and every merged cell, must be an integer in [0, 2^32): otherwise TP_ERR_ARG naming the
+ * chromosome and bins (fractional counts have no reads to draw).  Only cis contacts count (trans pixels are dropped at
+ * ingest).  The handle must be on a device of ctx; the work runs there.
+ *
+ * tp_genome_depth: reads_out[nchrom] = cis contacts (the sum of the counts) per chromosome. */
+int tp_genome_depth(tp_ctx *ctx, const tp_genome *g, unsigned long long *reads_out);
+/* A uniform subset of exactly `contacts` of src's reads (<= the total: otherwise TP_ERR_ARG): key(read) = first 64 bits
+ * (x0 << 32 | x1) of Philox4x32-10 on counter (r, i, j, 0xD5000000 | c) with key words (seed low 32 bits, seed high 32),
+ * and the reads with the `contacts` smallest (key, c, i, j, r) are kept.  *out holds, per chromosome, every cell that
+ * keeps a read with its number of kept reads as the count: raw integer counts, exactly the pixels a library with that many
+ * reads would give.  The draw is the multivariate hypergeometric one; it depends only on the merged cells, seed and
+ * contacts (not on pixel order or duplicate splitting), and is the same bits on every run and device.  *out has src's bin
+ * table, device, trans and below counts (tp_genome_stats), and is independent of src: either may be freed first.
+ * Device memory: 32 bytes per bucket entry of src (a hash table, rounded up to a power of two) + 28 per merged cell, then
+ * 16 per output pixel; TP_ERR_NOMEM when that does not fit. */
+int tp_genome_downsample(tp_ctx *ctx, const tp_genome *src, unsigned long long contacts, unsigned long long seed,
+                         tp_genome **out);
+/* bucket `chrom` (0-based) of g copied to the host: tp_genome_stats gives its length; order unspecified */
+int tp_genome_pixels(tp_ctx *ctx, const tp_genome *g, int chrom, int32_t *i_out, int32_t *j_out, double *count_out);
+
 /* The context is a device-resident pipeline handle: after tp_call / tp_call_arm / tp_pca the PC scores stay in HBM, and
  * after a sweep so do all k dendrograms (tp_get_dendro) and the score matrix (tp_get_sweep_scores).  tp_recall repeats
  * only the n_pcs sweep and the selection for another max_pcs (<= the number of PCs computed) and / or min_clusters:

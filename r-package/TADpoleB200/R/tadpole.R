@@ -265,22 +265,78 @@ TADpole_batch <- function(mats, max_pcs = 200, min_clusters = 2, bad_frac = 0.01
 # its call runs.  A named list of tadpole objects (bin-table order, or chroms order), attr(, "failed") = the messages
 # of the chromosomes whose call failed.  centromere_search = TRUE: as TADpole(centromere_search = TRUE) on each
 # chromosome; one that does not split fails.
+# pixels may also be a genome_load() result (bins is then not needed): it is called as it is and stays loaded.
 TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clusters = 2, bad_frac = 0.01, inflight = 8L,
                            centromere_search = FALSE, resident = FALSE) {
-    stopifnot(inherits(pixels, "tadpole_pixels"))
-    ctx <- .tp_ctx()
-    tab <- .tp_bin_table(bins)
+    loaded <- inherits(pixels, "tadpole_genome")
+    stopifnot(loaded || inherits(pixels, "tadpole_pixels"))
+    ctx <- if (loaded) attr(pixels, "ctx") else .tp_ctx()
+    tab <- if (loaded) list(names = attr(pixels, "chroms"), n = attr(pixels, "n")) else .tp_bin_table(bins)
     sel <- if (is.null(chroms)) tab$names else as.character(chroms)
     idx <- match(sel, tab$names)
     if (anyNA(idx)) stop("unknown chromosome(s): ", paste(sel[is.na(idx)], collapse = ", "))
-    g <- if (is.null(pixels$path)) .Call(C_tp_genome, ctx, tab$n, pixels$bin1, pixels$bin2, pixels$count, pixels$index_base)
-         else .Call(C_tp_genome_file, ctx, tab$n, path.expand(pixels$path), pixels$index_base)
+    h <- if (loaded) pixels else .tp_ingest_genome(ctx, pixels, tab)
     res <- .tp_with_resident(ctx, resident, function() if (centromere_search)
-        .Call(C_tp_call_genome_arms, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
+        .Call(C_tp_call_genome_arms, ctx, h, as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
               as.numeric(bad_frac), as.integer(inflight), FALSE)
-    else .Call(C_tp_call_genome, ctx, g[[1L]], as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
+    else .Call(C_tp_call_genome, ctx, h, as.integer(idx - 1L), as.integer(max_pcs), as.integer(min_clusters),
                as.numeric(bad_frac), as.integer(inflight), TRUE))
     .tp_genome_list(sel, res$items, res$batch, list())
+}
+
+# the buckets of sparse_counts() pixels with global bin ids over the bin table `tab`, on the GPU (an external pointer)
+.tp_ingest_genome <- function(ctx, pixels, tab) {
+    g <- if (is.null(pixels$path)) .Call(C_tp_genome, ctx, tab$n, pixels$bin1, pixels$bin2, pixels$count, pixels$index_base)
+         else .Call(C_tp_genome_file, ctx, tab$n, path.expand(pixels$path), pixels$index_base)
+    g[[1L]]
+}
+
+.tp_loaded <- function(handle, tab, ctx)
+    structure(handle, class = "tadpole_genome", chroms = tab$names, n = tab$n, ctx = ctx)
+
+# A genome-wide pixel list (sparse_counts() with global bin ids, as TADpole_genome() takes it) ingested once and kept on
+# the GPU: an external pointer whose finalizer releases it.  TADpole_genome() takes it in place of the pixels, and
+# genome_depth() / genome_downsample() / genome_pixels() read and subsample it.
+genome_load <- function(pixels, bins) {
+    stopifnot(inherits(pixels, "tadpole_pixels"))
+    ctx <- .tp_ctx()
+    tab <- .tp_bin_table(bins)
+    .tp_loaded(.tp_ingest_genome(ctx, pixels, tab), tab, ctx)
+}
+
+# cis contacts per chromosome of a loaded genome (named numeric vector; exact below 2^53)
+genome_depth <- function(g) {
+    stopifnot(inherits(g, "tadpole_genome"))
+    d <- .Call(C_tp_genome_depth, attr(g, "ctx"), g, length(attr(g, "n")))
+    names(d) <- attr(g, "chroms")
+    d
+}
+
+# A new loaded genome holding a uniform random subset of exactly `contacts` of g's cis contacts, or of
+# floor(fraction * total) of them: raw integer counts, the matrix a library with that many reads would give.  The draw
+# depends on the merged pixels, seed and contacts only (Philox keys, DESIGN S0d), not on R's random number stream.
+genome_downsample <- function(g, contacts = NULL, fraction = NULL, seed = 0) {
+    stopifnot(inherits(g, "tadpole_genome"))
+    if (is.null(contacts) == is.null(fraction)) stop("genome_downsample needs exactly one of contacts and fraction")
+    total <- sum(genome_depth(g))
+    if (!is.null(fraction)) {
+        if (!(fraction >= 0 && fraction <= 1)) stop("fraction must be in [0, 1]")
+        contacts <- floor(fraction * total)
+    }
+    if (!(contacts >= 0 && contacts <= total)) stop("contacts must be in 0..", format(total, scientific = FALSE))
+    tab <- list(names = attr(g, "chroms"), n = attr(g, "n"))
+    p <- .Call(C_tp_genome_downsample, attr(g, "ctx"), g, length(tab$n), as.numeric(contacts), as.numeric(seed))
+    .tp_loaded(p[[1L]], tab, attr(g, "ctx"))
+}
+
+# the pixels of chromosome `chrom` of a loaded genome: data.frame(i, j, count), chromosome-local 1-based bins, sorted
+genome_pixels <- function(g, chrom) {
+    stopifnot(inherits(g, "tadpole_genome"))
+    idx <- match(as.character(chrom), attr(g, "chroms"))
+    if (is.na(idx)) stop("unknown chromosome: ", chrom)
+    r <- .Call(C_tp_genome_pixels, attr(g, "ctx"), g, as.integer(idx - 1L), length(attr(g, "n")))
+    o <- order(r[[1L]], r[[2L]])
+    data.frame(i = r[[1L]][o] + 1L, j = r[[2L]][o] + 1L, count = r[[3L]][o])
 }
 
 # the named list TADpole_genome() returns from the items of a genome call or recall; failed: the earlier failures

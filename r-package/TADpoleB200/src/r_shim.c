@@ -13,6 +13,7 @@
 #include <R.h>
 #include <Rinternals.h>
 #include <R_ext/Rdynload.h>
+#include <math.h>
 #include <stdint.h>
 #include <string.h>
 #include "tadpole_b200.h"
@@ -511,6 +512,73 @@ SEXP C_tp_genome_file(SEXP ctx, SEXP chrom_bins, SEXP path, SEXP index_base) {
     return genome_result(ctx, g, length(chrom_bins));
 }
 
+static tp_genome *genome_of(SEXP p) {
+    tp_genome *g = (tp_genome *)R_ExternalPtrAddr(p);
+    if (!g) error("TADpole: the genome pixels have been released");
+    return g;
+}
+
+static int nchrom_of(SEXP nchrom) {
+    const int n = asInteger(nchrom);
+    if (n < 1 || n > (1 << 20)) error("TADpole: the number of chromosomes must be in 1..2^20");
+    return n;
+}
+
+/* a whole number in [0, 2^53] given as an R numeric (contacts, seeds) */
+static unsigned long long count_arg(SEXP x, const char *what) {
+    const double v = asReal(x);
+    if (!(v >= 0 && v <= 9007199254740992.0 && v == floor(v))) error("TADpole: %s must be a whole number >= 0", what);
+    return (unsigned long long)v;
+}
+
+/* cis contacts per chromosome of a C_tp_genome handle over `nchrom` chromosomes (tp_genome_depth), as doubles */
+SEXP C_tp_genome_depth(SEXP ctx, SEXP genome, SEXP nchrom) {
+    tp_ctx *c = ctx_of(ctx);
+    tp_genome *g = genome_of(genome);
+    const int n = nchrom_of(nchrom);
+    unsigned long long *tmp = (unsigned long long *)R_alloc((size_t)n, sizeof(unsigned long long));
+    if (tp_genome_depth(c, g, tmp) != TP_OK) error("%s", tp_last_error());
+    SEXP out = PROTECT(allocVector(REALSXP, n));
+    for (int i = 0; i < n; i++) REAL(out)[i] = (double)tmp[i];
+    UNPROTECT(1);
+    return out;
+}
+
+/* a uniform subset of exactly `contacts` of the genome's cis reads drawn with `seed` (tp_genome_downsample): what
+ * C_tp_genome returns, for the new buckets */
+SEXP C_tp_genome_downsample(SEXP ctx, SEXP genome, SEXP nchrom, SEXP contacts, SEXP seed) {
+    tp_ctx *c = ctx_of(ctx);
+    tp_genome *g = genome_of(genome);
+    const int n = nchrom_of(nchrom);
+    const unsigned long long k = count_arg(contacts, "contacts"), sd = count_arg(seed, "seed");
+    tp_genome *out = NULL;
+    if (tp_genome_downsample(c, g, k, sd, &out) != TP_OK) error("%s", tp_last_error());
+    return genome_result(ctx, out, n);
+}
+
+/* bucket `chrom` (0-based) of a genome over `nchrom` chromosomes: list(i, j, count), 0-based local bins, bucket order */
+SEXP C_tp_genome_pixels(SEXP ctx, SEXP genome, SEXP chrom, SEXP nchrom) {
+    tp_ctx *c = ctx_of(ctx);
+    tp_genome *g = genome_of(genome);
+    const int n = nchrom_of(nchrom), ch = asInteger(chrom);
+    if (ch < 0 || ch >= n) error("TADpole: chromosome index out of range");
+    unsigned long long *cis = (unsigned long long *)R_alloc((size_t)n, sizeof(unsigned long long));
+    if (tp_genome_stats(g, cis, NULL, NULL) != TP_OK) error("%s", tp_last_error());
+    if (cis[ch] > 2147483647ULL) error("TADpole: the bucket holds more than 2^31 - 1 pixels");
+    const int m = (int)cis[ch];
+    SEXP i = PROTECT(allocVector(INTSXP, m)), j = PROTECT(allocVector(INTSXP, m)), v = PROTECT(allocVector(REALSXP, m));
+    if (m > 0 && tp_genome_pixels(c, g, ch, INTEGER(i), INTEGER(j), REAL(v)) != TP_OK) {
+        UNPROTECT(3);
+        error("%s", tp_last_error());
+    }
+    SEXP out = PROTECT(allocVector(VECSXP, 3));
+    SET_VECTOR_ELT(out, 0, i);
+    SET_VECTOR_ELT(out, 1, j);
+    SET_VECTOR_ELT(out, 2, v);
+    UNPROTECT(4);
+    return out;
+}
+
 /* TADpole() on the chromosomes `chroms` (0-based) of a C_tp_genome handle, `inflight` calls per device in flight
  * (tp_call_genome with `centromere`).  Per chromosome, in chroms order: arms_item, or a character error message. */
 static SEXP call_genome(SEXP ctx, SEXP genome, SEXP chroms, SEXP max_pcs, SEXP min_clusters, SEXP bad_frac, SEXP inflight,
@@ -757,6 +825,9 @@ static const R_CallMethodDef call_table[] = {
     {"C_tp_ctx_set", (DL_FUNC)&C_tp_ctx_set, 3},
     {"C_tp_batch_recall", (DL_FUNC)&C_tp_batch_recall, 6},
     {"C_tp_batch_dendro", (DL_FUNC)&C_tp_batch_dendro, 4},
+    {"C_tp_genome_depth", (DL_FUNC)&C_tp_genome_depth, 3},
+    {"C_tp_genome_downsample", (DL_FUNC)&C_tp_genome_downsample, 5},
+    {"C_tp_genome_pixels", (DL_FUNC)&C_tp_genome_pixels, 4},
     {NULL, NULL, 0}};
 
 void R_init_TADpoleB200(DllInfo *dll) {

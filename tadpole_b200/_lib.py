@@ -33,7 +33,7 @@ EXPORTED = [
     "tp_batch_size", "tp_batch_device_ms", "tp_batch_launches", "tp_batch_status", "tp_batch_error", "tp_batch_dims", "tp_batch_get", "tp_batch_free", "tp_find_groups",
     "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
     "tp_centromere_split", "tp_batch_split", "tp_batch_recall", "tp_batch_dendro", "tp_batch_resident_bytes",
-    "tp_batch_resident_devices", "tp_ctx_get",
+    "tp_batch_resident_devices", "tp_ctx_get", "tp_genome_depth", "tp_genome_downsample", "tp_genome_pixels",
 ]
 
 
@@ -89,6 +89,9 @@ def load():
         "tp_genome_matrix": (c_int, [vp, vp, c_int, dp]),
         "tp_call_genome": (c_int, [vp, vp, ip, c_int, c_int, c_int, c_double, c_int, c_int, c_int, POINTER(vp)]),
         "tp_genome_free": (c_int, [vp]),
+        "tp_genome_depth": (c_int, [vp, vp, POINTER(ctypes.c_ulonglong)]),
+        "tp_genome_downsample": (c_int, [vp, vp, ctypes.c_ulonglong, ctypes.c_ulonglong, POINTER(vp)]),
+        "tp_genome_pixels": (c_int, [vp, vp, c_int, ip, ip, dp]),
         "tp_find_groups": (c_int, [dp, c_int, ip]),
         "tp_ctx_destroy": (c_int, [vp]),
         "tp_ctx_sync": (c_int, [vp]),
@@ -845,6 +848,25 @@ class Genome:
         out = np.empty((n, n))
         check(self.lib.tp_genome_matrix(self.ctx._h, self._h, int(chrom), _dp(out)))
         return out
+
+    def depth(self):
+        """cis contacts (sum of the integer counts) per chromosome (tp_genome_depth)"""
+        out = np.zeros(self.chrom_bins.size, dtype=np.uint64)
+        check(self.lib.tp_genome_depth(self.ctx._h, self._h, out.ctypes.data_as(POINTER(ctypes.c_ulonglong))))
+        return out
+
+    def downsample(self, contacts, seed=0):
+        """tp_genome_downsample: a new Genome holding a uniform subset of exactly `contacts` of the cis reads."""
+        h = c_void_p()
+        check(self.lib.tp_genome_downsample(self.ctx._h, self._h, int(contacts), int(seed) % 2 ** 64, ctypes.byref(h)))
+        return Genome(self.ctx, h, self.chrom_bins)
+
+    def pixels(self, chrom):
+        """(i, j, count) of bucket `chrom` (0-based), in the bucket's order (tp_genome_pixels)"""
+        n = int(self.stats()[0][chrom])
+        i, j, v = np.empty(n, np.int32), np.empty(n, np.int32), np.empty(n)
+        check(self.lib.tp_genome_pixels(self.ctx._h, self._h, int(chrom), _ip(i), _ip(j), _dp(v)))
+        return i, j, v
 
     def close(self):
         if getattr(self, "_h", None):

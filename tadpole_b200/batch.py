@@ -14,6 +14,7 @@ and each chromosome's dense matrix exists only in HBM, only while its call runs 
 """
 from __future__ import annotations
 
+import math
 import os
 
 import numpy as np
@@ -23,7 +24,8 @@ from .api import (NOSPLIT_MESSAGE, ResidentArm, Tadpole, _Obj, _arm_object, _bed
                   _messages_bad, _messages_optimal, _messages_split, get_context, message, read_matrix)
 from .hclust import Dendro
 
-__all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "TADpole_genome", "read_bins", "diffT_genome"]
+__all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "LoadedGenome", "TADpole_genome", "read_bins", "diffT_genome",
+           "equal_depth"]
 
 
 class ContextPool:
@@ -200,6 +202,109 @@ class GenomePixels:
     def _ingest(self, ctx):
         return ctx.genome_ingest(self.chrom_bins, self.bin1, self.bin2, self.count, self.index_base, self.path, self.sep)
 
+    def load(self, ctx=None, device=0):
+        """Ingest the pixels once and keep them on the GPU: a LoadedGenome, which TADpole_genome takes in place of the
+        pixels and which can be subsampled (downsample, equal_depth).  Without ctx, a context on `device` is made and
+        closed with the last LoadedGenome that uses it."""
+        ref = _CtxRef(ctx or _lib.Context(device), ctx is None)
+        try:
+            return LoadedGenome(self._ingest(ref.ctx), self.names, ref)
+        except BaseException:
+            ref.release()
+            raise
+
+
+class _CtxRef:
+    """The context of one or more LoadedGenomes; a context made for them is closed when the last one is closed."""
+
+    def __init__(self, ctx, own):
+        self.ctx, self.own, self.users = ctx, own, 0
+
+    def acquire(self):
+        self.users += 1
+        return self
+
+    def release(self):
+        self.users -= 1
+        if self.users <= 0 and self.own:
+            self.ctx.close()
+
+
+class LoadedGenome:
+    """A genome-wide pixel list held on the GPU, one bucket of cis pixels per chromosome (GenomePixels.load, or a
+    subsample of another LoadedGenome).  names / chrom_bins: the bin table's chromosomes and their bins.  TADpole_genome
+    takes it wherever it takes GenomePixels, and does not free it.  Close it (or use it as a context manager) to release
+    its device memory."""
+
+    def __init__(self, genome, names, ref):
+        self._g, self.names, self.chrom_bins = genome, list(names), np.asarray(genome.chrom_bins, dtype=np.int32)
+        self._ref = ref.acquire()
+        self.ctx = ref.ctx
+
+    def depth(self):
+        """{chromosome: cis contacts}: the sum of the integer counts of its pixels"""
+        return {nm: int(x) for nm, x in zip(self.names, self._g.depth())}
+
+    @property
+    def total_depth(self):
+        return sum(self.depth().values())
+
+    def downsample(self, contacts=None, fraction=None, seed=0):
+        """A new LoadedGenome holding a uniform random subset of exactly `contacts` of this genome's cis contacts, or of
+        floor(fraction * total_depth) of them: the counts stay raw integers, the matrix a library with that many reads
+        would give.  The draw is a function of the merged pixels, seed and contacts only (DESIGN S0d), on the GPU that
+        holds this genome.  Both genomes stay valid and either may be closed first."""
+        if (contacts is None) == (fraction is None):
+            raise ValueError("downsample needs exactly one of contacts and fraction")
+        total = self.total_depth
+        if fraction is not None:
+            f = float(fraction)
+            if not 0.0 <= f <= 1.0:
+                raise ValueError(f"fraction must be in [0, 1], not {fraction}")
+            contacts = math.floor(f * total)                 # in double precision, as R's floor(fraction * total)
+        contacts = int(contacts)
+        if not 0 <= contacts <= total:
+            raise ValueError(f"contacts must be in 0..{total} (the genome's cis contacts), not {contacts}")
+        return LoadedGenome(self._g.downsample(contacts, int(seed) % 2 ** 64), self.names, self._ref)
+
+    def pixels(self, chrom):
+        """(i, j, count) of chromosome `chrom` (a name): chromosome-local 0-based bins, sorted by (i, j)"""
+        if chrom not in self.names:
+            raise ValueError(f"unknown chromosome {chrom!r}: not in the bin table")
+        i, j, v = self._g.pixels(self.names.index(chrom))
+        o = np.lexsort((j, i))
+        return i[o], j[o], v[o]
+
+    def stats(self):
+        return self._g.stats()
+
+    def close(self):
+        if self._g is not None:
+            self._g.close()
+            self._g = None
+            self._ref.release()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def equal_depth(*genomes, seed=0):
+    """The LoadedGenomes at the same cis depth: every genome deeper than the shallowest is subsampled to the shallowest's
+    total (genome s with seed + s), the others are returned as they are.  Returns the list, in argument order."""
+    totals = [g.total_depth for g in genomes]
+    low = min(totals)
+    return [g.downsample(contacts=low, seed=(int(seed) + s) % 2 ** 64) if t > low else g
+            for s, (g, t) in enumerate(zip(genomes, totals))]
+
 
 class GenomeResult(dict):
     """{chromosome name: Tadpole}; .failed {name: message of the library}; .stats dict(cis={name: pixels}, trans=,
@@ -238,7 +343,8 @@ class GenomeResult(dict):
 
 def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, ctx=None, device=0, streams=4,
                    centromere_search=False, centromere_fix=False, resident=False):
-    """TADpole() on every chromosome of a genome-wide pixel list (GenomePixels), `streams` calls in flight per GPU.
+    """TADpole() on every chromosome of a genome-wide pixel list (GenomePixels, or a LoadedGenome: then with ctx=None the
+    call runs on the context the genome was loaded on, and the genome stays loaded), `streams` calls in flight per GPU.
     Each chromosome's Tadpole is the one TADpole() returns for that chromosome's dense matrix (with centromere_search /
     centromere_fix as TADpole() takes them: p, q and merging_arms; a chromosome that does not split fails with
     TADpole()'s message unless centromere_fix).  Returns a GenomeResult in bin-table order, or in `chroms` order when
@@ -250,17 +356,23 @@ def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.
     unknown = [c for c in sel if c not in index]
     if unknown:
         raise ValueError(f"unknown chromosome(s) {unknown}: not in the bin table")
+    loaded = isinstance(pixels, LoadedGenome)
+    if loaded and pixels._g is None:
+        raise ValueError("the LoadedGenome has been closed")
+    if loaded and ctx is None:
+        ctx = pixels.ctx
     own = ctx is None
     ctx = ctx or _lib.Context(device)
     try:
-        g = pixels._ingest(ctx)
+        g = pixels._g if loaded else pixels._ingest(ctx)
         try:
             cis, trans, below = g.stats()
             res = ctx.call_genome(g, [index[c] for c in sel], max_pcs=max_pcs, min_clusters=min_clusters, bad_frac=bad_frac,
                                   inflight=streams, centromere_search=centromere_search, centromere_fix=centromere_fix,
                                   resident=resident)
         finally:
-            g.close()
+            if not loaded:
+                g.close()
     finally:
         if own:
             ctx.close()

@@ -279,6 +279,9 @@ struct tp_genome {
 // the dense n_c x n_c row-major matrix of chromosome `chrom` into c->raw_own, on c's stream (a bucket held by another device
 // is first copied into c->icoo); *out = c->raw_own
 int tp_genome_dense(tp_ctx *c, const tp_genome *g, int chrom, double **out);
+// ingest.cu: TP_ERR_NOMEM naming `who` and `what` unless `bytes` fit in the free device memory plus `held` (bytes the
+// caller is about to release or reuse)
+int device_room(tp_ctx *ctx, double bytes, size_t held, const char *who, const char *what);
 int tp_upload_range(tp_ctx *ctx, void *dst, const void *src, size_t bytes, cudaStream_t st);   // filter.cu: pageable -> lanes
 int tp_stage_input(tp_ctx *ctx, const double *mat, int n, int colmajor);   // filter.cu: upload under the running call
 int tp_flags_reset(tp_ctx *ctx);                 // zero the status words (stream ordered)

@@ -12,6 +12,7 @@
 // All arithmetic is integer until the final division, so results are bit-identical to R.
 #include <algorithm>
 #include "common.cuh"
+#include "philox.cuh"
 
 #define DT_THREADS 256
 #define DT_EMPTY 0xffffffffffffffffULL
@@ -237,17 +238,7 @@ int tp_difft_batch(tp_ctx *ctx, const int32_t *labels_x, const int32_t *labels_y
 // the sorted borders and the label vector.  R's Mersenne-Twister stream cannot be reproduced, so draws differ from
 // R's sample(); the distribution (uniform subsets) is the same, and the oracle restates this generator exactly.
 __host__ __device__ __forceinline__ unsigned long long philox_key64(unsigned c0, unsigned c1, unsigned long long seed) {
-    unsigned k0 = (unsigned)seed, k1 = (unsigned)(seed >> 32);
-    unsigned x0 = c0, x1 = c1, x2 = 0u, x3 = 0x7adu;
-#pragma unroll
-    for (int r = 0; r < 10; r++) {
-        const unsigned long long p0 = (unsigned long long)0xD2511F53u * x0, p1 = (unsigned long long)0xCD9E8D57u * x2;
-        const unsigned y0 = (unsigned)(p1 >> 32) ^ x1 ^ k0, y1 = (unsigned)p1;
-        const unsigned y2 = (unsigned)(p0 >> 32) ^ x3 ^ k1, y3 = (unsigned)p0;
-        x0 = y0; x1 = y1; x2 = y2; x3 = y3;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    return ((unsigned long long)x0 << 32) | x1;
+    return philox4x32_key64(c0, c1, 0u, 0x7adu, seed);
 }
 
 #define RP_THREADS 256

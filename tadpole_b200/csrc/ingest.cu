@@ -595,7 +595,7 @@ static int open_text_file(const char *path, const char *who, TextSource *src) {
 
 // fail with a plain message when `bytes` more cannot fit on ctx's device (`held`: bytes of the buffer about to be grown,
 // which its reserve frees first)
-static int device_room(tp_ctx *ctx, double bytes, size_t held, const char *who, const char *what) {
+int device_room(tp_ctx *ctx, double bytes, size_t held, const char *who, const char *what) {
     size_t fr = 0, tot = 0;
     if (cudaMemGetInfo(&fr, &tot) != cudaSuccess) { (void)cudaGetLastError(); return TP_OK; }
     if (bytes > (double)fr + (double)held) {

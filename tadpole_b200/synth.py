@@ -15,7 +15,7 @@ from __future__ import annotations
 
 import numpy as np
 
-__all__ = ["synth_hic", "synth_hic_gpu", "synth_genome_pixels", "synth_partition_pairs", "write_tsv"]
+__all__ = ["synth_hic", "synth_hic_gpu", "synth_genome_pixels", "synth_sparse_genome_pixels", "synth_partition_pairs", "write_tsv"]
 
 
 def _random_blocks(rng, n, mean_len):
@@ -149,6 +149,30 @@ def synth_genome_pixels(sizes, seed=1, trans_per_chrom=100, centromere=None):
     perm = rng.permutation(b1.size)
     names = [f"chr{c + 1}" for c in range(len(sizes))]
     return names, (b1[perm].astype(np.int32), b2[perm].astype(np.int32), v[perm].astype(np.float64)), mats
+
+
+def synth_sparse_genome_pixels(sizes, band=50, mean_count=32.0, seed=1):
+    """A seeded genome-wide pixel list generated sparsely, for depths the dense generators cannot reach: chromosome c has
+    sizes[c] bins, and every cell (i, j) with 0 <= j - i < band gets a Poisson count with mean proportional to
+    1 / (1 + j - i), scaled so that the mean over the band is mean_count; cells drawn as 0 are left out.  About
+    sum(sizes) * band * mean_count cis reads (5e8 for GRCh38 at 10 kb with the defaults).  Global 0-based bin ids, in
+    chromosome then row order.  Returns (bin1, bin2, count): int32, int32, float64."""
+    rng = np.random.default_rng(seed)
+    d = np.arange(band)
+    lam = 1.0 / (1.0 + d)
+    lam *= mean_count / lam.mean()
+    start, b1, b2, v = 0, [], [], []
+    for n in (int(x) for x in sizes):
+        i = np.repeat(np.arange(n, dtype=np.int64), band)
+        dd = np.tile(d, n)
+        ok = i + dd < n
+        i, dd = i[ok], dd[ok]
+        cnt = rng.poisson(lam[dd])
+        nz = cnt > 0
+        b1.append((start + i[nz]).astype(np.int32)); b2.append((start + i[nz] + dd[nz]).astype(np.int32))
+        v.append(cnt[nz].astype(np.float64))
+        start += n
+    return np.concatenate(b1), np.concatenate(b2), np.concatenate(v)
 
 
 def synth_partition_pairs(npairs, length, ntads, seed=1, zero_frac=0.01):
