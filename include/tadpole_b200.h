@@ -366,6 +366,22 @@ int tp_genome_downsample(tp_ctx *ctx, const tp_genome *src, unsigned long long c
 /* bucket `chrom` (0-based) of g copied to the host: tp_genome_stats gives its length; order unspecified */
 int tp_genome_pixels(tp_ctx *ctx, const tp_genome *g, int chrom, int32_t *i_out, int32_t *j_out, double *count_out);
 
+/* ---- coarsening: the same genome at a multiple of its bin size (DESIGN S0e) --------------------------------------------
+ * *out = src at `factor` (>= 1) times its bin size.  Coarse chromosome c has ceil(n_c / factor) bins; coarse bin I covers
+ * fine bins I*factor .. min((I+1)*factor, n_c) - 1 (the last one is narrower when factor does not divide n_c, as cooler
+ * coarsen makes it).  Every bucket entry (c, i, j, v) adds to coarse cell (c, i / factor, j / factor) (integer division:
+ * I <= J holds).  A NaN count adds 0 (the reference's NA -> 0 applied at the fine resolution), a cell's count is the sum
+ * of its entries' counts, and cells whose sum is exactly 0 are not stored.  When every count is an integer and each
+ * cell's sum of |count| is below 2^53 the sums are exact: the same bits in any order, so coarsening by a and then b equals
+ * coarsening by a*b, and tp_genome_depth is unchanged.  Otherwise the rounding order is unspecified (as in the dense
+ * build); fractional counts are accepted.  factor = 1 gives src with duplicate cells merged.  *out has src's device,
+ * trans and below counts (tp_genome_stats), and is independent of src: either may be freed first.  The handle must be on
+ * a device of ctx (TP_ERR_ARG otherwise, and for a null argument or factor < 1); the work runs there.
+ * Device memory: 16 bytes per table slot (2 per bucket entry of src, rounded up to a power of two), and 16 per output
+ * cell while the output is written; the table is released before the call returns.  TP_ERR_NOMEM naming the table or
+ * the output buckets when they do not fit. */
+int tp_genome_coarsen(tp_ctx *ctx, const tp_genome *src, int factor, tp_genome **out);
+
 /* The context is a device-resident pipeline handle: after tp_call / tp_call_arm / tp_pca the PC scores stay in HBM, and
  * after a sweep so do all k dendrograms (tp_get_dendro) and the score matrix (tp_get_sweep_scores).  tp_recall repeats
  * only the n_pcs sweep and the selection for another max_pcs (<= the number of PCs computed) and / or min_clusters:

@@ -291,12 +291,12 @@ TADpole_genome <- function(pixels, bins, chroms = NULL, max_pcs = 200, min_clust
     g[[1L]]
 }
 
-.tp_loaded <- function(handle, tab, ctx)
-    structure(handle, class = "tadpole_genome", chroms = tab$names, n = tab$n, ctx = ctx)
+.tp_loaded <- function(handle, tab, ctx, factor = 1)
+    structure(handle, class = "tadpole_genome", chroms = tab$names, n = tab$n, ctx = ctx, factor = factor)
 
 # A genome-wide pixel list (sparse_counts() with global bin ids, as TADpole_genome() takes it) ingested once and kept on
 # the GPU: an external pointer whose finalizer releases it.  TADpole_genome() takes it in place of the pixels, and
-# genome_depth() / genome_downsample() / genome_pixels() read and subsample it.
+# genome_depth() / genome_downsample() / genome_coarsen() / genome_pixels() read, subsample and coarsen it.
 genome_load <- function(pixels, bins) {
     stopifnot(inherits(pixels, "tadpole_pixels"))
     ctx <- .tp_ctx()
@@ -326,7 +326,21 @@ genome_downsample <- function(g, contacts = NULL, fraction = NULL, seed = 0) {
     if (!(contacts >= 0 && contacts <= total)) stop("contacts must be in 0..", format(total, scientific = FALSE))
     tab <- list(names = attr(g, "chroms"), n = attr(g, "n"))
     p <- .Call(C_tp_genome_downsample, attr(g, "ctx"), g, length(tab$n), as.numeric(contacts), as.numeric(seed))
-    .tp_loaded(p[[1L]], tab, attr(g, "ctx"))
+    .tp_loaded(p[[1L]], tab, attr(g, "ctx"), attr(g, "factor"))
+}
+
+# A new loaded genome at `factor` times g's bin size (DESIGN S0e): chromosome c gets ceiling(n_c / factor) bins (the
+# last one narrower when factor does not divide n_c), and coarse cell (I, J) holds the sum of the counts of the cells
+# (i, j) with (i - 1) %/% factor + 1 = I and (j - 1) %/% factor + 1 = J (an NA count adds 0; cells that sum to 0 are left
+# out).  attr(, "factor") is the bin size as a multiple of the loaded file's: bin b covers the loaded bins
+# factor * (b - 1) + 1 .. min(factor * b, n).
+genome_coarsen <- function(g, factor) {
+    stopifnot(inherits(g, "tadpole_genome"))
+    if (!(is.numeric(factor) && length(factor) == 1L && !is.na(factor) && factor >= 1 && factor <= 2147483647 &&
+          factor == floor(factor))) stop("factor must be a whole number >= 1")
+    tab <- list(names = attr(g, "chroms"), n = as.integer(ceiling(attr(g, "n") / factor)))
+    p <- .Call(C_tp_genome_coarsen, attr(g, "ctx"), g, length(tab$n), as.numeric(factor))
+    .tp_loaded(p[[1L]], tab, attr(g, "ctx"), attr(g, "factor") * factor)
 }
 
 # the pixels of chromosome `chrom` of a loaded genome: data.frame(i, j, count), chromosome-local 1-based bins, sorted

@@ -556,6 +556,18 @@ SEXP C_tp_genome_downsample(SEXP ctx, SEXP genome, SEXP nchrom, SEXP contacts, S
     return genome_result(ctx, out, n);
 }
 
+/* the genome at `factor` times its bin size (tp_genome_coarsen): what C_tp_genome returns, for the new buckets */
+SEXP C_tp_genome_coarsen(SEXP ctx, SEXP genome, SEXP nchrom, SEXP factor) {
+    const double f = asReal(factor);
+    if (!(f >= 1 && f <= 2147483647.0 && f == floor(f))) error("TADpole: factor must be a whole number >= 1");
+    tp_ctx *c = ctx_of(ctx);
+    tp_genome *g = genome_of(genome);
+    const int n = nchrom_of(nchrom);
+    tp_genome *out = NULL;
+    if (tp_genome_coarsen(c, g, (int)f, &out) != TP_OK) error("%s", tp_last_error());
+    return genome_result(ctx, out, n);
+}
+
 /* bucket `chrom` (0-based) of a genome over `nchrom` chromosomes: list(i, j, count), 0-based local bins, bucket order */
 SEXP C_tp_genome_pixels(SEXP ctx, SEXP genome, SEXP chrom, SEXP nchrom) {
     tp_ctx *c = ctx_of(ctx);
@@ -828,6 +840,7 @@ static const R_CallMethodDef call_table[] = {
     {"C_tp_genome_depth", (DL_FUNC)&C_tp_genome_depth, 3},
     {"C_tp_genome_downsample", (DL_FUNC)&C_tp_genome_downsample, 5},
     {"C_tp_genome_pixels", (DL_FUNC)&C_tp_genome_pixels, 4},
+    {"C_tp_genome_coarsen", (DL_FUNC)&C_tp_genome_coarsen, 4},
     {NULL, NULL, 0}};
 
 void R_init_TADpoleB200(DllInfo *dll) {

@@ -34,6 +34,7 @@ EXPORTED = [
     "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
     "tp_centromere_split", "tp_batch_split", "tp_batch_recall", "tp_batch_dendro", "tp_batch_resident_bytes",
     "tp_batch_resident_devices", "tp_ctx_get", "tp_genome_depth", "tp_genome_downsample", "tp_genome_pixels",
+    "tp_genome_coarsen",
 ]
 
 
@@ -92,6 +93,7 @@ def load():
         "tp_genome_depth": (c_int, [vp, vp, POINTER(ctypes.c_ulonglong)]),
         "tp_genome_downsample": (c_int, [vp, vp, ctypes.c_ulonglong, ctypes.c_ulonglong, POINTER(vp)]),
         "tp_genome_pixels": (c_int, [vp, vp, c_int, ip, ip, dp]),
+        "tp_genome_coarsen": (c_int, [vp, vp, c_int, POINTER(vp)]),
         "tp_find_groups": (c_int, [dp, c_int, ip]),
         "tp_ctx_destroy": (c_int, [vp]),
         "tp_ctx_sync": (c_int, [vp]),
@@ -860,6 +862,12 @@ class Genome:
         h = c_void_p()
         check(self.lib.tp_genome_downsample(self.ctx._h, self._h, int(contacts), int(seed) % 2 ** 64, ctypes.byref(h)))
         return Genome(self.ctx, h, self.chrom_bins)
+
+    def coarsen(self, factor):
+        """tp_genome_coarsen: a new Genome at `factor` times the bin size, ceil(chrom_bins / factor) bins per chromosome."""
+        h = c_void_p()
+        check(self.lib.tp_genome_coarsen(self.ctx._h, self._h, int(factor), ctypes.byref(h)))
+        return Genome(self.ctx, h, (-(-self.chrom_bins.astype(np.int64) // int(factor))).astype(np.int32))
 
     def pixels(self, chrom):
         """(i, j, count) of bucket `chrom` (0-based), in the bucket's order (tp_genome_pixels)"""

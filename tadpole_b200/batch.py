@@ -232,12 +232,15 @@ class _CtxRef:
 
 class LoadedGenome:
     """A genome-wide pixel list held on the GPU, one bucket of cis pixels per chromosome (GenomePixels.load, or a
-    subsample of another LoadedGenome).  names / chrom_bins: the bin table's chromosomes and their bins.  TADpole_genome
-    takes it wherever it takes GenomePixels, and does not free it.  Close it (or use it as a context manager) to release
-    its device memory."""
+    subsample or coarsening of another LoadedGenome).  names / chrom_bins: the bin table's chromosomes and their bins.
+    factor: the bin size as a multiple of the ingested file's (1 after load(), multiplied by each coarsen(), kept by
+    downsample()); bin b (1-based) of a chromosome of n_fine ingested bins covers the ingested bins
+    factor * (b - 1) + 1 .. min(factor * b, n_fine).  TADpole_genome takes it wherever it takes GenomePixels, and does not
+    free it.  Close it (or use it as a context manager) to release its device memory."""
 
-    def __init__(self, genome, names, ref):
+    def __init__(self, genome, names, ref, factor=1):
         self._g, self.names, self.chrom_bins = genome, list(names), np.asarray(genome.chrom_bins, dtype=np.int32)
+        self.factor = factor
         self._ref = ref.acquire()
         self.ctx = ref.ctx
 
@@ -265,7 +268,24 @@ class LoadedGenome:
         contacts = int(contacts)
         if not 0 <= contacts <= total:
             raise ValueError(f"contacts must be in 0..{total} (the genome's cis contacts), not {contacts}")
-        return LoadedGenome(self._g.downsample(contacts, int(seed) % 2 ** 64), self.names, self._ref)
+        return LoadedGenome(self._g.downsample(contacts, int(seed) % 2 ** 64), self.names, self._ref, self.factor)
+
+    def coarsen(self, factor):
+        """A new LoadedGenome at `factor` times this genome's bin size, on the GPU that holds it (DESIGN S0e): chromosome c
+        gets ceil(chrom_bins[c] / factor) bins (the last one narrower when factor does not divide it), and coarse cell
+        (I, J) holds the sum of the counts of the cells (i, j) with i // factor = I and j // factor = J (a NaN count adds
+        0; cells that sum to 0 are left out).  Integer counts add exactly.  Both genomes stay valid and either may be
+        closed first."""
+        if isinstance(factor, bool) or not isinstance(factor, (int, np.integer, float, np.floating)):
+            raise ValueError(f"factor must be an integer >= 1, not {factor!r}")
+        if isinstance(factor, (float, np.floating)) and not float(factor).is_integer():
+            raise ValueError(f"factor must be an integer >= 1, not {factor!r}")
+        f = int(factor)
+        if not 1 <= f <= 2 ** 31 - 1:
+            raise ValueError(f"factor must be an integer in 1..2^31-1, not {factor!r}")
+        if self._g is None:
+            raise ValueError("the LoadedGenome has been closed")
+        return LoadedGenome(self._g.coarsen(f), self.names, self._ref, self.factor * f)
 
     def pixels(self, chrom):
         """(i, j, count) of chromosome `chrom` (a name): chromosome-local 0-based bins, sorted by (i, j)"""

@@ -23,10 +23,9 @@
 // three passes over the cells (N = 0 and N = T skip the select); memory: 16 bytes per table slot (2 slots per bucket
 // entry, rounded up to a power of two) + 28 bytes per cell, the table released before the output is built.
 #include <algorithm>
-#include "common.cuh"
+#include "genome_util.cuh"
 #include "philox.cuh"
 
-#define DS_THREADS 256
 #define DS_ITEMS 16
 #define DS_TILE (DS_THREADS * DS_ITEMS)      // reads per tile of the select passes; cells per tile of the scan
 #define DS_DIGIT 12
@@ -41,30 +40,7 @@ typedef unsigned long long u64;
 // [2] cells listed [3] reads tied with the threshold  [4] selection prefix [5] reads still needed at the prefix
 enum { DS_BAD = 0, DS_BIG, DS_NCELL, DS_NEQ, DS_PREFIX, DS_NEED, DS_NSTATUS = 8 };
 
-// largest c in [0, nchrom) with offs[c] <= e (the chromosome whose bucket holds entry e)
-__device__ __forceinline__ int ds_chrom_of_entry(const u64 *__restrict__ offs, int nchrom, u64 e) {
-    int lo = 0, hi = nchrom - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (__ldg(offs + mid) <= e) lo = mid; else hi = mid - 1;
-    }
-    return lo;
-}
-__device__ __forceinline__ int ds_chrom_of_bin(const int *__restrict__ starts, int nchrom, int x) {
-    int lo = 0, hi = nchrom - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (__ldg(starts + mid) <= x) lo = mid; else hi = mid - 1;
-    }
-    return lo;
-}
-
 __device__ __forceinline__ bool ds_is_count(double v) { return v >= 0.0 && v < 4294967296.0 && v == floor(v); }
-
-__device__ __forceinline__ u64 ds_hash(u64 key) {
-    key ^= key >> 33; key *= 0xff51afd7ed558ccdULL; key ^= key >> 33; key *= 0xc4ceb9fe1a85ec53ULL; key ^= key >> 33;
-    return key;
-}
 
 // exclusive scan of one u64 per thread over the CTA; *total = the sum
 __device__ __forceinline__ u64 ds_block_scan(u64 v, u64 *s_warp, u64 *total) {
@@ -402,23 +378,6 @@ ds_out_scatter_kernel(const int *__restrict__ cc, const int *__restrict__ ci, co
 }
 
 // ---- host side ------------------------------------------------------------------------------------------------------------
-// the member of ctx on the device that holds g (multi-device contexts: any of their devices), or an error
-static int ds_member(tp_ctx *ctx, const tp_genome *g, const char *who, tp_ctx **out) {
-    for (int r = 0; r < tp_group_size(ctx); r++) {
-        tp_ctx *m = tp_group_member(ctx, r);
-        if (m && m->device == g->device) { *out = m; return TP_OK; }
-    }
-    tp_set_error("%s: the handle is on device %d, which is not a device of the context", who, g->device);
-    return TP_ERR_ARG;
-}
-
-static unsigned ds_grid(const tp_ctx *c, u64 work) {
-    const u64 want = (work + DS_THREADS - 1) / DS_THREADS, cap = (u64)c->sm_count * 16;
-    return (unsigned)(want < 1 ? 1 : want < cap ? want : cap);
-}
-
-struct GenomeOwnerDs { tp_genome *g = nullptr; ~GenomeOwnerDs() { if (g) tp_genome_free(g); } };
-
 struct DsBufs {
     DevBuf aux, table, cells, kept, out_tmp;
     ~DsBufs() { aux.release(); table.release(); cells.release(); kept.release(); out_tmp.release(); }
