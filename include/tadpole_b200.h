@@ -382,6 +382,34 @@ int tp_genome_pixels(tp_ctx *ctx, const tp_genome *g, int chrom, int32_t *i_out,
  * the output buckets when they do not fit. */
 int tp_genome_coarsen(tp_ctx *ctx, const tp_genome *src, int factor, tp_genome **out);
 
+/* ---- read pairs: a genome binned at any bin size from the files a Hi-C pipeline writes (DESIGN S0f) -------------------
+ * *out = the cis contacts of the plain-text read-pair files paths[npaths] (4DN .pairs, HiC-Pro *.allValidPairs, Juicer
+ * merged_nodups.txt), binned at `binsize` (>= 1) bp over the chromosome table names[nchrom] / lengths[nchrom] (bp, table
+ * order).  cols = the 0-based columns (each <= 63, all four different) of chrom1, pos1, chrom2, pos2; a position p is
+ * index_base-based (0 or 1; the 4DN format is 1-based).  Chromosome c has ceil(lengths[c] / binsize) bins (the last one
+ * narrower when binsize does not divide the length) and p falls in bin (p - index_base) / binsize.
+ * A line whose first byte is '#' is a comment; a line of only spaces, tabs and '\r' is skipped; every other line is a
+ * pair, its fields separated by runs of spaces and tabs (a '\r' before the '\n' is ignored).  A pair naming a chromosome
+ * (exact bytes) that is not in the table is unplaced, else a pair on two chromosomes is trans: both are counted and
+ * dropped.  A cis pair adds 1 to cell (c, min(b1, b2), max(b1, b2)): a read pair is unordered.
+ * TP_ERR_ARG naming the file and the lowest 1-based line number (comment lines count) for: fewer fields than the largest
+ * column, a position that is not 1-18 ASCII digits, a position on a chromosome of the table outside index_base ..
+ * length - 1 + index_base, a line longer than the device window.  TP_ERR_ARG also for a gzip file (compressed input is
+ * not read), a file with no pair lines, and a chromosome table with a duplicate, empty or whitespace-holding name, a
+ * length < 1, or 2^31 - 1 or more bins in all.
+ * The result is an ordinary handle on ctx's device: every cell with count >= 1, as an exact integer in FP64 (bucket order
+ * unspecified).  tp_genome_stats: cis cells per chromosome, trans = trans pairs, below = 0.  counts_out (may be NULL) =
+ * {pair lines, cis, trans, unplaced}, pair lines = cis + trans + unplaced.  Several files give what their concatenation
+ * gives, in any order (line numbers in errors are per file); nothing depends on the window size or the file order.
+ * The files are streamed through device windows of 64 MB (environment variable TADPOLE_PAIRS_WINDOW: another size in
+ * bytes): device memory is the window, 8 bytes per line of a window and 16 bytes per slot of the cell table (2 to 4
+ * slots per distinct cell), then 16 bytes per cell for the buckets; TP_ERR_NOMEM when the table or the buckets do not
+ * fit.  tp_ingest_stats afterwards: [0] wall ms, [1] device ms of the per-window line-end and parse kernels, [2] bytes
+ * read, [3] windows. */
+int tp_genome_ingest_pairs_file(tp_ctx *ctx, const char *const *paths, int npaths, const char *const *names,
+                                const int64_t *lengths, int nchrom, int64_t binsize, const int cols[4], int index_base,
+                                unsigned long long counts_out[4], tp_genome **out);
+
 /* The context is a device-resident pipeline handle: after tp_call / tp_call_arm / tp_pca the PC scores stay in HBM, and
  * after a sweep so do all k dendrograms (tp_get_dendro) and the score matrix (tp_get_sweep_scores).  tp_recall repeats
  * only the n_pcs sweep and the selection for another max_pcs (<= the number of PCs computed) and / or min_clusters:

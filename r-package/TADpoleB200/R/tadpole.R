@@ -326,7 +326,9 @@ genome_downsample <- function(g, contacts = NULL, fraction = NULL, seed = 0) {
     if (!(contacts >= 0 && contacts <= total)) stop("contacts must be in 0..", format(total, scientific = FALSE))
     tab <- list(names = attr(g, "chroms"), n = attr(g, "n"))
     p <- .Call(C_tp_genome_downsample, attr(g, "ctx"), g, length(tab$n), as.numeric(contacts), as.numeric(seed))
-    .tp_loaded(p[[1L]], tab, attr(g, "ctx"), attr(g, "factor"))
+    out <- .tp_loaded(p[[1L]], tab, attr(g, "ctx"), attr(g, "factor"))
+    attr(out, "binsize") <- attr(g, "binsize")
+    out
 }
 
 # A new loaded genome at `factor` times g's bin size (DESIGN S0e): chromosome c gets ceiling(n_c / factor) bins (the
@@ -340,7 +342,59 @@ genome_coarsen <- function(g, factor) {
           factor == floor(factor))) stop("factor must be a whole number >= 1")
     tab <- list(names = attr(g, "chroms"), n = as.integer(ceiling(attr(g, "n") / factor)))
     p <- .Call(C_tp_genome_coarsen, attr(g, "ctx"), g, length(tab$n), as.numeric(factor))
-    .tp_loaded(p[[1L]], tab, attr(g, "ctx"), attr(g, "factor") * factor)
+    out <- .tp_loaded(p[[1L]], tab, attr(g, "ctx"), attr(g, "factor") * factor)
+    if (!is.null(attr(g, "binsize"))) attr(out, "binsize") <- attr(g, "binsize") * factor
+    out
+}
+
+# Read-pair files (4DN .pairs, HiC-Pro *.allValidPairs, Juicer merged_nodups.txt) binned at `binsize` bp on the GPU and
+# kept there (DESIGN S0f): a loaded genome like genome_load()'s, with attr(, "binsize") and attr(, "pairs") =
+# c(lines, cis, trans, unplaced).  Several files are pooled at read level.  chromsizes: a two-column chrom.sizes path, a
+# data.frame or list (name, length), a named numeric vector, or NULL for the '#chromsize:' header lines of the first
+# file.  Chromosome c gets ceiling(length / binsize) bins.  columns: the 1-based columns of chrom1, pos1, chrom2, pos2
+# (4DN pairs: 2:5; HiC-Pro validPairs: c(2, 3, 5, 6); Juicer merged_nodups: c(2, 3, 6, 7)); index_base: 1 (4DN) or 0.
+genome_load_pairs <- function(paths, chromsizes = NULL, binsize, columns = 2:5, index_base = 1L) {
+    paths <- as.character(paths)
+    if (length(paths) < 1L) stop("genome_load_pairs needs one or more file paths")
+    if (!(is.numeric(binsize) && length(binsize) == 1L && !is.na(binsize) && binsize >= 1 && binsize == floor(binsize)))
+        stop("binsize must be a whole number >= 1 (bp)")
+    if (!(is.numeric(columns) && length(columns) == 4L && !anyNA(columns) && all(columns >= 1 & columns <= 64) &&
+          all(columns == floor(columns)) && !anyDuplicated(columns)))
+        stop("columns must be four different 1-based column numbers in 1..64")
+    if (!(length(index_base) == 1L && index_base %in% c(0, 1))) stop("index_base must be 0 or 1")
+    tab <- .tp_chromsizes(chromsizes, paths[[1L]])
+    ctx <- .tp_ctx()
+    p <- .Call(C_tp_genome_pairs_file, ctx, paths, tab$name, tab$length, as.numeric(binsize),
+               as.integer(c(columns - 1L, index_base)))
+    g <- .tp_loaded(p[[1L]], list(names = tab$name, n = as.integer((tab$length - 1) %/% binsize + 1)), ctx)
+    attr(g, "binsize") <- binsize
+    attr(g, "pairs") <- stats::setNames(p[[4L]], c("lines", "cis", "trans", "unplaced"))
+    g
+}
+
+# data.frame(name, length) of a chromosome table given to genome_load_pairs()
+.tp_chromsizes <- function(chromsizes, first) {
+    if (is.null(chromsizes)) {
+        con <- file(first, "r")
+        on.exit(close(con))
+        hdr <- character(0)
+        repeat {
+            l <- readLines(con, n = 1L)
+            if (!length(l) || !startsWith(l, "#")) break
+            hdr <- c(hdr, l)
+        }
+        hdr <- grep("^#chromsize:", hdr, value = TRUE)
+        if (!length(hdr)) stop(first, " has no '#chromsize:' header lines: give the chromosome table (chromsizes =)")
+        f <- strsplit(trimws(sub("^#chromsize:", "", hdr)), "[ \t]+")
+        return(data.frame(name = vapply(f, `[`, "", 1L), length = as.numeric(vapply(f, `[`, "", 2L))))
+    }
+    if (is.character(chromsizes) && length(chromsizes) == 1L) {
+        t <- utils::read.table(chromsizes, colClasses = "character", comment.char = "")
+        return(data.frame(name = t[[1L]], length = as.numeric(t[[2L]])))
+    }
+    if (is.numeric(chromsizes) && !is.null(names(chromsizes)))
+        return(data.frame(name = names(chromsizes), length = as.numeric(chromsizes)))
+    data.frame(name = as.character(chromsizes[[1L]]), length = as.numeric(chromsizes[[2L]]))
 }
 
 # the pixels of chromosome `chrom` of a loaded genome: data.frame(i, j, count), chromosome-local 1-based bins, sorted

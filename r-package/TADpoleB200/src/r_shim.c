@@ -568,6 +568,38 @@ SEXP C_tp_genome_coarsen(SEXP ctx, SEXP genome, SEXP nchrom, SEXP factor) {
     return genome_result(ctx, out, n);
 }
 
+/* Read-pair files binned at `binsize` bp on the GPU (tp_genome_ingest_pairs_file): paths and names (character), lengths
+ * (numeric, bp), layout = integer c(chrom1, pos1, chrom2, pos2 columns (0-based), index_base).  Returns what C_tp_genome
+ * returns, and c(pair lines, cis, trans, unplaced) as a fourth element. */
+SEXP C_tp_genome_pairs_file(SEXP ctx, SEXP paths, SEXP names, SEXP lengths, SEXP binsize, SEXP layout) {
+    const int np = length(paths), nc = length(names);
+    if (np < 1) error("TADpole: at least one pairs file is needed");
+    if (nc < 1 || nc > (1 << 20) || !isReal(lengths) || length(lengths) != nc)
+        error("TADpole: the chromosome table needs 1..2^20 names and as many numeric lengths");
+    for (int c = 0; c < nc; c++) {
+        const double v = REAL(lengths)[c];
+        if (!(v >= 1 && v <= 9007199254740992.0 && v == floor(v))) error("TADpole: chromosome lengths must be whole numbers >= 1");
+    }
+    const double b = asReal(binsize);
+    if (!(b >= 1 && b <= 9007199254740992.0 && b == floor(b))) error("TADpole: binsize must be a whole number >= 1");
+    if (!isInteger(layout) || length(layout) != 5) error("TADpole: layout must be 4 column indices and index_base (integer)");
+    tp_ctx *c = ctx_of(ctx);
+    const char **pp = (const char **)R_alloc((size_t)np, sizeof(char *)), **nm = (const char **)R_alloc((size_t)nc, sizeof(char *));
+    int64_t *len = (int64_t *)R_alloc((size_t)nc, sizeof(int64_t));
+    for (int i = 0; i < np; i++) pp[i] = CHAR(STRING_ELT(paths, i));
+    for (int i = 0; i < nc; i++) { nm[i] = CHAR(STRING_ELT(names, i)); len[i] = (int64_t)REAL(lengths)[i]; }
+    unsigned long long counts[4] = {0, 0, 0, 0};
+    tp_genome *g = NULL;
+    if (tp_genome_ingest_pairs_file(c, pp, np, nm, len, nc, (int64_t)b, INTEGER(layout), INTEGER(layout)[4], counts, &g) != TP_OK)
+        error("%s", tp_last_error());
+    SEXP res = PROTECT(genome_result(ctx, g, nc)), cnt = PROTECT(allocVector(REALSXP, 4)), out = PROTECT(allocVector(VECSXP, 4));
+    for (int i = 0; i < 4; i++) REAL(cnt)[i] = (double)counts[i];
+    for (int i = 0; i < 3; i++) SET_VECTOR_ELT(out, i, VECTOR_ELT(res, i));
+    SET_VECTOR_ELT(out, 3, cnt);
+    UNPROTECT(3);
+    return out;
+}
+
 /* bucket `chrom` (0-based) of a genome over `nchrom` chromosomes: list(i, j, count), 0-based local bins, bucket order */
 SEXP C_tp_genome_pixels(SEXP ctx, SEXP genome, SEXP chrom, SEXP nchrom) {
     tp_ctx *c = ctx_of(ctx);
@@ -841,6 +873,7 @@ static const R_CallMethodDef call_table[] = {
     {"C_tp_genome_downsample", (DL_FUNC)&C_tp_genome_downsample, 5},
     {"C_tp_genome_pixels", (DL_FUNC)&C_tp_genome_pixels, 4},
     {"C_tp_genome_coarsen", (DL_FUNC)&C_tp_genome_coarsen, 4},
+    {"C_tp_genome_pairs_file", (DL_FUNC)&C_tp_genome_pairs_file, 6},
     {NULL, NULL, 0}};
 
 void R_init_TADpoleB200(DllInfo *dll) {

@@ -7,9 +7,10 @@ libtadpole_b200.so (hand-written CUDA for sm_100a behind a C ABI, include/tadpol
 from .api import TADpole, load_mat, diffT, diffT_batch, diffT_null, random_bed, random_bed_batch, read_matrix, bin_index, Tadpole, LoadedMatrix, SparseCounts, get_context
 from ._lib import Context, TadpoleError, assemble
 from .hclust import Dendro, find_groups, cutree
-from .batch import ContextPool, TADpole_batch, GenomePixels, LoadedGenome, TADpole_genome, read_bins, diffT_genome, equal_depth
+from .batch import (ContextPool, TADpole_batch, GenomePixels, GenomePairs, LoadedGenome, TADpole_genome, read_bins, read_chromsizes,
+                    diffT_genome, equal_depth)
 
 __all__ = ["TADpole", "load_mat", "diffT", "diffT_batch", "diffT_null", "random_bed", "random_bed_batch", "read_matrix", "bin_index", "Tadpole", "LoadedMatrix", "SparseCounts",
-           "get_context", "ContextPool", "TADpole_batch", "GenomePixels", "LoadedGenome", "TADpole_genome", "read_bins", "diffT_genome",
+           "get_context", "ContextPool", "TADpole_batch", "GenomePixels", "GenomePairs", "LoadedGenome", "TADpole_genome", "read_bins", "read_chromsizes", "diffT_genome",
            "equal_depth", "Context", "TadpoleError", "assemble", "Dendro", "find_groups", "cutree"]
 __version__ = "0.1.0"

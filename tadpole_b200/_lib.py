@@ -34,7 +34,7 @@ EXPORTED = [
     "tp_genome_ingest", "tp_genome_ingest_file", "tp_genome_stats", "tp_genome_matrix", "tp_call_genome", "tp_genome_free",
     "tp_centromere_split", "tp_batch_split", "tp_batch_recall", "tp_batch_dendro", "tp_batch_resident_bytes",
     "tp_batch_resident_devices", "tp_ctx_get", "tp_genome_depth", "tp_genome_downsample", "tp_genome_pixels",
-    "tp_genome_coarsen",
+    "tp_genome_coarsen", "tp_genome_ingest_pairs_file",
 ]
 
 
@@ -94,6 +94,8 @@ def load():
         "tp_genome_downsample": (c_int, [vp, vp, ctypes.c_ulonglong, ctypes.c_ulonglong, POINTER(vp)]),
         "tp_genome_pixels": (c_int, [vp, vp, c_int, ip, ip, dp]),
         "tp_genome_coarsen": (c_int, [vp, vp, c_int, POINTER(vp)]),
+        "tp_genome_ingest_pairs_file": (c_int, [vp, POINTER(c_char_p), c_int, POINTER(c_char_p), POINTER(c_longlong), c_int,
+                                                c_longlong, ip, c_int, POINTER(ctypes.c_ulonglong), POINTER(vp)]),
         "tp_find_groups": (c_int, [dp, c_int, ip]),
         "tp_ctx_destroy": (c_int, [vp]),
         "tp_ctx_sync": (c_int, [vp]),
@@ -690,6 +692,22 @@ class Context:
             check(self.lib.tp_genome_ingest(self._h, _ip(cb), cb.size, _ip(b1), _ip(b2), _dp(v), b1.size, int(index_base),
                                             ctypes.byref(h)))
         return Genome(self, h, cb)
+
+    def genome_ingest_pairs(self, paths, names, lengths, binsize, columns=(1, 2, 3, 4), index_base=1):
+        """tp_genome_ingest_pairs_file: the read-pair files `paths` binned at `binsize` bp over the chromosome table
+        (names, lengths in bp) on this context's (first) device.  Returns (Genome, dict(lines, cis, trans, unplaced))."""
+        enc = [os.fsencode(p) for p in paths]
+        cp = (c_char_p * len(enc))(*enc)
+        cn = (c_char_p * len(names))(*[str(nm).encode() for nm in names])
+        ln = np.ascontiguousarray(lengths, dtype=np.int64)
+        lp = ln.ctypes.data_as(POINTER(c_longlong))
+        cols = np.ascontiguousarray(columns, dtype=np.int32)
+        counts = (ctypes.c_ulonglong * 4)()
+        h = c_void_p()
+        check(self.lib.tp_genome_ingest_pairs_file(self._h, cp, len(enc), cn, lp, ln.size, int(binsize), _ip(cols),
+                                                   int(index_base), counts, ctypes.byref(h)))
+        bins = ((ln - 1) // int(binsize) + 1).astype(np.int32)
+        return Genome(self, h, bins), dict(zip(("lines", "cis", "trans", "unplaced"), (int(x) for x in counts)))
 
     def call_genome(self, genome, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, inflight=8, tables=True,
                     centromere_search=False, centromere_fix=False, resident=False):

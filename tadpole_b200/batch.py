@@ -10,7 +10,9 @@ calling TADpole() on each matrix in turn.
 
 TADpole_genome() starts from what Hi-C pipelines write for a whole genome: one pixel list with global bin ids (HiC-Pro
 *.matrix, cooler dump -t pixels) and its bin table.  The pixels are split by chromosome on the GPU (tp_genome_ingest),
-and each chromosome's dense matrix exists only in HBM, only while its call runs (tp_call_genome).
+and each chromosome's dense matrix exists only in HBM, only while its call runs (tp_call_genome).  GenomePairs starts one
+step earlier, from the read-pair files themselves (4DN .pairs, HiC-Pro *.allValidPairs, Juicer merged_nodups.txt), binned
+at any bin size on the GPU (tp_genome_ingest_pairs_file).
 """
 from __future__ import annotations
 
@@ -24,8 +26,8 @@ from .api import (NOSPLIT_MESSAGE, ResidentArm, Tadpole, _Obj, _arm_object, _bed
                   _messages_bad, _messages_optimal, _messages_split, get_context, message, read_matrix)
 from .hclust import Dendro
 
-__all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "LoadedGenome", "TADpole_genome", "read_bins", "diffT_genome",
-           "equal_depth"]
+__all__ = ["ContextPool", "TADpole_batch", "GenomePixels", "GenomePairs", "LoadedGenome", "TADpole_genome", "read_bins",
+           "read_chromsizes", "diffT_genome", "equal_depth"]
 
 
 class ContextPool:
@@ -214,6 +216,117 @@ class GenomePixels:
             raise
 
 
+def read_chromsizes(chromsizes, first_path=None):
+    """[(name, length in bp)] of a chromosome table: the path of a two-column chrom.sizes file, a list of (name, length),
+    a dict {name: length}, or None for the '#chromsize: <name> <length>' header lines at the top of `first_path` (the 4DN
+    pairs header; a file without them is a ValueError).  Names must be unique, non-empty and free of whitespace, lengths
+    whole numbers >= 1."""
+    if chromsizes is None:
+        table = []
+        with open(first_path, "rb") as fh:
+            for raw in fh:
+                if not raw.startswith(b"#"):
+                    break
+                if raw.startswith(b"#chromsize:"):
+                    f = raw[len(b"#chromsize:"):].split()
+                    if len(f) != 2:
+                        raise ValueError(f"{first_path}: malformed header line {raw.decode(errors='replace').strip()!r}")
+                    table.append((f[0].decode(), f[1].decode()))
+        if not table:
+            raise ValueError(f"{first_path} has no '#chromsize:' header lines: give the chromosome table (chromsizes=)")
+    elif isinstance(chromsizes, (str, os.PathLike)):
+        table = []
+        with open(chromsizes) as fh:
+            for line in fh:
+                f = line.split()
+                if not f:
+                    continue
+                if len(f) < 2:
+                    raise ValueError(f"{chromsizes}: a chrom.sizes line needs a name and a length: {line.strip()!r}")
+                table.append((f[0], f[1]))
+    elif isinstance(chromsizes, dict):
+        table = list(chromsizes.items())
+    else:
+        table = [tuple(x) for x in chromsizes]
+    out, seen = [], set()
+    for item in table:
+        if len(item) != 2:
+            raise ValueError(f"a chromosome table entry is (name, length), not {item!r}")
+        nm, ln = item
+        nm = str(nm)
+        if not nm or any(ch.isspace() for ch in nm):
+            raise ValueError(f"chromosome name {nm!r} is empty or contains whitespace")
+        if nm in seen:
+            raise ValueError(f"chromosome {nm!r} appears twice in the chromosome table")
+        seen.add(nm)
+        try:
+            n = int(ln)
+        except (TypeError, ValueError, OverflowError):
+            n = None
+        if n is None or isinstance(ln, bool) or n < 1 or (isinstance(ln, float) and ln != n):
+            raise ValueError(f"chromosome {nm!r} has length {ln!r}: a whole number >= 1 is needed")
+        out.append((nm, n))
+    if not out:
+        raise ValueError("the chromosome table is empty")
+    return out
+
+
+class GenomePairs:
+    """The contacts of a whole genome as the read-pair files a Hi-C pipeline writes, binned at `binsize` bp on the GPU:
+    a drop-in for GenomePixels (names, chrom_bins, load(), TADpole_genome()).  Several files are pooled at read level
+    (replicates), and the result is the same in any file order.  Plain text only (gzip input is refused).
+
+    paths: one path or a list.  chromsizes: see read_chromsizes (None: the '#chromsize:' header of the first file).
+    Chromosome c gets ceil(length / binsize) bins, and position p falls in bin (p - index_base) // binsize.
+    columns: the 0-based columns of (chrom1, pos1, chrom2, pos2):
+      4DN pairs (readID chrom1 pos1 chrom2 pos2 ...):                  (1, 2, 3, 4)
+      HiC-Pro validPairs (readID chr1 pos1 strand1 chr2 pos2 ...):     (1, 2, 4, 5)
+      Juicer merged_nodups (str1 chr1 pos1 frag1 str2 chr2 pos2 ...):  (1, 2, 5, 6)
+    index_base: 1 (the 4DN definition of positions) or 0.  Lines starting with '#' and blank lines are skipped; a pair on a
+    chromosome outside the table is unplaced and a pair between two chromosomes is trans: both are counted and dropped
+    (LoadedGenome.pair_counts).  DESIGN S0f has the whole spec."""
+
+    def __init__(self, paths, chromsizes=None, binsize=None, columns=(1, 2, 3, 4), index_base=1):
+        paths = [paths] if isinstance(paths, (str, os.PathLike)) else list(paths)
+        if not paths or not all(isinstance(p, (str, os.PathLike)) for p in paths):
+            raise ValueError("GenomePairs needs one or more file paths")
+        if binsize is None or isinstance(binsize, bool) or not isinstance(binsize, (int, np.integer)) or binsize < 1:
+            raise ValueError(f"binsize must be an integer >= 1 (bp), not {binsize!r}")
+        cols = tuple(columns) if isinstance(columns, (list, tuple, np.ndarray)) else ()
+        if len(cols) != 4 or not all(isinstance(c, (int, np.integer)) and not isinstance(c, bool) and 0 <= c <= 63
+                                     for c in cols) or len(set(int(c) for c in cols)) != 4:
+            raise ValueError(f"columns must be four different 0-based column indices in 0..63, not {columns!r}")
+        if isinstance(index_base, bool) or index_base not in (0, 1):
+            raise ValueError(f"index_base must be 0 or 1, not {index_base!r}")
+        self.paths = [os.fspath(p) for p in paths]
+        self.chromsizes = read_chromsizes(chromsizes, self.paths[0])
+        self.binsize, self.columns, self.index_base = int(binsize), tuple(int(c) for c in cols), int(index_base)
+        nb = [(ln - 1) // self.binsize + 1 for _, ln in self.chromsizes]
+        if sum(nb) >= 2 ** 31 - 1:
+            raise ValueError(f"{self.binsize} bp bins give {sum(nb)} bins in all; at most 2^31 - 2 are supported")
+        self.names = [nm for nm, _ in self.chromsizes]
+        self.chrom_bins = np.array(nb, dtype=np.int32)
+
+    def _load(self, ctx):
+        return ctx.genome_ingest_pairs(self.paths, self.names, [ln for _, ln in self.chromsizes], self.binsize,
+                                       self.columns, self.index_base)
+
+    def _ingest(self, ctx):
+        return self._load(ctx)[0]
+
+    def load(self, ctx=None, device=0):
+        """Read, bin and merge the pairs once and keep the cells on the GPU: a LoadedGenome with binsize and pair_counts
+        (dict(lines, cis, trans, unplaced)).  Without ctx, a context on `device` is made and closed with the last
+        LoadedGenome that uses it."""
+        ref = _CtxRef(ctx or _lib.Context(device), ctx is None)
+        try:
+            g, counts = self._load(ref.ctx)
+            return LoadedGenome(g, self.names, ref, binsize=self.binsize, pair_counts=counts)
+        except BaseException:
+            ref.release()
+            raise
+
+
 class _CtxRef:
     """The context of one or more LoadedGenomes; a context made for them is closed when the last one is closed."""
 
@@ -231,16 +344,18 @@ class _CtxRef:
 
 
 class LoadedGenome:
-    """A genome-wide pixel list held on the GPU, one bucket of cis pixels per chromosome (GenomePixels.load, or a
-    subsample or coarsening of another LoadedGenome).  names / chrom_bins: the bin table's chromosomes and their bins.
-    factor: the bin size as a multiple of the ingested file's (1 after load(), multiplied by each coarsen(), kept by
-    downsample()); bin b (1-based) of a chromosome of n_fine ingested bins covers the ingested bins
-    factor * (b - 1) + 1 .. min(factor * b, n_fine).  TADpole_genome takes it wherever it takes GenomePixels, and does not
-    free it.  Close it (or use it as a context manager) to release its device memory."""
+    """A genome-wide pixel list held on the GPU, one bucket of cis pixels per chromosome (GenomePixels.load,
+    GenomePairs.load, or a subsample or coarsening of another LoadedGenome).  names / chrom_bins: the bin table's
+    chromosomes and their bins.  factor: the bin size as a multiple of the ingested file's (1 after load(), multiplied by
+    each coarsen(), kept by downsample()); bin b (1-based) of a chromosome of n_fine ingested bins covers the ingested bins
+    factor * (b - 1) + 1 .. min(factor * b, n_fine).  binsize: the bin size in bp (None for a pixel-file load; multiplied
+    by coarsen(), kept by downsample()).  pair_counts: dict(lines, cis, trans, unplaced) of the files a GenomePairs load
+    read, else None.  TADpole_genome takes it wherever it takes GenomePixels, and does not free it.  Close it (or use it
+    as a context manager) to release its device memory."""
 
-    def __init__(self, genome, names, ref, factor=1):
+    def __init__(self, genome, names, ref, factor=1, binsize=None, pair_counts=None):
         self._g, self.names, self.chrom_bins = genome, list(names), np.asarray(genome.chrom_bins, dtype=np.int32)
-        self.factor = factor
+        self.factor, self.binsize, self.pair_counts = factor, binsize, pair_counts
         self._ref = ref.acquire()
         self.ctx = ref.ctx
 
@@ -268,7 +383,8 @@ class LoadedGenome:
         contacts = int(contacts)
         if not 0 <= contacts <= total:
             raise ValueError(f"contacts must be in 0..{total} (the genome's cis contacts), not {contacts}")
-        return LoadedGenome(self._g.downsample(contacts, int(seed) % 2 ** 64), self.names, self._ref, self.factor)
+        return LoadedGenome(self._g.downsample(contacts, int(seed) % 2 ** 64), self.names, self._ref, self.factor,
+                            self.binsize)
 
     def coarsen(self, factor):
         """A new LoadedGenome at `factor` times this genome's bin size, on the GPU that holds it (DESIGN S0e): chromosome c
@@ -285,7 +401,8 @@ class LoadedGenome:
             raise ValueError(f"factor must be an integer in 1..2^31-1, not {factor!r}")
         if self._g is None:
             raise ValueError("the LoadedGenome has been closed")
-        return LoadedGenome(self._g.coarsen(f), self.names, self._ref, self.factor * f)
+        return LoadedGenome(self._g.coarsen(f), self.names, self._ref, self.factor * f,
+                            None if self.binsize is None else self.binsize * f)
 
     def pixels(self, chrom):
         """(i, j, count) of chromosome `chrom` (a name): chromosome-local 0-based bins, sorted by (i, j)"""
@@ -363,8 +480,9 @@ class GenomeResult(dict):
 
 def TADpole_genome(pixels, chroms=None, max_pcs=200, min_clusters=2, bad_frac=0.01, ctx=None, device=0, streams=4,
                    centromere_search=False, centromere_fix=False, resident=False):
-    """TADpole() on every chromosome of a genome-wide pixel list (GenomePixels, or a LoadedGenome: then with ctx=None the
-    call runs on the context the genome was loaded on, and the genome stays loaded), `streams` calls in flight per GPU.
+    """TADpole() on every chromosome of a genome-wide pixel list (GenomePixels, GenomePairs, or a LoadedGenome: then with
+    ctx=None the call runs on the context the genome was loaded on, and the genome stays loaded), `streams` calls in
+    flight per GPU.
     Each chromosome's Tadpole is the one TADpole() returns for that chromosome's dense matrix (with centromere_search /
     centromere_fix as TADpole() takes them: p, q and merging_arms; a chromosome that does not split fails with
     TADpole()'s message unless centromere_fix).  Returns a GenomeResult in bin-table order, or in `chroms` order when

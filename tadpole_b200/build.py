@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtadpole_b200.so")
-SOURCES = ["api.cu", "filter.cu", "gemm.cu", "jacobi.cu", "cholinv.cu", "osj.cu", "pca.cu", "coniss.cu", "difft.cu", "comm.cu", "igemm.cu", "ingest.cu", "group.cu", "downsample.cu", "coarsen.cu"]
+SOURCES = ["api.cu", "filter.cu", "gemm.cu", "jacobi.cu", "cholinv.cu", "osj.cu", "pca.cu", "coniss.cu", "difft.cu", "comm.cu", "igemm.cu", "ingest.cu", "group.cu", "downsample.cu", "coarsen.cu", "pairs.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", *os.environ.get("TADPOLE_NVCC_EXTRA", "").split(),
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default"]
 

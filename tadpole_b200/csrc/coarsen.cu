@@ -7,18 +7,15 @@
 //   1. cs_insert_kernel: every entry is added into an open-addressing table in HBM on the coarse key
 //      ((S_c + I) << 31) | (S_c + J), S_c the first coarse bin of c, with CAS and native FP64 atomicAdd.  (Adding up the
 //      runs of one cell in the warp first, with __shfl_down_sync, measured no faster on sorted input: DESIGN S0e.)
-//   2. cs_count_kernel: the stored cells of each chromosome (warp-aggregated atomics); the host scans them into offsets.
-//   3. cs_scatter_kernel: (count, I, J) of every stored cell into its chromosome's bucket through per-chromosome cursors.
+//   2. cs_count_kernel (genome_util.cuh): the stored cells of each chromosome (warp-aggregated atomics); the host scans
+//      them into offsets.
+//   3. cs_scatter_kernel (genome_util.cuh): (count, I, J) of every stored cell into its chromosome's bucket through
+//      per-chromosome cursors.
 // Integer counts whose cell sums of |count| stay below 2^53 add exactly, so the result is the same bits in any order;
 // otherwise the rounding order is unspecified (as in coo_scatter_kernel).  Memory: 16 bytes per table slot (2 slots per
 // bucket entry, rounded up to a power of two), and 16 bytes per output cell while the buckets are written; the table is
 // released before the call returns.
 #include "genome_util.cuh"
-
-#define CS_EMPTY 0xffffffffffffffffULL
-#define CS_FULL 0xffffffffu
-
-typedef unsigned long long u64;
 
 // ---- 1. merge ---------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(DS_THREADS)
@@ -37,53 +34,6 @@ cs_insert_kernel(const double *__restrict__ cnt, const int *__restrict__ bi, con
             if (k == CS_EMPTY) k = atomicCAS(tkeys + s, CS_EMPTY, key);
             if (k == CS_EMPTY || k == key) { atomicAdd(tval + s, v); break; }
             s = (s + 1) & mask;
-        }
-    }
-}
-
-// the chromosome of table slot s when it holds a cell to store (a sum that is not exactly 0), else -1
-__device__ __forceinline__ int cs_slot_chrom(const u64 *__restrict__ tkeys, const double *__restrict__ tval, u64 cap, u64 s,
-                                             const int *__restrict__ cstarts, int nchrom, u64 *key, double *v) {
-    if (s >= cap) return -1;
-    *key = tkeys[s];
-    if (*key == CS_EMPTY) return -1;
-    *v = tval[s];
-    if (*v == 0.0) return -1;
-    return ds_chrom_of_bin(cstarts, nchrom, (int)(*key >> 31));
-}
-
-// ---- 2. stored cells per chromosome --------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(DS_THREADS)
-cs_count_kernel(const u64 *__restrict__ tkeys, const double *__restrict__ tval, u64 cap, const int *__restrict__ cstarts,
-                int nchrom, u64 *__restrict__ hist) {
-    const u64 stride = (u64)gridDim.x * DS_THREADS;
-    for (u64 base = (u64)blockIdx.x * DS_THREADS; base < cap; base += stride) {
-        u64 key = 0;
-        double v = 0.0;
-        const int c = cs_slot_chrom(tkeys, tval, cap, base + threadIdx.x, cstarts, nchrom, &key, &v);
-        const unsigned grp = __match_any_sync(CS_FULL, c);
-        if (c >= 0 && (threadIdx.x & 31) == __ffs(grp) - 1) atomicAdd(hist + c, (u64)__popc(grp));
-    }
-}
-
-// ---- 3. the new buckets ---------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(DS_THREADS)
-cs_scatter_kernel(const u64 *__restrict__ tkeys, const double *__restrict__ tval, u64 cap, const int *__restrict__ cstarts,
-                  int nchrom, u64 *__restrict__ cursor, double *__restrict__ ov, int *__restrict__ oi, int *__restrict__ oj) {
-    const u64 stride = (u64)gridDim.x * DS_THREADS;
-    const int lane = threadIdx.x & 31;
-    for (u64 base = (u64)blockIdx.x * DS_THREADS; base < cap; base += stride) {
-        u64 key = 0;
-        double v = 0.0;
-        const int c = cs_slot_chrom(tkeys, tval, cap, base + threadIdx.x, cstarts, nchrom, &key, &v);
-        const unsigned grp = __match_any_sync(CS_FULL, c);
-        const int leader = __ffs(grp) - 1;
-        u64 pos = 0;
-        if (c >= 0 && lane == leader) pos = atomicAdd(cursor + c, (u64)__popc(grp));
-        pos = __shfl_sync(CS_FULL, pos, leader) + (u64)__popc(grp & ((1u << lane) - 1));
-        if (c >= 0) {
-            const int s0 = __ldg(cstarts + c);
-            ov[pos] = v; oi[pos] = (int)(key >> 31) - s0; oj[pos] = (int)(key & 0x7fffffffULL) - s0;
         }
     }
 }

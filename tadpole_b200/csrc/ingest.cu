@@ -16,11 +16,10 @@
 // count matrices and for the usual 6-17 digit normalised matrices.  Algorithmic traffic: file bytes read once + 8 N^2 written.
 #include "common.cuh"
 #include "numparse.cuh"
-#include <errno.h>
+#include "text.cuh"
 #include <fcntl.h>
 #include <stdlib.h>
 #include <sys/stat.h>
-#include <unistd.h>
 #include <chrono>
 
 static const uint64_t h_pow5[] = {
@@ -287,29 +286,9 @@ __global__ void scatter_f64_kernel(double *__restrict__ out, const unsigned *__r
 }
 
 // ---- host side -----------------------------------------------------------------------------------------------------
-struct TextSource {
-    const unsigned char *mem = nullptr;
-    int fd = -1;
-    size_t size = 0;
-    int fetch(size_t off, size_t len, void *dst) const {
-        if (mem) { memcpy(dst, mem + off, len); return TP_OK; }
-        size_t got = 0;
-        while (got < len) {
-            ssize_t k = pread(fd, (char *)dst + got, len - got, (off_t)(off + got));
-            if (k < 0 && errno == EINTR) continue;
-            if (k <= 0) { tp_set_error("tp_ingest_tsv_file: read failed at byte %zu (%s)", off + got, k < 0 ? strerror(errno) : "unexpected end of file"); return TP_ERR_ARG; }
-            got += (size_t)k;
-        }
-        return TP_OK;
-    }
-};
-
-// Upload the text (through the two pinned buffers) and count its rows: on return *text_out is the device copy with a
-// newline and IG_PAD readable bytes appended, offs[0..nb] the newline offsets per 16 KB tile (offs[nb] = rows).
-static int text_rows(tp_ctx *ctx, const TextSource &src, const char *who, unsigned char **text_out, size_t *nbytes_out,
-                     int *nb_out, long long **offs_out, long long *nrows_out) {
-    cudaStream_t st = ctx->stream;
-    // drop trailing newlines / blanks: the last row ends at the single '\n' appended on the device
+// The length of the text without its trailing newlines and blanks (the last row ends at the single '\n' that text_rows
+// appends on the device); an empty or too large text is an error.
+static int text_trimmed(const TextSource &src, const char *who, size_t *nbytes_out) {
     size_t nbytes = src.size;
     {
         unsigned char tail[4096];
@@ -324,6 +303,13 @@ static int text_rows(tp_ctx *ctx, const TextSource &src, const char *who, unsign
     }
     if (nbytes == 0) { tp_set_error("%s: the input holds no data", who); return TP_ERR_ARG; }
     if (nbytes >= ((size_t)1 << 40)) { tp_set_error("%s: input too large", who); return TP_ERR_ARG; }
+    *nbytes_out = nbytes;
+    return TP_OK;
+}
+
+int text_rows(tp_ctx *ctx, const TextSource &src, size_t base, size_t nbytes, unsigned char **text_out, int *nb_out,
+              long long **offs_out, long long *nrows_out) {
+    cudaStream_t st = ctx->stream;
     const long long limit = (long long)nbytes + 1;
     TP_TRY(ctx->itext.reserve(nbytes + IG_PAD + 16));
     unsigned char *text = ctx->itext.as<unsigned char>();
@@ -341,7 +327,7 @@ static int text_rows(tp_ctx *ctx, const TextSource &src, const char *who, unsign
         const int b = c & 1;
         const size_t k = nbytes - off < CH ? nbytes - off : CH;
         if (c >= 2) TP_CUDA(cudaEventSynchronize(ctx->ipin_ev[b]));
-        TP_TRY(src.fetch(off, k, ctx->ipin[b]));
+        TP_TRY(src.fetch(base + off, k, ctx->ipin[b]));
         TP_CUDA(cudaMemcpyAsync(text + off, ctx->ipin[b], k, cudaMemcpyHostToDevice, st));
         TP_CUDA(cudaEventRecord(ctx->ipin_ev[b], st));
     }
@@ -357,7 +343,18 @@ static int text_rows(tp_ctx *ctx, const TextSource &src, const char *who, unsign
     TP_CUDA(cudaMemcpyAsync(&nrows_ll, offs + nb, sizeof(long long), cudaMemcpyDeviceToHost, st));
     TP_CUDA(tp_stream_sync(ctx));
     ctx->launches += 2;
-    *text_out = text; *nbytes_out = nbytes; *nb_out = nb; *offs_out = offs; *nrows_out = nrows_ll;
+    *text_out = text; *nb_out = nb; *offs_out = offs; *nrows_out = nrows_ll;
+    return TP_OK;
+}
+
+int text_line_ends(tp_ctx *ctx, const unsigned char *text, size_t nbytes, int nb, const long long *offs, long long nrows,
+                   long long **row_end_out) {
+    TP_TRY(ctx->irows.reserve((size_t)nrows * sizeof(long long)));
+    long long *row_end = ctx->irows.as<long long>();
+    newline_pos_kernel<<<nb, IG_THREADS, 0, ctx->stream>>>(text, (long long)nbytes + 1, offs, row_end);
+    TP_CUDA(cudaGetLastError());
+    ctx->launches += 1;
+    *row_end_out = row_end;
     return TP_OK;
 }
 
@@ -396,7 +393,8 @@ static int ingest_core(tp_ctx *ctx, const TextSource &src, int sep, int *n_out) 
     size_t nbytes = 0;
     int nb = 0;
     long long *offs = nullptr, nrows_ll = 0;
-    TP_TRY(text_rows(ctx, src, "tp_ingest_tsv", &text, &nbytes, &nb, &offs, &nrows_ll));
+    TP_TRY(text_trimmed(src, "tp_ingest_tsv", &nbytes));
+    TP_TRY(text_rows(ctx, src, 0, nbytes, &text, &nb, &offs, &nrows_ll));
     const long long limit = (long long)nbytes + 1;
     TP_ARG(nrows_ll >= 2, "tp_ingest_tsv: the matrix must have at least 2 rows");
     TP_ARG(nrows_ll <= 200000, "tp_ingest_tsv: more than 200000 rows");
@@ -575,7 +573,7 @@ extern "C" int tp_ingest_coo(tp_ctx *ctx, const int32_t *bin1, const int32_t *bi
     return TP_OK;
 }
 
-static int open_text_file(const char *path, const char *who, TextSource *src) {
+int open_text_file(const char *path, const char *who, TextSource *src) {
     src->fd = open(path, O_RDONLY);
     if (src->fd < 0) {
         tp_set_error("%s: cannot open '%s' (%s)", who, path, strerror(errno));
@@ -617,7 +615,8 @@ static int coo_text_pixels(tp_ctx *ctx, const TextSource &src, int sep, const ch
     size_t nbytes = 0;
     int nb = 0;
     long long *offs = nullptr, nrows = 0;
-    TP_TRY(text_rows(ctx, src, who, &text, &nbytes, &nb, &offs, &nrows));
+    TP_TRY(text_trimmed(src, who, &nbytes));
+    TP_TRY(text_rows(ctx, src, 0, nbytes, &text, &nb, &offs, &nrows));
     if (nrows < 1 || nrows >= 0x7fffffffLL) {
         tp_set_error("%s: the file must hold between 1 and 2^31 - 2 rows", who);
         return TP_ERR_ARG;
@@ -804,7 +803,7 @@ genome_bucket_kernel(const int *__restrict__ b1, const int *__restrict__ b2, con
     if (c >= 0) { ov[pos] = v[e]; oi[pos] = li; oj[pos] = lj; }
 }
 
-static int genome_new(const int32_t *chrom_bins, int nchrom, int index_base, const char *who, tp_genome **out) {
+int genome_new(const int32_t *chrom_bins, int nchrom, int index_base, const char *who, tp_genome **out) {
     if (!(nchrom >= 1 && nchrom <= (1 << 20))) { tp_set_error("%s: the number of chromosomes must be in 1..2^20", who); return TP_ERR_ARG; }
     if (index_base != 0 && index_base != 1) { tp_set_error("%s: index_base must be 0 or 1", who); return TP_ERR_ARG; }
     long long total = 0;
